@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the conditional-Glow hot path (BASELINE.json metric: train frames/sec, final_model.yaml).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gemm fp32|bf16x3|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--gemm fp32|bf16x3|bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one optimizer step (forward + NLL + backward + clip_grad_norm 20 + Adam) on a batch of 256 synthetic
@@ -51,7 +51,38 @@ def parse():
     ap.add_argument("--ncu-step", action="store_true",
                     help="profiling helper: warm up, then run ONE step between cudaProfilerStart/Stop and exit "
                          "(use with ncu --profile-from-start off); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed training step returned as DIR/<name>.npy: loss, "
+                         "grad_norm and params (a fixed sample of the updated parameters); inputs and seeds do not change "
+                         "between runs, so two builds can be compared output for output (bench_outputs/<build> in the "
+                         "checkout is ignored by git)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.ncu_step):
+        ap.error("--dump-outputs writes the outputs of the timed GPU training step: not with --impl reference or --ncu-step")
+    return a
+
+
+DUMP_PARAMS = 1 << 22   # parameters written by --dump-outputs (16 MB as float32; the final model has 17.6 M)
+
+
+def dump_outputs(out_dir, model, trainer, loss):
+    """What a caller of Trainer.step holds after the last timed step: its loss, the gradient norm the step clipped with, and
+    the updated parameters (the step writes them in place), flattened in `named_parameters` order.  Larger models are
+    sampled at DUMP_PARAMS positions drawn from a fixed seed, in ascending order."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    params = torch.cat([p.detach().reshape(-1) for _, p in model.named_parameters()])
+    if params.numel() > DUMP_PARAMS:
+        pick = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_PARAMS].sort().values
+        params = params[pick.to(params.device)]
+    out = {"loss": np.float64(loss.item()), "grad_norm": np.float64(trainer.grad_norm().item()),
+           "params": params.float().cpu().numpy()}
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def peaks():
@@ -301,12 +332,19 @@ def run_ours(a):
         torch.cuda.synchronize()
         torch.cuda.profiler.stop()
         return
+    last = {}
+
+    def headline_step():
+        last["loss"] = trainer.step(dbatch)
+
     n0 = L.lfi_launch_count()
     t_w0 = time.time()
-    ms = timed(lambda: trainer.step(dbatch), a.steps)
+    ms = timed(headline_step, a.steps)
     t_w1 = time.time()
     launches = L.lfi_launch_count() - n0
     clk = clocks.stop((t_w0, t_w1))
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, model, trainer, last["loss"])
     frames_step = B * Tp * world
     value = frames_step * a.steps / (ms / 1e3)
 

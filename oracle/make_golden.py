@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY — generates `tests/golden/*.npz` by running the UNMODIFIED reference
-(`/root/reference/code/glow_pytorch/glow`) on the CPU of the authoring container.
+(`code/glow_pytorch/glow` of a jonepatr/lets_face_it checkout) on the CPU.
 
-    python oracle/make_golden.py            # writes tests/golden/kat_full.npz, kat_small_*.npz
+    LFI_REFERENCE_ROOT=<checkout> python oracle/make_golden.py    # writes tests/golden/kat_full.npz, kat_small_*.npz
 
 Recipe = SURVEY.md §8(c): torch/numpy seed 1234 (code/config.toml:4), LinearZeros perturbed from
 Generator(7), encoder dropout disabled (or replaced by injected masks), data from Generator(1),
@@ -21,6 +21,7 @@ import torch.nn as nn
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import glow_oracle as O  # noqa: E402
 from oracle.ref_shim import import_reference, load_reference_hparams  # noqa: E402
+from tests.kat import fingerprint  # noqa: E402  (the stored fingerprints and the test must sum alike)
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
@@ -90,11 +91,6 @@ def build_reference_model(hp, models, modules):
         if isinstance(mod, models.ModalityEncoder):
             mod.dropout = None
     return m
-
-
-def fingerprint(sd):
-    names = sorted(sd.keys())
-    return names, np.array([[float(sd[n].double().sum()), float(sd[n].double().abs().sum())] for n in names])
 
 
 def run_case(hp, B, T, infer_len, with_masks, full_tensors, tag):

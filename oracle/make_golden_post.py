@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY — golden vectors for the rows of SURVEY.md §8(f) ranks 2-3 (output wire format of sampling,
-training-step glue), produced by the UNMODIFIED reference in the authoring container:
+training-step glue), produced by the UNMODIFIED reference (a jonepatr/lets_face_it checkout):
 
-    python oracle/make_golden_post.py        # writes tests/golden/kat_post.npz
+    LFI_REFERENCE_ROOT=<checkout> python oracle/make_golden_post.py    # writes tests/golden/kat_post.npz
 
 * `expand_face_dim` is executed from the reference's own source text (`code/glow_pytorch/generate_motion_from_model.py`:
   the module itself imports rendering / Lightning / optuna packages that are absent here, so only that function's `def`

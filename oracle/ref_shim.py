@@ -1,30 +1,31 @@
-"""TEST INFRASTRUCTURE ONLY — import shim for the *live* reference (container only).
+"""TEST INFRASTRUCTURE ONLY — import shim for the *live* reference.
 
-Makes `/root/reference/code/glow_pytorch/glow/{models,modules}.py` importable without editing
+The reference is a checkout of jonepatr/lets_face_it named by the environment variable
+LFI_REFERENCE_ROOT; it is not part of this repository, and without the variable the tests marked
+`reference` skip.  Makes `$LFI_REFERENCE_ROOT/code/glow_pytorch/glow/{models,modules}.py` importable without editing
 the reference: `glow/__init__.py:2` pulls in `glow/utils.py`, which imports `jsmin` and
 `pytorch_lightning.Trainer` (utils.py:7,9); both are absent here, so two stub modules are
-inserted first (SURVEY.md §8(c)).  `/root/reference` does not exist on the GPU box: nothing
-that runs there may import this file.  Used by `oracle/make_golden.py` and by the
-container-only pinning tests.
+inserted first (SURVEY.md §8(c)).  Used by `oracle/make_golden.py` and by the
+reference-only pinning tests.
 """
 import argparse
 import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("LFI_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("LFI_REFERENCE_ROOT", "")
 REF_CODE = os.path.join(REF_ROOT, "code")
 REF_YAML_DIR = os.path.join(REF_CODE, "glow_pytorch", "hparams")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF_CODE, "glow_pytorch", "glow", "models.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_CODE, "glow_pytorch", "glow", "models.py"))
 
 
 def import_reference():
     """Returns (models, modules) of the unmodified reference."""
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REF_ROOT)
+        raise RuntimeError("reference tree not found: set LFI_REFERENCE_ROOT to a checkout of jonepatr/lets_face_it (now %r)" % REF_ROOT)
     if "jsmin" not in sys.modules:
         m = types.ModuleType("jsmin")
         m.jsmin = lambda s: s

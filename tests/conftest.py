@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the live reference tree (authoring container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the original project named by LFI_REFERENCE_ROOT")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -24,4 +24,4 @@ def pytest_collection_modifyitems(config, items):
         if "gpu" in it.keywords and not has_gpu:
             it.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference" in it.keywords and not has_ref:
-            it.add_marker(pytest.mark.skip(reason="live reference tree not present"))
+            it.add_marker(pytest.mark.skip(reason="LFI_REFERENCE_ROOT does not name a checkout of the original project"))

@@ -27,9 +27,23 @@ def build_kat_model(hp, device=None):
     return m
 
 
+# torch splits a large CPU reduction into one partial sum per intra-op thread, so the last bits of a double-precision sum
+# depend on the thread count: the stored fingerprints (tests/golden/kat_*.npz) were summed with 8 threads, and summing
+# with 16 threads moves them by ~2e-12.  Pinning the count is necessary, not sufficient: the order also follows the vector
+# width of the CPU kernel torch dispatches to (the same results were seen under AVX2 and AVX-512, not on other ISAs), and
+# OpenMP must grant all 8 threads (OMP_THREAD_LIMIT, OMP_DYNAMIC).  The parameters themselves are bit-identical, so a
+# host where the sums still differ needs a comparison within a few ulp, not a looser parameter check.
+FINGERPRINT_THREADS = 8
+
+
 def fingerprint(sd):
     names = sorted(sd.keys())
-    return names, np.array([[float(sd[n].double().sum()), float(sd[n].double().abs().sum())] for n in names])
+    threads = torch.get_num_threads()
+    torch.set_num_threads(FINGERPRINT_THREADS)
+    try:
+        return names, np.array([[float(sd[n].double().sum()), float(sd[n].double().abs().sum())] for n in names])
+    finally:
+        torch.set_num_threads(threads)
 
 
 def to_device(batch, device):

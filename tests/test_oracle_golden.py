@@ -1,5 +1,5 @@
 """CPU: pins oracle/glow_oracle.py to vectors produced by the unmodified reference
-(oracle/make_golden.py), and — in the authoring container — to the live reference."""
+(oracle/make_golden.py), and — where LFI_REFERENCE_ROOT names a checkout of it — to the live reference."""
 import numpy as np
 import pytest
 import torch
@@ -165,11 +165,27 @@ def test_oracle_three_optimizer_steps_match_reference_vectors():
         assert float((got - ref).norm()) <= 0.02 * float(ref.norm()) + 1e-12, n
 
 
+def test_packaged_final_model_yaml_matches_values_the_reference_recorded():
+    """The packaged final_model.yaml against what the reference's runs on its own final_model.yaml stored in the golden
+    vectors: the learning rate of its optimizer steps (kat_steps_full), the face-parameter split of its output side and the
+    modalities its mismatched-NLL probe shuffles (kat_post).  The shape-bearing Conditioning / Glow values are pinned by
+    the bit-identical parameters test_cabi_symbols.py::test_dropin_constructor_reproduces_reference_parameters builds."""
+    from lets_face_it_b200.glow.utils import get_mismatched_modalities
+    from lets_face_it_b200.hparams import load_hparams
+
+    hp = load_hparams()
+    steps, post = load_golden("kat_steps_full"), load_golden("kat_post")
+    assert hp.lr == float(steps["lr"])
+    assert [hp.Data[k] for k in ("expression_dim", "jaw_dim", "neck_dim")] == [int(v) for v in post["data_dims"]]
+    mods, name = get_mismatched_modalities(hp)
+    assert mods == [str(m) for m in post["mismatched_modalities"]] and name == str(post["mismatched_name"])
+
+
 @pytest.mark.reference
 def test_reference_yaml_files_load_unchanged():
     """The reference's own hparams files (code/glow_pytorch/hparams/*.yaml, 159 lines each) load through
     `lets_face_it_b200.hparams.load_hparams` and build the drop-in SeqGlow; for final_model.yaml the result has exactly the
-    shapes of the packaged subset (authoring container only: the GPU box has no reference tree)."""
+    shapes of the packaged subset (runs only where LFI_REFERENCE_ROOT names a checkout of the reference)."""
     import os
 
     from lets_face_it_b200.glow import SeqGlow
