@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 5
+#define LFI_ABI_VERSION 6
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -182,6 +182,61 @@ int lfi_flowstep_bwd(const lfi_shape *s, const void *derived, const lfi_params *
                      const float *c_in, const float *dy, const float *dlogdet, const float *dh_out, const float *dc_out, float *dx,
                      float *dcond, float *dh_in, float *dc_in, lfi_params *g, int B, void *stash, size_t stash_bytes, void *ws,
                      size_t ws_bytes, void *stream);
+
+/* ---- stand-alone modules under autograd (modules.py ActNorm2d / InvertibleConv1x1 / LinearZeros, models.py f_seq) ---------
+ * Backward passes of lfi_actnorm and of LinearZeros, and f_seq.forward (models.py:204-214) with its backward, each on the
+ * module's own tensors.  GEMMs run in LFI_GEMM_FP32, as in lfi_flowstep.  Parameter gradients are WRITTEN, not accumulated.
+ * Every reduction over the B rows runs in a fixed order (no atomics): the same call twice gives bit-identical gradients. */
+/* ActNorm2d backward on [B,C]; x / y = input / output of the lfi_actnorm call (reverse=0 reads y, reverse=1 reads x; the
+ * other may be NULL).  dbias, dlogs [C]:
+ *   reverse=0:  dx = dy e^{logs},   dbias =  sum_B dy e^{logs},  dlogs =  sum_B dy y
+ *   reverse=1:  dx = dy e^{-logs},  dbias = -sum_B dy,           dlogs = -sum_B dy x e^{-logs}
+ * The parameter-only log-det term C * sum(logs) is the caller's. */
+int lfi_actnorm_bwd(const float *x, const float *y, const float *logs, const float *dy, float *dx, float *dbias, float *dlogs,
+                    int B, int C, int reverse, void *stream);
+/* LinearZeros backward (modules.py:93-95): out = (h W^T + b) e^{f logs}, h [B,In], W [Out,In], f = logscale_factor.  Given
+ * out and dout [B,Out]: dh [B,In] = g W, dW [Out,In] = g^T h, db [Out] = sum_B g, dlogs [Out] = f sum_B dout out, with
+ * g = dout e^{f logs} (workspace: lfi_linear_zeros_bwd_ws_bytes). */
+size_t lfi_linear_zeros_bwd_ws_bytes(int B, int Out);
+int lfi_linear_zeros_bwd(const float *h, const float *w, const float *logs, const float *out, const float *dout, float logscale_factor,
+                         float *dh, float *dw, float *db, float *dlogs, int B, int In, int Out, void *ws, size_t ws_bytes,
+                         void *stream);
+
+/* Shapes of one stand-alone f_seq (models.py:148-194). */
+typedef struct lfi_fseq_shape {
+  int32_t In;             /* input_size: width of z                                   */
+  int32_t Out;            /* output_size: LinearZeros output                          */
+  int32_t H;              /* hidden_size                                              */
+  int32_t D;              /* cond_dim: cond_transform output                          */
+  int32_t F;              /* feature_encoder_dim: width of the conditioning           */
+  int32_t G;              /* 3 = GRUCell (r,z,n), 4 = LSTMCell (i,f,g,o)               */
+  float logscale_factor;  /* final_linear.logscale_factor (3 by default)              */
+} lfi_fseq_shape;
+
+/* Parameters of one f_seq, as the module holds them (not the [K, ...] blocks of lfi_params). */
+typedef struct lfi_fseq_params {
+  float *wc, *bc;         /* [D,F],[D]         cond_transform.0.{weight,bias}  */
+  float *w_ih, *b_ih;     /* [G*H,In+D],[G*H]  rnn.{weight_ih,bias_ih}         */
+  float *w_hh, *b_hh;     /* [G*H,H],[G*H]     rnn.{weight_hh,bias_hh}         */
+  float *wf, *bf, *lf;    /* [Out,H],[Out],[Out] final_linear.{weight,bias,logs} */
+} lfi_fseq_params;
+
+/* f_seq.forward: out [B,Out] = LinearZeros(cell([z | LeakyReLU(cond W_c^T + b_c)], state)), z [B,In], cond [B,F];
+ * h_in (c_in) [B,H] or NULL = zeros (f_seq.init_rnn_hidden; the LSTM zero state of FlowStep), h_out (c_out) [B,H].
+ * stash NULL (inference) or lfi_fseq_stash_bytes(s, B) bytes, caller owned and opaque, for lfi_fseq_bwd. */
+size_t lfi_fseq_ws_bytes(const lfi_fseq_shape *s, int B);
+size_t lfi_fseq_stash_bytes(const lfi_fseq_shape *s, int B);
+size_t lfi_fseq_bwd_ws_bytes(const lfi_fseq_shape *s, int B);
+int lfi_fseq_fwd(const lfi_fseq_shape *s, const lfi_fseq_params *p, const float *z, const float *cond, const float *h_in,
+                 const float *c_in, float *h_out, float *c_out, float *out, int B, void *stash, size_t stash_bytes, void *ws,
+                 size_t ws_bytes, void *stream);
+/* Backward of the above: dout [B,Out], dh_out / dc_out [B,H] = dL/d(new state) (NULL = 0); z, cond, h_in, c_in as passed to
+ * the forward.  dz [B,In], dcond [B,F], dh_in / dc_in [B,H] (each NULL = not wanted); all nine parameter gradients are
+ * written into g (dW_hh = 0 when h_in is NULL). */
+int lfi_fseq_bwd(const lfi_fseq_shape *s, const lfi_fseq_params *p, const float *z, const float *cond, const float *h_in,
+                 const float *c_in, const float *dout, const float *dh_out, const float *dc_out, float *dz, float *dcond,
+                 float *dh_in, float *dc_in, lfi_fseq_params *g, int B, const void *stash, size_t stash_bytes, void *ws,
+                 size_t ws_bytes, void *stream);
 
 /* ---- primitives exposed for the module API and unit parity --------------------------------- */
 /* ActNorm2d.forward (modules.py:45-80) on [B,C]: reverse=0  y=(x+bias)*exp(logs); reverse=1 y=x*exp(-logs)-bias */

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "liblfi_b200.so")
 NMOD = 4
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 GEMM_FP32, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
 EPI_BIAS, EPI_LRELU, EPI_ACCUM, EPI_LRELU_BWD = 1, 2, 4, 8
@@ -37,6 +37,18 @@ class Params(C.Structure):
     ]
 
 
+class FseqShape(C.Structure):
+    _fields_ = [("In", C.c_int32), ("Out", C.c_int32), ("H", C.c_int32), ("D", C.c_int32), ("F", C.c_int32), ("G", C.c_int32),
+                ("logscale_factor", C.c_float)]
+
+
+FSEQ_PARAMS = ("wc", "bc", "w_ih", "b_ih", "w_hh", "b_hh", "wf", "bf", "lf")
+
+
+class FseqParams(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in FSEQ_PARAMS]
+
+
 class Batch(C.Structure):
     _fields_ = [("x", C.c_void_p * NMOD), ("mask", C.c_void_p * NMOD), ("B", C.c_int32), ("T", C.c_int32)]
 
@@ -44,6 +56,7 @@ class Batch(C.Structure):
 # name -> (restype, argtypes); every symbol include/lfi_b200.h declares
 _P, _SZ, _I, _F, _L = C.c_void_p, C.c_size_t, C.c_int, C.c_float, C.c_long
 _SH, _PR, _BT = C.POINTER(Shape), C.POINTER(Params), C.POINTER(Batch)
+_FS, _FP = C.POINTER(FseqShape), C.POINTER(FseqParams)
 SYMBOLS = {
     "lfi_last_error": (C.c_char_p, []),
     "lfi_abi_version": (_I, []),
@@ -77,6 +90,14 @@ SYMBOLS = {
     "lfi_actnorm": (_I, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "lfi_matmul": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "lfi_nll": (_I, [_P, _P, _P, _I, _I, _P]),
+    "lfi_actnorm_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
+    "lfi_linear_zeros_bwd_ws_bytes": (_SZ, [_I, _I]),
+    "lfi_linear_zeros_bwd": (_I, [_P, _P, _P, _P, _P, _F, _P, _P, _P, _P, _I, _I, _I, _P, _SZ, _P]),
+    "lfi_fseq_ws_bytes": (_SZ, [_FS, _I]),
+    "lfi_fseq_stash_bytes": (_SZ, [_FS, _I]),
+    "lfi_fseq_bwd_ws_bytes": (_SZ, [_FS, _I]),
+    "lfi_fseq_fwd": (_I, [_FS, _FP, _P, _P, _P, _P, _P, _P, _P, _I, _P, _SZ, _P, _SZ, _P]),
+    "lfi_fseq_bwd": (_I, [_FS, _FP, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _FP, _I, _P, _SZ, _P, _SZ, _P]),
     "lfi_gather_batch": (_I, [_P, _P, _I, _I, _I, _P, _P]),
     "lfi_jerk": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "lfi_clip_adam": (_I, [_P, _P, _P, _P, _SZ, _F, _F, _F, _F, _F, _F, _I, _P, _P]),

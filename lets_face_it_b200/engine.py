@@ -491,10 +491,12 @@ class Engine:
                 "wf": Co * H, "bf": Co, "lf": Co}
 
     @_on_own_device
-    def flowstep_train(self, k, x, cond, h_in, c_in, want_scale=False):
+    def flowstep_train(self, k, x, cond, h_in, c_in, want_scale=False, refresh=True):
         """Forward of one FlowStep on one frame WITH the stash `flowstep_backward` needs (lfi_flowstep_fwd_train).
-        Returns (y, ld [B] coupling log-det term, h_out, c_out, scale, stash)."""
-        self.refresh(False)
+        Returns (y, ld [B] coupling log-det term, h_out, c_out, scale, stash).  refresh=False: the derived cache is current
+        (FlowNet.encode rebuilds it once per call)."""
+        if refresh:
+            self.refresh(False)
         L, st = cabi.lib(), cabi.stream_ptr()
         P = self._params_struct(self.theta, self.W)
         dev = self.theta.device

@@ -8,11 +8,14 @@ three fused device paths reached through the C ABI (`engine.py` / `_cabi.py`):
   SeqGlow.forward   -> lfi_seq_train_fwd / lfi_seq_train_bwd  (autograd.Function below)
   SeqGlow.inference -> lfi_seq_sample (persistent autoregressive sampler)
   SeqGlow.invert    -> lfi_seq_sample (teacher forced)
-  FlowStep / FlowNet / Glow single-frame calls -> lfi_flowstep
+  FlowStep / FlowNet / Glow single-frame calls -> lfi_flowstep (under autograd lfi_flowstep_fwd_train / lfi_flowstep_bwd)
+  f_seq.forward on its own                     -> lfi_fseq_fwd (under autograd lfi_fseq_bwd as well)
 
 CUDA tensors only; there is no CPU / eager fallback.
 """
 from __future__ import annotations
+
+import ctypes
 
 import numpy as np
 import torch
@@ -202,10 +205,63 @@ class _SingleModality:
         return torch.cat([out, out], dim=1) if E else out
 
 
+def _fseq_run(shape, params, z, cond, h_in, c_in, want_stash):
+    """lfi_fseq_fwd on device tensors (fp32, contiguous): returns (out, h, c or None, stash or None)."""
+    L = cabi.lib()
+    B, dev = z.shape[0], z.device
+    h = torch.empty(B, shape.H, dtype=torch.float32, device=dev)
+    c = torch.empty(B, shape.H, dtype=torch.float32, device=dev) if shape.G == 4 else None
+    out = torch.empty(B, shape.Out, dtype=torch.float32, device=dev)
+    stash = torch.empty(L.lfi_fseq_stash_bytes(ctypes.byref(shape), B), dtype=torch.uint8, device=dev) if want_stash else None
+    ws = torch.empty(L.lfi_fseq_ws_bytes(ctypes.byref(shape), B), dtype=torch.uint8, device=dev)
+    P = cabi.FseqParams(*[cabi.ptr(t) for t in params])
+    cabi.check(L.lfi_fseq_fwd(ctypes.byref(shape), ctypes.byref(P), cabi.ptr(z), cabi.ptr(cond), cabi.ptr(h_in), cabi.ptr(c_in), cabi.ptr(h),
+                              cabi.ptr(c), cabi.ptr(out), B, stash.data_ptr() if want_stash else None, stash.numel() if want_stash else 0, ws.data_ptr(),
+                              ws.numel(), cabi.stream_ptr()), "lfi_fseq_fwd")
+    return out, h, c, stash
+
+
+class _FSeqFn(torch.autograd.Function):
+    """f_seq.forward under autograd (reference models.py:204-214 differentiated by torch): forward = lfi_fseq_fwd with a stash,
+    backward = lfi_fseq_bwd.  Inputs after `c_in` are the nine parameters in `f_seq._params()` order."""
+
+    @staticmethod
+    def forward(ctx, shape, z, cond, h_in, c_in, *params):
+        out, h, c, stash = _fseq_run(shape, [p.detach() for p in params], z.detach(), cond.detach(),
+                                     h_in.detach() if h_in is not None else None, c_in.detach() if c_in is not None else None, True)
+        ctx.shape, ctx.stash = shape, stash
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(z, cond, h_in, c_in, *params)
+        return (out, h) + ((c,) if c is not None else ())
+
+    @staticmethod
+    def backward(ctx, dout, dh, dc=None):
+        shape, stash = ctx.shape, ctx.stash
+        z, cond, h_in, c_in, *params = ctx.saved_tensors
+        B, dev = z.shape[0], z.device
+        f32 = lambda t: t.to(dtype=torch.float32).contiguous() if t is not None else None
+        dout = f32(dout) if dout is not None else torch.zeros(B, shape.Out, dtype=torch.float32, device=dev)
+        dh, dc = f32(dh), f32(dc)
+        dz, dcond = torch.empty_like(z), torch.empty_like(cond)
+        dh_in = torch.empty_like(h_in) if h_in is not None else None
+        dc_in = torch.empty_like(c_in) if c_in is not None else None
+        grads = [torch.empty_like(p) for p in params]
+        L = cabi.lib()
+        ws = torch.empty(L.lfi_fseq_bwd_ws_bytes(ctypes.byref(shape), B), dtype=torch.uint8, device=dev)
+        P = cabi.FseqParams(*[cabi.ptr(t) for t in params])
+        Gr = cabi.FseqParams(*[cabi.ptr(t) for t in grads])
+        cabi.check(L.lfi_fseq_bwd(ctypes.byref(shape), ctypes.byref(P), cabi.ptr(z), cabi.ptr(cond), cabi.ptr(h_in), cabi.ptr(c_in),
+                                  cabi.ptr(dout), cabi.ptr(dh), cabi.ptr(dc), cabi.ptr(dz), cabi.ptr(dcond), cabi.ptr(dh_in), cabi.ptr(dc_in),
+                                  ctypes.byref(Gr), B, stash.data_ptr(), stash.numel(), ws.data_ptr(), ws.numel(), cabi.stream_ptr()),
+                   "lfi_fseq_bwd")
+        return (None, dz, dcond, dh_in, dc_in) + tuple(grads)
+
+
 class f_seq(nn.Module):
     """Coupling network: Linear+LeakyReLU on the conditioning, GRUCell/LSTMCell over frames, LinearZeros
-    (reference models.py:148-214).  Holds the parameters and the carried RNN state; it is evaluated inside
-    the fused flow-step kernels, never on its own."""
+    (reference models.py:148-214).  Holds the parameters and the carried RNN state.  Inside a FlowStep it is evaluated by the
+    fused flow-step kernels; `forward` runs it on its own (lfi_fseq_fwd, under autograd lfi_fseq_bwd as well) and leaves the
+    state where FlowStep.forward of the same step reads it next."""
 
     def __init__(self, input_size, output_size, hidden_size, cond_dim, feature_encoder_dim, rnn_type):
         super().__init__()
@@ -229,8 +285,39 @@ class f_seq(nn.Module):
         self.hidden = None
         self.cell = None
 
+    def _params(self):
+        ct, fl = self.cond_transform[0], self.final_linear
+        return [ct.weight, ct.bias, self.rnn.weight_ih, self.rnn.bias_ih, self.rnn.weight_hh, self.rnn.bias_hh, fl.weight, fl.bias, fl.logs]
+
+    def _shape(self):
+        sh = cabi.FseqShape()
+        ct = self.cond_transform[0]
+        sh.In, sh.Out, sh.H, sh.D, sh.F = self.input_size, self.output_size, self.hidden_size, ct.out_features, ct.in_features
+        sh.G = 3 if self.rnn_type == "gru" else 4
+        sh.logscale_factor = float(self.final_linear.logscale_factor)
+        return sh
+
     def forward(self, z, condition):
-        raise NotImplementedError("f_seq is evaluated inside the fused FlowStep kernel (call FlowStep.forward)")
+        """z [B, input_size], condition [B, feature_encoder_dim] -> [B, output_size]; updates self.hidden (and self.cell)."""
+        params = self._params()
+        h_in, c_in = self.hidden, (self.cell if self.rnn_type == "lstm" else None)
+        dev = z.device
+        sh = self._shape()
+        B = z.shape[0]
+        if z.shape[1] != sh.In or condition.shape != (B, sh.F):
+            raise RuntimeError("f_seq expects z [B,%d] and condition [B,%d], got %s / %s" % (sh.In, sh.F, tuple(z.shape), tuple(condition.shape)))
+        for name, t in (("hidden", h_in), ("cell", c_in)):
+            if t is not None and t.shape != (B, sh.H):
+                raise RuntimeError("f_seq.%s has shape %s, expected [%d, %d]" % (name, tuple(t.shape), B, sh.H))
+        if modules._needs_grad(z, condition, h_in, c_in, *params):
+            f32 = lambda t: modules._f32g(t, dev) if t is not None else None
+            outs = _FSeqFn.apply(sh, f32(z), f32(condition), f32(h_in), f32(c_in), *[f32(p) for p in params])
+            out, h, c = outs[0], outs[1], (outs[2] if sh.G == 4 else None)
+        else:
+            f32 = lambda t: modules._f32c(t, dev) if t is not None else None
+            out, h, c, _ = _fseq_run(sh, [f32(p) for p in params], f32(z), f32(condition), f32(h_in), f32(c_in), False)
+        self.hidden, self.cell = h, c
+        return out
 
 
 class _FlowStepFn(torch.autograd.Function):
@@ -239,8 +326,8 @@ class _FlowStepFn(torch.autograd.Function):
     step's parameters in `FlowStep._autograd_params()` order (graph connectivity; values are read from the flat buffer)."""
 
     @staticmethod
-    def forward(ctx, eng, k, want_scale, n_lu, x, cond, h_in, c_in, *params):
-        y, ld, h_out, c_out, scale, saved = eng.flowstep_train(k, x, cond, h_in, c_in, want_scale)
+    def forward(ctx, eng, k, want_scale, n_lu, refresh, x, cond, h_in, c_in, *params):
+        y, ld, h_out, c_out, scale, saved = eng.flowstep_train(k, x, cond, h_in, c_in, want_scale, refresh=refresh)
         ctx.eng, ctx.k, ctx.saved, ctx.n_lu = eng, k, saved, n_lu
         ctx.has_c = c_out is not None
         outs = (y, ld, h_out) + ((c_out,) if c_out is not None else ()) + ((scale,) if scale is not None else ())
@@ -266,7 +353,7 @@ class _FlowStepFn(torch.autograd.Function):
         out += [g["wc"].view(D, F), g["bc"], g["w_ih"].view(GH, In), g["b_ih"], g["w_hh"].view(GH, H), g["b_hh"],
                 g["wf"].view(Co, H), g["bf"], g["lf"]]
         _, h_in, c_in = ctx.saved[1], ctx.saved[2], ctx.saved[3]
-        return (None, None, None, None, dx, dcond, dh_in if h_in is not None else None,
+        return (None, None, None, None, None, dx, dcond, dh_in if h_in is not None else None,
                 dc_in if (c_in is not None and dc_in is not None) else None) + tuple(out)
 
 
@@ -313,12 +400,14 @@ class FlowStep(nn.Module):
                                                               f.rnn.weight_hh, f.rnn.bias_hh, f.final_linear.weight, f.final_linear.bias,
                                                               f.final_linear.logs]
 
-    def _forward_autograd(self, eng, input_, cond, logdet):
+    def _forward_autograd(self, eng, input_, cond, logdet, refresh=True):
         """normal_flow under autograd: kernels for everything data dependent, torch for the parameter-only log-det terms
-        C * sum(logs) + C * sum(log_s) (modules.py:62, 171) so that autograd owns their gradients."""
+        C * sum(logs) + C * sum(log_s) (modules.py:62, 171) so that autograd owns their gradients.  refresh=False: the caller
+        (FlowNet.encode) has rebuilt the derived cache for this call already."""
         params = self._autograd_params()
         h_in, c_in = self.f.hidden, self.f.cell
-        outs = _FlowStepFn.apply(eng, self._k, bool(self.scale_logging), 1 if self.invconv.LU else 0, input_, cond, h_in, c_in, *params)
+        outs = _FlowStepFn.apply(eng, self._k, bool(self.scale_logging), 1 if self.invconv.LU else 0, bool(refresh), input_, cond, h_in, c_in,
+                                 *params)
         y, ld, h = outs[0], outs[1], outs[2]
         i = 3
         c = None
@@ -344,7 +433,7 @@ class FlowStep(nn.Module):
         if not reverse and torch.is_grad_enabled() and (
                 input_.requires_grad or audio_features.requires_grad or any(p.requires_grad for p in self._autograd_params())
                 or (self.f.hidden is not None and self.f.hidden.requires_grad)):
-            return self._forward_autograd(eng, input_, audio_features, logdet)
+            return self._forward_autograd(eng, input_, audio_features, logdet, _refresh)
         y, logdet, h, c, scale = eng.flowstep(self._k, input_, audio_features, self.f.hidden, self.f.cell, logdet, bool(reverse),
                                               want_scale=self.scale_logging, refresh=_refresh)
         self.f.hidden, self.f.cell = h, c
