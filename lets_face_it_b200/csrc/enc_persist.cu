@@ -1,9 +1,9 @@
-// Persistent windowed encoder GRU, forward and backward (ModalityEncoder `enc: rnn`: a one-layer batch-first nn.GRU run from a zero state over
-// the `history` frames of every window, reference models.py:21-27 and 55-69; gate equations of torch nn.GRU, order r, z, n).
+// Persistent windowed encoder GRU, forward only (ModalityEncoder `enc: rnn`: a one-layer batch-first nn.GRU run from a zero state
+// over the `history` frames of every window, reference models.py:21-27 and 55-69; gate equations of torch nn.GRU, order r, z, n).
+// Sampling and feature encoding use it; training runs the per-step launches, which also write the stash of the backward pass.
 //
-// Round 1 ran one launch per window step (recurrent product + gate math), so the state h, its operand planes and the input
-// projections made a round trip through HBM / L2 24 + 2 + 16 times per training step.  Here ONE launch per modality walks all
-// window steps:
+// The per-step form runs one launch per window step (recurrent product + gate math), so the state h, its operand planes and the
+// input projections make a round trip through HBM / L2 once per step.  Here ONE launch per modality walks all window steps:
 //   * a 2-CTA thread-block cluster owns a tile of 128 windows (rows m = t' * B + b) for the whole window; CTA c owns the hidden
 //     units [c * E/2, (c+1) * E/2), i.e. the r, u, n columns of those units (3 E/2 <= 384 fp32 accumulator columns in TMEM);
 //   * the state h lives in shared memory as split-bf16 (hi, lo) operand planes in the canonical K-major 128-byte-swizzled UMMA
@@ -13,9 +13,8 @@
 //     runs ahead across step boundaries; one elected thread issues the MMAs (a = a_hi + a_lo: a_hi b_hi + a_lo b_hi + a_hi b_lo,
 //     fp32 accumulation in TMEM), eight warps do the gate math straight from TMEM (thread = window x 16-unit chunks);
 //   * the input projections xp are read from L2 (63 MB for the widest modality, re-used by every window that contains the
-//     frame), the stash for the backward pass (16-bit gates, h-side n pre-activation, state) is the only HBM traffic.  Both use
-//     the row-interleaved layouts of enc_persist.cuh, so that the thread-per-window accesses of a warp are contiguous (the first
-//     version used row-major arrays: 32 lines per warp access, 62 k cycles of gate phase per step against 18 k of products).
+//     frame) in the row-interleaved layout of enc_persist.cuh, so that the thread-per-window accesses of a warp are contiguous
+//     (row-major: 32 lines per warp access).  Only the final state leaves the kernel, into the cond columns.
 // Synchronisation per step: mbarriers only (no cluster-wide barrier): `a_ready` (16 warp arrivals: both CTAs have written
 // their halves of h_s into THIS CTA's planes and this CTA's accumulator reads are done) gates the next product; `mma_done`
 // (2 arrivals: this CTA's and the peer's products of the step have completed, so nobody reads h_{s-1} any more) gates the
@@ -36,15 +35,13 @@ using namespace tcp;
 namespace {
 
 constexpr int kRows = 128;            // windows per cluster tile (UMMA M)
-constexpr int kEpiWarps = 8;
-constexpr int kThreads = 32 * (kEpiWarps + 2);  // + TMA producer warp + MMA issuer warp
 constexpr int kKB = 64;               // bf16 elements per k-block (one 128-byte swizzle span)
 constexpr int kAKB = kRows * 128;     // bytes of one k-block of one A plane
 constexpr int kTmemCols = 512;
-// The gate phase is issue-latency bound (ncu: 2 gate warps per scheduler sustain ~0.3 instructions per cycle): the forward kernel
-// runs 16 gate warps (4 per scheduler, 96 registers each) instead of 8.
+// The gate phase is issue-latency bound (ncu: 2 gate warps per scheduler sustain ~0.3 instructions per cycle), but 16 gate warps
+// (4 per scheduler, 96 registers each) measured slower than 8.
 constexpr int kFwdGateWarps = 8;
-constexpr int kFwdThreads = 32 * (kFwdGateWarps + 2);
+constexpr int kFwdThreads = 32 * (kFwdGateWarps + 2);  // + TMA producer warp + MMA issuer warp
 
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
@@ -101,7 +98,6 @@ __device__ __forceinline__ void unpack8(const uint4 &hi, const uint4 &lo, float 
   v[4] = bf_lo(hi.z) + bf_lo(lo.z); v[5] = bf_hi(hi.z) + bf_hi(lo.z);
   v[6] = bf_lo(hi.w) + bf_lo(lo.w); v[7] = bf_hi(hi.w) + bf_hi(lo.w);
 }
-__device__ __forceinline__ uint32_t pack_u16(unsigned short a, unsigned short b) { return (uint32_t)a | ((uint32_t)b << 16); }
 
 constexpr int kStageBytes = 192 * 128;  // forward ring stage: one 64-unit half (r, u, n rows) of one k-block of one W_hh plane
 constexpr int kMaxStages = 8;
@@ -123,9 +119,7 @@ __host__ __device__ inline SmemPlan plan(int E) {
   return p;
 }
 
-// 16 consecutive columns n0 .. n0+15 of row `row` of a tiled fp32 array of width W (enc_persist.cuh)
-// 8-column variants (two 4-column groups)
-// L1 policy: with 225 KB of shared memory per CTA the L1 is a few tens of KB.  The streams (input projections, stash) pass it
+// L1 policy: with 225 KB of shared memory per CTA the L1 is a few tens of KB.  The input projections pass it
 // without allocating; the bias vectors, which every chunk of every step re-reads, are asked to stay (evict-last).
 __device__ __forceinline__ float4 ld_stream4(const float *p) {
   float4 v;
@@ -137,21 +131,11 @@ __device__ __forceinline__ float4 ld_keep4(const float *p) {
   asm volatile("ld.global.nc.L1::evict_last.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
   return v;
 }
-__device__ __forceinline__ void st_stream4(float *p, float a, float b, float c, float d) {
-  asm volatile("st.global.L1::no_allocate.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-__device__ __forceinline__ void st_stream_u4(void *p, uint4 v) {
-  asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
+// 8 consecutive columns n0 .. n0+7 of row `row` of a tiled fp32 array of width W (enc_persist.cuh)
 __device__ __forceinline__ void ldt8(const float *base, size_t row, int n0, int W, float *v) {
   const float *p = base + ((row >> 5) * (size_t)(W >> 2) + (size_t)(n0 >> 2)) * 128 + (row & 31) * 4;
   const float4 t0 = ld_stream4(p), t1 = ld_stream4(p + 128);
   v[0] = t0.x; v[1] = t0.y; v[2] = t0.z; v[3] = t0.w; v[4] = t1.x; v[5] = t1.y; v[6] = t1.z; v[7] = t1.w;
-}
-__device__ __forceinline__ void stt8(float *base, size_t row, int n0, int W, const float *v) {
-  float *p = base + ((row >> 5) * (size_t)(W >> 2) + (size_t)(n0 >> 2)) * 128 + (row & 31) * 4;
-  st_stream4(p, v[0], v[1], v[2], v[3]);
-  st_stream4(p + 128, v[4], v[5], v[6], v[7]);
 }
 __device__ __forceinline__ void ldg8(const float *p, float *v) {
   const float4 t0 = ld_keep4(p), t1 = ld_keep4(p + 4);
@@ -165,9 +149,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {  // la
                : "memory");
 #pragma unroll
   for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ unsigned short *u16_ptr(void *base, size_t row, int n0, int W) {
-  return reinterpret_cast<unsigned short *>(base) + ((row >> 5) * (size_t)(W >> 3) + (size_t)(n0 >> 3)) * 256 + (row & 31) * 8;
 }
 
 }  // namespace
@@ -274,7 +255,6 @@ enc_gru_fwd_persist(const FwdArgs a, const __grid_constant__ CUtensorMap map_hi,
     const uint32_t tlane = tmem + ((uint32_t)(32 * q) << 16);
     const uint32_t ready_own = mapa_u32(smem_u32(a_ready), my_rank), ready_peer = mapa_u32(smem_u32(a_ready), peer_rank);
     const bool cond_vec = a.cond && (((uintptr_t)a.cond & 15) == 0) && (a.cond_ld % 4 == 0);
-    const size_t Mp = tiled_rows((size_t)a.M);
     const bool tm = (a.timing & 1) && blockIdx.x == 0 && blockIdx.y == 0 && tid == 0;
     long long t_wait = 0, t_epi = 0;
     const int ug_first = c * UH + sub * UQ;
@@ -325,7 +305,7 @@ enc_gru_fwd_persist(const FwdArgs a, const __grid_constant__ CUtensorMap map_hi,
             hn[i] = ng[i] + au[i] * (hp[i] - ng[i]);                                                        // h' = (1 - u) n + u h
           }
         }
-        if (j + 1 < nch) {  // the next chunk's input projections travel while this chunk's state / stash is packed and stored
+        if (j + 1 < nch) {  // the next chunk's input projections travel while this chunk's state is packed and stored
           const int ugn = ug + 8;
           ldt8(a.xp, xr_row, ugn, 3 * E, xr); ldt8(a.xp, xr_row, E + ugn, 3 * E, xu); ldt8(a.xp, xr_row, 2 * E + ugn, 3 * E, xn);
         }
@@ -335,42 +315,14 @@ enc_gru_fwd_persist(const FwdArgs a, const __grid_constant__ CUtensorMap map_hi,
           *reinterpret_cast<uint4 *>(sA + o0) = hi0; *reinterpret_cast<uint4 *>(sA + pl.a_plane + o0) = lo0;
           *reinterpret_cast<uint4 *>(peerA + o0) = hi0; *reinterpret_cast<uint4 *>(peerA + pl.a_plane + o0) = lo0;
         }
-        if (row_ok) {
-          if (a.stash) {
-            if (a.hs) stt8(a.hs + (size_t)s * Mp * E, m, ug, E, hn);
-            if (a.hp_hi) {
-              const size_t o1e = ((size_t)s * a.M + m) * E + ug;
-              st_stream_u4((__nv_bfloat16 *)a.hp_hi + o1e, hi0);
-              if (a.hp_lo) st_stream_u4((__nv_bfloat16 *)a.hp_lo + o1e, lo0);
-            }
-            if (a.gates) {
-              float *gstep = reinterpret_cast<float *>(a.gates) + (size_t)s * Mp * 3 * E;  // per-step blocks of Mp * 3E floats in both formats
-              if (a.gates16) {
-                uint32_t w[4];
+        if (row_ok && lastStep && a.cond) {
+          float *cd = a.cond + m * a.cond_ld + ug;
+          if (cond_vec) {
+            *reinterpret_cast<float4 *>(cd) = make_float4(hn[0], hn[1], hn[2], hn[3]);
+            *reinterpret_cast<float4 *>(cd + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
+          } else {
 #pragma unroll
-                for (int g = 0; g < 3; ++g) {
-                  const float *src = g == 0 ? ar : (g == 1 ? au : ng);
-#pragma unroll
-                  for (int i = 0; i < 4; ++i)  // sigmoid / tanh outputs already lie in [0, 1] / [-1, 1]: no clamp needed
-                    w[i] = g < 2 ? pack_u16((unsigned short)__float2uint_rn(src[2 * i] * 65535.0f), (unsigned short)__float2uint_rn(src[2 * i + 1] * 65535.0f))
-                                 : pack_u16((unsigned short)(short)__float2int_rn(src[2 * i] * 32767.0f), (unsigned short)(short)__float2int_rn(src[2 * i + 1] * 32767.0f));
-                  st_stream_u4(u16_ptr(gstep, m, g * E + ug, 3 * E), make_uint4(w[0], w[1], w[2], w[3]));
-                }
-              } else {
-                stt8(gstep, m, ug, 3 * E, ar); stt8(gstep, m, E + ug, 3 * E, au); stt8(gstep, m, 2 * E + ug, 3 * E, ng);
-              }
-            }
-            if (a.ahn) stt8(a.ahn + (size_t)s * Mp * E, m, ug, E, an);
-          }
-          if (lastStep && a.cond) {
-            float *cd = a.cond + m * a.cond_ld + ug;
-            if (cond_vec) {
-              *reinterpret_cast<float4 *>(cd) = make_float4(hn[0], hn[1], hn[2], hn[3]);
-              *reinterpret_cast<float4 *>(cd + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
-            } else {
-#pragma unroll
-              for (int i = 0; i < 8; ++i) cd[i] = hn[i];
-            }
+            for (int i = 0; i < 8; ++i) cd[i] = hn[i];
           }
         }
       }
@@ -406,8 +358,7 @@ int launch_fwd(const FwdArgs &a, cudaStream_t st) {
   LFI_REQUIRE(a.E == 128 || a.E == 256, LFI_ERR_SHAPE, "enc_persist: E=%d unsupported", a.E);
   LFI_REQUIRE(a.xp && a.b_ih && a.b_hh && a.whh_hi && (a.nplanes == 1 || a.whh_lo), LFI_ERR_ARG, "enc_persist: null argument");
   auto al16 = [](const void *p) { return p == nullptr || ((uintptr_t)p & 15) == 0; };
-  LFI_REQUIRE(al16(a.xp) && al16(a.b_ih) && al16(a.b_hh) && al16(a.hs) && al16(a.hp_hi) && al16(a.hp_lo) && al16(a.gates) && al16(a.ahn),
-              LFI_ERR_ARG, "enc_persist: misaligned pointer");
+  LFI_REQUIRE(al16(a.xp) && al16(a.b_ih) && al16(a.b_hh), LFI_ERR_ARG, "enc_persist: misaligned pointer");
   const SmemPlan p = plan(a.E);
   LFI_REQUIRE(p.stages >= 2 && p.total <= 227 * 1024, LFI_ERR_SHAPE, "enc_persist: shared-memory plan does not fit");
   CUtensorMap mhi, mlo;
@@ -427,448 +378,6 @@ int launch_fwd(const FwdArgs &a, cudaStream_t st) {
   const int smem = p.total < 120 * 1024 ? 120 * 1024 : p.total;
   dim3 grid(2, ntiles, 1);
   enc_gru_fwd_persist<<<grid, kFwdThreads, smem, st>>>(at, mhi, mlo);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
-}
-
-// ================================================================================================
-// Backward: one CTA per tile of 128 windows walks the window steps in reverse.  The hidden units are processed in chunks of 32:
-// the gate warps (thread = window x 16 units) turn dh_s into the gate gradients of the chunk and write them as split-bf16
-// operand planes [128 windows x (da_r | da_u | da_n r) of 32 units] into one of two shared-memory buffers; the MMA warp
-// accumulates dh_{s-1} += dA_h(chunk) W_hh[chunk rows, :] into the other of two TMEM accumulators ([128 x E] fp32 each) while
-// the gate warps work on the next chunk.  W_hh streams from L2 as MN-major operand blocks (TMA boxes of 32 rows x 64 columns).
-// The direct part dh_s * u_s travels through an L2-resident tiled scratch (same thread writes and re-reads it); the gate
-// gradients leave for the weight-gradient GEMMs through a per-warp shared-memory transpose, so that the global stores cover
-// whole 96-byte row segments instead of one 16-byte piece per line.
-namespace {
-
-constexpr int kCU = 32;                          // hidden units per chunk
-constexpr int kAGate = kRows * 64;               // bytes of one gate block [128 windows x 32 units] of one plane (64-byte swizzle)
-constexpr int kABuf = 2 * 3 * kAGate;            // one chunk buffer: 2 planes x 3 gates
-constexpr int kStgRow = 112;                     // staging row pitch in bytes (96 + 16: conflict-free 128-bit accesses)
-constexpr int kStgWarp = 32 * kStgRow;
-
-struct BwdPlan {
-  int acc_off, stg_off, b_off, stage_bytes, stages, bar_off, total;
-};
-__host__ __device__ inline BwdPlan bwd_plan(int E) {
-  BwdPlan p;
-  p.acc_off = 2 * kABuf;                          // bias-gradient accumulators [4][E] fp32
-  p.stg_off = p.acc_off + 4 * E * 4;
-  p.b_off = (p.stg_off + kEpiWarps * kStgWarp + 1023) & ~1023;
-  p.stage_bytes = (E / 64) * 32 * 128;            // W_hh rows [g*E + 32j, +32) x all E columns of one plane: E/64 boxes of [32][64]
-  const int budget = 227 * 1024 - 1024 - 256 - p.b_off;
-  p.stages = budget / p.stage_bytes;
-  if (p.stages > kMaxStages) p.stages = kMaxStages;
-  p.bar_off = p.b_off + p.stages * p.stage_bytes;
-  p.total = p.bar_off + 256 + 1024;
-  return p;
-}
-
-// MN-major operand block (rows = K index, 64 MN elements = 128 bytes per row, 128-byte swizzle): LBO = stride between
-// 64-element MN chunks, SBO = 8 K-rows (gemm_tc.cu: make_sdesc with b_mn)
-__device__ __forceinline__ uint64_t make_sdesc_mn(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= 1ull << 46;
-  d |= 2ull << 61;  // SWIZZLE_128B
-  return d;
-}
-
-// Sum over the 32 lanes of 64 values per lane; lane l ends up with the totals of indices 2l and 2l+1 (in v[0], v[1]).
-
-// Sum over the 32 lanes of 32 values per lane; lane l ends up with the total of index l (in v[0]).
-__device__ __forceinline__ void warp_reduce32(float (&v)[32], int lane) {
-#pragma unroll
-  for (int half = 16, bit = 16; half >= 1; half >>= 1, bit >>= 1) {
-    const bool upper = (lane & bit) != 0;
-#pragma unroll
-    for (int i = 0; i < half; ++i) {
-      const float send = upper ? v[i] : v[i + half];
-      const float keep = upper ? v[i + half] : v[i];
-      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, bit);
-    }
-  }
-}
-
-}  // namespace
-
-template <bool G16>  // gate stash in 16-bit fixed point (the tensor-core modes' default) or fp32
-__global__ void __launch_bounds__(kThreads, 1)
-enc_gru_bwd_persist(const BwdArgs a, const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo) {
-  extern __shared__ __align__(16) uint8_t smraw[];
-  uint8_t *smb = (uint8_t *)(((uintptr_t)smraw + 1023) & ~(uintptr_t)1023);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int E = a.E, hist = a.hist, nch = E / kCU;
-  const BwdPlan pl = bwd_plan(E);
-  uint8_t *sA = smb, *sB = smb + pl.b_off;
-  float *bacc = (float *)(smb + pl.acc_off);
-  uint64_t *bars = (uint64_t *)(smb + pl.bar_off);
-  uint64_t *full = bars, *empty = bars + kMaxStages, *a_full = bars + 2 * kMaxStages, *a_empty = a_full + 2, *acc_full = a_full + 4;
-  uint32_t *tmem_slot = (uint32_t *)(a_full + 5);
-
-  if (tid == 0) {
-    for (int s = 0; s < pl.stages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int b = 0; b < 2; ++b) { mbar_init(&a_full[b], kEpiWarps); mbar_init(&a_empty[b], 1); }
-    mbar_init(acc_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  for (int i = tid; i < 4 * E; i += kThreads) bacc[i] = 0.f;
-  if (warp == kEpiWarps + 1) tmem_alloc(tmem_slot, kTmemCols);
-  fence_before();
-  __syncthreads();
-  fence_after();
-  const uint32_t tmem = *tmem_slot;
-  const int tile = blockIdx.x;
-  const int nit = hist - 1;  // iterations with a product (it = hist-1-s for s >= 1)
-
-  if (warp == kEpiWarps) {
-    // ============================== TMA producer: W_hh rows of (chunk, plane, gate) as MN-major blocks ===================
-    if (lane == 0) {
-      // The stash of a step is read once, 2 GB after it was written: it comes from HBM.  One thread asks the L2 for the NEXT
-      // step's blocks of this tile (the row-interleaved layout makes them whole contiguous ranges per 32-window group) while
-      // the gate warps work on the current one, so that their loads pay L2 latency instead of HBM latency.
-      const size_t Mp = tiled_rows((size_t)a.M);
-      const size_t g0 = (size_t)blockIdx.x * (kRows / 32), g1 = min(g0 + kRows / 32, Mp / 32);
-      auto prefetch_step = [&](int s) {
-        if (s < 0) return;
-        const size_t gbytes = (size_t)3 * E * (a.gates16 ? 64 : 128), ebytes = (size_t)E * 128;  // bytes per 32-window group
-        const char *gb = reinterpret_cast<const char *>(a.gates) + (size_t)s * Mp * 3 * E * sizeof(float);
-        const char *ab = reinterpret_cast<const char *>(a.ahn + (size_t)s * Mp * E);
-        for (size_t gq = g0; gq < g1; ++gq) {
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gb + gq * gbytes), "r"((uint32_t)gbytes) : "memory");
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(ab + gq * ebytes), "r"((uint32_t)ebytes) : "memory");
-          if (s > 0) {
-            const char *hb = reinterpret_cast<const char *>(a.hs + (size_t)(s - 1) * Mp * E);
-            asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(hb + gq * ebytes), "r"((uint32_t)ebytes) : "memory");
-          }
-        }
-      };
-      prefetch_step(hist - 1);
-      prefetch_step(hist - 2);
-      int st = 0; uint32_t ph = 0;
-      for (int it = 0; it < nit; ++it) {
-        prefetch_step(hist - 3 - it);
-        for (int j = 0; j < nch; ++j)
-          for (int p = 0; p < a.nplanes; ++p)
-            for (int g = 0; g < 3; ++g) {
-              mbar_wait(&empty[st], ph ^ 1);
-              mbar_expect_tx(&full[st], (uint32_t)pl.stage_bytes);
-              uint8_t *dst = sB + (size_t)st * pl.stage_bytes;
-              const CUtensorMap *mp = p ? &map_lo : &map_hi;
-              for (int i = 0; i < E / 64; ++i) tma_load_3d(dst + i * 4096, mp, &full[st], 64 * i, g * E + kCU * j, 0);
-              if (++st == pl.stages) { st = 0; ph ^= 1; }
-            }
-      }
-    }
-  } else if (warp == kEpiWarps + 1) {
-    // ============================== MMA issuer ==============================================================================
-    if (lane == 0) {
-      const uint32_t sAu = smem_u32(sA), sBu = smem_u32(sB);
-      // D fp32, A / B bf16, A K-major, B MN-major, N = E, M = 128
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((uint32_t)(E >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-      int st = 0; uint32_t ph = 0;
-      int cc = 0;
-      for (int it = 0; it < nit; ++it) {
-        const uint32_t d_tmem = tmem + (uint32_t)(((it + 1) & 1) * 256);
-        uint32_t acc = 0;
-        for (int j = 0; j < nch; ++j, ++cc) {
-          const int buf = cc & 1;
-          mbar_wait(&a_full[buf], (uint32_t)((cc >> 1) & 1));  // the chunk's gate gradients are in the operand planes
-          fence_after();
-          fence_async_smem();
-          for (int p = 0; p < a.nplanes; ++p)
-            for (int g = 0; g < 3; ++g) {
-              mbar_wait(&full[st], ph);
-              fence_after();
-              const uint32_t bbase = sBu + (uint32_t)st * pl.stage_bytes;
-              const int na = (p == 0 && a.nplanes == 2) ? 2 : 1;
-              for (int pa = 0; pa < na; ++pa) {
-                const uint32_t abase = sAu + (uint32_t)buf * kABuf + (uint32_t)pa * (3 * kAGate) + (uint32_t)g * kAGate;
-#pragma unroll
-                for (int ks = 0; ks < kCU / 16; ++ks) {
-                  umma_bf16(d_tmem, make_sdesc(abase + ks * 32, 512, kSw64), make_sdesc_mn(bbase + ks * 2048, 4096, 1024), idesc, acc);
-                  acc = 1;
-                }
-              }
-              umma_commit(&empty[st]);
-              if (++st == pl.stages) { st = 0; ph ^= 1; }
-            }
-          umma_commit(&a_empty[buf]);  // the chunk buffer may be overwritten once the products above have read it
-        }
-        umma_commit(acc_full);         // dh_{s-1} (product part) is complete
-      }
-    }
-  } else {
-    // ============================== gate backward: thread = window x 16 units of the chunk ===================================
-    const int q = warp & 3, sub = warp >> 2;
-    const int L = 32 * q + lane;
-    const size_t m_raw = (size_t)tile * kRows + L;
-    const bool row_ok = m_raw < (size_t)a.M;
-    const size_t m = row_ok ? m_raw : (size_t)a.M - 1;
-    const size_t Mp = tiled_rows((size_t)a.M);
-    const uint32_t tlane = tmem + ((uint32_t)(32 * q) << 16);
-    uint8_t *stg = smb + pl.stg_off + warp * kStgWarp;
-    const size_t row0 = (size_t)tile * kRows + 32 * q;  // first window of this warp
-    const bool extra_vec = a.dh_extra && (((uintptr_t)a.dh_extra & 15) == 0) && (a.dh_extra_ld % 4 == 0);
-    const bool tm = a.timing && blockIdx.x == 0 && tid == 0;
-    long long t_wait = 0, t_gate = 0;
-    int cc = 0;
-    // raw stash of one sub-chunk (8 units of this window): requested one sub-chunk ahead, so that its latency (L2: the TMA warp
-    // prefetches each step's stash from HBM) overlaps the packing / stores / reduction of the previous sub-chunk
-    struct Raw { uint4 g[3]; float gf[3][8]; float an[8], hp[8], dd[8]; };
-    auto load_raw = [&](int s, int it, int ug, uint4 (&g16)[3], float (&gf)[3][G16 ? 1 : 8], float (&an)[8], float (&hp)[8], float (&dd)[8]) {
-      const float *gstep = reinterpret_cast<const float *>(a.gates) + (size_t)s * Mp * 3 * E;
-      if constexpr (G16) {
-        const unsigned short *base = reinterpret_cast<const unsigned short *>(gstep);
-#pragma unroll
-        for (int g = 0; g < 3; ++g)
-          asm volatile("ld.global.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];"
-                       : "=r"(g16[g].x), "=r"(g16[g].y), "=r"(g16[g].z), "=r"(g16[g].w)
-                       : "l"(base + ((m >> 5) * (size_t)((3 * E) >> 3) + (size_t)((g * E + ug) >> 3)) * 256 + (m & 31) * 8));
-      } else {
-#pragma unroll
-        for (int g = 0; g < 3; ++g) {
-          float t[8];
-          ldt8(gstep, m, g * E + ug, 3 * E, t);
-#pragma unroll
-          for (int i = 0; i < (G16 ? 1 : 8); ++i) gf[g][i] = t[i];
-        }
-      }
-      ldt8(a.ahn + (size_t)s * Mp * E, m, ug, E, an);
-      if (s > 0) ldt8(a.hs + (size_t)(s - 1) * Mp * E, m, ug, E, hp);
-      else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) hp[i] = 0.f;
-      }
-      if (it > 0) ldt8(a.dhd, m, ug, E, dd);
-      else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) dd[i] = 0.f;
-      }
-    };
-    uint4 ng16[3]; float ngf[3][G16 ? 1 : 8], nan_[8], nhp[8], ndd[8];  // "next" register set
-    load_raw(hist - 1, 0, 16 * sub, ng16, ngf, nan_, nhp, ndd);
-    const int nsub = 2 * nch;  // sub-chunks per step
-    for (int it = 0; it < hist; ++it) {
-      const int s = hist - 1 - it;
-      const long long c0 = tm ? clock64() : 0;
-      if (it > 0) {
-        mbar_wait(acc_full, (uint32_t)((it - 1) & 1));
-        fence_after();
-      }
-      const long long c1 = tm ? clock64() : 0;
-      t_wait += c1 - c0;
-      const uint32_t tcur = tlane + (uint32_t)((it & 1) * 256);
-      for (int i2 = 0; i2 < nsub; ++i2) {
-        const int j = i2 >> 1, half = i2 & 1;
-        const int ug = kCU * j + 16 * sub + 8 * half;
-        float rg[8], ugt[8], ng[8], an[8], hp[8], dh[8];
-        // ---- this sub-chunk's operands (requested one sub-chunk ago) ----
-        if constexpr (G16) {
-#pragma unroll
-          for (int g = 0; g < 3; ++g) {
-            const uint32_t w[4] = {ng16[g].x, ng16[g].y, ng16[g].z, ng16[g].w};
-            float *dst = g == 0 ? rg : (g == 1 ? ugt : ng);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              if (g < 2) { dst[2 * i] = dq_unorm16((unsigned short)(w[i] & 0xffff)); dst[2 * i + 1] = dq_unorm16((unsigned short)(w[i] >> 16)); }
-              else { dst[2 * i] = dq_snorm16((unsigned short)(w[i] & 0xffff)); dst[2 * i + 1] = dq_snorm16((unsigned short)(w[i] >> 16)); }
-            }
-          }
-        } else {
-#pragma unroll
-          for (int i = 0; i < (G16 ? 1 : 8); ++i) { rg[i] = ngf[0][i]; ugt[i] = ngf[1][i]; ng[i] = ngf[2][i]; }
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { an[i] = nan_[i]; hp[i] = nhp[i]; }
-        if (it > 0) {
-          tmem_ld8(tcur + ug, dh);                  // (dA_h(s+1) W_hh)[:, ug..]
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 8; ++i) dh[i] += ndd[i];   // + dh_{s+1} * u_{s+1}
-        } else {
-          if (a.dh_extra) {
-            const float *ex = a.dh_extra + m * a.dh_extra_ld + ug;
-            if (extra_vec) {
-              const float4 t0 = *reinterpret_cast<const float4 *>(ex), t1 = *reinterpret_cast<const float4 *>(ex + 4);
-              dh[0] = t0.x; dh[1] = t0.y; dh[2] = t0.z; dh[3] = t0.w; dh[4] = t1.x; dh[5] = t1.y; dh[6] = t1.z; dh[7] = t1.w;
-            } else {
-#pragma unroll
-              for (int i = 0; i < 8; ++i) dh[i] = ex[i];
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) dh[i] = 0.f;
-          }
-        }
-        // ---- request the next sub-chunk (of this step, or the first one of the next step) ----
-        if (i2 + 1 < nsub) load_raw(s, it, kCU * ((i2 + 1) >> 1) + 16 * sub + 8 * ((i2 + 1) & 1), ng16, ngf, nan_, nhp, ndd);
-        else if (s > 0) load_raw(s - 1, it + 1, 16 * sub, ng16, ngf, nan_, nhp, ndd);
-        // ---- gate backward (aux::enc_gate_bwd2 semantics) ----
-        float dar[8], dau[8], dan[8], danr[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float dn = dh[i] * (1.0f - ugt[i]), du = dh[i] * (hp[i] - ng[i]);
-          dan[i] = dn * (1.0f - ng[i] * ng[i]);
-          dau[i] = du * ugt[i] * (1.0f - ugt[i]);
-          dar[i] = dan[i] * an[i] * rg[i] * (1.0f - rg[i]);
-          danr[i] = dan[i] * rg[i];
-          dh[i] *= ugt[i];                          // direct part for step s-1
-        }
-        if (s > 0 && row_ok) stt8(a.dhd, m, ug, E, dh);
-        // ---- operand planes of the chunk for dh_{s-1} += dA_h W_hh (K index = unit inside the chunk) ----
-        const int buf = cc & 1;
-        if (s > 0) {
-          if (half == 0) mbar_wait(&a_empty[buf], (uint32_t)(((cc >> 1) & 1) ^ 1));
-          uint8_t *ab = sA + buf * kABuf;
-          const uint32_t o0 = sw64_off(L, 2 * sub + half);
-#pragma unroll
-          for (int g = 0; g < 3; ++g) {
-            const float *src = g == 0 ? dar : (g == 1 ? dau : danr);
-            const float v0[8] = {src[0], src[1], src[2], src[3], src[4], src[5], src[6], src[7]};
-            uint4 h0, l0;
-            split8(v0, h0, l0);
-            *reinterpret_cast<uint4 *>(ab + g * kAGate + o0) = h0;
-            *reinterpret_cast<uint4 *>(ab + 3 * kAGate + g * kAGate + o0) = l0;
-          }
-          if (half == 1) {
-            fence_before();
-            fence_async_smem();
-            __syncwarp();
-            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&a_full[buf])) : "memory");
-          }
-        }
-        if (half == 1) ++cc;
-        // ---- gate gradients for the weight-gradient GEMMs: gate-interleaved columns (24 values = 3 pieces of 16 bytes per
-        //      window and plane), transposed through shared memory so that a store instruction covers whole 48-byte runs ----
-        {
-          __nv_bfloat16 *planes[2] = {(__nv_bfloat16 *)a.dah3_hi, (__nv_bfloat16 *)a.dah3_lo};
-#pragma unroll
-          for (int pp = 0; pp < 2; ++pp) {
-            if (planes[pp] == nullptr) continue;
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-              float v[8];
-#pragma unroll
-              for (int x = 0; x < 8; ++x) {
-                const int e = 8 * k + x, u = e / 3, g = e - 3 * u;
-                v[x] = g == 0 ? dar[u] : (g == 1 ? dau[u] : danr[u]);
-              }
-              uint4 hi, lo;
-              split8(v, hi, lo);
-              *reinterpret_cast<uint4 *>(stg + lane * kStgRow + 16 * k) = pp ? lo : hi;
-            }
-            __syncwarp();
-#pragma unroll
-            for (int k2 = 0; k2 < 3; ++k2) {
-              const int pc = k2 * 32 + lane, r = pc / 3, piece = pc - 3 * r;
-              const uint4 val = *reinterpret_cast<const uint4 *>(stg + r * kStgRow + 16 * piece);
-              const size_t mr = row0 + r;
-              if (mr < (size_t)a.M)
-                st_stream_u4(planes[pp] + ((size_t)s * a.M + mr) * 3 * E + 3 * ug + 8 * piece, val);
-            }
-            __syncwarp();
-          }
-          // da_n: 8 units = 1 piece per plane; staged as [hi lo] per window
-          {
-            uint4 h0, l0;
-            split8(dan, h0, l0);
-            *reinterpret_cast<uint4 *>(stg + lane * kStgRow) = h0; *reinterpret_cast<uint4 *>(stg + lane * kStgRow + 16) = l0;
-            __syncwarp();
-#pragma unroll
-            for (int k2 = 0; k2 < 2; ++k2) {
-              const int pc = k2 * 32 + lane, r = pc >> 1, piece = pc & 1;
-              const uint4 val = *reinterpret_cast<const uint4 *>(stg + r * kStgRow + 16 * piece);
-              const size_t mr = row0 + r;
-              __nv_bfloat16 *dst = (__nv_bfloat16 *)(piece == 0 ? a.dan_hi : a.dan_lo);
-              if (mr < (size_t)a.M && dst) st_stream_u4(dst + ((size_t)s * a.M + mr) * E + ug, val);
-            }
-            __syncwarp();
-          }
-        }
-        // ---- bias gradients: column sums over the warp's windows, then shared-memory accumulators ----
-        {
-          float v[32];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            v[i] = row_ok ? dar[i] : 0.f; v[8 + i] = row_ok ? dau[i] : 0.f; v[16 + i] = row_ok ? dan[i] : 0.f; v[24 + i] = row_ok ? danr[i] : 0.f;
-          }
-          warp_reduce32(v, lane);
-          atomicAdd(&bacc[(lane >> 3) * E + ug + (lane & 7)], v[0]);
-        }
-      }
-      if (tm) t_gate += clock64() - c1;
-    }
-    if (tm) printf("enc_persist bwd E=%d hist=%d: gate warp 0 per step: wait products %lld cycles, gate backward + stores %lld cycles\n", E, hist, t_wait / hist, t_gate / hist);
-  }
-
-  fence_before();
-  __syncthreads();
-  for (int i = tid; i < 4 * E; i += kThreads) {
-    const int type = i / E, u = i - type * E;
-    const float v = bacc[i];
-    if (type == 0) { atomicAdd(a.gb_ih + u, v); atomicAdd(a.gb_hh + u, v); }
-    else if (type == 1) { atomicAdd(a.gb_ih + E + u, v); atomicAdd(a.gb_hh + E + u, v); }
-    else if (type == 2) atomicAdd(a.gb_ih + 2 * E + u, v);
-    else atomicAdd(a.gb_hh + 2 * E + u, v);
-  }
-  if (warp == kEpiWarps + 1) {
-    fence_after();
-    tmem_dealloc(tmem, kTmemCols);
-  }
-}
-
-bool bwd_supported(int E, int hist, size_t M, int mode) {
-  if (!fwd_supported(E, hist, M, mode)) return false;
-  const BwdPlan p = bwd_plan(E);
-  return p.stages >= 3 && p.total <= 227 * 1024;
-}
-
-int launch_bwd(const BwdArgs &a, cudaStream_t st) {
-  LFI_REQUIRE(a.E == 128 || a.E == 256, LFI_ERR_SHAPE, "enc_persist bwd: E=%d unsupported", a.E);
-  LFI_REQUIRE(a.hs && a.gates && a.ahn && a.whh_hi && (a.nplanes == 1 || a.whh_lo) && a.dhd && a.dah3_hi && a.dan_hi && a.gb_ih && a.gb_hh,
-              LFI_ERR_ARG, "enc_persist bwd: null argument");
-  const BwdPlan p = bwd_plan(a.E);
-  LFI_REQUIRE(p.stages >= 3 && p.total <= 227 * 1024, LFI_ERR_SHAPE, "enc_persist bwd: shared-memory plan does not fit");
-  CUtensorMap mhi, mlo;
-  LFI_TRY(tc::make_plane_map(&mhi, a.whh_hi, 3 * a.E, a.E, a.E, 0, 1, 32));
-  if (a.nplanes == 2) LFI_TRY(tc::make_plane_map(&mlo, a.whh_lo, 3 * a.E, a.E, a.E, 0, 1, 32));
-  else mlo = mhi;
-  static const bool timing = env_flag("LFI_ENC_TIMING", false);
-  BwdArgs at = a;
-  at.timing = timing ? 1 : 0;
-  static bool attr_set = false;
-  if (!attr_set) {
-    LFI_CUDA(cudaFuncSetAttribute(enc_gru_bwd_persist<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    LFI_CUDA(cudaFuncSetAttribute(enc_gru_bwd_persist<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    attr_set = true;
-  }
-  const int ntiles = (a.M + kRows - 1) / kRows;
-  const int smem = p.total < 120 * 1024 ? 120 * 1024 : p.total;
-  if (a.gates16) enc_gru_bwd_persist<true><<<ntiles, kThreads, smem, st>>>(at, mhi, mlo);
-  else enc_gru_bwd_persist<false><<<ntiles, kThreads, smem, st>>>(at, mhi, mlo);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-__global__ void add_deinterleaved_rows_kernel(float *out, const float *in, int E, int ngates, int cols) {
-  const size_t n = (size_t)ngates * E * cols;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-    const int j = (int)(i % cols);
-    const size_t r = i / cols;
-    const int g = (int)(r / E), u = (int)(r - (size_t)g * E);
-    out[i] += in[((size_t)3 * u + g) * cols + j];
-  }
-}
-int add_deinterleaved_rows(float *out, const float *in, int E, int ngates, int cols, cudaStream_t st) {
-  const size_t n = (size_t)ngates * E * cols;
-  int blocks = (int)((n + 255) / 256);
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  add_deinterleaved_rows_kernel<<<blocks, 256, 0, st>>>(out, in, E, ngates, cols);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -1,12 +1,11 @@
-// Persistent windowed encoder GRU (ModalityEncoder `enc: rnn`, reference models.py:21-27, 55-69): ALL window steps of a tile of
-// 128 windows in ONE launch per direction, the recurrent state resident on chip between the steps (enc_persist.cu).
+// Persistent windowed encoder GRU, forward (ModalityEncoder `enc: rnn`, reference models.py:21-27, 55-69): ALL window steps of a
+// tile of 128 windows in ONE launch, the recurrent state resident on chip between the steps (enc_persist.cu).
 //
-// Row-interleaved ("tiled") layouts.  The kernels read their accumulators out of TMEM with thread = window (TMEM lane), so
-// every array that only these kernels touch is stored so that the 32 windows of a warp are contiguous per 4-float (16-byte)
-// column group - a warp-wide 128-bit access then covers 512 contiguous bytes instead of 32 separate lines:
+// Row-interleaved ("tiled") layout.  The kernel reads its accumulators out of TMEM with thread = window (TMEM lane), so the
+// input projections it reads are stored so that the 32 windows of a warp are contiguous per 4-float (16-byte) column group -
+// a warp-wide 128-bit access then covers 512 contiguous bytes instead of 32 separate lines:
 //   fp32, width W (W % 4 == 0):  element (m, n) at ((m >> 5) * (W >> 2) + (n >> 2)) * 128 + (m & 31) * 4 + (n & 3)       [floats]
-//   u16,  width W (W % 8 == 0):  element (m, n) at ((m >> 5) * (W >> 3) + (n >> 3)) * 256 + (m & 31) * 8 + (n & 7)       [u16]
-// Rows are padded to a multiple of 32 (Mp).  The input projections xp are TIME-major and tiled (row r = tau * B + b, written
+// Rows are padded to a multiple of 32.  The input projections xp are TIME-major and tiled (row r = tau * B + b, written
 // by the projection GEMM's row-interleaved epilogue, GemmArgs::c_tiled32): the raw frame of window m at step s is then row
 // m + (t0 - hist + 1 + s) * B - a constant offset per step, so the 32 windows of a warp read 32 consecutive rows.
 #pragma once
@@ -16,8 +15,6 @@ namespace lfi {
 namespace encp {
 
 __host__ __device__ inline size_t tiled_rows(size_t M) { return (M + 31) & ~(size_t)31; }
-__host__ __device__ inline size_t tiled_off_f32(size_t m, int n, int W) { return ((m >> 5) * (size_t)(W >> 2) + (size_t)(n >> 2)) * 128 + (m & 31) * 4 + (n & 3); }
-__host__ __device__ inline size_t tiled_off_u16(size_t m, int n, int W) { return ((m >> 5) * (size_t)(W >> 3) + (size_t)(n >> 3)) * 256 + (m & 31) * 8 + (n & 7); }
 
 struct FwdArgs {
   int E, hist, B, T, t0, M;       // hidden size, window length, batch geometry (row m = t' * B + b), rows
@@ -26,43 +23,12 @@ struct FwdArgs {
   const float *b_ih, *b_hh;       // [3E]
   const float *mask;              // [M][hist] frame-dropout mask (already scaled) or nullptr
   const void *whh_hi, *whh_lo;    // bf16 planes of W_hh [3E][E]
-  // outputs; the per-step arrays are [hist] blocks when stash != 0 and absent otherwise (sampling)
-  int stash;
-  float *hs;                      // [hist][Mp][E]  tiled fp32 state (h_{s-1} of the backward gate math)
-  void *hp_hi, *hp_lo;            // [hist][M][E]   row-major bf16 planes of the state (operand of dW_hh)
-  void *gates; int gates16;       // [hist] blocks of Mp*3E floats: r, u, n after activation, tiled fp32 or tiled 16-bit fixed point
-  float *ahn;                     // [hist][Mp][E]  tiled h-side n pre-activation
   float *cond; int cond_ld;       // final state -> cond[m * cond_ld + e]  (row-major)
   int timing;                     // debug (LFI_ENC_TIMING=1): block (0,0) prints its per-step phase cycles
 };
 
-// Backward of the above (BPTT over the window).  Per step s = hist-1 .. 0 and window m:
-//   dh_s = dh_extra (s = hist-1: d cond) + dh_{s+1} * u_{s+1} + (dA_h(s+1) W_hh)          [the product runs on the tensor cores]
-//   gate backward -> da_r, da_u, da_n, da_n * r ; dA_h(s) = (da_r, da_u, da_n * r)
-// Outputs for the batched weight-gradient GEMMs (row-major bf16 planes, gate-interleaved columns):
-//   dah3 [hist][M][3E]: column 3 * unit + g = (da_r, da_u, da_n * r)[g]    (dW_hh, and the r / u rows of dW_ih)
-//   dan  [hist][M][E] : da_n                                               (the n rows of dW_ih)
-// and the bias gradients (accumulated): gb_ih += (sum da_r, sum da_u, sum da_n), gb_hh += (sum da_r, sum da_u, sum da_n * r).
-struct BwdArgs {
-  int E, hist, M;
-  int nplanes;
-  const float *hs;                // forward stash (tiled), as FwdArgs
-  const void *gates; int gates16;
-  const float *ahn;
-  const void *whh_hi, *whh_lo;    // bf16 planes of W_hh [3E][E]
-  const float *dh_extra; int dh_extra_ld;  // d cond columns of this modality: row-major [M][ld]
-  float *dhd;                     // [Mp][E] tiled scratch: direct part dh_s * u_s between two steps
-  void *dah3_hi, *dah3_lo, *dan_hi, *dan_lo;
-  float *gb_ih, *gb_hh;           // [3E] accumulated
-  int timing;
-};
-
 bool fwd_supported(int E, int hist, size_t M, int mode);
 int launch_fwd(const FwdArgs &a, cudaStream_t st);
-bool bwd_supported(int E, int hist, size_t M, int mode);
-int launch_bwd(const BwdArgs &a, cudaStream_t st);
-// out[g * E + u][j] += in[3 * u + g][j]  (g < 3): rows of a weight gradient taken over gate-interleaved columns back to (gate, unit) order
-int add_deinterleaved_rows(float *out, const float *in, int E, int ngates, int cols, cudaStream_t st);
 
 }  // namespace encp
 

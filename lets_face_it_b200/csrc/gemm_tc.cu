@@ -288,7 +288,7 @@ __device__ __forceinline__ void gru_fwd_tile(const Params &p, const TileCoord &t
   const GruEpi &G = p.gru;
   const int E = G.E;
   const int rr = lane & 7, cg = (lane >> 3) * 4;
-  const int UT = p.bn / 3;  // hidden units per tile (64 or 32): TMEM columns [0,UT) r, [UT,2UT) u, [2UT,3UT) n
+  const int UT = p.bn / 3;  // hidden units per tile (64): TMEM columns [0,UT) r, [UT,2UT) u, [2UT,3UT) n
   const int u_base = (t.n0 / p.bn) * UT;
   const int mrow0 = t.m0 + q * 32;
   __nv_bfloat16 *hhi = (__nv_bfloat16 *)G.h_hi, *hlo = (__nv_bfloat16 *)G.h_lo;
@@ -372,80 +372,6 @@ __device__ __forceinline__ void gru_fwd_tile(const Params &p, const TileCoord &t
           else { cd[0] = hn[0]; cd[1] = hn[1]; cd[2] = hn[2]; cd[3] = hn[3]; }
         }
         if (hhi) st_planes4(hhi, hlo, o1, hn);
-      }
-    }
-  }
-  if (!waited) { mbar_wait(tfull, aph); tc_fence_after(); }
-}
-
-// Backward (aux::enc_gate_bwd2_kernel semantics): the accumulator tile is dA_h(s) W_hh for 128 windows x all E units;
-// dh_{s-1} = tile + dh (direct part), then the gate backward of step s-1.  Bias gradients: per-lane sums over its four
-// rows, butterfly over the eight row lanes, one atomic per column and warp.
-__device__ __forceinline__ void gru_bwd_tile(const Params &p, const TileCoord &t, uint32_t tbase, float *stg, int q, int half, int lane,
-                                             uint64_t *tfull, uint32_t aph, int nsub) {
-  const GruEpi &G = p.gru;
-  const int E = G.E;
-  const int rr = lane & 7, cg = (lane >> 3) * 4;
-  const int mrow0 = t.m0 + q * 32;
-  __nv_bfloat16 *dah_hi = (__nv_bfloat16 *)G.dah_hi, *dah_lo = (__nv_bfloat16 *)G.dah_lo;
-  __nv_bfloat16 *dan_hi = (__nv_bfloat16 *)G.dan_hi, *dan_lo = (__nv_bfloat16 *)G.dan_lo;
-  bool waited = false;
-  for (int sc = half; sc < E / 16; sc += nsub) {
-    const int e = 16 * sc + cg;
-    float4 d4[4], r4[4], u4[4], n4[4], a4[4], h4[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int m = min(mrow0 + rr + 8 * i, p.M - 1);
-      const size_t o1 = (size_t)m * E + e, o3 = (size_t)m * 3 * E + e;
-      d4[i] = ld4(G.dh + o1); r4[i] = ld4(G.bgates + o3); u4[i] = ld4(G.bgates + o3 + E); n4[i] = ld4(G.bgates + o3 + 2 * E);
-      a4[i] = ld4(G.bahn + o1);
-      h4[i] = G.bhprev ? ld4(G.bhprev + o1) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    if (!waited) { mbar_wait(tfull, aph); tc_fence_after(); waited = true; }
-    float acc[4][4];
-    chunk_to_rows(tbase + sc * 16, stg, lane, rr, cg, acc);
-    float s_r[4] = {0.f, 0.f, 0.f, 0.f}, s_u[4] = {0.f, 0.f, 0.f, 0.f}, s_n[4] = {0.f, 0.f, 0.f, 0.f}, s_nr[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int m = mrow0 + rr + 8 * i;
-      if (m < p.M) {
-        const size_t o1 = (size_t)m * E + e, o3 = (size_t)m * 3 * E + e;
-        const float dd[4] = {d4[i].x, d4[i].y, d4[i].z, d4[i].w}, rg[4] = {r4[i].x, r4[i].y, r4[i].z, r4[i].w}, uu[4] = {u4[i].x, u4[i].y, u4[i].z, u4[i].w};
-        const float nn[4] = {n4[i].x, n4[i].y, n4[i].z, n4[i].w}, aa[4] = {a4[i].x, a4[i].y, a4[i].z, a4[i].w}, hh[4] = {h4[i].x, h4[i].y, h4[i].z, h4[i].w};
-        float dar[4], dau[4], dan[4], dnr[4], dhn[4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const float dh = dd[c] + acc[i][c];
-          const float dn = dh * (1.0f - uu[c]), du = dh * (hh[c] - nn[c]);
-          dan[c] = dn * (1.0f - nn[c] * nn[c]);
-          dau[c] = du * uu[c] * (1.0f - uu[c]);
-          dar[c] = dan[c] * aa[c] * rg[c] * (1.0f - rg[c]);
-          dnr[c] = dan[c] * rg[c];
-          dhn[c] = dh * uu[c];
-          s_r[c] += dar[c]; s_u[c] += dau[c]; s_n[c] += dan[c]; s_nr[c] += dnr[c];
-        }
-        st4(G.dh + o1, dhn[0], dhn[1], dhn[2], dhn[3]);
-        st_planes4(dah_hi, dah_lo, o3, dar);
-        st_planes4(dah_hi, dah_lo, o3 + E, dau);
-        st_planes4(dah_hi, dah_lo, o3 + 2 * E, dnr);
-        st_planes4(dan_hi, dan_lo, o1, dan);
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-#pragma unroll
-      for (int o = 1; o < 8; o <<= 1) {
-        s_r[c] += __shfl_xor_sync(0xffffffffu, s_r[c], o);
-        s_u[c] += __shfl_xor_sync(0xffffffffu, s_u[c], o);
-        s_n[c] += __shfl_xor_sync(0xffffffffu, s_n[c], o);
-        s_nr[c] += __shfl_xor_sync(0xffffffffu, s_nr[c], o);
-      }
-    }
-    if (rr == 0) {
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        atomicAdd(G.gb_ih + e + c, s_r[c]); atomicAdd(G.gb_ih + E + e + c, s_u[c]); atomicAdd(G.gb_ih + 2 * E + e + c, s_n[c]);
-        atomicAdd(G.gb_hh + e + c, s_r[c]); atomicAdd(G.gb_hh + E + e + c, s_u[c]); atomicAdd(G.gb_hh + 2 * E + e + c, s_nr[c]);
       }
     }
   }
@@ -661,10 +587,9 @@ gemm_tc_kernel(const Params p, const __grid_constant__ CUtensorMap mapA0, const 
       const bool has_work = t.kb1 > t.kb0;
       const int mrow0 = t.m0 + q * 32;
       bool waited = false;
-      if constexpr (FUSE != LFI_FUSE_NONE) {
+      if constexpr (GRUF) {
         const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + as * 256;
-        if constexpr (GRUF) gru_fwd_tile<XF>(p, t, tb, stg, q, half, lane, &tfull[as], aph, EW / 4);
-        else gru_bwd_tile(p, t, tb, stg, q, half, lane, &tfull[as], aph, EW / 4);
+        gru_fwd_tile<XF>(p, t, tb, stg, q, half, lane, &tfull[as], aph, EW / 4);
         waited = true;
       }
       for (int sc = half; sc < p.bn / 16 && FUSE == LFI_FUSE_NONE; sc += EW / 4) {
@@ -907,19 +832,13 @@ static int launch_core(const Operand &A, const Operand &B, const GemmArgs &g, in
   const bool gruf = g.fuse == LFI_FUSE_GRU_FWD || g.fuse == LFI_FUSE_GRU_FWD_X;
   if (gruf) {
     LFI_REQUIRE(g.gru.E % 64 == 0 && g.N == 3 * g.gru.E && !B.mn && g.batch == 1, LFI_ERR_SHAPE, "gemm_tc: fused GRU forward needs E %% 64 == 0");
-    // 64 hidden units per tile, or 32 (LFI_GRU_TILE32=1): twice the tiles, half the epilogue per tile, a finer last wave
-    static const bool tile32 = env_flag("LFI_GRU_TILE32", false);
-    p.bn = tile32 ? 96 : 192;
+    p.bn = 192;  // 64 hidden units per tile
     if (g.fuse == LFI_FUSE_GRU_FWD_X)
       LFI_REQUIRE(g.gru.xa_hi && g.gru.xb_hi && (nplanes == 1 || (g.gru.xa_lo && g.gru.xb_lo)) && g.gru.xk >= 8 && g.gru.xk % 8 == 0 &&
                       g.gru.xa_ld % 8 == 0 && g.gru.xb_ld % 8 == 0,
                   LFI_ERR_ARG, "gemm_tc: fused GRU forward with input part needs the input / W_ih operand planes (pitch %% 8 == 0)");
     const float *cd = g.gru.cond;
     p.cond_vec = cd && (((uintptr_t)cd & 15) == 0) && g.gru.cond_ld % 4 == 0;
-  } else if (g.fuse == LFI_FUSE_GRU_BWD) {
-    LFI_REQUIRE(g.gru.E == g.N && (g.N == 64 || g.N == 128 || g.N == 192 || g.N == 256) && g.batch == 1, LFI_ERR_SHAPE,
-                "gemm_tc: fused GRU backward needs E in {64,128,192,256}");
-    p.bn = g.N;
   }
   p.nplanes = nplanes; p.a_mn = A.mn; p.b_mn = B.mn;
   if (!g_sms) {
@@ -1019,7 +938,6 @@ static int launch_core(const Operand &A, const Operand &B, const GemmArgs &g, in
     LFI_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<LFI_FUSE_NONE, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
     LFI_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<LFI_FUSE_GRU_FWD, 1, kGruEpiWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
     LFI_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<LFI_FUSE_GRU_FWD_X, 1, kGruEpiWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-    LFI_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<LFI_FUSE_GRU_BWD, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
     attr_set = true;
   }
   const long ntiles = tiles * p.splitk;
@@ -1028,7 +946,6 @@ static int launch_core(const Operand &A, const Operand &B, const GemmArgs &g, in
   const int smem_req = smem < 120 * 1024 ? 120 * 1024 : smem;
   if (g.fuse == LFI_FUSE_GRU_FWD) gemm_tc_kernel<LFI_FUSE_GRU_FWD, 1, kGruEpiWarps><<<grid, threads_for(kGruEpiWarps), smem_req, st>>>(p, mA0, mA1, mB0, mB1, mXA0, mXA1, mXB0, mXB1);
   else if (g.fuse == LFI_FUSE_GRU_FWD_X) gemm_tc_kernel<LFI_FUSE_GRU_FWD_X, 1, kGruEpiWarps><<<grid, threads_for(kGruEpiWarps), smem_req, st>>>(p, mA0, mA1, mB0, mB1, mXA0, mXA1, mXB0, mXB1);
-  else if (g.fuse == LFI_FUSE_GRU_BWD) gemm_tc_kernel<LFI_FUSE_GRU_BWD, 1><<<grid, kThreads, smem_req, st>>>(p, mA0, mA1, mB0, mB1, mXA0, mXA1, mXB0, mXB1);
   else if (pair) {
     // CTA pairs: one 256-row cta_group::2 tile per cluster
     cudaLaunchConfig_t cfg;

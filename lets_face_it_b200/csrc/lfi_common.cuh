@@ -134,13 +134,13 @@ struct PlaneRef {
 };
 
 // Fused encoder-GRU epilogues of the tcgen05 GEMM (ModalityEncoder nn.GRU, models.py:21-27, 63-64): the window step's
-// recurrent product h_{s-1} W_hh^T (forward) / dA_h W_hh (backward) leaves TMEM straight into the gate math, so the
-// [M, 3E] pre-activation matrix never travels through HBM.  Argument meaning as aux::EncStep / aux::EncStepBwd2.
+// recurrent product h_{s-1} W_hh^T leaves TMEM straight into the gate math, so the [M, 3E] pre-activation matrix never
+// travels through HBM.  Argument meaning as aux::EncStep.
 // LFI_FUSE_GRU_FWD_X: as _FWD, and the input projection of the step joins the same accumulator: the masked window inputs of
 // step s (operand planes [M, xk], as gathered for the dW_ih GEMMs) times W_ih^T run as extra k-blocks - r and u on top of the
 // recurrent product, the n gate's input part into a fourth column group (it stays outside r * (...)) - so the epilogue has no
 // [M, 3E] projection rows to fetch (three of its four 16-byte load streams).
-enum { LFI_FUSE_NONE = 0, LFI_FUSE_GRU_FWD = 1, LFI_FUSE_GRU_BWD = 2, LFI_FUSE_GRU_FWD_X = 3 };
+enum { LFI_FUSE_NONE = 0, LFI_FUSE_GRU_FWD = 1, LFI_FUSE_GRU_FWD_X = 3 };
 // 16-bit fixed-point gate stash of the encoder GRUs (tensor-core modes): r, u in [0,1] as unorm16 (|err| <= 7.7e-6), n in
 // [-1,1] as snorm16 (|err| <= 1.6e-5).  The forward pass itself uses the exact fp32 gates; only the backward pass reads
 // the stash, and its gradient tolerance (5e-3 relative L2 per tensor in bf16x3 mode) is ~100x above the induced error.
@@ -159,11 +159,6 @@ struct GruEpi {
   // LFI_FUSE_GRU_FWD_X: masked window inputs of this step [M, xk] and W_ih [3E, xk] as operand planes (pitches in elements)
   const void *xa_hi, *xa_lo, *xb_hi, *xb_lo; int xa_ld, xb_ld, xk;
   int x_only;  // window step 0: zero state, no recurrent product - the launch consists of the input part alone (hprev == nullptr)
-  // backward: the GEMM of step s yields dh_{s-1}; the epilogue runs the gate backward of step s-1
-  const float *bgates, *bahn, *bhprev;   // stash of step s-1 (bhprev = h_{s-2}, nullptr when s-1 == 0)
-  float *dh;                             // [M][E] in: direct part dh_s * u_s, out: dh_{s-1} * u_{s-1}
-  void *dah_hi, *dah_lo, *dan_hi, *dan_lo;
-  float *gb_ih, *gb_hh;
 };
 
 struct GemmArgs {

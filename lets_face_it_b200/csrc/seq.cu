@@ -93,11 +93,9 @@ struct EncWs {
   bool xfuse;             // the forward steps s >= 1 take their input projection inside the step GEMM (training, per-step path)
   float *xg32;            // the same in fp32 [hist][M][dim] (split source / fp32-mode operand)
   float *dhe;             // [M][E] running d h of the window recurrence
-  // persistent window-GRU kernels (enc_persist.cu): xp is time-major and row-interleaved, the stash (hs, gates, ahn, dhe) is
-  // row-interleaved with rows padded to 32, dah holds gate-interleaved columns
+  // persistent window-GRU forward (enc_persist.cu; sampling / feature encoding only): xp is time-major and row-interleaved
   bool persist;
   float *xT;              // [T*B][dim] raw frames in time-major order (input of the projection GEMM)
-  float *wscr;            // [3E][E + round_up(dim, 8)] weight gradients over gate-interleaved rows, before de-interleaving
 };
 
 // A modality's encoder runs on operand planes when every GEMM it issues is taken by the tcgen05 tiles.
@@ -108,17 +106,15 @@ static bool enc_use_planes(const lfi_shape *s, int m, size_t M, int mode) {
   GemmArgs g = gemm_args(0, 1, (int)M, 3 * E, E, nullptr, E, nullptr, E, nullptr, 3 * E);
   return gemm_tc_wants(g);
 }
-// The persistent window-GRU kernels take over a modality when its encoder runs on operand planes, the shape fits them and the
-// projection GEMM is taken by the tcgen05 tiles (only those write the row-interleaved xp).
-// Switches (read at call time): training uses them when LFI_ENC_PERSIST=1 - measured on B200 they tie with the per-step launches
-// on one GPU (11.08 vs 11.03 ms per step) and lose 1.3 % at two GPUs, because a 225 KB-shared-memory CTA per SM leaves no room for
-// the NCCL kernels that overlap the encoder backward (DESIGN.md section 4) - so the default for training is the per-step path.
-// Sampling / feature encoding (no stash to store) is 4 % faster with them: on by default (LFI_ENC_PERSIST_SAMPLE=0 turns them off).
-static bool enc_use_persist(const lfi_shape *s, int m, size_t M, size_t BT, int mode, bool need_bwd) {
-  if (!env_flag(need_bwd ? "LFI_ENC_PERSIST" : "LFI_ENC_PERSIST_SAMPLE", !need_bwd)) return false;
+// The persistent window-GRU forward kernel takes over a modality in sampling / feature encoding (no stash to store: 4 % faster
+// than the per-step launches; LFI_ENC_PERSIST_SAMPLE=0 turns it off, read at call time) when its encoder runs on operand planes,
+// the shape fits the kernel and the projection GEMM is taken by the tcgen05 tiles (only those write the row-interleaved xp).
+// Training always runs the per-step launches, which write the stash of the backward pass.
+static bool enc_use_persist(const lfi_shape *s, int m, size_t M, size_t BT, int mode) {
+  if (!env_flag("LFI_ENC_PERSIST_SAMPLE", true)) return false;
   if (!enc_use_planes(s, m, M, mode)) return false;
   const int E = s->ehid[m], hist = s->hist[m];
-  if (need_bwd ? !encp::bwd_supported(E, hist, M, mode) : !encp::fwd_supported(E, hist, M, mode)) return false;
+  if (!encp::fwd_supported(E, hist, M, mode)) return false;
   GemmArgs g = gemm_args(0, 1, (int)BT, 3 * E, s->dim[m], nullptr, s->dim[m], nullptr, s->dim[m], nullptr, 3 * E);
   return gemm_tc_wants(g);
 }
@@ -166,16 +162,12 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
     if (s->hist[m] <= 0 || s->ehid[m] <= 0) continue;
     const size_t E = s->ehid[m], h = s->hist[m];
     EncWs &e = w->enc[m];
-    const size_t Mp = encp::tiled_rows(M);
-    e.xp = b.take<float>(encp::tiled_rows((size_t)B * T) * 3 * E);
-    e.hs = b.take<float>(h * Mp * E);
-    e.gates = b.take<float>(h * Mp * 3 * E);
-    e.ahn = b.take<float>(h * Mp * E);
+    e.xp = b.take<float>((size_t)B * T * 3 * E);
+    e.hs = b.take<float>(h * M * E);
+    e.gates = b.take<float>(h * M * 3 * E);
+    e.ahn = b.take<float>(h * M * E);
     e.planes = enc_use_planes(s, m, M, mode);
-    e.persist = enc_use_persist(s, m, M, (size_t)B * T, mode, true);
-    e.xT = e.persist ? b.take<float>((size_t)B * T * s->dim[m]) : nullptr;
-    e.wscr = e.persist ? b.take<float>(3 * E * (E + round_up(s->dim[m], 8))) : nullptr;
-    e.gates16 = e.planes && E % 4 == 0 && env_flag("LFI_GATES16", true) && !env_flag("LFI_FUSED_GRU_BWD", false);
+    e.gates16 = e.planes && E % 4 == 0 && env_flag("LFI_GATES16", true);
     if (e.planes) {
       const bool lo = mode == LFI_GEMM_BF16X3;
       const size_t dimp = round_up(s->dim[m], 8);
@@ -187,13 +179,13 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
       e.wih_hi = take_bf16(b, 3 * E * dimp);        e.wih_lo = lo ? take_bf16(b, 3 * E * dimp) : nullptr;
       // input projection inside the fused step GEMM: the masked window inputs are gathered as operand planes in the forward pass
       // (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand; step 0 (no state yet) keeps the xp rows
-      e.xfuse = !e.persist && E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true) && env_flag("LFI_ENC_XFUSE", true);
+      e.xfuse = E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true) && env_flag("LFI_ENC_XFUSE", true);
     } else {
       e.dah32 = b.take<float>(h * M * 3 * E);
       e.dan32 = b.take<float>(h * M * E);
     }
     e.xg32 = b.take<float>(h * M * s->dim[m]);
-    e.dhe = b.take<float>(Mp * E);
+    e.dhe = b.take<float>(M * E);
     if (M * 3 * E > ghmax) ghmax = M * 3 * E;
     if (h * M * s->dim[m] > xgmax) xgmax = h * M * s->dim[m];
     if (E > emax) emax = E;
@@ -343,11 +335,6 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       a.E = E; a.hist = hist; a.B = B; a.T = T; a.t0 = t0; a.M = (int)M; a.nplanes = lo ? 2 : 1;
       a.xp = ew.xp; a.b_ih = p->enc_b_ih[m]; a.b_hh = p->enc_b_hh[m]; a.mask = bt->mask[m];
       a.whh_hi = ew.whh_hi; a.whh_lo = lo ? ew.whh_lo : nullptr;
-      a.stash = stash ? 1 : 0;
-      if (stash) {
-        a.hs = ew.hs; a.hp_hi = ew.hp_hi; a.hp_lo = lo ? ew.hp_lo : nullptr;
-        a.gates = ew.gates; a.gates16 = ew.gates16 ? 1 : 0; a.ahn = ew.ahn;
-      }
       a.cond = cond + d.enc_offe[m]; a.cond_ld = d.Fe;
       return encp::launch_fwd(a, cs);
     }
@@ -749,41 +736,7 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
       LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, d.start_ts, Tp, st));
     else
       LFI_TRY(aux::gather_windows(ew.xg32, dim, 1, bt->x[m], bt->mask[m], B, T, dim, hist, 1, d.start_ts, Tp, st));
-    if (ew.persist) {
-      // persistent BPTT over the window: one launch, then the weight gradients as long-K GEMMs over the gate-interleaved planes
-      encp::BwdArgs q;
-      memset(&q, 0, sizeof(q));
-      q.E = E; q.hist = hist; q.M = (int)M; q.nplanes = lo ? 2 : 1;
-      q.hs = ew.hs; q.gates = ew.gates; q.gates16 = ew.gates16 ? 1 : 0; q.ahn = ew.ahn;
-      q.whh_hi = ew.whh_hi; q.whh_lo = lo ? ew.whh_lo : nullptr;
-      q.dh_extra = w.dcond + d.enc_offe[m]; q.dh_extra_ld = d.Fe;
-      q.dhd = ew.dhe;
-      q.dah3_hi = ew.dah_hi; q.dah3_lo = lo ? ew.dah_lo : nullptr; q.dan_hi = ew.dan_hi; q.dan_lo = lo ? ew.dan_lo : nullptr;
-      q.gb_ih = g->enc_b_ih[m]; q.gb_hh = g->enc_b_hh[m];
-      LFI_TRY(encp::launch_bwd(q, st));
-      float *s_hh = ew.wscr, *s_ih = ew.wscr + (size_t)3 * E * E;
-      LFI_TRY(aux::fill(ew.wscr, 0.f, (size_t)3 * E * (E + dimp), st));
-      const int Kall = (int)(hist * M), Khh = (int)((hist - 1) * M);
-      if (hist > 1) {  // rows 3u+g of s_hh = sum_{s>=1} dA_h[s][:, (g, u)]^T h[s-1]
-        GemmArgs r = gemm_args(1, 0, 3 * E, E, Khh, nullptr, 3 * E, nullptr, E, s_hh, E, LFI_EPI_ACCUM);
-        r.pA = plane_ref(off16(ew.dah_hi, M * 3 * E), lo ? off16(ew.dah_lo, M * 3 * E) : nullptr, 3 * E);
-        r.pB = plane_ref(ew.hp_hi, ew.hp_lo, E);
-        LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
-        LFI_TRY(encp::add_deinterleaved_rows(g->enc_w_hh[m], s_hh, E, 3, E, st));
-      }
-      {  // r, u rows of dW_ih from the interleaved planes (the da_n r rows of the product are not used), n rows from da_n
-        GemmArgs r = gemm_args(1, 0, 3 * E, dim, Kall, nullptr, 3 * E, nullptr, dim, s_ih, dim, LFI_EPI_ACCUM);
-        r.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); r.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp);
-        LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
-        LFI_TRY(encp::add_deinterleaved_rows(g->enc_w_ih[m], s_ih, E, 2, dim, st));
-        GemmArgs n = gemm_args(1, 0, E, dim, Kall, nullptr, E, nullptr, dim, g->enc_w_ih[m] + (size_t)2 * E * dim, dim, LFI_EPI_ACCUM);
-        n.pA = plane_ref(ew.dan_hi, ew.dan_lo, E); n.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp);
-        LFI_TRY(gemm_dispatch(bmode, n, gws, gws_bytes, st));
-      }
-      return LFI_OK;
-    }
     LFI_TRY(aux::fill(ew.dhe, 0.f, M * E, st));
-    const bool fused = ew.planes && (E == 64 || E == 128 || E == 192 || E == 256) && env_flag("LFI_FUSED_GRU_BWD", false);
     for (int sidx = hist - 1; sidx >= 0; --sidx) {
       aux::EncStepBwd2 e;
       memset(&e, 0, sizeof(e));
@@ -797,21 +750,10 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
         e.dah32 = ew.dah32 + (size_t)sidx * M * 3 * E; e.dan32 = ew.dan32 + (size_t)sidx * M * E;
       }
       e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.gates16 ? 1 : 0;
-      if (!fused || sidx == hist - 1) LFI_TRY(aux::enc_gate_bwd2(e, st));
+      LFI_TRY(aux::enc_gate_bwd2(e, st));
       if (sidx) {  // dh_{s-1} += dA_h W_hh
         GemmArgs t = gemm_args(0, 0, (int)M, E, 3 * E, e.dah32, 3 * E, p->enc_w_hh[m], E, ew.dhe, E, LFI_EPI_ACCUM);
         if (ew.planes) { t.pA = plane_ref(e.dah_hi, e.dah_lo, 3 * E); t.pB = plane_ref(ew.whh_hi, ew.whh_lo, E); }
-        if (fused) {  // ... and the gate backward of step s-1 in the same launch
-          t.C = nullptr; t.epi = 0; t.fuse = LFI_FUSE_GRU_BWD;
-          GruEpi &q = t.gru;
-          q.E = E;
-          q.bgates = ew.gates + (size_t)(sidx - 1) * M * 3 * E; q.bahn = ew.ahn + (size_t)(sidx - 1) * M * E;
-          q.bhprev = sidx - 1 > 0 ? ew.hs + (size_t)(sidx - 2) * M * E : nullptr;
-          q.dh = ew.dhe;
-          q.dah_hi = off16(ew.dah_hi, (size_t)(sidx - 1) * M * 3 * E); q.dah_lo = lo ? off16(ew.dah_lo, (size_t)(sidx - 1) * M * 3 * E) : nullptr;
-          q.dan_hi = off16(ew.dan_hi, (size_t)(sidx - 1) * M * E);     q.dan_lo = lo ? off16(ew.dan_lo, (size_t)(sidx - 1) * M * E) : nullptr;
-          q.gb_ih = g->enc_b_ih[m]; q.gb_hh = g->enc_b_hh[m];
-        }
         LFI_TRY(gemm_dispatch(bmode, t, gws, gws_bytes, st));
       }
     }
@@ -889,7 +831,7 @@ static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chu
     e.xp = b.take<float>(encp::tiled_rows((size_t)B * T) * 3 * E);
     e.hs = b.take<float>(2 * Mc * E);
     e.planes = enc_use_planes(s, m, Mc, mode);
-    e.persist = enc_use_persist(s, m, Mc, (size_t)B * T, mode, false);
+    e.persist = enc_use_persist(s, m, Mc, (size_t)B * T, mode);
     e.xT = e.persist ? b.take<float>((size_t)B * T * s->dim[m]) : nullptr;
     if (e.planes) {
       const bool lo = mode == LFI_GEMM_BF16X3;

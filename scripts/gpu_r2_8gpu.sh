@@ -11,5 +11,3 @@ d=json.loads([l for l in open('gpurun_out/bench8_n$n.log') if l.startswith('{')]
 print('N=$n ms/step', d['ms_per_step'], 'value', d['value'], 'e2e', d['e2e']['value'], 'sample', d.get('sample',{}).get('value'))
 PY
 done
-LFI_ENC_PERSIST=1 timeout 900 python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29519 bench.py --gpus 8 --steps 20 --warmup 5 --no-sample > gpurun_out/bench8_n8_persist.log 2>&1
-python -c "import json;d=json.loads([l for l in open('gpurun_out/bench8_n8_persist.log') if l.startswith('{')][-1]);print('N=8 persist ms/step', d['ms_per_step'])"

@@ -14,5 +14,3 @@ tail -5 gpurun_out/smoke.log
 timeout 600 python bench.py --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 > gpurun_out/bench.log 2>&1
 echo "bench exit $?" >> gpurun_out/bench.log
 tail -3 gpurun_out/bench.log
-LFI_ENC_PERSIST=0 timeout 600 python bench.py --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 --no-sample > gpurun_out/bench_nopersist.log 2>&1
-tail -2 gpurun_out/bench_nopersist.log

@@ -3,8 +3,6 @@ mkdir -p gpurun_out
 timeout 600 python -m pytest tests/test_gpu_paths.py -m gpu -q --timeout 300 -k "persistent_encoder" > gpurun_out/pytest_enc.log 2>&1
 echo "pytest enc exit $?" >> gpurun_out/pytest_enc.log
 grep -E 'passed|failed|FAILED|ERROR|assert|Error|timed out' gpurun_out/pytest_enc.log | tail -20
-LFI_ENC_PERSIST_BWD=0 timeout 600 python -m pytest tests/test_gpu_paths.py -m gpu -q --timeout 300 -k "persistent_encoder and 256-bf16x3" > gpurun_out/pytest_enc_fwdonly.log 2>&1
-grep -E 'passed|failed|FAILED|ERROR|assert|Error|timed out' gpurun_out/pytest_enc_fwdonly.log | tail -5
 timeout 300 python scripts/step_phases.py > gpurun_out/phases.log 2>&1
 sort gpurun_out/phases.log | uniq -c | sort -rn | awk '{$1="";print}' | sort -u | head -20
 timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none --profile-from-start off --csv --log-file gpurun_out/launches.csv \

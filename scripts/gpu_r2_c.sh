@@ -1,7 +1,4 @@
 #!/bin/bash
 mkdir -p gpurun_out
-timeout 1500 ncu --set full --clock-control none --import-source on --profile-from-start off -k "regex:enc_gru_(fwd|bwd)_persist" -c 6 \
-  -f -o gpurun_out/prof_encp python bench.py --ncu-step > gpurun_out/ncu_full.log 2>&1
-echo "ncu exit $?"; tail -3 gpurun_out/ncu_full.log; ls -la gpurun_out/*.ncu-rep
 timeout 900 python -m pytest tests/test_gpu_autograd_api.py -m gpu -q --timeout 300 > gpurun_out/pytest_autograd.log 2>&1
 grep -E 'passed|failed|FAILED|ERROR|assert|Error' gpurun_out/pytest_autograd.log | tail -20

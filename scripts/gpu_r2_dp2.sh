@@ -3,13 +3,5 @@ mkdir -p gpurun_out
 nvidia-smi --query-gpu=index,name --format=csv
 timeout 900 python -m pytest tests/test_gpu_dp2.py -m gpu -q --timeout 600 > gpurun_out/pytest_dp2.log 2>&1
 grep -E 'passed|failed|skipped|FAILED|ERROR|assert|Error' gpurun_out/pytest_dp2.log | tail -8
-for mode in 1 0; do
-LFI_ENC_PERSIST=$mode timeout 900 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 bench.py --gpus 2 --steps 20 --warmup 5 --no-sample > gpurun_out/bench_2gpu_persist$mode.log 2>&1
-python - <<PY
-import json
-d=json.loads([l for l in open('gpurun_out/bench_2gpu_persist$mode.log') if l.startswith('{')][-1])
-print('persist=$mode 2 GPUs: ms/step', d['ms_per_step'], 'value', d['value'], 'e2e', d['e2e']['value'])
-PY
-done
 timeout 600 python bench.py --steps 20 --warmup 5 --no-cpu-baseline --no-bf16 --no-sample > gpurun_out/bench_1gpu.log 2>&1
 python -c "import json;d=json.loads(open('gpurun_out/bench_1gpu.log').read().strip().splitlines()[-1]);print('1 GPU ms/step', d['ms_per_step'])"

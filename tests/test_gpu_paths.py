@@ -163,11 +163,11 @@ def test_tensor_core_sampler_matches_fp32_sampler(mode, tol):
 
 @pytest.mark.parametrize("mode,tol", [("bf16x3", 2e-5), ("bf16", 5e-3)])
 @pytest.mark.parametrize("B", [256, 100])
-def test_persistent_encoder_matches_per_step_launches(mode, tol, B):
-    """The persistent window-GRU kernels (enc_persist.cu: all 24 / 2 / 16 window steps of a 128-window tile in one launch per
-    direction, state resident in shared memory, halves exchanged through DSMEM; LFI_ENC_PERSIST=1) against the chain of
-    per-step launches (LFI_ENC_PERSIST=0, the training default): encoded features, z / NLL and every gradient (the backward pass reads the stash the forward kernel
-    wrote).  Frame-dropout masks on.  B=100 leaves a ragged last tile (5,600 rows = 43.75 tiles)."""
+def test_persistent_encoder_feature_encode_matches_per_step_launches(mode, tol, B):
+    """Feature encoding on the persistent window-GRU forward kernel (enc_persist.cu: all 24 / 2 / 16 window steps of a
+    128-window tile in one launch, state resident in shared memory, halves exchanged through DSMEM; LFI_ENC_PERSIST_SAMPLE=1,
+    the sampling default) against the chain of per-step launches (LFI_ENC_PERSIST_SAMPLE=0, the path training runs): encoded
+    features.  Frame-dropout masks on.  B=100 leaves a ragged last tile (5,600 rows = 43.75 tiles)."""
     hp, m = _model(mode)
     hy = O.Hyper.from_hparams(hp)
     m.train()
@@ -176,19 +176,11 @@ def test_persistent_encoder_matches_per_step_launches(mode, tol, B):
     masks = O.make_masks(hy, B, T - hy.start_ts, seed=32)
     m.injected_masks = {k: (v.to(DEV) if v is not None else None) for k, v in masks.items()}
     eng = m.engine()
-    with _env(LFI_ENC_PERSIST="1", LFI_ENC_PERSIST_SAMPLE="1"):
+    with _env(LFI_ENC_PERSIST_SAMPLE="1"):
         c1 = eng.feature_encode(batch, hy.start_ts, T - hy.start_ts, m.injected_masks).clone()
-        z1, n1, g1 = _fwd_bwd(m, batch)
-    with _env(LFI_ENC_PERSIST="0", LFI_ENC_PERSIST_SAMPLE="0"):
+    with _env(LFI_ENC_PERSIST_SAMPLE="0"):
         c0 = eng.feature_encode(batch, hy.start_ts, T - hy.start_ts, m.injected_masks).clone()
-        z0, n0, g0 = _fwd_bwd(m, batch)
     assert relerr(c1, c0) < tol
-    assert relerr(z1, z0) < 5 * tol
-    assert relerr(n1, n0) < 1e-5 if mode == "bf16x3" else 1e-4
-    for k in g0:
-        ref = g0[k].double()
-        err = float((g1[k].double() - ref).norm() / ref.norm().clamp_min(1e-30))
-        assert err < (2e-3 if mode == "bf16x3" else 0.1), (k, err)
     # and the encoded features against the oracle on 8 sequences of the first two frames
     P = {k: v.detach() for k, v in oracle_params_from(m).items()}
     S = 8
