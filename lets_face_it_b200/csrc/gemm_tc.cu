@@ -1006,6 +1006,9 @@ int gemm_tc(int mode, const GemmArgs &g, void *ws, size_t ws_bytes, cudaStream_t
   LFI_REQUIRE(nplanes == 1 || ((!g.pA.hi || g.pA.lo) && (!g.pB.hi || g.pB.lo)), LFI_ERR_ARG, "gemm: split-bf16 mode needs lo planes");
   LFI_REQUIRE(!(g.epi & LFI_EPI_BIAS) || g.bias, LFI_ERR_ARG, "gemm: bias epilogue without bias");
   LFI_REQUIRE(!(g.epi & LFI_EPI_LRELU_BWD) || g.aux || g.auxp, LFI_ERR_ARG, "gemm: lrelu-bwd epilogue without aux");
+  // the vector epilogue would fold the old C into the sums when the launch is not split over K, split-K and the scalar
+  // epilogue would not: the result would depend on the split count, so the combination is refused
+  LFI_REQUIRE(!(g.colsum && (g.epi & LFI_EPI_ACCUM)), LFI_ERR_ARG, "gemm: column sums cannot be combined with the accumulate epilogue");
   // A: transA = 0 -> stored [M, K] (K-major); 1 -> stored [K, M] (MN-major).  B: transB = 1 -> [N, K] (K-major); 0 -> [K, N] (MN-major)
   tc::Operand A, B;
   A.mn = g.transA ? 1 : 0; A.rows = g.transA ? g.K : g.M; A.cols = g.transA ? g.M : g.K;
