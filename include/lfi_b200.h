@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 6
+#define LFI_ABI_VERSION 7
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -155,6 +155,31 @@ int lfi_seq_sample(const lfi_shape *s, const void *derived, const lfi_params *p,
 size_t lfi_feature_ws_bytes(const lfi_shape *s, int B, int T, int Tp, int gemm_mode);
 int lfi_feature_encode(const lfi_shape *s, const lfi_params *p, const lfi_batch *b, int t0, int Tp, float *cond,
                        void *ws, size_t ws_bytes, int gemm_mode, void *stream);
+
+/* ---- FeatureEncoder / ModalityEncoder.forward WITH autograd (models.py:12-145 differentiated by torch) -----------------------
+ * lfi_feature_encode_fwd_train computes the same folded cond [Tp*B, Fe] as lfi_feature_encode, with the window-GRU launches of the
+ * training step (per-step fused GRU GEMMs with the input projection inside in the tensor-core modes; never the persistent kernel,
+ * which keeps no stash), and fills `stash` (lfi_feature_stash_bytes, caller owned, opaque: h of every window step, the gate stash,
+ * the masked window inputs).  One stash per call: a per-frame loop that makes T forward calls before one backward keeps T of them.
+ * At final_model.yaml, B = 256, Tp = 1 a stash is 53.7 MB in fp32 mode, 66.5 MB in bf16x3 and 60.1 MB in bf16 mode, most of it
+ * p2_face (hist 24, E = 256: 31.5 MB in fp32, 39.1 MB in bf16x3); a 56-frame loop keeps all 56 alive until its backward.
+ * lfi_feature_encode_bwd is its backward; it must get the stash of the matching forward call and the same batch, masks and mode.
+ *   in : dcond [Tp*B, Fe] = dL/d(folded cond) (the caller sums the two copies of a GRU state of the unfolded vector)
+ *   out: dx[m] NULL or [B, T, dim[m]]: dL/d(raw stream m) over all T frames, zero where no window reads a frame (GRU and
+ *        "enc: none" modalities; dx itself may be NULL); the enc_* fields of g (layout of lfi_params, nothing else is read) are
+ *        WRITTEN, not accumulated.
+ * Both take a workspace of at least lfi_feature_bwd_ws_bytes bytes.  Numerics: the GEMMs run in gemm_mode.  In
+ * fp32 mode the forward equals lfi_feature_encode bitwise (same kernels); in the tensor-core modes lfi_feature_encode runs the
+ * persistent window-GRU kernel, so the two agree within the mode's bound only.  The backward has no atomics and no split-K
+ * (weight gradients written by one tile each, bias gradients as per-block partials reduced in a fixed order, the adjoint of the
+ * window gather one thread per element): the same call twice gives bit-identical gradients in every mode. */
+size_t lfi_feature_stash_bytes(const lfi_shape *s, int B, int T, int Tp, int gemm_mode);
+size_t lfi_feature_bwd_ws_bytes(const lfi_shape *s, int B, int T, int Tp, int gemm_mode);
+int lfi_feature_encode_fwd_train(const lfi_shape *s, const lfi_params *p, const lfi_batch *b, int t0, int Tp, float *cond,
+                                 void *stash, size_t stash_bytes, void *ws, size_t ws_bytes, int gemm_mode, void *stream);
+int lfi_feature_encode_bwd(const lfi_shape *s, const lfi_params *p, const lfi_batch *b, int t0, int Tp, const float *dcond,
+                           float *const dx[LFI_NMOD], lfi_params *g, void *stash, size_t stash_bytes, void *ws, size_t ws_bytes,
+                           int gemm_mode, void *stream);
 
 /* ---- single-frame module API (FlowStep.forward models.py:305-373, test_modules.py) ----------
  * One flow step k on one frame: x [B,C], cond [B,F] (raw, unfolded), h (and c) [B,H] in/out

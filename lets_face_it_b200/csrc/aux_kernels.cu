@@ -356,7 +356,9 @@ int enc_gate_bwd(const EncStepBwd &a, cudaStream_t st) {
 }
 
 // thread = hidden unit e (coalesced over e), block = a strip of rows; the four bias-gradient sums stay in registers
-__global__ void enc_gate_bwd2_kernel(EncStepBwd2 a, int rows_per_block) {
+// kPart: the block adds its sums into its own row of part [blocks][4E] instead of issuing atomics
+template <bool kPart>
+__global__ void enc_gate_bwd2_kernel(EncStepBwd2 a, int rows_per_block, float *part) {
   const int E = a.E;
   const int e = blockIdx.y * blockDim.x + threadIdx.x;
   if (e >= E) return;
@@ -393,13 +395,20 @@ __global__ void enc_gate_bwd2_kernel(EncStepBwd2 a, int rows_per_block) {
     a.dh[idx] = dh * ug;
     s_r += dar; s_u += dau; s_n += dan; s_nr += danr;
   }
+  if (kPart) {
+    float *q = part + (size_t)blockIdx.x * 4 * E + e;
+    q[0] += s_r; q[E] += s_u; q[2 * E] += s_n; q[3 * E] += s_nr;
+    return;
+  }
   atomicAdd(a.gb_ih + e, s_r); atomicAdd(a.gb_ih + E + e, s_u); atomicAdd(a.gb_ih + 2 * E + e, s_n);
   atomicAdd(a.gb_hh + e, s_r); atomicAdd(a.gb_hh + E + e, s_u); atomicAdd(a.gb_hh + 2 * E + e, s_nr);
 }
 // Vectorised variant (E % 4 == 0, 256 % (E/4) == 0): thread = 4 consecutive hidden units of one window, 128-bit loads,
 // 64-bit plane stores, grid-stride over the windows so that every SM keeps several independent rows in flight; the
-// bias-gradient sums are reduced over the block's row lanes in shared memory before the atomics.
-__global__ void __launch_bounds__(256) enc_gate_bwd2_v4_kernel(EncStepBwd2 a) {
+// bias-gradient sums are reduced over the block's row lanes in shared memory before the atomics (kPart: before the block
+// adds them into its own row of part [blocks][4E]).
+template <bool kPart>
+__global__ void __launch_bounds__(256) enc_gate_bwd2_v4_kernel(EncStepBwd2 a, float *part) {
   extern __shared__ float red[];  // [4 sums][rows per iteration][E]
   const int E = a.E, tpr = E >> 2, rpb = 256 / tpr;
   const int e = 4 * (threadIdx.x % tpr), rl = threadIdx.x / tpr;
@@ -469,32 +478,83 @@ __global__ void __launch_bounds__(256) enc_gate_bwd2_v4_kernel(EncStepBwd2 a) {
     const int which = i / E, u = i - which * E;
     float s = 0.f;
     for (int r = 0; r < rpb; ++r) s += red[(size_t)which * plane + (size_t)r * E + u];
-    if (which == 0) { atomicAdd(a.gb_ih + u, s); atomicAdd(a.gb_hh + u, s); }
+    if (kPart) part[(size_t)blockIdx.x * 4 * E + i] += s;
+    else if (which == 0) { atomicAdd(a.gb_ih + u, s); atomicAdd(a.gb_hh + u, s); }
     else if (which == 1) { atomicAdd(a.gb_ih + E + u, s); atomicAdd(a.gb_hh + E + u, s); }
     else if (which == 2) atomicAdd(a.gb_ih + 2 * E + u, s);
     else atomicAdd(a.gb_hh + 2 * E + u, s);
   }
 }
 
-int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st) {
+// Grids of the two enc_gate_bwd2 kernels: blocks of the vectorised kernel (0 when the shape does not fit it), and row
+// strip / blocks of the scalar kernel.
+static int bwd2_v4_blocks(int M, int E) {
+  const int tpr = E / 4;
+  if (E % 4 != 0 || tpr < 1 || tpr > 256 || 256 % tpr != 0) return 0;
+  const int rpb = 256 / tpr;
+  const int blocks = (M + rpb - 1) / rpb;
+  return blocks > 148 * 6 ? 148 * 6 : blocks;
+}
+static int bwd2_scalar_rpb(int M, int E, int *threads, int *cb) {
+  *threads = E >= 256 ? 256 : (E >= 128 ? 128 : 64);
+  *cb = (E + *threads - 1) / *threads;
+  int rpb = 32;
+  while ((long)((M + rpb - 1) / rpb) * *cb > 148 * 16 && rpb < 4096) rpb *= 2;
+  return rpb;
+}
+
+int enc_gate_bwd2_part_rows(int M, int E) {
+  int threads, cb;
+  const int rpb = bwd2_scalar_rpb(M, E, &threads, &cb), scalar = (M + rpb - 1) / rpb, v4 = bwd2_v4_blocks(M, E);
+  return scalar > v4 ? scalar : v4;
+}
+
+int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st, float *part) {
   auto al16 = [](const void *p) { return p == nullptr || ((uintptr_t)p & 15) == 0; };
-  const int tpr = a.E / 4;
-  if (a.E % 4 == 0 && tpr >= 1 && tpr <= 256 && 256 % tpr == 0 && al16(a.dh) && al16(a.gates) && al16(a.ahn) && al16(a.hprev) &&
+  const int v4 = bwd2_v4_blocks(a.M, a.E);
+  if (v4 > 0 && al16(a.dh) && al16(a.gates) && al16(a.ahn) && al16(a.hprev) &&
       al16(a.dah32) && al16(a.dan32) && al16(a.dh_extra) && (a.dh_extra == nullptr || a.dh_extra_ld % 4 == 0) &&
       (((uintptr_t)a.dah_hi | (uintptr_t)a.dah_lo | (uintptr_t)a.dan_hi | (uintptr_t)a.dan_lo) & 7) == 0) {
-    const int rpb = 256 / tpr;
-    int blocks = (a.M + rpb - 1) / rpb;
-    if (blocks > 148 * 6) blocks = 148 * 6;
-    const size_t smem = (size_t)4 * rpb * a.E * sizeof(float);
-    enc_gate_bwd2_v4_kernel<<<blocks, 256, smem, st>>>(a);
+    const size_t smem = (size_t)4 * (256 / (a.E / 4)) * a.E * sizeof(float);
+    if (part) enc_gate_bwd2_v4_kernel<true><<<v4, 256, smem, st>>>(a, part);
+    else enc_gate_bwd2_v4_kernel<false><<<v4, 256, smem, st>>>(a, nullptr);
     LFI_LAUNCH_CHECK();
     return LFI_OK;
   }
-  const int threads = a.E >= 256 ? 256 : (a.E >= 128 ? 128 : 64);
-  const int cb = (a.E + threads - 1) / threads;
-  int rpb = 32;
-  while ((long)((a.M + rpb - 1) / rpb) * cb > 148 * 16 && rpb < 4096) rpb *= 2;
-  enc_gate_bwd2_kernel<<<dim3((a.M + rpb - 1) / rpb, cb), threads, 0, st>>>(a, rpb);
+  int threads, cb;
+  const int rpb = bwd2_scalar_rpb(a.M, a.E, &threads, &cb);
+  const dim3 grid((a.M + rpb - 1) / rpb, cb);
+  if (part) enc_gate_bwd2_kernel<true><<<grid, threads, 0, st>>>(a, rpb, part);
+  else enc_gate_bwd2_kernel<false><<<grid, threads, 0, st>>>(a, rpb, nullptr);
+  LFI_LAUNCH_CHECK();
+  return LFI_OK;
+}
+
+// Adjoint of gather_windows: thread = one element dx[b][tau][c]; the (t', s) pairs whose window reads frame tau are visited
+// in increasing t', so every element is one thread's fixed-order sum (no atomics although windows overlap when Tp > 1).
+__global__ void window_grad_kernel(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim,
+                                   int hist, int off, int t0, int Tp) {
+  const size_t M = (size_t)Tp * B;
+  const size_t n = (size_t)B * T * dim;
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+    const int c = (int)(e % dim);
+    const size_t q = e / dim;
+    const int tau = (int)(q % T), b = (int)(q / T);
+    float acc = 0.f;
+    for (int tp = 0; tp < Tp; ++tp) {
+      const int s = tau - t0 - tp + hist - off;
+      if (s < 0 || s >= hist) continue;
+      const size_t m = (size_t)tp * B + b;
+      float v = layout_steps ? src[((size_t)s * M + m) * ld + c] : src[m * ld + (size_t)s * dim + c];
+      if (mask) v *= mask[m * hist + s];
+      acc += v;
+    }
+    dx[e] = acc;
+  }
+}
+int window_grad(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim, int hist, int off, int t0,
+                int Tp, cudaStream_t st) {
+  window_grad_kernel<<<blocks_for((size_t)B * T * dim), TB, 0, st>>>(dx, src, ld, layout_steps, mask, B, T, dim, hist, off, t0, Tp);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -68,7 +68,16 @@ struct EncStepBwd2 {
   int M, E;
   int gates16;                               // gates stash in 16-bit fixed point
 };
-int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st);
+// part != nullptr: bias gradients without atomics - every block adds its four sums (r, u, n, n*r blocks of E columns) into its
+// own row of part [enc_gate_bwd2_part_rows(M, E)][4E] (zeroed by the caller; the blocks of one launch own distinct rows and the
+// window steps are stream ordered) and gb_ih / gb_hh are not touched; one fixed-order column reduction finishes them.
+int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st, float *part = nullptr);
+int enc_gate_bwd2_part_rows(int M, int E);
+
+// Adjoint of gather_windows (same arguments, src in the layout gather_windows writes): dx [B][T][dim] is written for every frame,
+// dx[b][tau][c] = sum of mask * src over the (t', s) with tau = t0 + t' - hist + off + s, zero where no window reads the frame
+int window_grad(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim, int hist, int off, int t0,
+                int Tp, cudaStream_t st);
 
 // LU parametrisation helpers (modules.py:163-177)
 int lu_build(float *Lm, float *Um, const float *l, const float *u, const float *log_s, const float *sign_s, int K, int C, cudaStream_t st);

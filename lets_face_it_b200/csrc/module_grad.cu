@@ -257,6 +257,18 @@ bool fseq_params_ok(const lfi_fseq_params *p) {
 }
 
 }  // namespace
+
+// Bias gradients of an encoder GRU from the per-block partial sums of aux::enc_gate_bwd2 (part [rows][4E]: r, u, n, n*r blocks of
+// E columns): db_ih = (r, u, n), db_hh = (r, u, n*r), written; every column summed over the rows in a fixed order (one launch).
+int enc_bias_grads(const float *part, int rows, int E, float *gb_ih, float *gb_hh, cudaStream_t st) {
+  ColJobs j;
+  memset(&j, 0, sizeof(j));
+  j.j[0] = col_job(part, rows, 3 * E, 4 * E, gb_ih);
+  j.j[1] = col_job(part, rows, 2 * E, 4 * E, gb_hh);
+  j.j[2] = col_job(part + 3 * E, rows, E, 4 * E, gb_hh + 2 * E);
+  return launch_colgrad<COL_SUM>(j, 3, st);
+}
+
 }  // namespace lfi
 
 using namespace lfi;

@@ -16,6 +16,8 @@ namespace lfi {
 
 size_t gemm_ws_bytes(int mode, const GemmArgs &g);  // gemm_dispatch.cu: operand-plane scratch one GEMM needs
 static size_t gemm_ws_bytes_for(int mode, const GemmArgs &g) { return gemm_ws_bytes(mode, g); }
+int enc_bias_grads(const float *part, int rows, int E, float *gb_ih, float *gb_hh, cudaStream_t st);  // module_grad.cu
+static void *off16(void *base, size_t n) { return base ? (void *)((uint16_t *)base + n) : nullptr; }
 
 // ------------------------------------------------------------------------------------------------
 // derived cache layout (floats)
@@ -146,6 +148,40 @@ static bool core_planes_ok(const Dims &d, int mode) {
   return d.C % 8 == 0 && d.Co % 8 == 0 && d.H % 8 == 0 && d.D % 8 == 0;
 }
 
+// Where the training state of a modality's encoder lives.  The training step lays all of it out in its one workspace; the module
+// API (lfi_feature_encode_fwd_train / _bwd) splits it into the caller's stash (what the backward reads), forward-only scratch, the
+// weight planes that each of its calls builds for itself, and backward-only scratch.  A dry-run Bump (null base) only sizes its part.
+struct EncBumps { Bump *stash, *fwd, *wts, *bwd; };
+static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t M, int mode, const EncBumps &bb, EncWs &e) {
+  memset(&e, 0, sizeof(EncWs));
+  Bump &S = *bb.stash, &F = *bb.fwd, &W = *bb.wts, &K = *bb.bwd;
+  const size_t E = s->ehid[m], h = s->hist[m];
+  e.xp = F.take<float>(B * T * 3 * E);
+  e.hs = S.take<float>(h * M * E);
+  e.gates = S.take<float>(h * M * 3 * E);
+  e.ahn = S.take<float>(h * M * E);
+  e.planes = enc_use_planes(s, m, M, mode);
+  e.gates16 = e.planes && E % 4 == 0 && env_flag("LFI_GATES16", true);
+  if (e.planes) {
+    const bool lo = mode == LFI_GEMM_BF16X3;
+    const size_t dimp = round_up(s->dim[m], 8);
+    e.hp_hi = take_bf16(S, h * M * E);            e.hp_lo = lo ? take_bf16(S, h * M * E) : nullptr;
+    e.whh_hi = take_bf16(W, 3 * E * E);           e.whh_lo = lo ? take_bf16(W, 3 * E * E) : nullptr;
+    e.dah_hi = take_bf16(K, h * M * 3 * E);       e.dah_lo = lo ? take_bf16(K, h * M * 3 * E) : nullptr;
+    e.dan_hi = take_bf16(K, h * M * E);           e.dan_lo = lo ? take_bf16(K, h * M * E) : nullptr;
+    e.xg_hi = take_bf16(S, h * M * dimp);         e.xg_lo = lo ? take_bf16(S, h * M * dimp) : nullptr;
+    e.wih_hi = take_bf16(W, 3 * E * dimp);        e.wih_lo = lo ? take_bf16(W, 3 * E * dimp) : nullptr;
+    // input projection inside the fused step GEMM: the masked window inputs are gathered as operand planes in the forward pass
+    // (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand; step 0 (no state yet) keeps the xp rows
+    e.xfuse = E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true) && env_flag("LFI_ENC_XFUSE", true);
+  } else {
+    e.dah32 = K.take<float>(h * M * 3 * E);
+    e.dan32 = K.take<float>(h * M * E);
+  }
+  e.xg32 = K.take<float>(h * M * s->dim[m]);
+  e.dhe = K.take<float>(M * E);
+}
+
 static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode, void *ws, TrainWs *w) {
   Bump b(ws, 0);
   const size_t Tp = T - d.start_ts, M = Tp * B, K = d.K;
@@ -157,35 +193,12 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
   w->ld = b.take<float>(M);
   w->flags = b.take<int>(kFlagInts);
   size_t ghmax = 0, xgmax = 0, emax = 0;
+  const EncBumps eb = {&b, &b, &b, &b};
   for (int m = 0; m < LFI_NMOD; ++m) {
     memset(&w->enc[m], 0, sizeof(EncWs));
     if (s->hist[m] <= 0 || s->ehid[m] <= 0) continue;
     const size_t E = s->ehid[m], h = s->hist[m];
-    EncWs &e = w->enc[m];
-    e.xp = b.take<float>((size_t)B * T * 3 * E);
-    e.hs = b.take<float>(h * M * E);
-    e.gates = b.take<float>(h * M * 3 * E);
-    e.ahn = b.take<float>(h * M * E);
-    e.planes = enc_use_planes(s, m, M, mode);
-    e.gates16 = e.planes && E % 4 == 0 && env_flag("LFI_GATES16", true);
-    if (e.planes) {
-      const bool lo = mode == LFI_GEMM_BF16X3;
-      const size_t dimp = round_up(s->dim[m], 8);
-      e.hp_hi = take_bf16(b, h * M * E);            e.hp_lo = lo ? take_bf16(b, h * M * E) : nullptr;
-      e.whh_hi = take_bf16(b, 3 * E * E);           e.whh_lo = lo ? take_bf16(b, 3 * E * E) : nullptr;
-      e.dah_hi = take_bf16(b, h * M * 3 * E);       e.dah_lo = lo ? take_bf16(b, h * M * 3 * E) : nullptr;
-      e.dan_hi = take_bf16(b, h * M * E);           e.dan_lo = lo ? take_bf16(b, h * M * E) : nullptr;
-      e.xg_hi = take_bf16(b, h * M * dimp);         e.xg_lo = lo ? take_bf16(b, h * M * dimp) : nullptr;
-      e.wih_hi = take_bf16(b, 3 * E * dimp);        e.wih_lo = lo ? take_bf16(b, 3 * E * dimp) : nullptr;
-      // input projection inside the fused step GEMM: the masked window inputs are gathered as operand planes in the forward pass
-      // (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand; step 0 (no state yet) keeps the xp rows
-      e.xfuse = E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true) && env_flag("LFI_ENC_XFUSE", true);
-    } else {
-      e.dah32 = b.take<float>(h * M * 3 * E);
-      e.dan32 = b.take<float>(h * M * E);
-    }
-    e.xg32 = b.take<float>(h * M * s->dim[m]);
-    e.dhe = b.take<float>(M * E);
+    plan_enc_train(s, m, B, T, M, mode, eb, w->enc[m]);
     if (M * 3 * E > ghmax) ghmax = M * 3 * E;
     if (h * M * s->dim[m] > xgmax) xgmax = h * M * s->dim[m];
     if (E > emax) emax = E;
@@ -406,6 +419,86 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
     cudaStreamWaitEvent(st, ev_join[i], 0);
   }
   return rc;
+}
+
+// Encoder GRU of modality m, BPTT over the window (models.py:63-64), for frames t0 .. t0+Tp-1 given dcond (folded, ld Fe).  Per
+// step only the gate math and dh_prev = dA_h W_hh run; the gate gradients of all steps are kept so that every weight gradient is
+// ONE long-K GEMM (reduction over hist x M rows), and the bias gradients are summed inside the gate kernel.
+// The training step accumulates into g (split-K GEMMs, float atomics).  o.part set (module API): the gradients are written and
+// bit-reproducible - weight-gradient GEMMs with the plain store epilogue and dh_prev with ACCUM_PRE (neither ever splits K), bias
+// gradients through per-block partials o.part [o.part_rows][4E] and one fixed-order reduction.  o.dx set: also dL/d(raw stream)
+// [B][T][dim] through dXg = dA_h[:, :2E] W_ih[:2E] + dA_n W_ih[2E:] in o.dxg [hist*M][dim] (needs the W_ih planes in plane mode).
+struct EncBwdOpts {
+  float *part; int part_rows;
+  float *dxg, *dx;
+};
+static int enc_bwd(const lfi_shape *s, const Dims &d, const lfi_params *p, const lfi_batch *bt, int t0, int Tp, int m, EncWs &ew,
+                   const float *dcond, lfi_params *g, int mode, int bmode, void *gws, size_t gws_bytes, const EncBwdOpts &o,
+                   cudaStream_t st) {
+  const int B = bt->B, T = bt->T, hist = s->hist[m], E = s->ehid[m], dim = s->dim[m];
+  const size_t M = (size_t)Tp * B;
+  const bool lo = mode == LFI_GEMM_BF16X3;
+  const bool det = o.part != nullptr;
+  const int wepi = det ? 0 : LFI_EPI_ACCUM;
+  const int dimp = round_up(dim, 8);
+  if (ew.planes && ew.xfuse) {
+    // (gathered by the forward pass, which fed them to its fused step GEMMs)
+  } else if (ew.planes)  // masked window inputs straight into the operand planes of the dW_ih GEMMs
+    LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
+  else
+    LFI_TRY(aux::gather_windows(ew.xg32, dim, 1, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
+  LFI_TRY(aux::fill(ew.dhe, 0.f, M * E, st));
+  if (det) LFI_TRY(aux::fill(o.part, 0.f, (size_t)o.part_rows * 4 * E, st));
+  for (int sidx = hist - 1; sidx >= 0; --sidx) {
+    aux::EncStepBwd2 e;
+    memset(&e, 0, sizeof(e));
+    e.gates = ew.gates + (size_t)sidx * M * 3 * E; e.ahn = ew.ahn + (size_t)sidx * M * E;
+    e.hprev = sidx ? ew.hs + (size_t)(sidx - 1) * M * E : nullptr;
+    e.dh = ew.dhe; e.dh_extra = (sidx == hist - 1) ? dcond + d.enc_offe[m] : nullptr; e.dh_extra_ld = d.Fe;
+    if (ew.planes) {
+      e.dah_hi = off16(ew.dah_hi, (size_t)sidx * M * 3 * E); e.dah_lo = lo ? off16(ew.dah_lo, (size_t)sidx * M * 3 * E) : nullptr;
+      e.dan_hi = off16(ew.dan_hi, (size_t)sidx * M * E);     e.dan_lo = lo ? off16(ew.dan_lo, (size_t)sidx * M * E) : nullptr;
+    } else {
+      e.dah32 = ew.dah32 + (size_t)sidx * M * 3 * E; e.dan32 = ew.dan32 + (size_t)sidx * M * E;
+    }
+    e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.gates16 ? 1 : 0;
+    LFI_TRY(aux::enc_gate_bwd2(e, st, o.part));
+    if (sidx) {  // dh_{s-1} += dA_h W_hh
+      GemmArgs t = gemm_args(0, 0, (int)M, E, 3 * E, e.dah32, 3 * E, p->enc_w_hh[m], E, ew.dhe, E, det ? LFI_EPI_ACCUM_PRE : LFI_EPI_ACCUM);
+      if (ew.planes) { t.pA = plane_ref(e.dah_hi, e.dah_lo, 3 * E); t.pB = plane_ref(ew.whh_hi, ew.whh_lo, E); }
+      LFI_TRY(gemm_dispatch(bmode, t, gws, gws_bytes, st));
+    }
+  }
+  if (det) LFI_TRY(enc_bias_grads(o.part, o.part_rows, E, g->enc_b_ih[m], g->enc_b_hh[m], st));
+  const int Kall = (int)(hist * M), Khh = (int)((hist - 1) * M);
+  if (hist > 1) {  // dW_hh += sum_{s>=1} dA_h[s]^T h[s-1]
+    GemmArgs q = gemm_args(1, 0, 3 * E, E, Khh, ew.dah32 ? ew.dah32 + M * 3 * E : nullptr, 3 * E, ew.hs, E, g->enc_w_hh[m], E, wepi);
+    if (ew.planes) { q.pA = plane_ref(off16(ew.dah_hi, M * 3 * E), lo ? off16(ew.dah_lo, M * 3 * E) : nullptr, 3 * E); q.pB = plane_ref(ew.hp_hi, ew.hp_lo, E); }
+    LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
+  } else if (det) {
+    LFI_CUDA(cudaMemsetAsync(g->enc_w_hh[m], 0, (size_t)3 * E * E * sizeof(float), st));
+  }
+  {  // dW_ih rows [0,2E) += dA_h[:, :2E]^T x  (r, u blocks coincide with the i-side gradients); rows [2E,3E) += dA_n^T x
+    GemmArgs q = gemm_args(1, 0, 2 * E, dim, Kall, ew.dah32, 3 * E, ew.xg32, dim, g->enc_w_ih[m], dim, wepi);
+    if (ew.planes) { q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
+    LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
+    GemmArgs r = gemm_args(1, 0, E, dim, Kall, ew.dan32, E, ew.xg32, dim, g->enc_w_ih[m] + (size_t)2 * E * dim, dim, wepi);
+    if (ew.planes) { r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E); r.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
+    LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
+  }
+  if (o.dx) {  // dXg = dA_h[:, :2E] W_ih[:2E] + dA_n W_ih[2E:] (ACCUM_PRE: neither launch splits K), then the adjoint of the gather
+    GemmArgs q = gemm_args(0, 0, Kall, dim, 2 * E, ew.dah32, 3 * E, p->enc_w_ih[m], dim, o.dxg, dim, 0);
+    GemmArgs r = gemm_args(0, 0, Kall, dim, E, ew.dan32, E, p->enc_w_ih[m] + (size_t)2 * E * dim, dim, o.dxg, dim, LFI_EPI_ACCUM_PRE);
+    if (ew.planes) {
+      q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.wih_hi, ew.wih_lo, dimp);
+      r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E);
+      r.pB = plane_ref(off16(ew.wih_hi, (size_t)2 * E * dimp), lo ? off16(ew.wih_lo, (size_t)2 * E * dimp) : nullptr, dimp);
+    }
+    LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
+    LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
+    LFI_TRY(aux::window_grad(o.dx, o.dxg, dim, 1, bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
+  }
+  return LFI_OK;
 }
 
 // cond_transform for all K steps, then the c-part of the gate-ih product (models.py:187-190, 206-208)
@@ -636,7 +729,6 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   auto join_wgrads = [&]() {
     if (wg_par) { cudaEventRecord(wg_join, wg_stream); cudaStreamWaitEvent(st_main, wg_join, 0); }
   };
-  auto off16 = [](void *base, size_t n) -> void * { return base ? (void *)((uint16_t *)base + n) : nullptr; };
   auto wgrad = [&](int Mo, int No, size_t red, const float *A, int lda, long sA, const float *Bm, int ldb, long sB, float *Cm,
                    int ldc, long sC, PlaneRef pa = PlaneRef{nullptr, nullptr, 0, 0}, PlaneRef pb = PlaneRef{nullptr, nullptr, 0, 0}) -> int {
     GemmArgs q = gemm_args(1, 0, Mo, No, (int)red, A, lda, Bm, ldb, Cm, ldc, LFI_EPI_ACCUM);
@@ -720,58 +812,12 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
     LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
   }
 
-  // 4. encoder GRUs, BPTT over the window (models.py:63-64).  Per step only the gate math and dh_prev = dA_h W_hh
-  //    run; the gate gradients of all steps are kept so that every weight gradient is ONE long-K GEMM per modality
-  //    (reduction over hist x M rows), and the bias gradients are accumulated inside the gate kernel.
-  //    The modalities are independent chains of a latency-bound GEMM and an HBM-bound gate kernel per window step: with
-  //    every operand in plane form (no shared scratch) they run on parallel streams forked from / joined to the caller's.
-  auto enc_bwd = [&](int m, cudaStream_t st) -> int {
-    const int hist = s->hist[m], E = s->ehid[m], dim = s->dim[m];
-    EncWs &ew = w.enc[m];
-    const bool lo = gemm_mode == LFI_GEMM_BF16X3;
-    const int dimp = round_up(dim, 8);
-    if (ew.planes && ew.xfuse) {
-      // (gathered by the forward pass of this step, which fed them to its fused step GEMMs)
-    } else if (ew.planes)  // masked window inputs straight into the operand planes of the dW_ih GEMMs
-      LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, d.start_ts, Tp, st));
-    else
-      LFI_TRY(aux::gather_windows(ew.xg32, dim, 1, bt->x[m], bt->mask[m], B, T, dim, hist, 1, d.start_ts, Tp, st));
-    LFI_TRY(aux::fill(ew.dhe, 0.f, M * E, st));
-    for (int sidx = hist - 1; sidx >= 0; --sidx) {
-      aux::EncStepBwd2 e;
-      memset(&e, 0, sizeof(e));
-      e.gates = ew.gates + (size_t)sidx * M * 3 * E; e.ahn = ew.ahn + (size_t)sidx * M * E;
-      e.hprev = sidx ? ew.hs + (size_t)(sidx - 1) * M * E : nullptr;
-      e.dh = ew.dhe; e.dh_extra = (sidx == hist - 1) ? w.dcond + d.enc_offe[m] : nullptr; e.dh_extra_ld = d.Fe;
-      if (ew.planes) {
-        e.dah_hi = off16(ew.dah_hi, (size_t)sidx * M * 3 * E); e.dah_lo = lo ? off16(ew.dah_lo, (size_t)sidx * M * 3 * E) : nullptr;
-        e.dan_hi = off16(ew.dan_hi, (size_t)sidx * M * E);     e.dan_lo = lo ? off16(ew.dan_lo, (size_t)sidx * M * E) : nullptr;
-      } else {
-        e.dah32 = ew.dah32 + (size_t)sidx * M * 3 * E; e.dan32 = ew.dan32 + (size_t)sidx * M * E;
-      }
-      e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.gates16 ? 1 : 0;
-      LFI_TRY(aux::enc_gate_bwd2(e, st));
-      if (sidx) {  // dh_{s-1} += dA_h W_hh
-        GemmArgs t = gemm_args(0, 0, (int)M, E, 3 * E, e.dah32, 3 * E, p->enc_w_hh[m], E, ew.dhe, E, LFI_EPI_ACCUM);
-        if (ew.planes) { t.pA = plane_ref(e.dah_hi, e.dah_lo, 3 * E); t.pB = plane_ref(ew.whh_hi, ew.whh_lo, E); }
-        LFI_TRY(gemm_dispatch(bmode, t, gws, gws_bytes, st));
-      }
-    }
-    const int Kall = (int)(hist * M), Khh = (int)((hist - 1) * M);
-    if (hist > 1) {  // dW_hh += sum_{s>=1} dA_h[s]^T h[s-1]
-      GemmArgs q = gemm_args(1, 0, 3 * E, E, Khh, ew.dah32 ? ew.dah32 + M * 3 * E : nullptr, 3 * E, ew.hs, E, g->enc_w_hh[m], E, LFI_EPI_ACCUM);
-      if (ew.planes) { q.pA = plane_ref(off16(ew.dah_hi, M * 3 * E), lo ? off16(ew.dah_lo, M * 3 * E) : nullptr, 3 * E); q.pB = plane_ref(ew.hp_hi, ew.hp_lo, E); }
-      LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
-    }
-    {  // dW_ih rows [0,2E) += dA_h[:, :2E]^T x  (r, u blocks coincide with the i-side gradients); rows [2E,3E) += dA_n^T x
-      GemmArgs q = gemm_args(1, 0, 2 * E, dim, Kall, ew.dah32, 3 * E, ew.xg32, dim, g->enc_w_ih[m], dim, LFI_EPI_ACCUM);
-      if (ew.planes) { q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
-      LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
-      GemmArgs r = gemm_args(1, 0, E, dim, Kall, ew.dan32, E, ew.xg32, dim, g->enc_w_ih[m] + (size_t)2 * E * dim, dim, LFI_EPI_ACCUM);
-      if (ew.planes) { r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E); r.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
-      LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
-    }
-    return LFI_OK;
+  // 4. encoder GRUs, BPTT over the window (enc_bwd).  The modalities are independent chains of a latency-bound GEMM and an
+  //    HBM-bound gate kernel per window step: with every operand in plane form (no shared scratch) they run on parallel streams
+  //    forked from / joined to the caller's.
+  const EncBwdOpts accumulate = {nullptr, 0, nullptr, nullptr};
+  auto enc_chain = [&](int m, cudaStream_t cs) -> int {
+    return enc_bwd(s, d, p, bt, d.start_ts, Tp, m, w.enc[m], w.dcond, g, gemm_mode, bmode, gws, gws_bytes, accumulate, cs);
   };
   int mods[LFI_NMOD], nmods = 0;
   bool all_planes = true;
@@ -782,14 +828,14 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   const bool par = nmods > 1 && all_planes && env_flag("LFI_ENC_STREAMS", true);
   if (!par) {
     int rc = LFI_OK;
-    for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_bwd(mods[i], st);
+    for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], st);
     join_wgrads();
     return rc;
   }
   LFI_CUDA(cudaEventRecord(ev_fork, st));
   for (int i = 1; i < nmods; ++i) LFI_CUDA(cudaStreamWaitEvent(side[i], ev_fork, 0));
   int rc = LFI_OK;
-  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_bwd(mods[i], i == 0 ? st : side[i]);
+  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], i == 0 ? st : side[i]);
   for (int i = 1; i < nmods; ++i) {  // always join, also on error
     cudaEventRecord(ev_join[i], side[i]);
     cudaStreamWaitEvent(st, ev_join[i], 0);
@@ -1304,6 +1350,167 @@ int lfi_flowstep_bwd(const lfi_shape *s, const void *derived, const lfi_params *
   LFI_TRY(wg(D, F, dC, D, cond, F, g->wc + (size_t)k * D * F, F));
   GemmArgs u = gemm_args(0, 0, B, F, D, dC, D, p->wc + (size_t)k * D * F, F, dcond, F, 0);
   LFI_TRY(gemm_simt(u, st));
+  return LFI_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------------
+// FeatureEncoder / ModalityEncoder.forward with autograd (module API): the window GRUs with the training step's per-step launches
+// and stash, and their backward with written, bit-reproducible gradients and the gradient of the raw streams.
+namespace lfi {
+struct FeatPlan {
+  EncWs enc[LFI_NMOD];
+  float *gh;                  // forward: [M][3E] recurrent products of the unfused window steps
+  float *part, *dxg;          // backward: bias-gradient partials and dXg of the largest modality (modalities run one after another)
+  int part_rows[LFI_NMOD];
+  size_t stash_bytes, ws_bytes;  // (ws_bytes: the call's workspace before its GEMM scratch)
+};
+// The stash layout depends on (shape, B, Tp, mode) only, so the forward and the backward call find the same arrays in it.
+static void plan_feature(const lfi_shape *s, int B, int T, int Tp, int mode, void *stash, void *ws, bool bwd, FeatPlan *f) {
+  Bump S(stash, 0), W(ws, 0), none(nullptr, 0);
+  const EncBumps eb = {&S, bwd ? &none : &W, &W, bwd ? &W : &none};
+  const size_t M = (size_t)Tp * B;
+  size_t ghmax = 0, partmax = 0, xgmax = 0;
+  for (int m = 0; m < LFI_NMOD; ++m) {
+    memset(&f->enc[m], 0, sizeof(EncWs));
+    f->part_rows[m] = 0;
+    if (s->hist[m] <= 0 || s->ehid[m] <= 0) continue;
+    const size_t E = s->ehid[m];
+    plan_enc_train(s, m, B, T, M, mode, eb, f->enc[m]);
+    f->part_rows[m] = aux::enc_gate_bwd2_part_rows((int)M, (int)E);
+    ghmax = ghmax > M * 3 * E ? ghmax : M * 3 * E;
+    partmax = partmax > f->part_rows[m] * 4 * E ? partmax : f->part_rows[m] * 4 * E;
+    xgmax = xgmax > s->hist[m] * M * s->dim[m] ? xgmax : s->hist[m] * M * s->dim[m];
+  }
+  f->gh = bwd ? nullptr : W.take<float>(ghmax);
+  f->part = bwd ? W.take<float>(partmax) : nullptr;
+  f->dxg = bwd ? W.take<float>(xgmax) : nullptr;
+  f->stash_bytes = round_up_sz(S.off, 256);
+  f->ws_bytes = round_up_sz(W.off, 256);
+}
+
+// Operand-plane scratch of the backward GEMMs: only modalities whose encoder does not run on operand planes split fp32 operands.
+static size_t feature_bwd_scratch(const lfi_shape *s, const FeatPlan &f, int Tp, int B, int mode) {
+  size_t need = 0;
+  const int M = Tp * B;
+  for (int m = 0; m < LFI_NMOD; ++m) {
+    if (s->hist[m] <= 0 || s->ehid[m] <= 0 || f.enc[m].planes) continue;
+    const int E = s->ehid[m], dim = s->dim[m], h = s->hist[m];
+    const GemmArgs gs[] = {gemm_args(0, 0, M, E, 3 * E, nullptr, 3 * E, nullptr, E, nullptr, E),
+                           gemm_args(1, 0, 3 * E, E, (h - 1) * M, nullptr, 3 * E, nullptr, E, nullptr, E),
+                           gemm_args(1, 0, 2 * E, dim, h * M, nullptr, 3 * E, nullptr, dim, nullptr, dim),
+                           gemm_args(0, 0, h * M, dim, 2 * E, nullptr, 3 * E, nullptr, dim, nullptr, dim)};
+    for (const GemmArgs &g : gs) need = need > gemm_ws_bytes_for(mode, g) ? need : gemm_ws_bytes_for(mode, g);
+  }
+  return need;
+}
+static size_t feature_fwd_need(const lfi_shape *s, const Dims &d, int B, int T, int Tp, int mode) {
+  FeatPlan f;
+  plan_feature(s, B, T, Tp, mode, nullptr, nullptr, false, &f);
+  return f.ws_bytes + gemm_scratch_bound(s, d, (size_t)Tp * B, (size_t)B * T, mode);
+}
+static size_t feature_bwd_need(const lfi_shape *s, int B, int T, int Tp, int mode) {
+  FeatPlan f;
+  plan_feature(s, B, T, Tp, mode, nullptr, nullptr, true, &f);
+  return f.ws_bytes + feature_bwd_scratch(s, f, Tp, B, mode);
+}
+
+// One workspace size serves both calls (lfi_feature_bwd_ws_bytes).
+static size_t feature_ws_need(const lfi_shape *s, const Dims &d, int B, int T, int Tp, int mode) {
+  const size_t a = feature_fwd_need(s, d, B, T, Tp, mode), b = feature_bwd_need(s, B, T, Tp, mode);
+  return a > b ? a : b;
+}
+
+static int feature_train_dims(const lfi_shape *s, int B, int Tp, int mode, Dims *d) {
+  LFI_TRY(make_dims(s, d));
+  LFI_REQUIRE(s->f_raw <= 0, LFI_ERR_SHAPE, "feature encoder: the shape has no encoders (f_raw = %d)", s->f_raw);
+  LFI_REQUIRE(B >= 1 && Tp >= 1, LFI_ERR_SHAPE, "feature encoder: B=%d Tp=%d must be >= 1", B, Tp);
+  LFI_REQUIRE(mode >= LFI_GEMM_FP32 && mode <= LFI_GEMM_BF16, LFI_ERR_ARG, "feature encoder: unknown gemm mode %d", mode);
+  return LFI_OK;
+}
+
+// Arguments both calls share: frames inside the batch, every stream the shape names present, the GRU weights (and gradients) set.
+static int feature_check(const lfi_shape *s, const Dims &d, const lfi_params *p, const lfi_batch *bt, int t0, int Tp, const lfi_params *g,
+                         const char *what) {
+  LFI_REQUIRE(t0 >= d.start_ts && t0 + Tp <= bt->T, LFI_ERR_SHAPE, "%s: frames [%d,%d) outside [%d,%d)", what, t0, t0 + Tp, d.start_ts, bt->T);
+  for (int m = 0; m < LFI_NMOD; ++m) {
+    if (s->hist[m] <= 0) continue;
+    LFI_REQUIRE(bt->x[m], LFI_ERR_ARG, "%s: batch modality %d missing", what, m);
+    if (s->ehid[m] <= 0) continue;
+    LFI_REQUIRE(p->enc_w_ih[m] && p->enc_w_hh[m] && p->enc_b_ih[m] && p->enc_b_hh[m], LFI_ERR_ARG, "%s: encoder %d weights missing", what, m);
+    LFI_REQUIRE(!g || (g->enc_w_ih[m] && g->enc_w_hh[m] && g->enc_b_ih[m] && g->enc_b_hh[m]), LFI_ERR_ARG,
+                "%s: encoder %d gradients missing", what, m);
+  }
+  return LFI_OK;
+}
+}  // namespace lfi
+
+extern "C" {
+
+size_t lfi_feature_stash_bytes(const lfi_shape *s, int B, int T, int Tp, int gemm_mode) {
+  Dims d;
+  if (feature_train_dims(s, B, Tp, gemm_mode, &d) != LFI_OK) return 0;
+  FeatPlan f;
+  plan_feature(s, B, T, Tp, gemm_mode, nullptr, nullptr, false, &f);
+  return f.stash_bytes;
+}
+
+size_t lfi_feature_bwd_ws_bytes(const lfi_shape *s, int B, int T, int Tp, int gemm_mode) {
+  Dims d;
+  if (feature_train_dims(s, B, Tp, gemm_mode, &d) != LFI_OK) return 0;
+  return feature_ws_need(s, d, B, T, Tp, gemm_mode);
+}
+
+int lfi_feature_encode_fwd_train(const lfi_shape *s, const lfi_params *p, const lfi_batch *bt, int t0, int Tp, float *cond, void *stash,
+                                 size_t stash_bytes, void *ws, size_t ws_bytes, int gemm_mode, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  LFI_REQUIRE(s && p && bt && cond && stash && ws, LFI_ERR_ARG, "lfi_feature_encode_fwd_train: null argument");
+  Dims d;
+  LFI_TRY(feature_train_dims(s, bt->B, Tp, gemm_mode, &d));
+  LFI_TRY(feature_check(s, d, p, bt, t0, Tp, nullptr, "lfi_feature_encode_fwd_train"));
+  FeatPlan f;
+  plan_feature(s, bt->B, bt->T, Tp, gemm_mode, stash, ws, false, &f);
+  LFI_REQUIRE(stash_bytes >= f.stash_bytes, LFI_ERR_WORKSPACE, "lfi_feature_encode_fwd_train: stash too small: %zu < %zu", stash_bytes,
+              f.stash_bytes);
+  const size_t need = feature_ws_need(s, d, bt->B, bt->T, Tp, gemm_mode);
+  LFI_REQUIRE(ws_bytes >= need, LFI_ERR_WORKSPACE, "lfi_feature_encode_fwd_train: workspace too small: %zu < %zu", ws_bytes, need);
+  return build_cond(s, d, p, bt, t0, Tp, cond, f.enc, f.gh, true, false, true, gemm_mode, (char *)ws + f.ws_bytes, ws_bytes - f.ws_bytes, st);
+}
+
+int lfi_feature_encode_bwd(const lfi_shape *s, const lfi_params *p, const lfi_batch *bt, int t0, int Tp, const float *dcond,
+                           float *const dx[LFI_NMOD], lfi_params *g, void *stash, size_t stash_bytes, void *ws, size_t ws_bytes,
+                           int gemm_mode, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  LFI_REQUIRE(s && p && bt && dcond && g && stash && ws, LFI_ERR_ARG, "lfi_feature_encode_bwd: null argument");
+  Dims d;
+  LFI_TRY(feature_train_dims(s, bt->B, Tp, gemm_mode, &d));
+  LFI_TRY(feature_check(s, d, p, bt, t0, Tp, g, "lfi_feature_encode_bwd"));
+  const int B = bt->B, T = bt->T;
+  FeatPlan f;
+  plan_feature(s, B, T, Tp, gemm_mode, stash, ws, true, &f);
+  LFI_REQUIRE(stash_bytes >= f.stash_bytes, LFI_ERR_WORKSPACE, "lfi_feature_encode_bwd: stash too small: %zu < %zu", stash_bytes, f.stash_bytes);
+  const size_t need = feature_ws_need(s, d, B, T, Tp, gemm_mode);
+  LFI_REQUIRE(ws_bytes >= need, LFI_ERR_WORKSPACE, "lfi_feature_encode_bwd: workspace too small: %zu < %zu", ws_bytes, need);
+  void *gws = (char *)ws + f.ws_bytes;
+  const size_t gws_bytes = ws_bytes - f.ws_bytes;
+  const bool lo = gemm_mode == LFI_GEMM_BF16X3;
+  for (int m = 0; m < LFI_NMOD; ++m) {
+    if (s->hist[m] <= 0) continue;
+    float *dxm = dx ? dx[m] : nullptr;
+    const int hist = s->hist[m], dim = s->dim[m], E = s->ehid[m];
+    if (E <= 0) {  // "enc: none": the window itself is the feature block
+      if (dxm) LFI_TRY(aux::window_grad(dxm, dcond + d.enc_offe[m], d.Fe, 0, bt->mask[m], B, T, dim, hist, m == 0 ? 0 : 1, t0, Tp, st));
+      continue;
+    }
+    EncWs &ew = f.enc[m];
+    if (ew.planes) {  // the operand planes of W_hh (dh_prev) and W_ih (dXg) belong to this call's workspace
+      LFI_TRY(split_to_planes(p->enc_w_hh[m], 3 * E, E, E, 0, 1, ew.whh_hi, lo ? ew.whh_lo : nullptr, st));
+      if (dxm) LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * E, dim, dim, 0, 1, ew.wih_hi, lo ? ew.wih_lo : nullptr, st));
+    }
+    const EncBwdOpts o = {f.part, f.part_rows[m], f.dxg, dxm};
+    LFI_TRY(enc_bwd(s, d, p, bt, t0, Tp, m, ew, dcond, g, gemm_mode, gemm_mode, gws, gws_bytes, o, st));
+  }
   return LFI_OK;
 }
 

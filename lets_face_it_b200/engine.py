@@ -59,6 +59,45 @@ def _on_own_device(fn):
     return wrapped
 
 
+def feature_train_fwd(shape, P, bt, keep, t0, Tp, mode, dev):
+    """lfi_feature_encode_fwd_train for a filled Params / Batch pair (`keep` holds the tensors they point into): returns
+    (cond [Tp*B, Fe] folded, saved) with `saved` what `feature_train_bwd` needs (the stash included)."""
+    L, st = cabi.lib(), cabi.stream_ptr()
+    B, T = bt.B, bt.T
+    cond = torch.empty(Tp * B, L.lfi_feature_dim_folded(ctypes.byref(shape)), dtype=torch.float32, device=dev)
+    stash = torch.empty(max(256, L.lfi_feature_stash_bytes(ctypes.byref(shape), B, T, Tp, mode)), dtype=torch.uint8, device=dev)
+    ws = torch.empty(max(256, L.lfi_feature_bwd_ws_bytes(ctypes.byref(shape), B, T, Tp, mode)), dtype=torch.uint8, device=dev)
+    cabi.check(L.lfi_feature_encode_fwd_train(ctypes.byref(shape), ctypes.byref(P), ctypes.byref(bt), t0, Tp, cond.data_ptr(), stash.data_ptr(),
+                                              stash.numel(), ws.data_ptr(), ws.numel(), mode, st), "lfi_feature_encode_fwd_train")
+    return cond, (shape, P, bt, keep, t0, Tp, mode, stash)
+
+
+def feature_train_bwd(saved, dcond, want_dx):
+    """lfi_feature_encode_bwd: returns (dx, grads).  dx[i] = dL/d(stream i) [B, T, dim] or None where want_dx[i] is false or absent;
+    grads[i] = (weight_ih, weight_hh, bias_ih, bias_hh) gradients of GRU modality i (written, not accumulated), None elsewhere."""
+    shape, P, bt, keep, t0, Tp, mode, stash = saved
+    L, st = cabi.lib(), cabi.stream_ptr()
+    B, T = bt.B, bt.T
+    dev = stash.device
+    dcond = dcond.to(dtype=torch.float32).contiguous()
+    dx, grads = [None] * cabi.NMOD, [None] * cabi.NMOD
+    DX = (ctypes.c_void_p * cabi.NMOD)()
+    G = cabi.Params()
+    for i in range(cabi.NMOD):
+        h, d, E = shape.hist[i], shape.dim[i], shape.ehid[i]
+        if h > 0 and i < len(want_dx) and want_dx[i]:
+            dx[i] = torch.empty(B, T, d, dtype=torch.float32, device=dev)
+            DX[i] = dx[i].data_ptr()
+        if h > 0 and E > 0:
+            grads[i] = (torch.empty(3 * E, d, device=dev), torch.empty(3 * E, E, device=dev), torch.empty(3 * E, device=dev),
+                        torch.empty(3 * E, device=dev))
+            G.enc_w_ih[i], G.enc_w_hh[i], G.enc_b_ih[i], G.enc_b_hh[i] = [t.data_ptr() for t in grads[i]]
+    ws = torch.empty(max(256, L.lfi_feature_bwd_ws_bytes(ctypes.byref(shape), B, T, Tp, mode)), dtype=torch.uint8, device=dev)
+    cabi.check(L.lfi_feature_encode_bwd(ctypes.byref(shape), ctypes.byref(P), ctypes.byref(bt), t0, Tp, dcond.data_ptr(), DX, ctypes.byref(G),
+                                        stash.data_ptr(), stash.numel(), ws.data_ptr(), ws.numel(), mode, st), "lfi_feature_encode_bwd")
+    return dx, grads
+
+
 class Engine:
     """One engine per top-level module (SeqGlow, or a stand-alone Glow/FlowNet/FlowStep)."""
 
@@ -440,6 +479,22 @@ class Engine:
         cabi.check(L.lfi_feature_encode(ctypes.byref(self.shape), ctypes.byref(P), ctypes.byref(bt), t0, Tp, cond.data_ptr(),
                                         ws.data_ptr(), ws.numel(), self.gemm_mode, st), "lfi_feature_encode")
         return cond
+
+    @_on_own_device
+    def feature_encode_train(self, data, t0, Tp, masks=None):
+        """`feature_encode` with the stash `feature_encode_backward` needs (lfi_feature_encode_fwd_train): (cond, saved)."""
+        self.ensure()
+        P = self._params_struct(self.theta, self.W)
+        x0 = data["p1_face"]
+        B, T = x0.shape[0], x0.shape[1]
+        bt, keep = self._batch_struct(data, B, T, masks)
+        return feature_train_fwd(self.shape, P, bt, keep, t0, Tp, self.gemm_mode, self.theta.device)
+
+    @_on_own_device
+    def feature_encode_backward(self, saved, dcond, want_dx):
+        """Backward of `feature_encode_train` (lfi_feature_encode_bwd): dL/d(stream) [B, T, dim] per modality (None where
+        want_dx[i] is false) and the encoder gradients as `feature_train_bwd` returns them."""
+        return feature_train_bwd(saved, dcond, want_dx)
 
     def unfold_features(self, cond):
         """[M, Fe] folded -> [M, F] as the reference lays it out (GRU state concatenated twice, models.py:64)."""

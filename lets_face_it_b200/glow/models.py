@@ -23,7 +23,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _cabi as cabi
-from ..engine import MODALITIES, Engine
+from ..engine import MODALITIES, Engine, feature_train_bwd, feature_train_fwd
 from . import modules, thops
 from .modules import GaussianDiag
 from .utils import get_longest_history
@@ -72,7 +72,11 @@ class ModalityEncoder(nn.Module):
         if self.enc_type not in ("rnn", "none"):
             raise NotImplementedError("enc=%r is outside the accelerated path" % self.enc_type)
         fe = _SingleModality(self)
-        return fe.encode(x, self.draw_mask(x.shape[:1], x.device))
+        mask = self.draw_mask(x.shape[:1], x.device)
+        params = fe.gru_params()
+        if modules._needs_grad(x, *params):
+            return fe.encode_autograd(x, mask, params)
+        return fe.encode(x, mask)
 
 
 class FeatureEncoder(nn.Module):
@@ -133,26 +137,47 @@ class FeatureEncoder(nn.Module):
             out[m] = enc.draw_mask(lead_shape, device) if enc is not None else None
         return out if any(v is not None for v in out.values()) else None
 
+    def gru_params(self):
+        """The GRU parameters of every GRU-encoded modality, MODALITIES order, (weight_ih, weight_hh, bias_ih, bias_hh) each."""
+        out = []
+        for m in MODALITIES:
+            gru = self.gru_of(m)
+            if gru is not None:
+                out += [gru.weight_ih_l0, gru.weight_hh_l0, gru.bias_ih_l0, gru.bias_hh_l0]
+        return out
+
     def forward(self, condition):
-        """condition: {"prev_p1_face": [B,h0,C], "p2_face": [B,h,d], "p1_speech": ..., "p2_speech": ...} -> [B, dim]."""
+        """condition: {"prev_p1_face": [B,h0,C], "p2_face": [B,h,d], "p1_speech": ..., "p2_speech": ...} -> [B, dim].
+        With grad mode on and a window or a GRU parameter requiring grad, the call is one autograd node (_FeatureEncodeFn)."""
         eng = self._engine if self._engine is not None else _encoder_only_engine(self)
         x0 = condition["prev_p1_face"]
         B, dev = x0.shape[0], x0.device
         st = eng.start_ts
-        data = {}
+        wins, data = {}, {}
         for m in MODALITIES:
             h = self._hist[m]
             if m != "p1_face" and not h:
                 continue
-            win = condition["prev_p1_face" if m == "p1_face" else m].float()
+            win = condition["prev_p1_face" if m == "p1_face" else m]
+            wins[m] = win
             buf = torch.zeros(B, st + 1, win.shape[2], device=dev)
             if m == "p1_face":
-                buf[:, st - h:st] = win      # window [t-h, t)
+                buf[:, st - h:st] = win.float()      # window [t-h, t)
             else:
-                buf[:, st - h + 1:st + 1] = win  # window (t-h, t]
+                buf[:, st - h + 1:st + 1] = win.float()  # window (t-h, t]
             data[m] = buf
         masks = self.draw_masks((1, B), dev)
-        return eng.unfold_features(eng.feature_encode(data, st, 1, masks))
+        params = self.gru_params()
+        if not modules._needs_grad(*wins.values(), *params):
+            return eng.unfold_features(eng.feature_encode(data, st, 1, masks))
+        # the window gradients leave the node as gradients of the padded buffers; the slice assignments above carry them back
+        bufs = [data.get(m) for m in MODALITIES]
+
+        def fwd(bs):
+            return eng.feature_encode_train({m: b for m, b in zip(MODALITIES, bs) if b is not None}, st, 1, masks)
+
+        cond = _FeatureEncodeFn.apply(fwd, eng.feature_encode_backward, len(bufs), *bufs, *params)
+        return eng.unfold_features(cond)
 
 
 def _encoder_only_engine(fe):
@@ -162,43 +187,94 @@ def _encoder_only_engine(fe):
     return eng
 
 
+class _FeatureEncodeFn(torch.autograd.Function):
+    """The window encoders under autograd (reference models.py:55-80 differentiated by torch): forward = `fwd(bufs)` over
+    lfi_feature_encode_fwd_train, backward = `bwd(saved, dcond, want_dx)` over lfi_feature_encode_bwd.  Inputs after `n` are
+    the n padded stream buffers [B, T, dim] (MODALITIES order, None where absent) and then the GRU parameters in
+    `FeatureEncoder.gru_params()` order (graph connectivity; the calls read the values through their own pointers).  The node
+    keeps its stash and masks; the backward runs in the forward's gemm mode."""
+
+    @staticmethod
+    def forward(ctx, fwd, bwd, n, *tensors):
+        cond, saved = fwd(tensors[:n])
+        ctx.bwd, ctx.saved, ctx.n = bwd, saved, n
+        return cond
+
+    @staticmethod
+    def backward(ctx, dcond):
+        n = ctx.n
+        want = ctx.needs_input_grad[3:3 + n]
+        dx, grads = ctx.bwd(ctx.saved, dcond, want)
+        dparams = [g for gs in grads if gs is not None for g in gs]
+        return (None, None, None) + tuple(dx[:n]) + tuple(dparams)
+
+
 class _SingleModality:
-    """Runs one ModalityEncoder window through lfi_feature_encode (a p1_face dummy fills slot 0)."""
+    """Runs one ModalityEncoder window through lfi_feature_encode (a p1_face dummy fills slot 0), under autograd through
+    lfi_feature_encode_fwd_train / lfi_feature_encode_bwd."""
 
     def __init__(self, enc: ModalityEncoder):
         self.enc = enc
 
-    def encode(self, x, mask):
-        import ctypes
+    def gru_params(self):
+        g = self.enc.encoder if self.enc.enc_type == "rnn" else None
+        return [g.weight_ih_l0, g.weight_hh_l0, g.bias_ih_l0, g.bias_hh_l0] if g is not None else []
+
+    def _call(self, xb, mask, params):
+        """Shape, Params and Batch of the one-modality call: xb [B, h+1, d] = the window after one zero frame (slot 1), params fp32
+        on xb's device."""
         enc = self.enc
-        B, h, d = x.shape
-        dev = x.device
+        B, T, d = xb.shape
+        h = T - 1
+        dev = xb.device
         sh = cabi.Shape()
         sh.C, sh.K, sh.H, sh.D, sh.G, sh.affine, sh.scale_eps, sh.f_raw = 2, 1, 4, 4, 3, 1, 1e-4, 0
         sh.hist[0], sh.dim[0], sh.ehid[0] = 1, 2, 0
         E = enc.encoder.hidden_size if enc.enc_type == "rnn" else 0
         sh.hist[1], sh.dim[1], sh.ehid[1] = h, d, E
         P = cabi.Params()
-        keep = []
-        if E:
-            for name, attr in (("enc_w_ih", "weight_ih_l0"), ("enc_w_hh", "weight_hh_l0"), ("enc_b_ih", "bias_ih_l0"), ("enc_b_hh", "bias_hh_l0")):
-                t = getattr(enc.encoder, attr).detach().to(device=dev, dtype=torch.float32).contiguous()
-                keep.append(t)
-                getattr(P, name)[1] = cabi.ptr(t)
-        T = h + 1
+        keep = list(params)
+        for name, t in zip(("enc_w_ih", "enc_w_hh", "enc_b_ih", "enc_b_hh"), params):
+            getattr(P, name)[1] = cabi.ptr(t)
         bt = cabi.Batch()
         bt.B, bt.T = B, T
         dummy = torch.zeros(B, T, 2, device=dev)
-        xb = torch.zeros(B, T, d, device=dev)
-        xb[:, 1:] = x.float()
+        keep += [dummy, xb]
         bt.x[0], bt.x[1] = cabi.ptr(dummy), cabi.ptr(xb)
         if mask is not None:
             mk = mask.reshape(1, B, h).float().contiguous()
+            keep.append(mk)
             bt.mask[1] = cabi.ptr(mk)
+        return sh, P, bt, keep
+
+    def encode_autograd(self, x, mask, params):
+        B, h, d = x.shape
+        dev = x.device
+        xb = torch.zeros(B, h + 1, d, device=dev)
+        xb[:, 1:] = x.float()
+        params = [modules._f32g(p, dev) for p in params]
+
+        def fwd(bs):
+            sh, P, bt, keep = self._call(bs[1].detach(), mask, [p.detach() for p in params])
+            return feature_train_fwd(sh, P, bt, keep, h, 1, cabi.GEMM_FP32, dev)
+
+        cond = _FeatureEncodeFn.apply(fwd, feature_train_bwd, 2, None, xb, *params)
+        out = cond[:, 2:]
+        return torch.cat([out, out], dim=1) if params else out
+
+    def encode(self, x, mask):
+        import ctypes
+        B, h, d = x.shape
+        dev = x.device
+        E = self.enc.encoder.hidden_size if self.enc.enc_type == "rnn" else 0
+        xb = torch.zeros(B, h + 1, d, device=dev)
+        xb[:, 1:] = x.float()
+        sh, P, bt, keep = self._call(xb, mask, [modules._f32c(p, dev) for p in self.gru_params()])
+        T = h + 1
         L = cabi.lib()
         Fe = L.lfi_feature_dim_folded(ctypes.byref(sh))
         cond = torch.empty(B, Fe, device=dev)
-        ws = torch.empty(L.lfi_feature_ws_bytes(ctypes.byref(sh), B, T, 1), dtype=torch.uint8, device=dev)
+        ws = torch.empty(L.lfi_feature_ws_bytes(ctypes.byref(sh), B, T, 1, cabi.GEMM_FP32), dtype=torch.uint8, device=dev)
         cabi.check(L.lfi_feature_encode(ctypes.byref(sh), ctypes.byref(P), ctypes.byref(bt), h, 1, cabi.ptr(cond), ws.data_ptr(),
                                         ws.numel(), cabi.GEMM_FP32, cabi.stream_ptr()), "lfi_feature_encode")
         out = cond[:, 2:]
