@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 7
+#define LFI_ABI_VERSION 8
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -136,6 +136,22 @@ int lfi_seq_train_fwd(const lfi_shape *s, const void *derived, const lfi_params 
 int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *b,
                       const float *z, const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, int gemm_mode,
                       void *stream);
+/* The same backward that also gives dL/d(input streams) (SeqGlow.forward differentiated with respect to its batch, as torch
+ * differentiates the reference's per-frame loop).  Arguments as lfi_seq_train_bwd, plus
+ *   dx[m]  NULL (not wanted) or [B, T, dim[m]] batch-first: dL/d(b->x[m]), WRITTEN over all T frames.  p1_face gets the gradient
+ *          of its windows and of the flow input (frame start_ts + t') as one sum; frames that no window and no flow input reads
+ *          are exact zeros.  Dropout masks scale the gradients as they scaled the inputs.  A non-NULL entry for an absent
+ *          modality (hist 0) is an argument error.
+ *   dws    scratch of lfi_train_dx_ws_bytes bytes (the dXg products of each GRU encoder, whose chains run concurrently).
+ * Null required pointers and a too-small ws / dws return a status before anything is launched.  The parameter gradients are
+ * those of lfi_seq_train_bwd (same kernels; reduction order may differ in the last bits) and the grad-ready event is recorded at
+ * the same point.  Like the parameter gradients of the encoders, the input gradients of GRU modalities are not bit-reproducible
+ * (their dh chains accumulate with split-K atomics).  At final_model.yaml, B = 256, T = 80 the scratch is 108.0 MB in every mode (p2_face 77.1, p2_speech 27.5, p1_speech
+ * 3.4 MB); with every modality "enc: none" it is the minimal 256 bytes. */
+size_t lfi_train_dx_ws_bytes(const lfi_shape *s, int B, int T, int gemm_mode);
+int lfi_seq_train_bwd_dx(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *b,
+                         const float *z, const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, float *const dx[LFI_NMOD],
+                         void *dws, size_t dws_bytes, int gemm_mode, void *stream);
 
 /* ---- SeqGlow.inference (models.py:567-596): persistent autoregressive sampler ---------------
  * faces [B, seq_len, C] in/out: the first start_ts frames hold the seed (data["p1_face"]), frames

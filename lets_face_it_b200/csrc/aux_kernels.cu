@@ -532,8 +532,10 @@ int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st, float *part) {
 
 // Adjoint of gather_windows: thread = one element dx[b][tau][c]; the (t', s) pairs whose window reads frame tau are visited
 // in increasing t', so every element is one thread's fixed-order sum (no atomics although windows overlap when Tp > 1).
+// ADD: the term add[tau - t0] of frames t0 <= tau < t0 + Tp comes last.
+template <bool ADD>
 __global__ void window_grad_kernel(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim,
-                                   int hist, int off, int t0, int Tp) {
+                                   int hist, int off, int t0, int Tp, const float *add) {
   const size_t M = (size_t)Tp * B;
   const size_t n = (size_t)B * T * dim;
   for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
@@ -549,12 +551,16 @@ __global__ void window_grad_kernel(float *dx, const float *src, int ld, int layo
       if (mask) v *= mask[m * hist + s];
       acc += v;
     }
+    if (ADD && tau >= t0 && tau < t0 + Tp) acc += add[((size_t)(tau - t0) * B + b) * dim + c];
     dx[e] = acc;
   }
 }
 int window_grad(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim, int hist, int off, int t0,
-                int Tp, cudaStream_t st) {
-  window_grad_kernel<<<blocks_for((size_t)B * T * dim), TB, 0, st>>>(dx, src, ld, layout_steps, mask, B, T, dim, hist, off, t0, Tp);
+                int Tp, cudaStream_t st, const float *add) {
+  if (add)
+    window_grad_kernel<true><<<blocks_for((size_t)B * T * dim), TB, 0, st>>>(dx, src, ld, layout_steps, mask, B, T, dim, hist, off, t0, Tp, add);
+  else
+    window_grad_kernel<false><<<blocks_for((size_t)B * T * dim), TB, 0, st>>>(dx, src, ld, layout_steps, mask, B, T, dim, hist, off, t0, Tp, nullptr);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

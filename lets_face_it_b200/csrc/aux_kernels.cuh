@@ -75,9 +75,11 @@ int enc_gate_bwd2(const EncStepBwd2 &a, cudaStream_t st, float *part = nullptr);
 int enc_gate_bwd2_part_rows(int M, int E);
 
 // Adjoint of gather_windows (same arguments, src in the layout gather_windows writes): dx [B][T][dim] is written for every frame,
-// dx[b][tau][c] = sum of mask * src over the (t', s) with tau = t0 + t' - hist + off + s, zero where no window reads the frame
+// dx[b][tau][c] = sum of mask * src over the (t', s) with tau = t0 + t' - hist + off + s, zero where no window reads the frame.
+// add != nullptr: [Tp][B][dim], add[t'][b][c] joins the sum of frame tau = t0 + t' as its last term (p1_face: the gradient of the
+// flow input), so each element stays one thread's fixed-order sum
 int window_grad(float *dx, const float *src, int ld, int layout_steps, const float *mask, int B, int T, int dim, int hist, int off, int t0,
-                int Tp, cudaStream_t st);
+                int Tp, cudaStream_t st, const float *add = nullptr);
 
 // LU parametrisation helpers (modules.py:163-177)
 int lu_build(float *Lm, float *Um, const float *l, const float *u, const float *log_s, const float *sign_s, int K, int C, cudaStream_t st);

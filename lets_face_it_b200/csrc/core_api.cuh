@@ -112,6 +112,9 @@ struct BwdArgs {
   // the cell kernel then leaves that product out (skip_hh set by the launcher)
   WaveTc wtc;
   int skip_hh;
+  // whole-sequence backward: nullptr, or [Tp][B][C] that receives dL/d(input of step 0) = dL/d(p1_face frame start_ts + t),
+  // written by the cells (0, t) after their ActNorm backward (the gradient of the flow input of every frame)
+  float *dx_in;
 };
 
 int fwd_smem_bytes(const Dims &d, int R);

@@ -9,7 +9,8 @@
 namespace lfi {
 namespace core {
 
-template <int RPT, int KC>
+// DXIN: the cells (0, t) also store the gradient of the flow input (BwdArgs.dx_in); the instantiation without it is the plain backward
+template <int RPT, int KC, bool DXIN>
 __global__ void __launch_bounds__(NT) core_bwd_wave(BwdArgs a, int wave, int kmin) {
   extern __shared__ __align__(16) float sm[];
   constexpr int R = Tile<RPT>::R, RS = Tile<RPT>::RS;
@@ -246,11 +247,17 @@ __global__ void __launch_bounds__(NT) core_bwd_wave(BwdArgs a, int wave, int kmi
         const int r = e / C, c = e - r * C;
         a.dx0_out[(size_t)(row0 + r) * C + c] = dxr[r * pC + c];
       }
-  } else if (k > 0)
+  } else if (k > 0) {
     for (int e = tid; e < nrows * C; e += NT) {
       const int r = e / C, c = e - r * C;
       a.dx[(cell * B + row0 + r) * C + c] = dxr[r * pC + c];
     }
+  } else if (DXIN) {  // step 0: the gradient of the flow input of frame t (cell == t)
+    for (int e = tid; e < nrows * C; e += NT) {
+      const int r = e / C, c = e - r * C;
+      a.dx_in[(cell * B + row0 + r) * C + c] = dxr[r * pC + c];
+    }
+  }
   for (int c = tid; c < C; c += NT) {
     float s1 = 0.f, s2 = 0.f;
     for (int r = 0; r < nrows; ++r) { s1 += dxr[r * pC + c]; s2 += prod[r * pO + c]; }
@@ -262,7 +269,8 @@ __global__ void __launch_bounds__(NT) core_bwd_wave(BwdArgs a, int wave, int kmi
 template <int RPT, int KC> static int launch_bwd_t(const BwdArgs &a, cudaStream_t st) {
   constexpr int R = Tile<RPT>::R;
   const int bytes = plan_smem(a.d, R, true, false, KC).total * (int)sizeof(float);
-  LFI_CUDA(cudaFuncSetAttribute(core_bwd_wave<RPT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  auto kern = a.dx_in ? core_bwd_wave<RPT, KC, true> : core_bwd_wave<RPT, KC, false>;
+  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   const int tiles = (a.B + R - 1) / R, K = a.d.K;
   const bool tcw = a.wtc.mode != 0 && a.single < 0;
   BwdArgs aw = a;
@@ -270,7 +278,7 @@ template <int RPT, int KC> static int launch_bwd_t(const BwdArgs &a, cudaStream_
   for (int wave = a.Tp + K - 2; wave >= 0; --wave) {
     const int k0 = max(0, wave - a.Tp + 1), k1 = min(K - 1, wave);
     dim3 grid(tiles, k1 - k0 + 1);
-    core_bwd_wave<RPT, KC><<<grid, NT, bytes, st>>>(aw, wave, k0);
+    kern<<<grid, NT, bytes, st>>>(aw, wave, k0);
     if (!tcw) continue;
     // cells (k, t = wave - k) with t >= 1 wrote the direct part of d h[k][t-1] into a.dh[k][t]; add dA_h[k][t] W_hh[k]  (batch over k)
     const int kb0 = k0, kb1 = min(k1, wave - 1);
@@ -293,8 +301,8 @@ template <int RPT, int KC> static int launch_bwd_t(const BwdArgs &a, cudaStream_
 template <int RPT, int KC> static int launch_bwd_single_t(const BwdArgs &a, cudaStream_t st) {
   constexpr int R = Tile<RPT>::R;
   const int bytes = plan_smem(a.d, R, true, false, KC).total * (int)sizeof(float);
-  LFI_CUDA(cudaFuncSetAttribute(core_bwd_wave<RPT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  core_bwd_wave<RPT, KC><<<dim3((a.B + R - 1) / R, 1), NT, bytes, st>>>(a, a.single, a.single);  // wave = k: t = 0
+  LFI_CUDA(cudaFuncSetAttribute(core_bwd_wave<RPT, KC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  core_bwd_wave<RPT, KC, false><<<dim3((a.B + R - 1) / R, 1), NT, bytes, st>>>(a, a.single, a.single);  // wave = k: t = 0
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -47,6 +47,8 @@ __host__ __device__ inline PipePlanB plan_pipe_bwd(const Dims &d) {
   return p;
 }
 
+// DXIN: stage 0 also stores the gradient of the flow input (BwdArgs.dx_in); the instantiation without it is the plain backward
+template <bool DXIN>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PNT, 1)
 core_bwd_pipe(const BwdArgs a, const int P, const int ntiles, int *progress) {
   extern __shared__ __align__(16) float sm[];
@@ -408,6 +410,7 @@ core_bwd_pipe(const BwdArgs a, const int P, const int ntiles, int *progress) {
                 gab[j] += dxv;
                 gal[j] += dy[i][j] * yv[i][j];
                 if (k > 0) a.dx[off + j] = dxv;
+                else if (DXIN) a.dx_in[off + j] = dxv;  // stage 0 (cell == t): gradient of the flow input
               }
             }
           }
@@ -503,11 +506,12 @@ int launch_bwd_pipe(const BwdArgs &a, cudaStream_t st) {
   int P = nsm / (2 * K);
   if (P > ntiles) P = ntiles;
   LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * (K + 1) * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
-  LFI_CUDA(cudaFuncSetAttribute(core_bwd_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  auto kern = a.dx_in ? core_bwd_pipe<true> : core_bwd_pipe<false>;
+  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * (K + 1) * 2 * sizeof(int), st));
   dim3 grid(2, K, P);
-  LFI_TRY(pipe_check_residency(core_bwd_pipe, PNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe"));
-  core_bwd_pipe<<<grid, PNT, bytes, st>>>(a, P, ntiles, a.flags);
+  LFI_TRY(pipe_check_residency(kern, PNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe"));
+  kern<<<grid, PNT, bytes, st>>>(a, P, ntiles, a.flags);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -72,6 +72,8 @@ __device__ int g_core_timing_bt = 0;
 
 }  // namespace
 
+// DXIN: stage 0 also stores the gradient of the flow input (BwdArgs.dx_in); the instantiation without it is the plain backward
+template <bool DXIN>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(BNT, 1)
 core_bwd_pipe_tc(const BwdArgs a, const int P, const int ntiles, int *progress) {
   extern __shared__ __align__(16) uint8_t smraw[];
@@ -526,6 +528,7 @@ core_bwd_pipe_tc(const BwdArgs a, const int P, const int ntiles, int *progress) 
                 gab[j] += dxv;
                 gal[j] += dy[i][j] * yv[i][j];
                 if (k > 0) a.dx[off + j] = dxv;
+                else if (DXIN) a.dx_in[off + j] = dxv;  // stage 0 (cell == t): gradient of the flow input
               }
             }
           }
@@ -618,11 +621,12 @@ int launch_bwd_pipe_tc(const BwdArgs &a, cudaStream_t st) {
   if (P > ntiles) P = ntiles;
   LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * (K + 1) * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
   LFI_REQUIRE(a.stash_tiled && a.pdG_hi && a.pdAh_hi, LFI_ERR_ARG, "tensor-core backward pipeline needs the tiled stash and plane outputs");
-  LFI_CUDA(cudaFuncSetAttribute(core_bwd_pipe_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  auto kern = a.dx_in ? core_bwd_pipe_tc<true> : core_bwd_pipe_tc<false>;
+  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * (K + 1) * 2 * sizeof(int), st));
   dim3 grid(2, K, P);
-  LFI_TRY(pipe_check_residency(core_bwd_pipe_tc, BNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe_tc"));
-  core_bwd_pipe_tc<<<grid, BNT, bytes, st>>>(a, P, ntiles, a.flags);
+  LFI_TRY(pipe_check_residency(kern, BNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe_tc"));
+  kern<<<grid, BNT, bytes, st>>>(a, P, ntiles, a.flags);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

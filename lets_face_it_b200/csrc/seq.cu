@@ -1,6 +1,6 @@
 // Host-side orchestration of the hot path behind the C ABI (include/lfi_b200.h):
 //   lfi_derive            derived weight cache
-//   lfi_seq_train_fwd/bwd SeqGlow.forward (models.py:534-561) and its backward
+//   lfi_seq_train_fwd/bwd SeqGlow.forward (models.py:534-561) and its backward (lfi_seq_train_bwd_dx: also d input streams)
 //   lfi_seq_sample        SeqGlow.inference / SeqGlow.invert (models.py:567-645)
 //   lfi_flowstep          FlowStep.forward on one frame (models.py:305-373)
 //   lfi_invconv_compose   InvertibleConv1x1.get_weight (modules.py:149-178) and its chain rule
@@ -669,12 +669,24 @@ int lfi_seq_train_fwd(const lfi_shape *s, const void *derived, const lfi_params 
   return core::launch_fwd(a, st);
 }
 
-int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *bt, const float *z,
-                      const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, int gemm_mode, void *stream) {
-  cudaStream_t st = (cudaStream_t)stream;
+// Backward of lfi_seq_train_fwd.  dx == nullptr: parameter gradients only (lfi_seq_train_bwd).  Otherwise (lfi_seq_train_bwd_dx)
+// also dL/d(raw stream m) into every non-null dx[m] [B][T][dim]: the flow core keeps the gradient of its input (step 0), d cond is
+// formed for the "enc: none" columns as well, and the window adjoints (aux::window_grad, inside enc_bwd for the GRU modalities)
+// scatter d cond back onto the frames; dws holds the dXg scratch of each GRU modality (plan_train_dx).
+struct TrainDxWs { float *dxg[LFI_NMOD]; size_t bytes; };
+static void plan_train_dx(const lfi_shape *s, size_t M, void *dws, TrainDxWs *x) {
+  Bump b(dws, 0);
+  for (int m = 0; m < LFI_NMOD; ++m)
+    x->dxg[m] = (s->hist[m] > 0 && s->ehid[m] > 0) ? b.take<float>((size_t)s->hist[m] * M * s->dim[m]) : nullptr;
+  x->bytes = round_up_sz(b.off > 256 ? b.off : 256, 256);
+}
+
+static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *bt, const float *z,
+                         const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, int gemm_mode, cudaStream_t st,
+                         float *const *dx, void *dws, size_t dws_bytes, const char *what) {
   Dims d;
   LFI_TRY(make_dims(s, &d));
-  LFI_REQUIRE(derived && p && z && dnll && g && ws, LFI_ERR_ARG, "lfi_seq_train_bwd: null argument");
+  LFI_REQUIRE(derived && p && z && dnll && g && ws, LFI_ERR_ARG, "%s: null argument", what);
   LFI_TRY(check_batch(s, d, bt, d.start_ts + 1));
   const int B = bt->B, T = bt->T, Tp = T - d.start_ts, K = d.K, C = d.C, Ci = d.Ci, GH = d.GH, H = d.H, D = d.D, Co = d.Co;
   const int In = Ci + D;
@@ -682,6 +694,18 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   TrainWs w;
   plan_train(s, d, B, T, gemm_mode, ws, &w);
   LFI_REQUIRE(ws_bytes >= w.bytes + gemm_scratch_bound(s, d, M, (size_t)B * T, gemm_mode), LFI_ERR_WORKSPACE, "train workspace too small");
+  TrainDxWs xw;
+  memset(&xw, 0, sizeof(xw));
+  bool none_dx = false;  // an "enc: none" modality wants the gradient of its stream
+  if (dx) {
+    for (int m = 0; m < LFI_NMOD; ++m) {
+      LFI_REQUIRE(!dx[m] || s->hist[m] > 0, LFI_ERR_ARG, "%s: dx[%d] given for an absent modality", what, m);
+      none_dx = none_dx || (dx[m] && s->ehid[m] == 0);
+    }
+    plan_train_dx(s, M, dws, &xw);
+    LFI_REQUIRE(dws, LFI_ERR_ARG, "%s: null dx workspace", what);
+    LFI_REQUIRE(dws_bytes >= xw.bytes, LFI_ERR_WORKSPACE, "%s: dx workspace too small: %zu < %zu", what, dws_bytes, xw.bytes);
+  }
   void *gws = (char *)ws + w.bytes;
   const size_t gws_bytes = ws_bytes - w.bytes;
   const DerivedLayout L = derived_layout(d);
@@ -709,6 +733,9 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   if (w.wave_tc) {  // planes of W_hh were built by the forward call of this step
     a.wtc.mode = gemm_mode; a.wtc.whh_hi = w.wt_hi; a.wtc.whh_lo = w.wt_lo; a.wtc.ghbuf = w.ghbuf; a.wtc.gws = gws; a.wtc.gws_bytes = gws_bytes;
   }
+  // d(flow input) of every frame into the step-0 slot of the hand-off buffer, which nothing else writes or reads
+  float *dflow = (dx && dx[0]) ? w.dx : nullptr;
+  a.dx_in = dflow;
   LFI_TRY(core::launch_bwd(a, st));
 
   // 2. weight gradients of the per-step matrices as batched (over k) reductions over the M rows.  With every operand in
@@ -801,23 +828,42 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
       }
     }
   }
-  // d cond for the encoder columns only (inputs carry no gradient)
+  // d cond for the encoder columns [enc_lo, Fe)
   int enc_lo = -1;
   for (int m = 0; m < LFI_NMOD; ++m)
     if (s->hist[m] > 0 && s->ehid[m] > 0) { enc_lo = d.enc_offe[m]; break; }
-  if (enc_lo < 0) { join_wgrads(); return LFI_OK; }
-  {
-    GemmArgs q = gemm_args(0, 0, (int)M, d.Fe - enc_lo, K * D, w.dC, K * D, WcF + enc_lo, d.Fe, w.dcond + enc_lo, d.Fe, 0);
+  if (enc_lo < 0 && !none_dx) { join_wgrads(); return LFI_OK; }
+  auto dcond_gemm = [&](int lo, int hi) -> int {
+    GemmArgs q = gemm_args(0, 0, (int)M, hi - lo, K * D, w.dC, K * D, WcF + lo, d.Fe, w.dcond + lo, d.Fe, 0);
     if (w.cp) q.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
-    LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
-  }
+    return gemm_dispatch(bmode, q, gws, gws_bytes, st);
+  };
+  if (enc_lo >= 0) LFI_TRY(dcond_gemm(enc_lo, d.Fe));
+  // "enc: none" streams: d cond of the columns before enc_lo in a launch of its own (one GEMM over all Fe columns would change the
+  // tile split, and in the tensor-core modes the numerics, of the encoder columns), then the adjoint of the window gather (p1_face:
+  // its window excludes frame t, and the gradient of the flow input of frame start_ts + t' joins the same fixed-order sum).
+  // Reads only final values: dC and the flow-core output.
+  auto none_grads = [&]() -> int {
+    if (none_dx && enc_lo != 0) LFI_TRY(dcond_gemm(0, enc_lo < 0 ? d.Fe : enc_lo));
+    for (int m = 0; dx && m < LFI_NMOD; ++m)
+      if (dx[m] && s->ehid[m] == 0)
+        LFI_TRY(aux::window_grad(dx[m], w.dcond + d.enc_offe[m], d.Fe, 0, bt->mask[m], B, T, s->dim[m], s->hist[m], m == 0 ? 0 : 1,
+                                 d.start_ts, Tp, st, m == 0 ? dflow : nullptr));
+    return LFI_OK;
+  };
 
   // 4. encoder GRUs, BPTT over the window (enc_bwd).  The modalities are independent chains of a latency-bound GEMM and an
   //    HBM-bound gate kernel per window step: with every operand in plane form (no shared scratch) they run on parallel streams
   //    forked from / joined to the caller's.
-  const EncBwdOpts accumulate = {nullptr, 0, nullptr, nullptr};
+  //    With dx[m] set the chain also forms dL/d(stream m) (EncBwdOpts.dx, its own dXg scratch: the chains run concurrently).
   auto enc_chain = [&](int m, cudaStream_t cs) -> int {
-    return enc_bwd(s, d, p, bt, d.start_ts, Tp, m, w.enc[m], w.dcond, g, gemm_mode, bmode, gws, gws_bytes, accumulate, cs);
+    float *dxm = dx ? dx[m] : nullptr;
+    EncWs &ew = w.enc[m];
+    if (dxm && ew.planes && !ew.xfuse)  // (the fused forward steps built the W_ih planes already)
+      LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * s->ehid[m], s->dim[m], s->dim[m], 0, 1, ew.wih_hi,
+                              gemm_mode == LFI_GEMM_BF16X3 ? ew.wih_lo : nullptr, cs));
+    const EncBwdOpts o = {nullptr, 0, dxm ? xw.dxg[m] : nullptr, dxm};
+    return enc_bwd(s, d, p, bt, d.start_ts, Tp, m, ew, w.dcond, g, gemm_mode, bmode, gws, gws_bytes, o, cs);
   };
   int mods[LFI_NMOD], nmods = 0;
   bool all_planes = true;
@@ -829,6 +875,7 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   if (!par) {
     int rc = LFI_OK;
     for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], st);
+    if (rc == LFI_OK) rc = none_grads();
     join_wgrads();
     return rc;
   }
@@ -836,12 +883,36 @@ int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params 
   for (int i = 1; i < nmods; ++i) LFI_CUDA(cudaStreamWaitEvent(side[i], ev_fork, 0));
   int rc = LFI_OK;
   for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], i == 0 ? st : side[i]);
+  if (rc == LFI_OK) rc = none_grads();
   for (int i = 1; i < nmods; ++i) {  // always join, also on error
     cudaEventRecord(ev_join[i], side[i]);
     cudaStreamWaitEvent(st, ev_join[i], 0);
   }
   join_wgrads();
   return rc;
+}
+
+int lfi_seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *bt, const float *z,
+                      const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, int gemm_mode, void *stream) {
+  return seq_train_bwd(s, derived, p, bt, z, dnll, g, ws, ws_bytes, gemm_mode, (cudaStream_t)stream, nullptr, nullptr, 0,
+                       "lfi_seq_train_bwd");
+}
+
+size_t lfi_train_dx_ws_bytes(const lfi_shape *s, int B, int T, int gemm_mode) {
+  (void)gemm_mode;  // (the dXg scratch is fp32 in every mode)
+  Dims d;
+  if (make_dims(s, &d) != LFI_OK || T <= d.start_ts || B < 1) return 0;
+  TrainDxWs x;
+  plan_train_dx(s, (size_t)(T - d.start_ts) * B, nullptr, &x);
+  return x.bytes;
+}
+
+int lfi_seq_train_bwd_dx(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *bt, const float *z,
+                         const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, float *const dx[LFI_NMOD], void *dws,
+                         size_t dws_bytes, int gemm_mode, void *stream) {
+  LFI_REQUIRE(dx, LFI_ERR_ARG, "lfi_seq_train_bwd_dx: null dx");
+  return seq_train_bwd(s, derived, p, bt, z, dnll, g, ws, ws_bytes, gemm_mode, (cudaStream_t)stream, dx, dws, dws_bytes,
+                       "lfi_seq_train_bwd_dx");
 }
 
 // ------------------------------------------------------------------------------------------------

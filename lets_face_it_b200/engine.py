@@ -376,8 +376,9 @@ class Engine:
         return z, nll
 
     @_on_own_device
-    def train_backward(self, z, dnll, gflat, token=None):
-        """Accumulates dL/dtheta into gflat (layout of new_flat_grad) given dL/dnll [T',B]."""
+    def train_backward(self, z, dnll, gflat, token=None, dx=None):
+        """Accumulates dL/dtheta into gflat (layout of new_flat_grad) given dL/dnll [T',B].  dx: None, or one entry per modality,
+        None or a [B, T, dim] fp32 tensor that receives dL/d(stream) (lfi_seq_train_bwd_dx; written, not accumulated)."""
         if token is not None and token != self._fwd_token:
             raise RuntimeError("backward called after another forward on the same engine: the activation stash was overwritten")
         L, st = cabi.lib(), cabi.stream_ptr()
@@ -386,9 +387,16 @@ class Engine:
         Gs = self._params_struct(gflat, dW)
         dnll = dnll.to(dtype=torch.float32).contiguous()
         ws = self._workspace(("train", B, T), 0)
-        cabi.check(L.lfi_seq_train_bwd(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), ctypes.byref(bt),
-                                       z.data_ptr(), dnll.data_ptr(), ctypes.byref(Gs), ws.data_ptr(), ws.numel(), self.gemm_mode, st),
-                   "lfi_seq_train_bwd")
+        if dx is None:
+            cabi.check(L.lfi_seq_train_bwd(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), ctypes.byref(bt),
+                                           z.data_ptr(), dnll.data_ptr(), ctypes.byref(Gs), ws.data_ptr(), ws.numel(), self.gemm_mode, st),
+                       "lfi_seq_train_bwd")
+        else:
+            DX = (ctypes.c_void_p * cabi.NMOD)(*[cabi.ptr(t) for t in dx])
+            dws = self._workspace(("train_dx",), L.lfi_train_dx_ws_bytes(ctypes.byref(self.shape), B, T, self.gemm_mode))
+            cabi.check(L.lfi_seq_train_bwd_dx(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), ctypes.byref(bt),
+                                              z.data_ptr(), dnll.data_ptr(), ctypes.byref(Gs), ws.data_ptr(), ws.numel(), DX,
+                                              dws.data_ptr(), dws.numel(), self.gemm_mode, st), "lfi_seq_train_bwd_dx")
         # the parameter-only constant: nll -= C * (sum logs + sum log_s) / ln2   for every (t, b)
         coef = -(float(self.C) / LN2) * dnll.sum()
         self.block("an_logs", gflat).add_(coef)

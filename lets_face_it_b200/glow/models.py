@@ -5,7 +5,8 @@ Class names, constructor signatures, parameter names/shapes and the `forward` co
 a drop-in for `glow_pytorch.glow`; the per-frame Python loops of the reference are replaced by
 three fused device paths reached through the C ABI (`engine.py` / `_cabi.py`):
 
-  SeqGlow.forward   -> lfi_seq_train_fwd / lfi_seq_train_bwd  (autograd.Function below)
+  SeqGlow.forward   -> lfi_seq_train_fwd / lfi_seq_train_bwd  (autograd.Function below; lfi_seq_train_bwd_dx when a batch
+                       stream requires grad)
   SeqGlow.inference -> lfi_seq_sample (persistent autoregressive sampler)
   SeqGlow.invert    -> lfi_seq_sample (teacher forced)
   FlowStep / FlowNet / Glow single-frame calls -> lfi_flowstep (under autograd lfi_flowstep_fwd_train / lfi_flowstep_bwd)
@@ -616,14 +617,16 @@ class Glow(nn.Module):
 
 
 class _SeqGlowFn(torch.autograd.Function):
-    """z, nll = SeqGlow core.  Inputs after `masks` are the engine's parameters (for graph connectivity;
-    their values are read from the flat buffer they alias)."""
+    """z, nll = SeqGlow core.  `mods` lists the modalities (indices into MODALITIES) whose streams follow it as inputs, each
+    the [B, T, dim] fp32 device tensor that `batch` holds for it: their gradients come from lfi_seq_train_bwd_dx.  The remaining
+    inputs are the engine's parameters (for graph connectivity; their values are read from the flat buffer they alias)."""
 
     @staticmethod
-    def forward(ctx, eng, batch, masks, scale_out, *params):
+    def forward(ctx, eng, batch, masks, scale_out, mods, *inputs):
         z, nll = eng.train_forward(batch, masks, scale_out)
         nll = nll - eng.logdet_const().detach() / LN2
-        ctx.eng, ctx.token = eng, eng._fwd_token
+        ctx.eng, ctx.token, ctx.mods = eng, eng._fwd_token, mods
+        ctx.T = batch["p1_face"].shape[1]
         ctx.save_for_backward(z)
         ctx.mark_non_differentiable(z)
         return z, nll
@@ -633,8 +636,15 @@ class _SeqGlowFn(torch.autograd.Function):
         eng = ctx.eng
         (z,) = ctx.saved_tensors
         g = eng.new_flat_grad()
-        eng.train_backward(z, dnll, g, ctx.token)
-        return (None, None, None, None) + tuple(eng.grad_views(g))
+        if not ctx.mods:
+            eng.train_backward(z, dnll, g, ctx.token)
+            return (None, None, None, None, None) + tuple(eng.grad_views(g))
+        B = z.shape[1]
+        dx = [None] * cabi.NMOD
+        for i in ctx.mods:
+            dx[i] = torch.empty(B, ctx.T, eng.shape.dim[i], dtype=torch.float32, device=z.device)
+        eng.train_backward(z, dnll, g, ctx.token, dx=dx)
+        return (None, None, None, None, None) + tuple(dx[i] for i in ctx.mods) + tuple(eng.grad_views(g))
 
 
 class SeqGlow(nn.Module):
@@ -692,7 +702,22 @@ class SeqGlow(nn.Module):
         scale_out = None
         if self.hparams.Validation["scale_logging"] and eng.affine:
             scale_out = torch.empty(eng.K, B, eng.Cz, device=eng.theta.device)
-        z, nll = _SeqGlowFn.apply(eng, batch, masks, scale_out, *eng.param_list())
+        # Streams that require grad enter the autograd node as inputs (lfi_seq_train_bwd_dx gives their gradients).  They are
+        # converted and cut to T frames here, with torch ops, so that the gradient flows back through the dtype / device copy
+        # and the slice; the engine then finds them ready and reads them in place.
+        mods, streams = (), ()
+        if torch.is_grad_enabled():
+            mods = tuple(i for i, m in enumerate(MODALITIES)
+                         if eng.shape.hist[i] > 0 and isinstance(batch.get(m), torch.Tensor) and batch[m].requires_grad)
+        if mods:
+            batch = dict(batch)
+            for i in mods:
+                x = batch[MODALITIES[i]].to(device=eng.theta.device, dtype=torch.float32)
+                if i > 0 and x.dim() == 3 and x.shape[1] > T:
+                    x = x[:, :T]
+                batch[MODALITIES[i]] = x.contiguous()
+            streams = tuple(batch[MODALITIES[i]] for i in mods)
+        z, nll = _SeqGlowFn.apply(eng, batch, masks, scale_out, mods, *streams, *eng.param_list())
         if scale_out is not None:
             for k, layer in enumerate(self.glow.flow.layers):
                 layer.scale = scale_out[k]
