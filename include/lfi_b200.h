@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 8
+#define LFI_ABI_VERSION 9
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -223,6 +223,24 @@ int lfi_flowstep_bwd(const lfi_shape *s, const void *derived, const lfi_params *
                      const float *c_in, const float *dy, const float *dlogdet, const float *dh_out, const float *dc_out, float *dx,
                      float *dcond, float *dh_in, float *dc_in, lfi_params *g, int B, void *stash, size_t stash_bytes, void *ws,
                      size_t ws_bytes, void *stream);
+
+/* ---- FlowStep.forward(reverse=True) WITH autograd (FlowStep.reverse_flow models.py:345-373 and FlowNet.decode 444-462 under
+ * torch autograd).  lfi_flowstep_rev_fwd_train = lfi_flowstep with reverse=1 (same kernels, bitwise the same outputs) that also
+ * fills `stash` (lfi_flowstep_stash_bytes bytes) with the activations of the call; lfi_flowstep_rev_bwd is its backward, with
+ * the arguments of lfi_flowstep_bwd (dy = dL/d(output), dx = dL/d(input)) and a workspace of lfi_flowstep_rev_bwd_ws_bytes.
+ * Differences from lfi_flowstep_bwd: the parameter gradients of step k are WRITTEN, not accumulated (g->w still receives dL/dW
+ * of the composed FORWARD weight, read through W^-1 from the derived cache, which lfi_derive must have built with winv); the
+ * reverse log-det subtracts the coupling terms, and the parameter-only terms C*sum(logs), C*sum(log_s) are the host's; every
+ * reduction over the B rows runs in a fixed order (no atomics, no split-K), so the same call twice gives bit-identical
+ * gradients.  A null pointer, a short stash or a short workspace returns a status before anything is launched. */
+size_t lfi_flowstep_rev_bwd_ws_bytes(const lfi_shape *s, int B);
+int lfi_flowstep_rev_fwd_train(const lfi_shape *s, const void *derived, const lfi_params *p, int k, const float *x, const float *cond,
+                               const float *h_in, const float *c_in, float *h_out, float *c_out, float *y, float *logdet, int B,
+                               void *stash, size_t stash_bytes, void *ws, size_t ws_bytes, void *stream);
+int lfi_flowstep_rev_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, int k, const float *cond, const float *h_in,
+                         const float *c_in, const float *dy, const float *dlogdet, const float *dh_out, const float *dc_out, float *dx,
+                         float *dcond, float *dh_in, float *dc_in, lfi_params *g, int B, void *stash, size_t stash_bytes, void *ws,
+                         size_t ws_bytes, void *stream);
 
 /* ---- stand-alone modules under autograd (modules.py ActNorm2d / InvertibleConv1x1 / LinearZeros, models.py f_seq) ---------
  * Backward passes of lfi_actnorm and of LinearZeros, and f_seq.forward (models.py:204-214) with its backward, each on the

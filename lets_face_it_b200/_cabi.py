@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "liblfi_b200.so")
 NMOD = 4
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 GEMM_FP32, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
 EPI_BIAS, EPI_LRELU, EPI_ACCUM, EPI_LRELU_BWD = 1, 2, 4, 8
@@ -79,6 +79,9 @@ SYMBOLS = {
     "lfi_flowstep_bwd_ws_bytes": (_SZ, [_SH, _I]),
     "lfi_flowstep_fwd_train": (_I, [_SH, _P, _PR, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P, _SZ, _P, _SZ, _P]),
     "lfi_flowstep_bwd": (_I, [_SH, _P, _PR, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _PR, _I, _P, _SZ, _P, _SZ, _P]),
+    "lfi_flowstep_rev_bwd_ws_bytes": (_SZ, [_SH, _I]),
+    "lfi_flowstep_rev_fwd_train": (_I, [_SH, _P, _PR, _I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _P, _SZ, _P, _SZ, _P]),
+    "lfi_flowstep_rev_bwd": (_I, [_SH, _P, _PR, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _PR, _I, _P, _SZ, _P, _SZ, _P]),
     "lfi_derive": (_I, [_SH, _PR, _P, _P, _I, _P]),
     "lfi_invconv_compose": (_I, [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "lfi_invconv_compose_bwd": (_I, [_I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),

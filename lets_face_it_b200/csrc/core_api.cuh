@@ -73,6 +73,11 @@ struct InvArgs {
   float *faces_out; long fo_sb, fo_st;        // where frame t_abs is written
   float *hstate, *cstate;     // [K][B][H] carried RNN state (in/out)
   float *logdet_out;          // [T'][B] or nullptr (coupling terms only)
+  // Module API (lfi_flowstep_rev_fwd_train: ONE frame, ONE step): nullptr, or the step's activations for its backward, all
+  // [B][width], in the conventions of the forward stash (core::Stash): x1 = zc W^-1 (input of the reverse ActNorm), zc (coupling
+  // output, input of the inverse 1x1 conv), post-activation gates, ahn (GRU), o after its exp(3 logs) scale.  Set together; a
+  // launch with st_x1 set runs the kernels' stash instantiation.
+  float *st_x1, *st_zc, *st_gates, *st_ahn, *st_o;
 };
 
 struct BwdArgs {

@@ -221,7 +221,9 @@ __global__ void __launch_bounds__(NT) core_fwd_wave(FwdArgs a, int wave, int kmi
 
 // ------------------------------------------------------------------------------------------------
 // Persistent inverse kernel: one CTA per sequence tile, all frames of a chunk x all K steps.
-template <int RPT>
+// STASH: also store the activations of the step (InvArgs.st_x1 ...; one frame, one step); the instantiation without it is the
+// plain inverse
+template <int RPT, bool STASH>
 __global__ void __launch_bounds__(NT) core_inv_persistent(InvArgs a) {
   extern __shared__ __align__(16) float sm[];
   constexpr int R = Tile<RPT>::R, RS = Tile<RPT>::RS;
@@ -285,9 +287,10 @@ __global__ void __launch_bounds__(NT) core_inv_persistent(InvArgs a) {
       } else {
         Grow = a.G + ((size_t)tc * B + row0) * a.g_ld + (size_t)(k - a.g_k0) * GH;
       }
-      coupling_net<RPT>(d, w, sp, sm, nrows, Grow, a.g_ld, nullptr, nullptr,
+      coupling_net<RPT>(d, w, sp, sm, nrows, Grow, a.g_ld, STASH ? a.st_gates + (size_t)row0 * GH : nullptr,
+                        STASH && a.st_ahn ? a.st_ahn + (size_t)row0 * H : nullptr,
                         a.hstate + ((size_t)k * B + row0) * H, d.G == 4 ? a.cstate + ((size_t)k * B + row0) * H : nullptr,
-                        nullptr);
+                        STASH ? a.st_o + (size_t)row0 * d.Co : nullptr);
       // inverse coupling (models.py:358-366): z2 = z2 / scale - shift
       const float *orow = sm + sp.orow;
       for (int r = warp; r < R; r += NT / 32) {
@@ -311,6 +314,11 @@ __global__ void __launch_bounds__(NT) core_inv_persistent(InvArgs a) {
       }
       // 1x1 conv inverse then ActNorm inverse (modules.py:175-177, 189-193, 76-78)
       tile_gemm<RPT>(xs, w.Winv, d.Cp, C, C, sm + sp.wst, [&](int r, int j, float v) {
+        if (STASH && r < nrows) {  // xs = zc is complete and unchanged while the product runs ([B][C] of one step: int offsets)
+          const int o = (row0 + r) * C + j;
+          a.st_zc[o] = xs[j * RS + r];
+          a.st_x1[o] = v;
+        }
         const float x = v * expf(-w.an_logs[j]) - w.an_bias[j];
         zrow[r * pC + j] = x;
         if (j < Ci) zact[j * RS + r] = x;
@@ -426,8 +434,9 @@ int launch_fwd(const FwdArgs &a, cudaStream_t st) {
 template <int RPT> static int launch_inv_t(const InvArgs &a, cudaStream_t st) {
   constexpr int R = Tile<RPT>::R;
   const int bytes = plan_smem(a.d, R, false, a.cstatic != nullptr).total * (int)sizeof(float);
-  LFI_CUDA(cudaFuncSetAttribute(core_inv_persistent<RPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  core_inv_persistent<RPT><<<(a.B + R - 1) / R, NT, bytes, st>>>(a);
+  auto kern = a.st_x1 ? core_inv_persistent<RPT, true> : core_inv_persistent<RPT, false>;
+  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  kern<<<(a.B + R - 1) / R, NT, bytes, st>>>(a);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -74,7 +74,9 @@ __device__ __forceinline__ void bulk_load(float *dst, const float *src, unsigned
                : "memory");
 }
 
-template <int RR>
+// STASH: also store the activations of the step (InvArgs.st_x1 ...; one frame, one step); the instantiation without it is the
+// plain inverse
+template <int RR, bool STASH>
 __global__ void core_inv_rows(InvArgs a) {
   extern __shared__ __align__(16) float sm[];
   const Dims &d = a.d;
@@ -192,6 +194,11 @@ __global__ void core_inv_rows(InvArgs a) {
         const float hn = ng + ug * (hp - ng);
         hs[m * RR + r] = hn;
         if (r < nrows) a.hstate[((size_t)k * B + row0 + r) * H + m] = hn;
+        if (STASH && r < nrows) {
+          float *g = a.st_gates + (size_t)(row0 + r) * GH;
+          g[m] = rg; g[H + m] = ug; g[2 * H + m] = ng;
+          a.st_ahn[(size_t)(row0 + r) * H + m] = sh[2 * H + m];
+        }
       }
       __syncthreads();
       // ---- 3. LinearZeros (modules.py:93-95): reduction split over 4 thread groups --------------------------------------
@@ -235,8 +242,21 @@ __global__ void core_inv_rows(InvArgs a) {
           v = z2 - osum(q);
         }
         xs[(Ci + q) * RR + r] = v;
+        if (STASH && r < nrows) a.st_zc[(size_t)(row0 + r) * C + Ci + q] = v;
       }
-      for (int e = tid; e < RR * Ci; e += NTH) { const int r = e / Ci, c = e - r * Ci; xs[c * RR + r] = zs[c * RR + r]; }
+      for (int e = tid; e < RR * Ci; e += NTH) {
+        const int r = e / Ci, c = e - r * Ci;
+        xs[c * RR + r] = zs[c * RR + r];
+        if (STASH && r < nrows) a.st_zc[(size_t)(row0 + r) * C + c] = zs[c * RR + r];
+      }
+      // o as a loop of its own: a stored product inside the loop above would no longer contract into its FMAs, and the
+      // coupling output would differ in the last bit from the plain instantiation's
+      if (STASH)
+        for (int e = tid; e < nrows * Co; e += NTH) {
+          const int r = e / Co, jj = e - r * Co;
+          a.st_o[(size_t)(row0 + r) * Co + jj] = (part[(0 * RR + r) * Cm + jj] + part[(1 * RR + r) * Cm + jj] + part[(2 * RR + r) * Cm + jj] +
+                                                  part[(3 * RR + r) * Cm + jj] + bfs[jj]) * e3[jj];
+        }
       __syncthreads();
       // ---- 5. 1x1 conv inverse, ActNorm inverse (modules.py:175-177, 189-193, 76-78) ----------------------------------------
       {
@@ -265,6 +285,7 @@ __global__ void core_inv_rows(InvArgs a) {
       for (int e = tid; e < RR * C; e += NTH) {
         const int r = e / C, c = e - r * C;
         const float v = part[(0 * RR + r) * Cm + c] + part[(1 * RR + r) * Cm + c] + part[(2 * RR + r) * Cm + c] + part[(3 * RR + r) * Cm + c];
+        if (STASH && r < nrows) a.st_x1[(size_t)(row0 + r) * C + c] = v;
         zs[c * RR + r] = v * einv[c] - anb[c];
       }
       __syncthreads();
@@ -293,8 +314,9 @@ bool inv_rows_supported(const InvArgs &a) {
 
 template <int RR> static int launch_inv_rows_t(const InvArgs &a, cudaStream_t st) {
   const int bytes = plan_rows(a.d, RR).total * (int)sizeof(float);
-  if (bytes > 48 * 1024) LFI_CUDA(cudaFuncSetAttribute(core_inv_rows<RR>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  core_inv_rows<RR><<<(a.B + RR - 1) / RR, round_up(a.d.GH, 32), bytes, st>>>(a);
+  auto kern = a.st_x1 ? core_inv_rows<RR, true> : core_inv_rows<RR, false>;
+  if (bytes > 48 * 1024) LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  kern<<<(a.B + RR - 1) / RR, round_up(a.d.GH, 32), bytes, st>>>(a);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

@@ -125,6 +125,27 @@ struct Bump {
   bool ok() const { return base == nullptr || off <= cap; }
 };
 
+// ---- module API: activations of one FlowStep.forward call on [B] rows (caller-owned, opaque, lfi_flowstep_stash_bytes) ----
+// Forward direction (lfi_flowstep_fwd_train): y = ActNorm output, zf = 1x1 conv output.  Reverse direction
+// (lfi_flowstep_rev_fwd_train): y = x1 = zc W^-1 (input of the reverse ActNorm), zf = zc (coupling output).  Both: Cact = the
+// cond_transform output, h / c = the new state, gates / ahn / o as the flow-core stash (core::Stash).
+struct StepStash {
+  float *Cact, *y, *zf, *h, *c, *gates, *ahn, *o;
+  size_t bytes;
+};
+inline void plan_step_stash(const Dims &d, int B, void *base, StepStash *s) {
+  Bump b(base, 0);
+  s->Cact = b.take<float>((size_t)B * d.D);
+  s->y = b.take<float>((size_t)B * d.C);
+  s->zf = b.take<float>((size_t)B * d.C);
+  s->h = b.take<float>((size_t)B * d.H);
+  s->c = b.take<float>((size_t)B * d.H);
+  s->gates = b.take<float>((size_t)B * d.GH);
+  s->ahn = b.take<float>((size_t)B * d.H);
+  s->o = b.take<float>((size_t)B * d.Co);
+  s->bytes = round_up_sz(b.off, 256);
+}
+
 // ---- generic GEMM (gemm_simt.cu / gemm_tc.cu) ---------------------------------------------------
 // bf16 operand planes of the tensor-core modes: value = hi (+ lo in the split-bf16 x3 mode); layout as the fp32
 // operand they stand for (same rows / cols / transposition), pitch ld in elements (multiple of 8), 16-byte aligned.

@@ -1,5 +1,7 @@
 // Stand-alone module API under autograd: the backward passes of ActNorm2d / InvertibleConv1x1 / LinearZeros
-// (modules.py:45-95, 122-194) and f_seq.forward with its backward (models.py:148-214), each on its own parameters.
+// (modules.py:45-95, 122-194) and f_seq.forward with its backward (models.py:148-214), each on its own parameters; and the
+// backward of FlowStep.forward in the reverse direction (FlowStep.reverse_flow, models.py:345-373) on one step of a flat
+// parameter block.
 //
 // Every reduction over the B rows is deterministic: one CTA owns 32 columns and all rows of them, its 8 row groups sum in
 // a fixed order and are combined in a fixed order (no atomics), and the weight-gradient GEMMs write their output tiles
@@ -8,6 +10,8 @@
 #include "lfi_common.cuh"
 
 namespace lfi {
+const float *derived_winv(const Dims &d, const void *derived, int k);  // seq.cu
+
 namespace {
 
 // ---- column-reduction kernels -------------------------------------------------------------------
@@ -256,6 +260,121 @@ bool fseq_params_ok(const lfi_fseq_params *p) {
   return p && p->wc && p->bc && p->w_ih && p->b_ih && p->w_hh && p->b_hh && p->wf && p->bf && p->lf;
 }
 
+// Backward of f_seq on B rows (lfi_fseq_bwd, and the coupling network inside lfi_flowstep_rev_bwd), arguments checked by the
+// caller.  z has row pitch z_ld; dz (nullable) has row pitch dz_ld and is written (dz_epi = 0) or added to (LFI_EPI_ACCUM_PRE:
+// no split-K, unlike LFI_EPI_ACCUM).
+int fseq_bwd_rows(const FseqDims &d, const lfi_fseq_params *p, const float *z, int z_ld, const float *cond, const float *h_in,
+                  const float *c_in, const float *dout, const float *dh_out, const float *dc_out, float *dz, int dz_ld, int dz_epi,
+                  float *dcond, float *dh_in, float *dc_in, lfi_fseq_params *g, int B, const FseqStash &q, const FseqBwdWs &w,
+                  cudaStream_t st) {
+  const int GH = d.GH, In = d.In, D = d.D, H = d.H, F = d.F, Out = d.Out, Wl = In + D;
+  // LinearZeros: g = dout e^{f logs}, db_f, dlogs (one pass), dW_f = g^T h', dh' = g W_f
+  ColJobs j;
+  memset(&j, 0, sizeof(j));
+  j.j[0] = col_job(dout, B, Out, Out, g->bf);
+  j.j[0].b = q.out; j.j[0].v = p->lf; j.j[0].o = w.g; j.j[0].s2 = g->lf; j.j[0].f = d.lf;
+  LFI_TRY(launch_colgrad<COL_LINZ>(j, 1, st));
+  LFI_TRY(gemm32(1, 0, Out, H, B, w.g, Out, q.h, H, g->wf, H, 0, nullptr, st));
+  LFI_TRY(gemm32(0, 0, B, H, Out, w.g, Out, p->wf, H, w.dh, H, 0, nullptr, st));
+  // cell backward: gate gradients, the direct part of dh_in, dc_in
+  CellBwd a;
+  memset(&a, 0, sizeof(a));
+  a.act = q.act; a.ahn = q.ahn; a.c_st = q.c; a.h_prev = h_in; a.c_prev = c_in; a.dh = w.dh; a.dh_ext = dh_out;
+  a.dc_ext = d.G == 4 ? dc_out : nullptr; a.dai = w.dai; a.dah = w.dah; a.dh_dir = dh_in; a.dc_prev = d.G == 4 ? dc_in : nullptr;
+  a.B = B; a.H = H; a.G = d.G;
+  cell_bwd_kernel<<<grid_for((size_t)B * H), 256, 0, st>>>(a);
+  LFI_LAUNCH_CHECK();
+  if (dh_in) LFI_TRY(gemm32(0, 0, B, H, GH, w.dah, GH, p->w_hh, H, dh_in, H, LFI_EPI_ACCUM_PRE, nullptr, st));
+  if (h_in) LFI_TRY(gemm32(1, 0, GH, H, B, w.dah, GH, h_in, H, g->w_hh, H, 0, nullptr, st));
+  else LFI_CUDA(cudaMemsetAsync(g->w_hh, 0, (size_t)GH * H * sizeof(float), st));
+  // gate-ih product over [z | c]: dW_ih in two column blocks, dz, and dc through LeakyReLU'
+  LFI_TRY(gemm32(1, 0, GH, In, B, w.dai, GH, z, z_ld, g->w_ih, Wl, 0, nullptr, st));
+  LFI_TRY(gemm32(1, 0, GH, D, B, w.dai, GH, q.cact, D, g->w_ih + In, Wl, 0, nullptr, st));
+  if (dz) LFI_TRY(gemm32(0, 0, B, In, GH, w.dai, GH, p->w_ih, Wl, dz, dz_ld, dz_epi, nullptr, st));
+  LFI_TRY(gemm32(0, 0, B, D, GH, w.dai, GH, p->w_ih + In, Wl, w.dc, D, LFI_EPI_LRELU_BWD, nullptr, st, q.cact, D));
+  // bias gradients: db_ih = sum dai, db_hh = sum dah, db_c = sum dc (one launch)
+  memset(&j, 0, sizeof(j));
+  j.j[0] = col_job(w.dai, B, GH, GH, g->b_ih);
+  j.j[1] = col_job(w.dah, B, GH, GH, g->b_hh);
+  j.j[2] = col_job(w.dc, B, D, D, g->bc);
+  LFI_TRY(launch_colgrad<COL_SUM>(j, 3, st));
+  // cond_transform: dW_c = dc^T cond, dcond = dc W_c
+  LFI_TRY(gemm32(1, 0, D, F, B, w.dc, D, cond, F, g->wc, F, 0, nullptr, st));
+  if (dcond) LFI_TRY(gemm32(0, 0, B, F, D, w.dc, D, p->wc, F, dcond, F, 0, nullptr, st));
+  return LFI_OK;
+}
+
+// ---- FlowStep.reverse_flow backward -------------------------------------------------------------
+// Backward of the inverse coupling (models.py:358-366) on [B] rows, one thread per (row, channel pair q < Cz) that also
+// passes column q < Ci through.  zc = [z1 | zc2] [B][C] and o [B][Co] (after its exp(3 logs) scale) come from the stash,
+// dzc [B][C] = dL/dzc, dld [B] = dL/d(logdet) (nullable).
+//   affine:   (shift, a) = (o[:, 0::2], o[:, 1::2]), s = max(sigmoid(a + 2), eps), zc2 = z2 / s - shift, ld -= sum log s
+//   additive: zc2 = z2 - o
+// z2 / s is recovered as zc2 + shift.  Writes dx [B][C] = (dL/dzc1, dL/dz2) - the f_seq path adds its dz1 to the first block
+// later - and dO [B][Co] = dL/do (interleaved like o; the clamp passes the gradient where sigmoid(a + 2) >= eps, as torch's
+// clamp does), and leaves dzc negated in place: the operand of dW = x1^T (-dzc).
+__global__ void __launch_bounds__(256) coupling_rev_bwd_kernel(const float *zc, const float *o, float *dzc, const float *dld,
+                                                                float *dx, float *dO, int B, int C, int Ci, int Co, int affine,
+                                                                float eps) {
+  const int Cz = C - Ci;
+  const size_t n = (size_t)B * Cz;
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+    const int b = (int)(e / Cz), q = (int)(e % Cz);
+    const size_t r = (size_t)b * C;
+    if (q < Ci) {
+      const float g1 = dzc[r + q];
+      dx[r + q] = g1;
+      dzc[r + q] = -g1;
+    }
+    const float g = dzc[r + Ci + q];
+    float *dOr = dO + (size_t)b * Co;
+    if (affine) {
+      const float shift = o[(size_t)b * Co + 2 * q], sg = sigm(o[(size_t)b * Co + 2 * q + 1] + 2.0f);
+      const float s = fmaxf(sg, eps);
+      const float ds = -(g * (zc[r + Ci + q] + shift) + (dld ? dld[b] : 0.f)) / s;
+      dOr[2 * q] = -g;
+      dOr[2 * q + 1] = sg >= eps ? ds * sg * (1.f - sg) : 0.f;
+      dx[r + Ci + q] = g / s;
+    } else {
+      dOr[q] = -g;
+      dx[r + Ci + q] = g;
+    }
+    dzc[r + Ci + q] = -g;
+  }
+}
+
+struct RevBwdWs {
+  float *dx1, *dzc, *dO;
+  FseqBwdWs f;
+  size_t bytes;
+};
+void plan_rev_bwd_ws(const Dims &d, const FseqDims &fd, int B, void *base, RevBwdWs *w) {
+  Bump b(base, 0);
+  w->dx1 = b.take<float>((size_t)B * d.C);
+  w->dzc = b.take<float>((size_t)B * d.C);
+  w->dO = b.take<float>((size_t)B * d.Co);
+  const size_t off = round_up_sz(b.off, 256);
+  plan_fseq_bwd_ws(fd, B, base ? (char *)base + off : nullptr, &w->f);
+  w->bytes = off + w->f.bytes;
+}
+
+// f_seq of step k: its shape, and its parameters (or their gradients) inside a flat [K, ...] block
+FseqDims step_fseq_dims(const Dims &d) {
+  FseqDims f;
+  f.In = d.Ci; f.Out = d.Co; f.H = d.H; f.D = d.D; f.F = d.F; f.G = d.G; f.GH = d.GH; f.lf = 3.0f;
+  return f;
+}
+template <class P>
+lfi_fseq_params step_fseq_params(const Dims &d, P *p, int k) {
+  const size_t GH = d.GH, In = d.Ci + d.D;
+  lfi_fseq_params f;
+  f.wc = p->wc + (size_t)k * d.D * d.F; f.bc = p->bc + (size_t)k * d.D;
+  f.w_ih = p->w_ih + k * GH * In; f.b_ih = p->b_ih + k * GH;
+  f.w_hh = p->w_hh + k * GH * d.H; f.b_hh = p->b_hh + k * GH;
+  f.wf = p->wf + (size_t)k * d.Co * d.H; f.bf = p->bf + (size_t)k * d.Co; f.lf = p->lf + (size_t)k * d.Co;
+  return f;
+}
+
 }  // namespace
 
 // Bias gradients of an encoder GRU from the per-block partial sums of aux::enc_gate_bwd2 (part [rows][4E]: r, u, n, n*r blocks of
@@ -387,41 +506,61 @@ int lfi_fseq_bwd(const lfi_fseq_shape *s, const lfi_fseq_params *p, const float 
   FseqBwdWs w;
   plan_fseq_bwd_ws(d, B, ws, &w);
   LFI_REQUIRE(ws_bytes >= w.bytes, LFI_ERR_WORKSPACE, "lfi_fseq_bwd: workspace too small: %zu < %zu", ws_bytes, w.bytes);
-  const int GH = d.GH, In = d.In, D = d.D, H = d.H, F = d.F, Out = d.Out, Wl = In + D;
-  // LinearZeros: g = dout e^{f logs}, db_f, dlogs (one pass), dW_f = g^T h', dh' = g W_f
+  return fseq_bwd_rows(d, p, z, d.In, cond, h_in, c_in, dout, dh_out, dc_out, dz, d.In, 0, dcond, dh_in, dc_in, g, B, q, w, st);
+}
+
+size_t lfi_flowstep_rev_bwd_ws_bytes(const lfi_shape *s, int B) {
+  Dims d;
+  if (make_dims(s, &d) != LFI_OK || B < 1) return 0;
+  RevBwdWs w;
+  plan_rev_bwd_ws(d, step_fseq_dims(d), B, nullptr, &w);
+  return w.bytes;
+}
+
+int lfi_flowstep_rev_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, int k, const float *cond, const float *h_in,
+                         const float *c_in, const float *dy, const float *dlogdet, const float *dh_out, const float *dc_out, float *dx,
+                         float *dcond, float *dh_in, float *dc_in, lfi_params *g, int B, void *stash, size_t stash_bytes, void *ws,
+                         size_t ws_bytes, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  Dims d;
+  LFI_TRY(make_dims(s, &d));
+  LFI_REQUIRE(derived && p && cond && dy && dx && dcond && dh_in && g && stash && ws, LFI_ERR_ARG, "lfi_flowstep_rev_bwd: null argument");
+  LFI_REQUIRE(p->an_logs && p->wc && p->bc && p->w_ih && p->b_ih && p->w_hh && p->b_hh && p->wf && p->bf && p->lf, LFI_ERR_ARG,
+              "lfi_flowstep_rev_bwd: null parameter block");
+  LFI_REQUIRE(g->an_bias && g->an_logs && g->w && g->wc && g->bc && g->w_ih && g->b_ih && g->w_hh && g->b_hh && g->wf && g->bf && g->lf,
+              LFI_ERR_ARG, "lfi_flowstep_rev_bwd: null gradient block");
+  LFI_REQUIRE(k >= 0 && k < d.K && B >= 1, LFI_ERR_ARG, "lfi_flowstep_rev_bwd: bad step %d / batch %d", k, B);
+  LFI_REQUIRE(d.G == 3 || dc_in, LFI_ERR_ARG, "lfi_flowstep_rev_bwd: LSTM needs dc_in");
+  StepStash q;
+  plan_step_stash(d, B, stash, &q);
+  LFI_REQUIRE(stash_bytes >= q.bytes, LFI_ERR_WORKSPACE, "flowstep stash too small: %zu < %zu", stash_bytes, q.bytes);
+  const FseqDims fd = step_fseq_dims(d);
+  RevBwdWs w;
+  plan_rev_bwd_ws(d, fd, B, ws, &w);
+  LFI_REQUIRE(ws_bytes >= w.bytes, LFI_ERR_WORKSPACE, "flowstep reverse backward workspace too small: %zu < %zu", ws_bytes, w.bytes);
+  const int C = d.C;
+  const size_t kC = (size_t)k * C;
+  // 1. reverse ActNorm, out = x1 e^{-logs} - bias: dx1, d bias, d logs (one pass)
   ColJobs j;
   memset(&j, 0, sizeof(j));
-  j.j[0] = col_job(dout, B, Out, Out, g->bf);
-  j.j[0].b = q.out; j.j[0].v = p->lf; j.j[0].o = w.g; j.j[0].s2 = g->lf; j.j[0].f = d.lf;
-  LFI_TRY(launch_colgrad<COL_LINZ>(j, 1, st));
-  LFI_TRY(gemm32(1, 0, Out, H, B, w.g, Out, q.h, H, g->wf, H, 0, nullptr, st));
-  LFI_TRY(gemm32(0, 0, B, H, Out, w.g, Out, p->wf, H, w.dh, H, 0, nullptr, st));
-  // cell backward: gate gradients, the direct part of dh_in, dc_in
-  CellBwd a;
-  memset(&a, 0, sizeof(a));
-  a.act = q.act; a.ahn = q.ahn; a.c_st = q.c; a.h_prev = h_in; a.c_prev = c_in; a.dh = w.dh; a.dh_ext = dh_out;
-  a.dc_ext = d.G == 4 ? dc_out : nullptr; a.dai = w.dai; a.dah = w.dah; a.dh_dir = dh_in; a.dc_prev = d.G == 4 ? dc_in : nullptr;
-  a.B = B; a.H = H; a.G = d.G;
-  cell_bwd_kernel<<<grid_for((size_t)B * H), 256, 0, st>>>(a);
+  j.j[0] = col_job(dy, B, C, C, g->an_bias + kC);
+  j.j[0].b = q.y; j.j[0].v = p->an_logs + kC; j.j[0].o = w.dx1; j.j[0].s2 = g->an_logs + kC;
+  LFI_TRY(launch_colgrad<COL_ACTNORM_REV>(j, 1, st));
+  // 2. inverse 1x1 conv, x1 = zc W^-1: dzc = dx1 W^-T
+  LFI_TRY(gemm32(0, 1, B, C, C, w.dx1, C, derived_winv(d, derived, k), d.Cp, w.dzc, C, 0, nullptr, st));
+  // 3. inverse coupling: dO, dL/dz2, the pass-through dL/dz1 (and -dzc for step 5)
+  coupling_rev_bwd_kernel<<<grid_for((size_t)B * d.Cz), 256, 0, st>>>(q.zf, q.o, w.dzc, dlogdet, dx, w.dO, B, C, d.Ci, d.Co, d.affine,
+                                                                      d.eps);
   LFI_LAUNCH_CHECK();
-  if (dh_in) LFI_TRY(gemm32(0, 0, B, H, GH, w.dah, GH, p->w_hh, H, dh_in, H, LFI_EPI_ACCUM_PRE, nullptr, st));
-  if (h_in) LFI_TRY(gemm32(1, 0, GH, H, B, w.dah, GH, h_in, H, g->w_hh, H, 0, nullptr, st));
-  else LFI_CUDA(cudaMemsetAsync(g->w_hh, 0, (size_t)GH * H * sizeof(float), st));
-  // gate-ih product over [z | c]: dW_ih in two column blocks, dz, and dc through LeakyReLU'
-  LFI_TRY(gemm32(1, 0, GH, In, B, w.dai, GH, z, In, g->w_ih, Wl, 0, nullptr, st));
-  LFI_TRY(gemm32(1, 0, GH, D, B, w.dai, GH, q.cact, D, g->w_ih + In, Wl, 0, nullptr, st));
-  if (dz) LFI_TRY(gemm32(0, 0, B, In, GH, w.dai, GH, p->w_ih, Wl, dz, In, 0, nullptr, st));
-  LFI_TRY(gemm32(0, 0, B, D, GH, w.dai, GH, p->w_ih + In, Wl, w.dc, D, LFI_EPI_LRELU_BWD, nullptr, st, q.cact, D));
-  // bias gradients: db_ih = sum dai, db_hh = sum dah, db_c = sum dc (one launch)
-  memset(&j, 0, sizeof(j));
-  j.j[0] = col_job(w.dai, B, GH, GH, g->b_ih);
-  j.j[1] = col_job(w.dah, B, GH, GH, g->b_hh);
-  j.j[2] = col_job(w.dc, B, D, D, g->bc);
-  LFI_TRY(launch_colgrad<COL_SUM>(j, 3, st));
-  // cond_transform: dW_c = dc^T cond, dcond = dc W_c
-  LFI_TRY(gemm32(1, 0, D, F, B, w.dc, D, cond, F, g->wc, F, 0, nullptr, st));
-  if (dcond) LFI_TRY(gemm32(0, 0, B, F, D, w.dc, D, p->wc, F, dcond, F, 0, nullptr, st));
-  return LFI_OK;
+  // 4. f_seq on z1 = zc[:, :Ci] with step k's parameters; its dz1 is added to dx[:, :Ci]
+  FseqStash fq;
+  fq.cact = q.Cact; fq.act = q.gates; fq.ahn = q.ahn; fq.h = q.h; fq.c = q.c; fq.out = q.o; fq.bytes = q.bytes;
+  const lfi_fseq_params fp = step_fseq_params(d, p, k);
+  lfi_fseq_params fg = step_fseq_params(d, g, k);
+  LFI_TRY(fseq_bwd_rows(fd, &fp, q.zf, C, cond, h_in, c_in, w.dO, dh_out, dc_out, dx, C, LFI_EPI_ACCUM_PRE, dcond, dh_in, dc_in, &fg, B,
+                        fq, w.f, st));
+  // 5. dW of the forward weight: with Winv = W^-1, dW = -W^-T (zc^T dx1) W^-T = -(zc W^-1)^T (dx1 W^-T) = x1^T (-dzc)
+  return gemm32(1, 0, C, C, B, q.y, C, w.dzc, C, g->w + (size_t)k * C * C, C, 0, nullptr, st);
 }
 
 }  // extern "C"

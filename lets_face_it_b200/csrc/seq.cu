@@ -55,6 +55,11 @@ static core::DerivedView make_view(const Dims &d, const void *derived, const lfi
   return v;
 }
 
+// W^-1 of step k in the derived cache, [C] rows of pitch Cp (written by lfi_derive with winv); read by lfi_flowstep_rev_bwd
+const float *derived_winv(const Dims &d, const void *derived, int k) {
+  return (const float *)derived + derived_layout(d).Winv + (size_t)k * d.C * d.Cp;
+}
+
 static int derive_impl(const lfi_shape *s, const lfi_params *p, const float *winv, void *derived, cudaStream_t st) {
   Dims d;
   LFI_TRY(make_dims(s, &d));
@@ -1104,10 +1109,13 @@ size_t lfi_flowstep_ws_bytes(const lfi_shape *s, int B) {
   return round_up_sz(b.off, 256) + 256;
 }
 
-int lfi_flowstep(const lfi_shape *s, const void *derived, const lfi_params *p, int k, int reverse, const float *x,
-                 const float *cond, const float *h_in, const float *c_in, float *h_out, float *c_out, float *y,
-                 float *logdet, float *scale_out, int B, void *ws, size_t ws_bytes, void *stream) {
-  cudaStream_t st = (cudaStream_t)stream;
+}  // extern "C"
+
+// lfi_flowstep; q (reverse direction only, lfi_flowstep_rev_fwd_train): also fill that stash.  The stash changes where the
+// cond_transform output lives and which kernel instantiation runs, not what is computed.
+static int flowstep_impl(const lfi_shape *s, const void *derived, const lfi_params *p, int k, int reverse, const float *x,
+                         const float *cond, const float *h_in, const float *c_in, float *h_out, float *c_out, float *y,
+                         float *logdet, float *scale_out, int B, void *ws, size_t ws_bytes, const StepStash *q, cudaStream_t st) {
   Dims d;
   LFI_TRY(make_dims(s, &d));
   LFI_REQUIRE(derived && p && x && cond && h_out && y && logdet && ws, LFI_ERR_ARG, "lfi_flowstep: null argument");
@@ -1116,6 +1124,7 @@ int lfi_flowstep(const lfi_shape *s, const void *derived, const lfi_params *p, i
   LFI_REQUIRE(ws_bytes >= lfi_flowstep_ws_bytes(s, B), LFI_ERR_WORKSPACE, "flowstep workspace too small");
   Bump b(ws, ws_bytes);
   float *Cact = b.take<float>((size_t)B * d.D);
+  if (q) Cact = q->Cact;
   float *G = b.take<float>((size_t)B * d.GH);
   float *xin = b.take<float>((size_t)B * d.C * 2);
   float *ldtmp = b.take<float>((size_t)B);
@@ -1156,10 +1165,24 @@ int lfi_flowstep(const lfi_shape *s, const void *derived, const lfi_params *p, i
   a.faces_out = y; a.fo_sb = d.C; a.fo_st = 0;
   a.hstate = h_out - koffH; a.cstate = c_out ? c_out - koffH : nullptr;
   a.logdet_out = ldtmp;
+  if (q) { a.st_x1 = q->y; a.st_zc = q->zf; a.st_gates = q->gates; a.st_ahn = d.G == 3 ? q->ahn : nullptr; a.st_o = q->o; }
   LFI_TRY(core::launch_inv(a, st));
+  if (q) {
+    LFI_CUDA(cudaMemcpyAsync(q->h, h_out, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (d.G == 4) LFI_CUDA(cudaMemcpyAsync(q->c, c_out, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  }
   // logdet += (-sum log s) computed by the kernel
   LFI_TRY(aux::colsum(logdet, ldtmp, B, 1, B, 1.0f, st));
   return LFI_OK;
+}
+
+extern "C" {
+
+int lfi_flowstep(const lfi_shape *s, const void *derived, const lfi_params *p, int k, int reverse, const float *x,
+                 const float *cond, const float *h_in, const float *c_in, float *h_out, float *c_out, float *y,
+                 float *logdet, float *scale_out, int B, void *ws, size_t ws_bytes, void *stream) {
+  return flowstep_impl(s, derived, p, k, reverse, x, cond, h_in, c_in, h_out, c_out, y, logdet, scale_out, B, ws, ws_bytes, nullptr,
+                       (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1286,26 +1309,8 @@ int lfi_gemm(int mode, int transA, int transB, int M, int N, int Kd, const float
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------
-// FlowStep.forward with autograd (module API): forward with a stash, and the backward of one cell.
-namespace lfi {
-struct StepStash {  // caller-owned, opaque: activations of one FlowStep.forward call on [B] rows
-  float *Cact, *y, *zf, *h, *c, *gates, *ahn, *o;
-  size_t bytes;
-};
-static void plan_step_stash(const Dims &d, int B, void *base, StepStash *s) {
-  Bump b(base, 0);
-  s->Cact = b.take<float>((size_t)B * d.D);
-  s->y = b.take<float>((size_t)B * d.C);
-  s->zf = b.take<float>((size_t)B * d.C);
-  s->h = b.take<float>((size_t)B * d.H);
-  s->c = b.take<float>((size_t)B * d.H);
-  s->gates = b.take<float>((size_t)B * d.GH);
-  s->ahn = b.take<float>((size_t)B * d.H);
-  s->o = b.take<float>((size_t)B * d.Co);
-  s->bytes = round_up_sz(b.off, 256);
-}
-}  // namespace lfi
-
+// FlowStep.forward with autograd (module API): forward with a stash (lfi_flowstep_rev_fwd_train: the reverse direction), and the
+// backward of one cell (the reverse direction's backward, lfi_flowstep_rev_bwd, is in module_grad.cu).
 extern "C" {
 
 size_t lfi_flowstep_stash_bytes(const lfi_shape *s, int B) {
@@ -1370,6 +1375,20 @@ int lfi_flowstep_fwd_train(const lfi_shape *s, const void *derived, const lfi_pa
   LFI_CUDA(cudaMemcpyAsync(h_out, q.h, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
   if (d.G == 4) LFI_CUDA(cudaMemcpyAsync(c_out, q.c, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return LFI_OK;
+}
+
+int lfi_flowstep_rev_fwd_train(const lfi_shape *s, const void *derived, const lfi_params *p, int k, const float *x, const float *cond,
+                               const float *h_in, const float *c_in, float *h_out, float *c_out, float *y, float *logdet, int B,
+                               void *stash, size_t stash_bytes, void *ws, size_t ws_bytes, void *stream) {
+  Dims d;
+  LFI_TRY(make_dims(s, &d));
+  LFI_REQUIRE(stash, LFI_ERR_ARG, "lfi_flowstep_rev_fwd_train: null stash");
+  LFI_REQUIRE(B >= 1, LFI_ERR_ARG, "lfi_flowstep_rev_fwd_train: bad batch %d", B);
+  StepStash q;
+  plan_step_stash(d, B, stash, &q);
+  LFI_REQUIRE(stash_bytes >= q.bytes, LFI_ERR_WORKSPACE, "flowstep stash too small: %zu < %zu", stash_bytes, q.bytes);
+  return flowstep_impl(s, derived, p, k, 1, x, cond, h_in, c_in, h_out, c_out, y, logdet, nullptr, B, ws, ws_bytes, &q,
+                       (cudaStream_t)stream);
 }
 
 int lfi_flowstep_bwd(const lfi_shape *s, const void *derived, const lfi_params *p, int k, const float *cond, const float *h_in,

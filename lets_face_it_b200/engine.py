@@ -554,12 +554,12 @@ class Engine:
                 "wf": Co * H, "bf": Co, "lf": Co}
 
     @_on_own_device
-    def flowstep_train(self, k, x, cond, h_in, c_in, want_scale=False, refresh=True):
-        """Forward of one FlowStep on one frame WITH the stash `flowstep_backward` needs (lfi_flowstep_fwd_train).
-        Returns (y, ld [B] coupling log-det term, h_out, c_out, scale, stash).  refresh=False: the derived cache is current
-        (FlowNet.encode rebuilds it once per call)."""
+    def flowstep_train(self, k, x, cond, h_in, c_in, want_scale=False, refresh=True, reverse=False):
+        """Forward of one FlowStep on one frame WITH the stash `flowstep_backward` needs (lfi_flowstep_fwd_train; reverse=True:
+        lfi_flowstep_rev_fwd_train, which has no scale).  Returns (y, ld [B] coupling log-det term, h_out, c_out, scale, stash).
+        refresh=False: the derived cache is current (FlowNet.encode / decode rebuild it once per call)."""
         if refresh:
-            self.refresh(False)
+            self.refresh(reverse)
         L, st = cabi.lib(), cabi.stream_ptr()
         P = self._params_struct(self.theta, self.W)
         dev = self.theta.device
@@ -574,9 +574,15 @@ class Engine:
         h_out = torch.empty(B, self.H, dtype=torch.float32, device=dev)
         c_out = torch.empty(B, self.H, dtype=torch.float32, device=dev) if self.G == 4 else None
         ld = torch.zeros(B, dtype=torch.float32, device=dev)
-        scale = torch.empty(B, self.Cz, dtype=torch.float32, device=dev) if (want_scale and self.affine) else None
+        scale = torch.empty(B, self.Cz, dtype=torch.float32, device=dev) if (want_scale and self.affine and not reverse) else None
         stash = torch.empty(L.lfi_flowstep_stash_bytes(ctypes.byref(self.shape), B), dtype=torch.uint8, device=dev)
         ws = self._workspace(("step", B), L.lfi_flowstep_ws_bytes(ctypes.byref(self.shape), B))
+        if reverse:
+            cabi.check(L.lfi_flowstep_rev_fwd_train(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), k, x.data_ptr(),
+                                                    cond.data_ptr(), cabi.ptr(h_in), cabi.ptr(c_in), h_out.data_ptr(), cabi.ptr(c_out),
+                                                    y.data_ptr(), ld.data_ptr(), B, stash.data_ptr(), stash.numel(), ws.data_ptr(), ws.numel(),
+                                                    st), "lfi_flowstep_rev_fwd_train")
+            return y, ld, h_out, c_out, scale, (stash, cond, h_in, c_in)
         cabi.check(L.lfi_flowstep_fwd_train(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), k, x.data_ptr(), cond.data_ptr(),
                                             cabi.ptr(h_in), cabi.ptr(c_in), h_out.data_ptr(), c_out.data_ptr() if c_out is not None else None,
                                             y.data_ptr(), ld.data_ptr(), scale.data_ptr() if scale is not None else None, B,
@@ -584,9 +590,10 @@ class Engine:
         return y, ld, h_out, c_out, scale, (stash, cond, h_in, c_in)
 
     @_on_own_device
-    def flowstep_backward(self, k, saved, dy, dld, dh_out, dc_out):
-        """Backward of `flowstep_train` (lfi_flowstep_bwd).  Returns (dx, dcond, dh_in, dc_in, grads) with grads a dict
-        block name -> gradient tensor of step k's block (dW of the composed 1x1 weight under "w")."""
+    def flowstep_backward(self, k, saved, dy, dld, dh_out, dc_out, reverse=False):
+        """Backward of `flowstep_train` (lfi_flowstep_bwd; reverse=True: lfi_flowstep_rev_bwd).  Returns (dx, dcond, dh_in, dc_in,
+        grads) with grads a dict block name -> gradient tensor of step k's block (dW of the composed 1x1 weight under "w", in both
+        directions)."""
         L, st = cabi.lib(), cabi.stream_ptr()
         stash, cond, h_in, c_in = saved
         dev = self.theta.device
@@ -608,11 +615,12 @@ class Engine:
         G = cabi.Params()
         for n in self._STEP_GRAD_BLOCKS:  # the C side indexes [K, ...] blocks: base moved back by k blocks
             setattr(G, n, gbuf.data_ptr() + 4 * offs[n] - 4 * k * numel[n])
-        ws = self._workspace(("stepbwd", B), L.lfi_flowstep_bwd_ws_bytes(ctypes.byref(self.shape), B))
-        cabi.check(L.lfi_flowstep_bwd(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), k, cond.data_ptr(), cabi.ptr(h_in),
-                                      cabi.ptr(c_in), dy.data_ptr(), cabi.ptr(dld), cabi.ptr(dh_out), cabi.ptr(dc_out), dx.data_ptr(),
-                                      dcond.data_ptr(), dh_in.data_ptr(), dc_in.data_ptr() if dc_in is not None else None, ctypes.byref(G), B,
-                                      stash.data_ptr(), stash.numel(), ws.data_ptr(), ws.numel(), st), "lfi_flowstep_bwd")
+        name, size = ("lfi_flowstep_rev_bwd", L.lfi_flowstep_rev_bwd_ws_bytes) if reverse else ("lfi_flowstep_bwd", L.lfi_flowstep_bwd_ws_bytes)
+        ws = self._workspace(("stepbwd", B), size(ctypes.byref(self.shape), B))
+        cabi.check(getattr(L, name)(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), k, cond.data_ptr(), cabi.ptr(h_in),
+                                    cabi.ptr(c_in), dy.data_ptr(), cabi.ptr(dld), cabi.ptr(dh_out), cabi.ptr(dc_out), dx.data_ptr(),
+                                    dcond.data_ptr(), dh_in.data_ptr(), dc_in.data_ptr() if dc_in is not None else None, ctypes.byref(G), B,
+                                    stash.data_ptr(), stash.numel(), ws.data_ptr(), ws.numel(), st), name)
         grads = {n: gbuf[offs[n]:offs[n] + numel[n]] for n in self._STEP_GRAD_BLOCKS}
         return dx, dcond, dh_in, dc_in, grads
 

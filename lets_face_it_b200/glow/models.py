@@ -9,7 +9,8 @@ three fused device paths reached through the C ABI (`engine.py` / `_cabi.py`):
                        stream requires grad)
   SeqGlow.inference -> lfi_seq_sample (persistent autoregressive sampler)
   SeqGlow.invert    -> lfi_seq_sample (teacher forced)
-  FlowStep / FlowNet / Glow single-frame calls -> lfi_flowstep (under autograd lfi_flowstep_fwd_train / lfi_flowstep_bwd)
+  FlowStep / FlowNet / Glow single-frame calls -> lfi_flowstep (under autograd lfi_flowstep_fwd_train / lfi_flowstep_bwd, in the
+                                                  reverse direction lfi_flowstep_rev_fwd_train / lfi_flowstep_rev_bwd)
   f_seq.forward on its own                     -> lfi_fseq_fwd (under autograd lfi_fseq_bwd as well)
 
 CUDA tensors only; there is no CPU / eager fallback.
@@ -398,14 +399,18 @@ class f_seq(nn.Module):
 
 
 class _FlowStepFn(torch.autograd.Function):
-    """One FlowStep on one frame under autograd (reference: FlowStep.normal_flow, models.py:311-342, differentiated by
-    torch): forward = lfi_flowstep_fwd_train, backward = lfi_flowstep_bwd + the LU chain rule.  Inputs after `c_in` are the
-    step's parameters in `FlowStep._autograd_params()` order (graph connectivity; values are read from the flat buffer)."""
+    """One FlowStep on one frame under autograd (reference: FlowStep.normal_flow, models.py:311-342, or with reverse set
+    FlowStep.reverse_flow, models.py:345-373, differentiated by torch): forward = lfi_flowstep_fwd_train / lfi_flowstep_rev_fwd_train,
+    backward = lfi_flowstep_bwd / lfi_flowstep_rev_bwd + the LU chain rule.  Inputs after `c_in` are the step's parameters in
+    `FlowStep._autograd_params()` order (graph connectivity; values are read from the flat buffer).  The reverse node also saves
+    them, so that an in-place update between its forward and backward raises instead of differentiating the wrong W^-1."""
 
     @staticmethod
-    def forward(ctx, eng, k, want_scale, n_lu, refresh, x, cond, h_in, c_in, *params):
-        y, ld, h_out, c_out, scale, saved = eng.flowstep_train(k, x, cond, h_in, c_in, want_scale, refresh=refresh)
-        ctx.eng, ctx.k, ctx.saved, ctx.n_lu = eng, k, saved, n_lu
+    def forward(ctx, eng, k, want_scale, n_lu, refresh, reverse, x, cond, h_in, c_in, *params):
+        y, ld, h_out, c_out, scale, saved = eng.flowstep_train(k, x, cond, h_in, c_in, want_scale, refresh=refresh, reverse=reverse)
+        ctx.eng, ctx.k, ctx.saved, ctx.n_lu, ctx.reverse = eng, k, saved, n_lu, reverse
+        if reverse:
+            ctx.save_for_backward(*params)
         ctx.has_c = c_out is not None
         outs = (y, ld, h_out) + ((c_out,) if c_out is not None else ()) + ((scale,) if scale is not None else ())
         if scale is not None:
@@ -418,7 +423,9 @@ class _FlowStepFn(torch.autograd.Function):
         eng, k = ctx.eng, ctx.k
         dy, dld, dh_out = grads[0], grads[1], grads[2]
         dc_out = grads[3] if ctx.has_c else None
-        dx, dcond, dh_in, dc_in, g = eng.flowstep_backward(k, ctx.saved, dy, dld, dh_out, dc_out)
+        if ctx.reverse:
+            ctx.saved_tensors  # raises if a parameter changed in place since the forward
+        dx, dcond, dh_in, dc_in, g = eng.flowstep_backward(k, ctx.saved, dy, dld, dh_out, dc_out, reverse=ctx.reverse)
         C = eng.C
         out = [g["an_bias"].view(1, C), g["an_logs"].view(1, C)]
         if ctx.n_lu:
@@ -430,7 +437,7 @@ class _FlowStepFn(torch.autograd.Function):
         out += [g["wc"].view(D, F), g["bc"], g["w_ih"].view(GH, In), g["b_ih"], g["w_hh"].view(GH, H), g["b_hh"],
                 g["wf"].view(Co, H), g["bf"], g["lf"]]
         _, h_in, c_in = ctx.saved[1], ctx.saved[2], ctx.saved[3]
-        return (None, None, None, None, None, dx, dcond, dh_in if h_in is not None else None,
+        return (None, None, None, None, None, None, dx, dcond, dh_in if h_in is not None else None,
                 dc_in if (c_in is not None and dc_in is not None) else None) + tuple(out)
 
 
@@ -477,24 +484,29 @@ class FlowStep(nn.Module):
                                                               f.rnn.weight_hh, f.rnn.bias_hh, f.final_linear.weight, f.final_linear.bias,
                                                               f.final_linear.logs]
 
-    def _forward_autograd(self, eng, input_, cond, logdet, refresh=True):
-        """normal_flow under autograd: kernels for everything data dependent, torch for the parameter-only log-det terms
-        C * sum(logs) + C * sum(log_s) (modules.py:62, 171) so that autograd owns their gradients.  refresh=False: the caller
-        (FlowNet.encode) has rebuilt the derived cache for this call already."""
+    def _forward_autograd(self, eng, input_, cond, logdet, refresh=True, reverse=False):
+        """normal_flow (reverse_flow) under autograd: kernels for everything data dependent, torch for the parameter-only log-det
+        terms C * sum(logs) + C * sum(log_s) (modules.py:62, 171) so that autograd owns their gradients.  refresh=False: the caller
+        (FlowNet.encode / decode) has rebuilt the derived cache for this call already."""
         params = self._autograd_params()
         h_in, c_in = self.f.hidden, self.f.cell
-        outs = _FlowStepFn.apply(eng, self._k, bool(self.scale_logging), 1 if self.invconv.LU else 0, bool(refresh), input_, cond, h_in, c_in,
-                                 *params)
+        outs = _FlowStepFn.apply(eng, self._k, bool(self.scale_logging) and not reverse, 1 if self.invconv.LU else 0, bool(refresh),
+                                 bool(reverse), input_, cond, h_in, c_in, *params)
         y, ld, h = outs[0], outs[1], outs[2]
         i = 3
         c = None
         if eng.G == 4:
             c = outs[i]
             i += 1
-        if self.scale_logging and eng.affine:
+        if self.scale_logging and eng.affine and not reverse:
             self.scale = outs[i]
         self.f.hidden, self.f.cell = h, c
         C = float(eng.C)
+        if reverse:  # the terms of Engine.step_logdet_const, in its order, so that the values are those of the no-grad call
+            s = self.actnorm.logs.sum() + (self.invconv.log_s.sum() if self.invconv.LU else torch.slogdet(self.invconv.weight)[1])
+            if logdet is not None:
+                logdet = logdet + (ld - s * C)
+            return y, logdet
         const = self.actnorm.logs.sum() * C
         const = const + (self.invconv.log_s.sum() * C if self.invconv.LU else torch.slogdet(self.invconv.weight)[1] * C)
         if logdet is not None:
@@ -511,6 +523,8 @@ class FlowStep(nn.Module):
                 input_.requires_grad or audio_features.requires_grad or any(p.requires_grad for p in self._autograd_params())
                 or (self.f.hidden is not None and self.f.hidden.requires_grad)):
             return self._forward_autograd(eng, input_, audio_features, logdet, _refresh)
+        if reverse and modules._needs_grad(input_, audio_features, self.f.hidden, self.f.cell, *self._autograd_params()):
+            return self._forward_autograd(eng, input_, audio_features, logdet, _refresh, reverse=True)
         y, logdet, h, c, scale = eng.flowstep(self._k, input_, audio_features, self.f.hidden, self.f.cell, logdet, bool(reverse),
                                               want_scale=self.scale_logging, refresh=_refresh)
         self.f.hidden, self.f.cell = h, c
