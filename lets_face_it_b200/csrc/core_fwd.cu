@@ -351,11 +351,9 @@ constexpr int kMaxSmem = 227 * 1024;
 int fwd_smem_bytes(const Dims &d, int R) { return plan_smem(d, R, false, false).total * (int)sizeof(float); }
 
 // Rows per CTA = 4*RPT.  Larger tiles amortise the weight stream, smaller tiles expose more CTAs;
-// take the largest tile that still gives every SM a CTA (LFI_RPT overrides for experiments).  The wavefront cell kernels
+// take the largest tile that still gives every SM a CTA.  The wavefront cell kernels
 // may also halve the weight ring (kc = 8) when that is what lets a tile fit (wide shapes: H = 256, LSTM).
 int choose_tile(const Dims &d, int B, bool bwd, bool sampler, int *kc_out) {
-  int forced = 0;
-  if (const char *e = getenv(sampler ? "LFI_RPT_SAMPLE" : (bwd ? "LFI_RPT_BWD" : "LFI_RPT"))) forced = atoi(e);
   const int cand[4] = {8, 4, 2, 1};
   int best = 0, best_kc = KC16;
   for (int i = 0; i < 4; ++i) {
@@ -365,7 +363,6 @@ int choose_tile(const Dims &d, int B, bool bwd, bool sampler, int *kc_out) {
       kc = 8;
       if (sampler || !kc_out || plan_smem(d, R, bwd, sampler, kc).total * (int)sizeof(float) > kMaxSmem) continue;
     }
-    if (forced == rpt) { best = rpt; best_kc = kc; break; }
     const long ctas = (long)((B + R - 1) / R) * (sampler ? 1 : d.K);
     best = rpt; best_kc = kc;
     if (ctas >= (sampler ? 120 : 148)) break;

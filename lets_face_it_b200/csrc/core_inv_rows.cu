@@ -322,8 +322,7 @@ template <int RR> static int launch_inv_rows_t(const InvArgs &a, cudaStream_t st
 }
 
 int launch_inv_rows(const InvArgs &a, cudaStream_t st) {
-  int rr = ((a.B + 7) / 8 >= 120 && plan_rows(a.d, 8).total * (int)sizeof(float) <= 227 * 1024) ? 8 : 4;
-  if (const char *e = getenv("LFI_INV_RR")) rr = atoi(e) == 8 ? 8 : 4;
+  const int rr = ((a.B + 7) / 8 >= 120 && plan_rows(a.d, 8).total * (int)sizeof(float) <= 227 * 1024) ? 8 : 4;
   return rr == 8 ? launch_inv_rows_t<8>(a, st) : launch_inv_rows_t<4>(a, st);
 }
 

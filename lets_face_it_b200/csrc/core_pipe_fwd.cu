@@ -354,8 +354,7 @@ static int sm_count() {
 }
 
 bool pipe_supported(const Dims &d, int nk, bool bwd) {
-  if (const char *e = getenv("LFI_CORE_PIPE"))
-    if (atoi(e) == 0) return false;
+  if (!env_flag("LFI_CORE_PIPE", true)) return false;
   if (d.G != 3 || d.H != 2 * PUC) return false;
   if (d.C > 64 || d.Co > 64 || d.C < 2) return false;
   if (d.affine && (d.Co & 1)) return false;

@@ -850,9 +850,8 @@ static int launch_core(const Operand &A, const Operand &B, const GemmArgs &g, in
   // pulls from L2 per MMA cycle - the bound of the 128-row tiles in the split-bf16 mode (64 B/clk/SM needed, ~43 available).
   // Needs a B tile that splits into two halves of whole swizzle atoms (K-major) / 64-wide chunks (MN-major) and enough
   // tiles to fill the machine with pairs.
-  static const bool pair_on = env_flag("LFI_GEMM_PAIR", true);
   bool pair = false;
-  if (pair_on && g.fuse == LFI_FUSE_NONE) {
+  if (g.fuse == LFI_FUSE_NONE) {
     int bn2 = p.bn;
     if (B.mn && bn2 % 128 != 0) bn2 = g.N > 128 ? 256 : 128;
     if (!B.mn && bn2 % 16 != 0) bn2 = round_up(bn2, 16);
@@ -862,9 +861,8 @@ static int launch_core(const Operand &A, const Operand &B, const GemmArgs &g, in
   if (!pair && g.fuse == LFI_FUSE_NONE && p.bn == 256 && g.N % 128 == 0) {
     // one 128 x 256 tile per CTA and fewer tiles than SMs: the launch is the serial latency of one tile (loads -> MMAs -> epilogue).
     // Half-width tiles give every CTA two or more, so that the mainloop of one overlaps the epilogue of the previous.
-    static const bool narrow_on = env_flag("LFI_GEMM_NARROW", true);
     const long t256 = (long)((g.M + BM - 1) / BM) * ((g.N + 255) / 256) * g.batch;
-    if (narrow_on && t256 < g_sms && t256 * 2 > g_sms) p.bn = 128;
+    if (t256 < g_sms && t256 * 2 > g_sms) p.bn = 128;
   }
   const int CL = pair ? 2 : 1;
   p.tiles_m = (g.M + BM - 1) / BM; p.tiles_n = (g.N + p.bn - 1) / p.bn;

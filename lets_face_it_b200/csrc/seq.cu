@@ -87,9 +87,9 @@ struct EncWs {
   float *hs;     // [hist][M][E]   (training) or [2][M][E] ping-pong (sampling)
   float *gates;  // [hist][M][3E]  (training only)
   float *ahn;    // [hist][M][E]   (training only)
-  // tensor-core modes (planes == true): bf16 operand planes written by the producers themselves, never re-split
+  // tensor-core modes (planes == true): bf16 operand planes written by the producers themselves, never re-split; the
+  // training stash keeps the gates in 16-bit fixed point (the fp32 mode keeps exact fp32 gates)
   bool planes;
-  bool gates16;           // gates stash in 16-bit fixed point (planes mode; the fp32 mode keeps exact fp32 gates)
   void *hp_hi, *hp_lo;    // h          [hist | 2][M][E]
   void *whh_hi, *whh_lo;  // W_hh       [3E][E]  (K-major B of the step GEMM, MN-major B of dh_prev = dA_h W_hh)
   // backward (training only): gate gradients of every window step, kept for the batched weight-gradient GEMMs
@@ -97,7 +97,7 @@ struct EncWs {
   void *dah_hi, *dah_lo, *dan_hi, *dan_lo;  // planes, same shapes
   void *xg_hi, *xg_lo;    // masked window inputs [hist][M][round_up(dim, 8)]
   void *wih_hi, *wih_lo;  // W_ih       [3E][round_up(dim, 8)]  (input part of the fused forward step, LFI_FUSE_GRU_FWD_X)
-  bool xfuse;             // the forward steps s >= 1 take their input projection inside the step GEMM (training, per-step path)
+  bool xfuse;             // the forward steps take their input projection inside the step GEMM (planes, training, per-step path)
   float *xg32;            // the same in fp32 [hist][M][dim] (split source / fp32-mode operand)
   float *dhe;             // [M][E] running d h of the window recurrence
   // persistent window-GRU forward (enc_persist.cu; sampling / feature encoding only): xp is time-major and row-interleaved
@@ -148,7 +148,7 @@ struct TrainWs {
 };
 
 static bool core_planes_ok(const Dims &d, int mode) {
-  if (mode == LFI_GEMM_FP32 || !env_flag("LFI_CORE_PLANES", true)) return false;
+  if (mode == LFI_GEMM_FP32) return false;
   if (!core::pipe_supported(d, d.K, false) || !core::pipe_supported(d, d.K, true)) return false;
   return d.C % 8 == 0 && d.Co % 8 == 0 && d.H % 8 == 0 && d.D % 8 == 0;
 }
@@ -166,7 +166,6 @@ static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t
   e.gates = S.take<float>(h * M * 3 * E);
   e.ahn = S.take<float>(h * M * E);
   e.planes = enc_use_planes(s, m, M, mode);
-  e.gates16 = e.planes && E % 4 == 0 && env_flag("LFI_GATES16", true);
   if (e.planes) {
     const bool lo = mode == LFI_GEMM_BF16X3;
     const size_t dimp = round_up(s->dim[m], 8);
@@ -178,7 +177,7 @@ static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t
     e.wih_hi = take_bf16(W, 3 * E * dimp);        e.wih_lo = lo ? take_bf16(W, 3 * E * dimp) : nullptr;
     // input projection inside the fused step GEMM: the masked window inputs are gathered as operand planes in the forward pass
     // (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand; step 0 (no state yet) keeps the xp rows
-    e.xfuse = E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true) && env_flag("LFI_ENC_XFUSE", true);
+    e.xfuse = E % 64 == 0 && env_flag("LFI_ENC_XFUSE", true);
   } else {
     e.dah32 = K.take<float>(h * M * 3 * E);
     e.dan32 = K.take<float>(h * M * E);
@@ -325,20 +324,20 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, enc[m].xT, dim, p->enc_w_ih[m], dim, enc[m].xp, 3 * E);
       g.c_tiled32 = 1;
       LFI_TRY(gemm_dispatch(mode, g, gws, gws_bytes, st));
-    } else if (project && !(stash && enc[m].planes && enc[m].xfuse && enc[m].xg_hi)) {  // (fused into the step GEMMs otherwise)
+    } else if (project && !(stash && enc[m].xfuse)) {  // (fused into the step GEMMs otherwise)
       GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, bt->x[m], dim, p->enc_w_ih[m], dim, enc[m].xp, 3 * E);
       LFI_TRY(gemm_dispatch(mode, g, gws, gws_bytes, st));
     }
     EncWs &ew = enc[m];
     if (ew.planes && project)  // W_hh planes: once per call (weights change every optimizer step)
       LFI_TRY(split_to_planes(p->enc_w_hh[m], 3 * E, E, E, 0, 1, ew.whh_hi, lo ? ew.whh_lo : nullptr, st));
-    if (ew.planes && stash && ew.xfuse && ew.xg_hi) {
+    if (stash && ew.xfuse) {
       const int dimp = round_up(dim, 8);
       LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
       LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * E, dim, dim, 0, 1, ew.wih_hi, lo ? ew.wih_lo : nullptr, st));
     }
     mods[nmods++] = m;
-    all_fused = all_fused && ew.planes && (ew.persist || (E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true)));
+    all_fused = all_fused && ew.planes && (ew.persist || E % 64 == 0);
   }
   // ---- phase 2: the window recurrences.  With the fused GRU launches (operands in plane form, no shared scratch) the
   //      modalities are independent chains: they run on parallel streams forked from / joined to the caller's, so that the
@@ -361,8 +360,8 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       const int cur = stash ? sidx : (sidx & 1), prv = stash ? sidx - 1 : ((sidx - 1) & 1);
       hcur = ew.hs + (size_t)cur * M * E;
       if (sidx) hprev = ew.hs + (size_t)prv * M * E;
-      const bool xf = stash && ew.planes && ew.xfuse && ew.xg_hi;  // input projection inside the step GEMM: also step 0 (input part alone)
-      const bool fused = (sidx || xf) && ew.planes && E % 64 == 0 && env_flag("LFI_FUSED_GRU_FWD", true);
+      const bool xf = stash && ew.xfuse;  // input projection inside the step GEMM: also step 0 (input part alone)
+      const bool fused = ew.planes && E % 64 == 0 && (sidx || xf);
       if (sidx && !fused) {
         GemmArgs gg = gemm_args(0, 1, (int)M, 3 * E, E, hprev, E, p->enc_w_hh[m], E, gh, 3 * E);
         if (ew.planes) {
@@ -380,7 +379,7 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       a.h_hi = ew.planes ? (void *)((uint16_t *)ew.hp_hi + (size_t)cur * M * E) : nullptr;
       a.h_lo = (ew.planes && lo) ? (void *)((uint16_t *)ew.hp_lo + (size_t)cur * M * E) : nullptr;
       a.s = sidx; a.hist = hist; a.B = B; a.T = T; a.Tp = Tp; a.t0 = t0; a.E = E;
-      a.gates16 = (stash && ew.gates16) ? 1 : 0;
+      a.gates16 = (stash && ew.planes) ? 1 : 0;
       if (fused) {
         // recurrent product and gate math in one launch: the [M, 3E] pre-activations stay in TMEM
         GemmArgs gg = gemm_args(0, 1, (int)M, 3 * E, E, nullptr, E, nullptr, E, nullptr, 3 * E);
@@ -389,7 +388,7 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
         gg.pB = plane_ref(ew.whh_hi, ew.whh_lo, E);
         gg.fuse = LFI_FUSE_GRU_FWD;
         GruEpi &q = gg.gru;
-        if (stash && ew.xfuse && ew.xg_hi) {
+        if (xf) {
           const int dimp = round_up(s->dim[m], 8);
           gg.fuse = LFI_FUSE_GRU_FWD_X;
           q.xa_hi = (uint16_t *)ew.xg_hi + (size_t)sidx * M * dimp; q.xa_lo = lo ? (uint16_t *)ew.xg_lo + (size_t)sidx * M * dimp : nullptr;
@@ -406,7 +405,7 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
     }
     return LFI_OK;
   };
-  const bool par = nmods > 1 && all_fused && env_flag("LFI_ENC_STREAMS", true);
+  const bool par = nmods > 1 && all_fused;
   if (!par) {
     for (int i = 0; i < nmods; ++i) LFI_TRY(chain(mods[i], st));
     return LFI_OK;
@@ -466,7 +465,7 @@ static int enc_bwd(const lfi_shape *s, const Dims &d, const lfi_params *p, const
     } else {
       e.dah32 = ew.dah32 + (size_t)sidx * M * 3 * E; e.dan32 = ew.dan32 + (size_t)sidx * M * E;
     }
-    e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.gates16 ? 1 : 0;
+    e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.planes ? 1 : 0;
     LFI_TRY(aux::enc_gate_bwd2(e, st, o.part));
     if (sidx) {  // dh_{s-1} += dA_h W_hh
       GemmArgs t = gemm_args(0, 0, (int)M, E, 3 * E, e.dah32, 3 * E, p->enc_w_hh[m], E, ew.dhe, E, det ? LFI_EPI_ACCUM_PRE : LFI_EPI_ACCUM);
@@ -545,52 +544,6 @@ static int check_batch(const lfi_shape *s, const Dims &d, const lfi_batch *b, in
   LFI_REQUIRE(b->T >= min_T, LFI_ERR_SHAPE, "batch: T=%d shorter than needed (%d)", b->T, min_T);
   (void)s; (void)d;
   return LFI_OK;
-}
-
-// Runs `body` (launches on `st` only) as one CUDA graph when possible; falls back to direct launches when the stream is
-// already being captured, the capture is refused, or LFI_SAMPLE_GRAPH=0.  Executable graphs are destroyed lazily, once the
-// event recorded behind their launch has completed (no host synchronisation inside the call).
-template <class F> static int run_frames_graphed(F &&body, int nframes, cudaStream_t st) {
-  struct Pending { cudaGraphExec_t ex; cudaEvent_t ev; };
-  static Pending pend[64];
-  static int npend = 0;
-  for (int i = 0; i < npend;) {  // reap finished graphs
-    if (cudaEventQuery(pend[i].ev) == cudaSuccess) {
-      cudaGraphExecDestroy(pend[i].ex);
-      cudaEventDestroy(pend[i].ev);
-      pend[i] = pend[--npend];
-    } else {
-      cudaGetLastError();
-      ++i;
-    }
-  }
-  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-  const bool want = nframes > 1 && npend < 60 && env_flag("LFI_SAMPLE_GRAPH", false) &&
-                    cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusNone;
-  if (!want) return body();
-  if (cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed) != cudaSuccess) {
-    cudaGetLastError();
-    return body();
-  }
-  const long launches_before = lfi_launch_count();
-  const int rc = body();
-  cudaGraph_t g = nullptr;
-  const cudaError_t e = cudaStreamEndCapture(st, &g);
-  cudaGraphExec_t ex = nullptr;
-  if (rc == LFI_OK && e == cudaSuccess && g && cudaGraphInstantiate(&ex, g, 0) == cudaSuccess) {
-    cudaGraphDestroy(g);
-    LFI_CUDA(cudaGraphLaunch(ex, st));
-    cudaEvent_t ev;
-    LFI_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    LFI_CUDA(cudaEventRecord(ev, st));
-    pend[npend++] = Pending{ex, ev};
-    return LFI_OK;
-  }
-  if (g) cudaGraphDestroy(g);
-  cudaGetLastError();
-  if (rc != LFI_OK) return rc;      // a real error of the body: report it
-  count_launches(launches_before - lfi_launch_count());  // the captured launches never ran: do not count them twice
-  return body();                    // capture refused: plain stream-ordered launches
 }
 
 }  // namespace lfi
@@ -751,7 +704,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   LFI_TRY(dev_res(&dr));
   cudaStream_t wg_stream = dr->wg_stream;
   cudaEvent_t wg_fork = dr->wg_fork, wg_join = dr->wg_join;
-  const bool wg_par = w.cp && env_flag("LFI_WGRAD_STREAM", true);
+  const bool wg_par = w.cp;
   cudaStream_t st_main = st;
   if (wg_par) {
     LFI_CUDA(cudaEventRecord(wg_fork, st_main));
@@ -806,7 +759,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
     if (w.cp) r.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
     size_t side_off = 0;
     bool wc_side = false;
-    if (wg_par && env_flag("LFI_DWC_STREAM", true)) {
+    if (wg_par) {
       GemmArgs qd = gemm_args(0, 0, (int)M, d.Fe, K * D, nullptr, K * D, WcF, d.Fe, nullptr, d.Fe, 0);
       side_off = round_up_sz(gemm_ws_bytes_for(gemm_mode, qd), 1024);
       wc_side = side_off + gemm_ws_bytes_for(gemm_mode, r) <= gws_bytes;
@@ -876,7 +829,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
     if (s->hist[m] > 0 && s->ehid[m] > 0) { mods[nmods++] = m; all_planes = all_planes && w.enc[m].planes; }
   cudaStream_t *side = dr->enc_side;
   cudaEvent_t ev_fork = dr->enc_fork, *ev_join = dr->enc_join;
-  const bool par = nmods > 1 && all_planes && env_flag("LFI_ENC_STREAMS", true);
+  const bool par = nmods > 1 && all_planes;
   if (!par) {
     int rc = LFI_OK;
     for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], st);
@@ -934,7 +887,7 @@ struct SampleWs {
   size_t bytes;
 };
 static bool sample_tc_ar(const Dims &d, int mode) {
-  return mode != LFI_GEMM_FP32 && d.Far > 0 && d.Far % 8 == 0 && d.D % 8 == 0 && env_flag("LFI_SAMPLE_TC", true);
+  return mode != LFI_GEMM_FP32 && d.Far > 0 && d.Far % 8 == 0 && d.D % 8 == 0;
 }
 static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chunk, int mode, void *ws, SampleWs *w) {
   Bump b(ws, 0);
@@ -1066,29 +1019,25 @@ int lfi_seq_sample(const lfi_shape *s, const void *derived, const lfi_params *p,
       }
       a.cstatic = nullptr; a.faces = nullptr;
       a.Tc = 1; a.G = w.G; a.g_ld = (long)K * d.GH;
-      auto frames = [&]() -> int {
-        for (int tc = 0; tc < Tc; ++tc) {
-          LFI_TRY(aux::gather_windows(w.car, d.Far, 0, faces, nullptr, B, seq_len, d.C, hist0, 0, t0 + tc, 1, st));
-          float *Cf = w.Cs + (size_t)tc * B * K * d.D;  // static pre-activation of this frame (bias included), updated in place
-          GemmArgs q = gemm_args(0, 1, B, K * d.D, d.Far, w.car, d.Far, nullptr, d.Far, Cf, K * d.D, LFI_EPI_ACCUM_PRE | LFI_EPI_LRELU);
-          q.pB = plane_ref(w.war_hi, w.war_lo, d.Far);
-          q.pOut = plane_ref(w.cact_hi, w.cact_lo, K * d.D);
-          LFI_TRY(gemm_dispatch(gemm_mode, q, gws, gws_bytes, st));
-          GemmArgs h = gemm_args(0, 1, B, d.GH, d.D, nullptr, K * d.D, nullptr, d.D, w.G, K * d.GH, LFI_EPI_BIAS, p->b_ih);
-          h.batch = K; h.sC = d.GH; h.sBias = d.GH;
-          h.pA = plane_ref(w.cact_hi, w.cact_lo, K * d.D, d.D);
-          h.pB = plane_ref(w.wihc_hi, w.wihc_lo, d.D, (long)d.GH * d.D);
-          LFI_TRY(gemm_dispatch(gemm_mode, h, gws, gws_bytes, st));
-          core::InvArgs af = a;
-          af.t_abs0 = t0 + tc; af.t_rel0 = c0 + tc;
-          LFI_TRY(core::launch_inv(af, st));
-        }
-        return LFI_OK;
-      };
-      // The frame chain is ~6 short, strictly dependent launches per frame.  LFI_SAMPLE_GRAPH=1 captures the whole chunk into
-      // ONE CUDA graph (every pointer and shape is fixed for the call).  Measured on B200 (1,024 sequences x 750 frames): 322.9 ms
-      // with and without the graph - the chain is bound by the kernels themselves, not by launch gaps - so it is off by default.
-      LFI_TRY(run_frames_graphed(frames, Tc, st));
+      // The frame chain is ~6 short, strictly dependent launches per frame, issued directly: capturing a chunk of it into one
+      // CUDA graph was measured on B200 (1,024 sequences x 750 frames) at 322.9 ms with and without the graph - the chain is
+      // bound by the kernels themselves, not by launch gaps.
+      for (int tc = 0; tc < Tc; ++tc) {
+        LFI_TRY(aux::gather_windows(w.car, d.Far, 0, faces, nullptr, B, seq_len, d.C, hist0, 0, t0 + tc, 1, st));
+        float *Cf = w.Cs + (size_t)tc * B * K * d.D;  // static pre-activation of this frame (bias included), updated in place
+        GemmArgs q = gemm_args(0, 1, B, K * d.D, d.Far, w.car, d.Far, nullptr, d.Far, Cf, K * d.D, LFI_EPI_ACCUM_PRE | LFI_EPI_LRELU);
+        q.pB = plane_ref(w.war_hi, w.war_lo, d.Far);
+        q.pOut = plane_ref(w.cact_hi, w.cact_lo, K * d.D);
+        LFI_TRY(gemm_dispatch(gemm_mode, q, gws, gws_bytes, st));
+        GemmArgs h = gemm_args(0, 1, B, d.GH, d.D, nullptr, K * d.D, nullptr, d.D, w.G, K * d.GH, LFI_EPI_BIAS, p->b_ih);
+        h.batch = K; h.sC = d.GH; h.sBias = d.GH;
+        h.pA = plane_ref(w.cact_hi, w.cact_lo, K * d.D, d.D);
+        h.pB = plane_ref(w.wihc_hi, w.wihc_lo, d.D, (long)d.GH * d.D);
+        LFI_TRY(gemm_dispatch(gemm_mode, h, gws, gws_bytes, st));
+        core::InvArgs af = a;
+        af.t_abs0 = t0 + tc; af.t_rel0 = c0 + tc;
+        LFI_TRY(core::launch_inv(af, st));
+      }
       continue;
     }
     LFI_TRY(core::launch_inv(a, st));

@@ -11,7 +11,6 @@ from __future__ import annotations
 
 import ctypes
 import math
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -335,20 +334,16 @@ class Engine:
         dev = self.theta.device
         # The derived cache (composed 1x1 weights, folded W_c, transposes: ~25 short launches) is rebuilt on a side stream: the
         # conditioning encoders, which open the forward call, do not read it, and the call waits for the event only in front
-        # of its first consumer (lfi_set_derived_ready_event).  LFI_DERIVE_STREAM=0: everything on the caller's stream.
-        ready = None
-        if dev.type == "cuda" and os.environ.get("LFI_DERIVE_STREAM", "1") != "0":
-            if self._derive_stream is None or self._derive_stream.device != dev:
-                self._derive_stream = torch.cuda.Stream(device=dev)
-                self._derive_event = torch.cuda.Event()
-            side = self._derive_stream
-            side.wait_stream(torch.cuda.current_stream(dev))  # after the optimizer update, and after every reader of the old cache
-            with torch.cuda.stream(side):
-                P = self.refresh(False)
-                self._derive_event.record(side)
-            ready = self._derive_event
-        else:
+        # of its first consumer (lfi_set_derived_ready_event).
+        if self._derive_stream is None or self._derive_stream.device != dev:
+            self._derive_stream = torch.cuda.Stream(device=dev)
+            self._derive_event = torch.cuda.Event()
+        side = self._derive_stream
+        side.wait_stream(torch.cuda.current_stream(dev))  # after the optimizer update, and after every reader of the old cache
+        with torch.cuda.stream(side):
             P = self.refresh(False)
+            self._derive_event.record(side)
+        ready = self._derive_event
         st = cabi.stream_ptr()
         x0 = batch["p1_face"]
         B, T = x0.shape[0], x0.shape[1]
@@ -360,16 +355,14 @@ class Engine:
         z = torch.empty(Tp, B, self.C, dtype=torch.float32, device=dev)
         nll = torch.empty(Tp, B, dtype=torch.float32, device=dev)
         ws = self._workspace(("train", B, T), L.lfi_train_ws_bytes(ctypes.byref(self.shape), B, T, self.gemm_mode))
-        if ready is not None:
-            L.lfi_set_derived_ready_event(ready.cuda_event)
+        L.lfi_set_derived_ready_event(ready.cuda_event)
         try:
             rc = L.lfi_seq_train_fwd(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), ctypes.byref(bt),
                                      z.data_ptr(), nll.data_ptr(), scale_out.data_ptr() if scale_out is not None else None,
                                      ws.data_ptr(), ws.numel(), self.gemm_mode, st)
         finally:
-            if ready is not None:
-                L.lfi_set_derived_ready_event(None)
-                torch.cuda.current_stream(dev).wait_event(ready)  # (a failed call may not have consumed it)
+            L.lfi_set_derived_ready_event(None)
+            torch.cuda.current_stream(dev).wait_event(ready)  # (a failed call may not have consumed it)
         cabi.check(rc, "lfi_seq_train_fwd")
         self._fwd_token += 1
         self._last = (bt, keep, B, T, P)

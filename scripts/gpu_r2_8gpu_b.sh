@@ -23,6 +23,6 @@ grep -o "NVLS[^ ]*\|Using network[^,]*\|[0-9]* coll channels[^,]*\|Connected all
 run cta4 NCCL_MAX_CTAS=4 -- --steps 20 --warmup 5 --no-cpu-baseline --no-bf16 --no-sample
 run cta16 NCCL_MAX_CTAS=16 -- --steps 20 --warmup 5 --no-cpu-baseline --no-bf16 --no-sample
 run ring NCCL_ALGO=Ring -- --steps 20 --warmup 5 --no-cpu-baseline --no-bf16 --no-sample
-run widelstm LFI_X=0 -- --variant wide-lstm --gemm bf16 --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 --no-sample
-run widegru LFI_X=0 -- --variant wide-gru --gemm bf16 --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 --no-sample
+run widelstm -- --variant wide-lstm --gemm bf16 --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 --no-sample
+run widegru -- --variant wide-gru --gemm bf16 --steps 10 --warmup 3 --no-cpu-baseline --no-bf16 --no-sample
 cp gpurun_out/b8_widelstm.log gpurun_out/b8_widelstm_line.json 2>/dev/null
