@@ -122,13 +122,30 @@ struct BwdArgs {
   float *dx_in;
 };
 
+// The kernel that runs one direction of the flow core.
+enum class CoreKernel : int {
+  Wave = 0,    // anti-diagonal wavefront launches (core_fwd.cu / core_bwd.cu)
+  WaveHybrid,  // the same, with the recurrent products of each wavefront as one batched tcgen05 GEMM (FwdArgs::wtc)
+  Pipe,        // persistent stage pipeline, FFMA gate products (core_pipe_fwd.cu / core_pipe_bwd.cu)
+  PipeTc       // persistent stage pipeline, tcgen05 gate products (core_pipe_fwd_tc.cu / core_pipe_bwd_tc.cu)
+};
+struct CorePlan {
+  CoreKernel fwd, bwd;
+  bool planes;  // the GEMM operands of the flow-step contractions are bf16 planes written by their producers (both pipelines run)
+  bool tiled;   // stash (gates / ahn / h) and G in the tiled layouts of the tensor-core pipelines (fwd == PipeTc)
+};
+// The one place that decides the flow-core path of whole-sequence training (core_plan.cu): shape, GEMM mode, the switches of
+// DESIGN.md §9.  The forward and backward calls of a training step plan alike, so they agree on the workspace layout.
+CorePlan plan_core(const Dims &d, int B, int gemm_mode);
+
 int fwd_smem_bytes(const Dims &d, int R);
 int choose_rpt(const Dims &d, int B, bool bwd, bool sampler);
 int choose_tile(const Dims &d, int B, bool bwd, bool sampler, int *kc_out);  // + weight-ring depth (16 or 8 rows per stage)
-int launch_fwd(const FwdArgs &a, cudaStream_t st);
+int launch_fwd(const FwdArgs &a, CoreKernel kern, cudaStream_t st);
 int launch_inv(const InvArgs &a, cudaStream_t st);
-int launch_bwd(const BwdArgs &a, cudaStream_t st);
+int launch_bwd(const BwdArgs &a, CoreKernel kern, cudaStream_t st);
 int launch_bwd_single(const BwdArgs &a, cudaStream_t st);  // a.single >= 0: one cell through the wavefront kernel
+bool use_inv_rows(const InvArgs &a);                        // the sampler's kernel: core_inv_rows or core_inv_persistent
 bool inv_rows_supported(const InvArgs &a);
 int launch_inv_rows(const InvArgs &a, cudaStream_t st);
 

@@ -266,13 +266,12 @@ __global__ void __launch_bounds__(NT) core_bwd_wave(BwdArgs a, int wave, int kmi
   }
 }
 
-template <int RPT, int KC> static int launch_bwd_t(const BwdArgs &a, cudaStream_t st) {
+template <int RPT, int KC> static int launch_bwd_t(const BwdArgs &a, bool tcw, cudaStream_t st) {  // tcw: hybrid wavefronts
   constexpr int R = Tile<RPT>::R;
   const int bytes = plan_smem(a.d, R, true, false, KC).total * (int)sizeof(float);
   auto kern = a.dx_in ? core_bwd_wave<RPT, KC, true> : core_bwd_wave<RPT, KC, false>;
   LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   const int tiles = (a.B + R - 1) / R, K = a.d.K;
-  const bool tcw = a.wtc.mode != 0 && a.single < 0;
   BwdArgs aw = a;
   aw.skip_hh = tcw ? 1 : 0;
   for (int wave = a.Tp + K - 2; wave >= 0; --wave) {
@@ -325,25 +324,34 @@ int launch_bwd_single(const BwdArgs &a, cudaStream_t st) {
   return LFI_ERR_SHAPE;
 }
 
-int launch_bwd(const BwdArgs &a, cudaStream_t st) {
-  if (a.flags && pipe_supported(a.d, a.d.K, true)) {
-    if (a.stash_tiled && a.pdG_hi && pipe_bwd_tc_supported(a.d)) return launch_bwd_pipe_tc(a, st);  // tensor-core GEMM modes
-    return launch_bwd_pipe(a, st);
-  }
+static int launch_bwd_wave(const BwdArgs &a, bool tcw, cudaStream_t st) {
   int kc = KC16;
   const int rpt = choose_tile(a.d, a.B, true, false, &kc);
   switch (rpt * 100 + kc) {
-    case 816: return launch_bwd_t<8, 16>(a, st);
-    case 416: return launch_bwd_t<4, 16>(a, st);
-    case 216: return launch_bwd_t<2, 16>(a, st);
-    case 116: return launch_bwd_t<1, 16>(a, st);
-    case 808: return launch_bwd_t<8, 8>(a, st);
-    case 408: return launch_bwd_t<4, 8>(a, st);
-    case 208: return launch_bwd_t<2, 8>(a, st);
-    case 108: return launch_bwd_t<1, 8>(a, st);
+    case 816: return launch_bwd_t<8, 16>(a, tcw, st);
+    case 416: return launch_bwd_t<4, 16>(a, tcw, st);
+    case 216: return launch_bwd_t<2, 16>(a, tcw, st);
+    case 116: return launch_bwd_t<1, 16>(a, tcw, st);
+    case 808: return launch_bwd_t<8, 8>(a, tcw, st);
+    case 408: return launch_bwd_t<4, 8>(a, tcw, st);
+    case 208: return launch_bwd_t<2, 8>(a, tcw, st);
+    case 108: return launch_bwd_t<1, 8>(a, tcw, st);
   }
   set_error("flow core backward: shape does not fit shared memory (H=%d G=%d C=%d)", a.d.H, a.d.G, a.d.C);
   return LFI_ERR_SHAPE;
+}
+
+int launch_bwd(const BwdArgs &a, CoreKernel kern, cudaStream_t st) {
+  switch (kern) {
+    case CoreKernel::Wave: return launch_bwd_wave(a, false, st);
+    case CoreKernel::WaveHybrid:
+      LFI_REQUIRE(a.single < 0 && a.wtc.mode && a.wtc.whh_hi, LFI_ERR_ARG, "flow core backward: hybrid wavefronts need W_hh planes");
+      return launch_bwd_wave(a, true, st);
+    case CoreKernel::Pipe: return launch_bwd_pipe(a, st);
+    case CoreKernel::PipeTc: return launch_bwd_pipe_tc(a, st);
+  }
+  set_error("flow core backward: unknown kernel %d", (int)kern);
+  return LFI_ERR_ARG;
 }
 
 }  // namespace core

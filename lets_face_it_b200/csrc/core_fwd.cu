@@ -373,13 +373,12 @@ int choose_tile(const Dims &d, int B, bool bwd, bool sampler, int *kc_out) {
 
 int choose_rpt(const Dims &d, int B, bool bwd, bool sampler) { return choose_tile(d, B, bwd, sampler, nullptr); }
 
-template <int RPT, int KC> static int launch_fwd_t(const FwdArgs &a, cudaStream_t st) {
+template <int RPT, int KC> static int launch_fwd_t(const FwdArgs &a, bool tcw, cudaStream_t st) {  // tcw: hybrid wavefronts
   constexpr int R = Tile<RPT>::R;
   const int bytes = plan_smem(a.d, R, false, false, KC).total * (int)sizeof(float);
   LFI_CUDA(cudaFuncSetAttribute(core_fwd_wave<RPT, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   const int tiles = (a.B + R - 1) / R;
   const int nk = a.k_last - a.k_first + 1;
-  const bool tcw = a.wtc.mode != 0 && a.k_first == 0 && !a.h0 && !a.c0;  // hybrid wavefronts: whole-sequence training forward only
   for (int wave = 0; wave < a.Tp + nk - 1; ++wave) {
     // active steps: k_first + i with 0 <= wave - i < Tp
     const int i0 = max(0, wave - a.Tp + 1), i1 = min(nk - 1, wave);
@@ -410,22 +409,37 @@ template <int RPT, int KC> static int launch_fwd_t(const FwdArgs &a, cudaStream_
   return LFI_OK;
 }
 
-int launch_fwd(const FwdArgs &a, cudaStream_t st) {
-  if (a.flags && !a.h0 && !a.c0 && pipe_supported(a.d, a.k_last - a.k_first + 1, false)) return launch_fwd_pipe(a, st);
+static int launch_fwd_wave(const FwdArgs &a, bool tcw, cudaStream_t st) {
   int kc = KC16;
   const int rpt = choose_tile(a.d, a.B, false, false, &kc);
   switch (rpt * 100 + kc) {
-    case 816: return launch_fwd_t<8, 16>(a, st);
-    case 416: return launch_fwd_t<4, 16>(a, st);
-    case 216: return launch_fwd_t<2, 16>(a, st);
-    case 116: return launch_fwd_t<1, 16>(a, st);
-    case 808: return launch_fwd_t<8, 8>(a, st);
-    case 408: return launch_fwd_t<4, 8>(a, st);
-    case 208: return launch_fwd_t<2, 8>(a, st);
-    case 108: return launch_fwd_t<1, 8>(a, st);
+    case 816: return launch_fwd_t<8, 16>(a, tcw, st);
+    case 416: return launch_fwd_t<4, 16>(a, tcw, st);
+    case 216: return launch_fwd_t<2, 16>(a, tcw, st);
+    case 116: return launch_fwd_t<1, 16>(a, tcw, st);
+    case 808: return launch_fwd_t<8, 8>(a, tcw, st);
+    case 408: return launch_fwd_t<4, 8>(a, tcw, st);
+    case 208: return launch_fwd_t<2, 8>(a, tcw, st);
+    case 108: return launch_fwd_t<1, 8>(a, tcw, st);
   }
   set_error("flow core: shape does not fit shared memory (H=%d G=%d C=%d)", a.d.H, a.d.G, a.d.C);
   return LFI_ERR_SHAPE;
+}
+
+int launch_fwd(const FwdArgs &a, CoreKernel kern, cudaStream_t st) {
+  // only the plain wavefronts start from a given state (module API); the other kernels run whole-sequence training
+  LFI_REQUIRE(kern == CoreKernel::Wave || (!a.h0 && !a.c0), LFI_ERR_ARG, "flow core: only the wavefront kernels take an initial state");
+  switch (kern) {
+    case CoreKernel::Wave: return launch_fwd_wave(a, false, st);
+    case CoreKernel::WaveHybrid:
+      LFI_REQUIRE(a.k_first == 0 && a.wtc.mode && a.wtc.whh_hi && a.wtc.ghbuf, LFI_ERR_ARG,
+                  "flow core: hybrid wavefronts need W_hh planes and product buffers from step 0");
+      return launch_fwd_wave(a, true, st);
+    case CoreKernel::Pipe: return launch_fwd_pipe(a, st);
+    case CoreKernel::PipeTc: return launch_fwd_pipe_tc(a, st);
+  }
+  set_error("flow core: unknown kernel %d", (int)kern);
+  return LFI_ERR_ARG;
 }
 
 template <int RPT> static int launch_inv_t(const InvArgs &a, cudaStream_t st) {
@@ -439,7 +453,7 @@ template <int RPT> static int launch_inv_t(const InvArgs &a, cudaStream_t st) {
 }
 
 int launch_inv(const InvArgs &a, cudaStream_t st) {
-  if (inv_rows_supported(a)) return launch_inv_rows(a, st);
+  if (use_inv_rows(a)) return launch_inv_rows(a, st);
   const int rpt = choose_rpt(a.d, a.B, false, true);
   switch (rpt) {
     case 8: return launch_inv_t<8>(a, st);

@@ -303,7 +303,6 @@ __global__ void core_inv_rows(InvArgs a) {
 
 bool inv_rows_supported(const InvArgs &a) {
   const Dims &d = a.d;
-  if (!env_flag("LFI_INV_ROWS", true)) return false;
   if (a.cstatic || !a.G || d.G != 3) return false;
   const int Cm = d.Co > d.C ? d.Co : d.C;
   const int nth = round_up(d.GH, 32);

@@ -123,14 +123,37 @@ inline int pipe_check_residency(Kern kern, int threads, int smem_bytes, int clus
   return LFI_OK;
 }
 
-bool pipe_supported(const Dims &d, int nk, bool bwd);
+int sm_count();  // SMs of the current device (core_plan.cu)
+
+// The part the four stage-pipeline launchers share: P pipelines of nk stage clusters (grid 2 x nk x P), as many as the SMs hold
+// and the tiles of 64 sequences need; flag_rows progress counters per pipeline and CTA, zeroed before the launch.
+template <typename Args>
+int launch_pipe(void (*kern)(Args, int, int, int *), const Args &a, int threads, int smem_bytes, int nk, int flag_rows,
+                const char *what, cudaStream_t st) {
+  const int ntiles = (a.B + PR - 1) / PR;
+  int P = sm_count() / (2 * nk);
+  if (P > ntiles) P = ntiles;
+  const size_t flag_bytes = (size_t)P * flag_rows * 2 * sizeof(int);
+  LFI_REQUIRE(a.flags, LFI_ERR_ARG, "%s: no progress flags", what);
+  LFI_REQUIRE(P >= 1 && flag_bytes <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
+  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  LFI_CUDA(cudaMemsetAsync(a.flags, 0, flag_bytes, st));
+  LFI_TRY(pipe_check_residency(kern, threads, smem_bytes, nk * P, what));
+  kern<<<dim3(2, nk, P), threads, smem_bytes, st>>>(a, P, ntiles, a.flags);
+  LFI_LAUNCH_CHECK();
+  return LFI_OK;
+}
+
+// Shape-only fit tests of the stage pipelines for whole-sequence training (K stages); each tests what it adds to the one
+// before it: pipe_supported, then pipe_tc_supported (forward) and pipe_bwd_tc_supported (backward).  Called by plan_core only.
+bool pipe_supported(const Dims &d, bool bwd);
+bool pipe_tc_supported(const Dims &d);
+bool pipe_bwd_tc_supported(const Dims &d);
 int pipe_bwd_smem_bytes(const Dims &d);
 int launch_fwd_pipe(const FwdArgs &a, cudaStream_t st);
 int launch_bwd_pipe(const BwdArgs &a, cudaStream_t st);
-// tensor-core variants (core_pipe_fwd_tc.cu): gate products as tcgen05.mma on split-bf16 operands, tensor-core GEMM modes only
-bool pipe_tc_supported(const Dims &d, int nk);
+// tensor-core variants (core_pipe_fwd_tc.cu, core_pipe_bwd_tc.cu): gate products as tcgen05.mma on split-bf16 operands
 int launch_fwd_pipe_tc(const FwdArgs &a, cudaStream_t st);
-bool pipe_bwd_tc_supported(const Dims &d);
 int launch_bwd_pipe_tc(const BwdArgs &a, cudaStream_t st);
 
 }  // namespace core

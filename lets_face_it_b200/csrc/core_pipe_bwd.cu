@@ -495,25 +495,10 @@ core_bwd_pipe(const BwdArgs a, const int P, const int ntiles, int *progress) {
 int pipe_bwd_smem_bytes(const Dims &d) { return plan_pipe_bwd(d).total * (int)sizeof(float); }
 
 int launch_bwd_pipe(const BwdArgs &a, cudaStream_t st) {
-  const int K = a.d.K;
   static const int timing = getenv("LFI_CORE_TIMING") ? atoi(getenv("LFI_CORE_TIMING")) : 0;
   if (timing) cudaMemcpyToSymbolAsync(g_core_timing_b, &timing, sizeof(int), 0, cudaMemcpyHostToDevice, st);
-  const int bytes = pipe_bwd_smem_bytes(a.d);
-  const int ntiles = (a.B + PR - 1) / PR;
-  int nsm = 0, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-  int P = nsm / (2 * K);
-  if (P > ntiles) P = ntiles;
-  LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * (K + 1) * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
   auto kern = a.dx_in ? core_bwd_pipe<true> : core_bwd_pipe<false>;
-  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * (K + 1) * 2 * sizeof(int), st));
-  dim3 grid(2, K, P);
-  LFI_TRY(pipe_check_residency(kern, PNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe"));
-  kern<<<grid, PNT, bytes, st>>>(a, P, ntiles, a.flags);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
+  return launch_pipe(kern, a, PNT, pipe_bwd_smem_bytes(a.d), a.d.K, a.d.K + 1, "core_bwd_pipe", st);
 }
 
 }  // namespace core

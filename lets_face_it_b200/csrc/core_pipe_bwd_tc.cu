@@ -602,33 +602,14 @@ core_bwd_pipe_tc(const BwdArgs a, const int P, const int ntiles, int *progress) 
 }
 
 // ------------------------------------------------------------------------------------------------
-bool pipe_bwd_tc_supported(const Dims &d) {
-  if (!env_flag("LFI_CORE_TC_BWD", true) || !pipe_tc_supported(d, d.K)) return false;
-  if (d.Ci > 32 || d.Co > 64 || d.C > 64) return false;
-  return plan_bt(d).total <= 227 * 1024;
-}
+bool pipe_bwd_tc_supported(const Dims &d) { return plan_bt(d).total <= 227 * 1024; }
 
 int launch_bwd_pipe_tc(const BwdArgs &a, cudaStream_t st) {
-  const int K = a.d.K;
+  LFI_REQUIRE(a.stash_tiled && a.pdG_hi && a.pdAh_hi, LFI_ERR_ARG, "tensor-core backward pipeline needs the tiled stash and plane outputs");
   static const int timing = getenv("LFI_CORE_TIMING") ? atoi(getenv("LFI_CORE_TIMING")) : 0;
   if (timing) cudaMemcpyToSymbolAsync(g_core_timing_bt, &timing, sizeof(int), 0, cudaMemcpyHostToDevice, st);
-  const int bytes = plan_bt(a.d).total;
-  const int ntiles = (a.B + PR - 1) / PR;
-  int nsm = 0, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-  int P = nsm / (2 * K);
-  if (P > ntiles) P = ntiles;
-  LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * (K + 1) * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
-  LFI_REQUIRE(a.stash_tiled && a.pdG_hi && a.pdAh_hi, LFI_ERR_ARG, "tensor-core backward pipeline needs the tiled stash and plane outputs");
   auto kern = a.dx_in ? core_bwd_pipe_tc<true> : core_bwd_pipe_tc<false>;
-  LFI_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * (K + 1) * 2 * sizeof(int), st));
-  dim3 grid(2, K, P);
-  LFI_TRY(pipe_check_residency(kern, BNT, bytes, (int)(grid.y * grid.z), "core_bwd_pipe_tc"));
-  kern<<<grid, BNT, bytes, st>>>(a, P, ntiles, a.flags);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
+  return launch_pipe(kern, a, BNT, plan_bt(a.d).total, a.d.K, a.d.K + 1, "core_bwd_pipe_tc", st);
 }
 
 }  // namespace core

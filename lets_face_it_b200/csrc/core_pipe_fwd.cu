@@ -342,23 +342,11 @@ core_fwd_pipe(const FwdArgs a, const int P, const int ntiles, int *progress) {
 // ------------------------------------------------------------------------------------------------
 constexpr int kPipeMaxSmem = 227 * 1024;
 
-static int sm_count() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
-
-bool pipe_supported(const Dims &d, int nk, bool bwd) {
-  if (!env_flag("LFI_CORE_PIPE", true)) return false;
+bool pipe_supported(const Dims &d, bool bwd) {
   if (d.G != 3 || d.H != 2 * PUC) return false;
   if (d.C > 64 || d.Co > 64 || d.C < 2) return false;
   if (d.affine && (d.Co & 1)) return false;
-  if (2 * nk > sm_count()) return false;
+  if (2 * d.K > sm_count()) return false;
   if (d.Ci > 32 || d.Cz > 32) return false;
   const int bytes = bwd ? pipe_bwd_smem_bytes(d) : plan_pipe(d).total * (int)sizeof(float);
   return bytes <= kPipeMaxSmem;
@@ -366,19 +354,7 @@ bool pipe_supported(const Dims &d, int nk, bool bwd) {
 
 int launch_fwd_pipe(const FwdArgs &a, cudaStream_t st) {
   const int nk = a.k_last - a.k_first + 1;
-  if (a.stash_tiled) return launch_fwd_pipe_tc(a, st);  // tensor-core GEMM modes (the caller checked pipe_tc_supported)
-  const int bytes = plan_pipe(a.d).total * (int)sizeof(float);
-  const int ntiles = (a.B + PR - 1) / PR;
-  int P = sm_count() / (2 * nk);
-  if (P > ntiles) P = ntiles;
-  LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * nk * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
-  LFI_CUDA(cudaFuncSetAttribute(core_fwd_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * nk * 2 * sizeof(int), st));
-  dim3 grid(2, nk, P);
-  LFI_TRY(pipe_check_residency(core_fwd_pipe, PNT, bytes, (int)(grid.y * grid.z), "core_fwd_pipe"));
-  core_fwd_pipe<<<grid, PNT, bytes, st>>>(a, P, ntiles, a.flags);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
+  return launch_pipe(core_fwd_pipe, a, PNT, plan_pipe(a.d).total * (int)sizeof(float), nk, nk, "core_fwd_pipe", st);
 }
 
 }  // namespace core

@@ -571,32 +571,14 @@ core_fwd_pipe_tc(const FwdArgs a, const int P, const int ntiles, int *progress) 
 }
 
 // ------------------------------------------------------------------------------------------------
-bool pipe_tc_supported(const Dims &d, int nk) {
-  if (!env_flag("LFI_CORE_TC", true) || !pipe_supported(d, nk, false)) return false;  // read at call time (tests toggle it)
-  if (d.Cip % 4 != 0 || d.Ci > 32 || d.Co > 64 || d.H != 2 * PUC) return false;
-  return plan_tc(d).total <= 227 * 1024;
-}
+bool pipe_tc_supported(const Dims &d) { return plan_tc(d).total <= 227 * 1024; }
 
 int launch_fwd_pipe_tc(const FwdArgs &a, cudaStream_t st) {
-  const int nk = a.k_last - a.k_first + 1;
-  const int bytes = plan_tc(a.d).total;
-  const int ntiles = (a.B + PR - 1) / PR;
-  int sms = 0, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (sms <= 0) sms = 148;
-  int P = sms / (2 * nk);
-  if (P > ntiles) P = ntiles;
-  LFI_REQUIRE(a.flags && P >= 1 && (size_t)P * nk * 2 * sizeof(int) <= a.flags_bytes, LFI_ERR_WORKSPACE, "flow core pipeline: flag buffer too small");
-  LFI_CUDA(cudaFuncSetAttribute(core_fwd_pipe_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  LFI_CUDA(cudaMemsetAsync(a.flags, 0, (size_t)P * nk * 2 * sizeof(int), st));
+  LFI_REQUIRE(a.stash_tiled, LFI_ERR_ARG, "tensor-core forward pipeline needs the tiled stash");
   static const int timing = getenv("LFI_CORE_TIMING") ? atoi(getenv("LFI_CORE_TIMING")) : 0;
   if (timing) cudaMemcpyToSymbolAsync(g_core_timing, &timing, sizeof(int), 0, cudaMemcpyHostToDevice, st);
-  dim3 grid(2, nk, P);
-  LFI_TRY(pipe_check_residency(core_fwd_pipe_tc, FNT, bytes, (int)(grid.y * grid.z), "core_fwd_pipe_tc"));
-  core_fwd_pipe_tc<<<grid, FNT, bytes, st>>>(a, P, ntiles, a.flags);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
+  const int nk = a.k_last - a.k_first + 1;
+  return launch_pipe(core_fwd_pipe_tc, a, FNT, plan_tc(a.d).total, nk, nk, "core_fwd_pipe_tc", st);
 }
 
 }  // namespace core

@@ -134,24 +134,18 @@ struct TrainWs {
   // backward
   float *dx, *dh, *dc, *dG, *dAh, *dO, *dzf, *dC, *dcond, *dWcF, *xg, *dhe, *dai, *dah;
   int *flags;  // progress counters of the stage-pipelined flow core
-  // tensor-core modes with the stage-pipelined core: GEMM operands of the flow-step contractions live as bf16 planes
-  // written by their producers (GEMM epilogues, core kernels), never re-split
-  bool cp, cp_lo;
-  bool st_tiled;  // gates / ahn / h stash in the tiled layout of the tensor-core flow-core pipeline
-  // hybrid wavefronts (shapes outside the stage pipelines, tensor-core modes): W_hh planes [K][GH][H] and the per-wavefront products
-  bool wave_tc;
+  // flow-core kernels; with plan.planes the GEMM operands of the flow-step contractions live as bf16 planes written by their
+  // producers (GEMM epilogues, core kernels), never re-split
+  core::CorePlan plan;
+  bool cp_lo;
+  // hybrid wavefronts (plan.fwd == WaveHybrid, which a backward on hybrid wavefronts implies): W_hh planes [K][GH][H] and the
+  // per-wavefront products
   void *wt_hi, *wt_lo;
   float *ghbuf;
   void *cact_hi, *cact_lo, *y_hi, *y_lo, *zf_hi, *zf_lo, *h_hi, *h_lo;
   void *dG_hi, *dG_lo, *dAh_hi, *dAh_lo, *dO_hi, *dO_lo, *dzf_hi, *dzf_lo, *dC_hi, *dC_lo;
   size_t bytes;
 };
-
-static bool core_planes_ok(const Dims &d, int mode) {
-  if (mode == LFI_GEMM_FP32) return false;
-  if (!core::pipe_supported(d, d.K, false) || !core::pipe_supported(d, d.K, true)) return false;
-  return d.C % 8 == 0 && d.Co % 8 == 0 && d.H % 8 == 0 && d.D % 8 == 0;
-}
 
 // Where the training state of a modality's encoder lives.  The training step lays all of it out in its one workspace; the module
 // API (lfi_feature_encode_fwd_train / _bwd) splits it into the caller's stash (what the backward reads), forward-only scratch, the
@@ -189,10 +183,11 @@ static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t
 static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode, void *ws, TrainWs *w) {
   Bump b(ws, 0);
   const size_t Tp = T - d.start_ts, M = Tp * B, K = d.K;
-  w->cp = core_planes_ok(d, mode); w->cp_lo = mode == LFI_GEMM_BF16X3;
+  w->plan = core::plan_core(d, B, mode); w->cp_lo = mode == LFI_GEMM_BF16X3;
+  const bool planes = w->plan.planes, hybrid = w->plan.fwd == core::CoreKernel::WaveHybrid;
   w->cond = b.take<float>(M * d.Fe);
   // operand-plane mode: the cond_transform activations and their gradients exist as bf16 planes only
-  w->Cact = w->cp ? nullptr : b.take<float>(M * K * d.D);
+  w->Cact = planes ? nullptr : b.take<float>(M * K * d.D);
   w->G = b.take<float>(round_up_sz(M, 32) * K * d.GH);  // (whole 32-row blocks: the row-interleaved layout of the tensor-core core)
   w->ld = b.take<float>(M);
   w->flags = b.take<int>(kFlagInts);
@@ -209,16 +204,13 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
   }
   w->gh = b.take<float>(ghmax);
   const size_t cells = K * M;
-  w->st_tiled = w->cp && core::pipe_tc_supported(d, d.K);
-  w->wave_tc = mode != LFI_GEMM_FP32 && !core::pipe_supported(d, d.K, false) && d.H % 8 == 0 && d.GH % 16 == 0 && B >= 16 &&
-               env_flag("LFI_WAVE_TC", true);
   w->wt_hi = w->wt_lo = nullptr; w->ghbuf = nullptr;
-  if (w->wave_tc) {
+  if (hybrid) {
     w->wt_hi = take_bf16(b, K * d.GH * d.H);
     w->wt_lo = mode == LFI_GEMM_BF16X3 ? take_bf16(b, K * d.GH * d.H) : nullptr;
     w->ghbuf = b.take<float>(2 * K * (size_t)B * d.GH);
   }
-  const size_t cells_t = w->st_tiled ? K * Tp * round_up_sz((size_t)B, 64) : cells;  // tiled stash: whole 64-sequence tiles
+  const size_t cells_t = w->plan.tiled ? K * Tp * round_up_sz((size_t)B, 64) : cells;  // tiled stash: whole 64-sequence tiles
   w->st.y = b.take<float>(cells * d.C);
   w->st.zf = b.take<float>(cells * d.C);
   w->st.h = b.take<float>(cells_t * d.H);
@@ -235,13 +227,13 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
   w->dAh = b.take<float>(cells * d.GH);
   w->dO = b.take<float>(cells * d.Co);
   w->dzf = b.take<float>(cells * d.C);
-  w->dC = w->cp ? nullptr : b.take<float>(M * K * d.D);
+  w->dC = planes ? nullptr : b.take<float>(M * K * d.D);
   w->dcond = b.take<float>(M * d.Fe);
   w->dWcF = b.take<float>(K * d.D * d.Fe);
   w->xg = b.take<float>(xgmax);
   w->dhe = b.take<float>(M * emax);
   w->dai = nullptr; w->dah = nullptr;
-  if (w->cp) {
+  if (planes) {
     auto two = [&](void *&hi, void *&lo_, size_t n) { hi = take_bf16(b, n); lo_ = w->cp_lo ? take_bf16(b, n) : nullptr; };
     two(w->cact_hi, w->cact_lo, M * K * d.D);
     two(w->y_hi, w->y_lo, cells * d.C); two(w->zf_hi, w->zf_lo, cells * d.C); two(w->h_hi, w->h_lo, cells * d.H);
@@ -251,7 +243,7 @@ static void plan_train(const lfi_shape *s, const Dims &d, int B, int T, int mode
   } else {
     w->cact_hi = w->cact_lo = w->y_hi = w->y_lo = w->zf_hi = w->zf_lo = w->h_hi = w->h_lo = nullptr;
     w->dG_hi = w->dG_lo = w->dAh_hi = w->dAh_lo = w->dO_hi = w->dO_lo = w->dzf_hi = w->dzf_lo = w->dC_hi = w->dC_lo = nullptr;
-    if (w->wave_tc) {  // hybrid wavefronts: the cells write the operands of the per-wavefront recurrent GEMMs (and of dW_hh, dWf) as planes
+    if (hybrid) {  // hybrid wavefronts: the cells write the operands of the per-wavefront recurrent GEMMs (and of dW_hh, dWf) as planes
       const bool lo = mode == LFI_GEMM_BF16X3;
       w->h_hi = take_bf16(b, cells * d.H);      w->h_lo = lo ? take_bf16(b, cells * d.H) : nullptr;
       w->dAh_hi = take_bf16(b, cells * d.GH);   w->dAh_lo = lo ? take_bf16(b, cells * d.GH) : nullptr;
@@ -604,8 +596,8 @@ int lfi_seq_train_fwd(const lfi_shape *s, const void *derived, const lfi_params 
   // the encoders read their parameters directly; the derived cache (composed 1x1 weights, folded W_c, transposes) is first needed
   // here - a caller that rebuilds it on another stream hands over the event to wait for (lfi_set_derived_ready_event)
   if (g_derived_ready_event) LFI_CUDA(cudaStreamWaitEvent(st, g_derived_ready_event, 0));
-  LFI_TRY(cond_to_gates(d, p, WcF, w.cond, M, w.Cact, w.G, gemm_mode, gws, gws_bytes, st, w.cp ? w.cact_hi : nullptr, w.cp ? w.cact_lo : nullptr,
-                        w.st_tiled));
+  LFI_TRY(cond_to_gates(d, p, WcF, w.cond, M, w.Cact, w.G, gemm_mode, gws, gws_bytes, st, w.plan.planes ? w.cact_hi : nullptr,
+                        w.plan.planes ? w.cact_lo : nullptr, w.plan.tiled));
 
   core::FwdArgs a;
   memset(&a, 0, sizeof(a));
@@ -616,15 +608,15 @@ int lfi_seq_train_fwd(const lfi_shape *s, const void *derived, const lfi_params 
   a.st_ahn = w.st.ahn; a.st_o = w.st.o; a.ld = w.ld; a.ld_accumulate = 0; a.nll = nll; a.z_out = z;
   a.scale_out = scale_out;
   a.flags = w.flags; a.flags_bytes = kFlagInts * sizeof(int);
-  if (w.cp) { a.py_hi = w.y_hi; a.py_lo = w.y_lo; a.pzf_hi = w.zf_hi; a.pzf_lo = w.zf_lo; a.ph_hi = w.h_hi; a.ph_lo = w.h_lo; }
-  a.stash_tiled = w.st_tiled ? 1 : 0;
-  a.g_tiled = w.st_tiled ? 1 : 0;
-  if (w.wave_tc) { a.ph_hi = w.h_hi; a.ph_lo = w.h_lo; }
-  if (w.wave_tc) {  // recurrent weights as operand planes, once per call (they change with every optimizer step)
+  if (w.plan.planes) { a.py_hi = w.y_hi; a.py_lo = w.y_lo; a.pzf_hi = w.zf_hi; a.pzf_lo = w.zf_lo; a.ph_hi = w.h_hi; a.ph_lo = w.h_lo; }
+  a.stash_tiled = w.plan.tiled ? 1 : 0;
+  a.g_tiled = w.plan.tiled ? 1 : 0;
+  if (w.plan.fwd == core::CoreKernel::WaveHybrid) {  // recurrent weights as operand planes, once per call (they change with every optimizer step)
+    a.ph_hi = w.h_hi; a.ph_lo = w.h_lo;
     LFI_TRY(split_to_planes(p->w_hh, d.GH, d.H, d.H, (long)d.GH * d.H, d.K, w.wt_hi, w.wt_lo, st));
     a.wtc.mode = gemm_mode; a.wtc.whh_hi = w.wt_hi; a.wtc.whh_lo = w.wt_lo; a.wtc.ghbuf = w.ghbuf; a.wtc.gws = gws; a.wtc.gws_bytes = gws_bytes;
   }
-  return core::launch_fwd(a, st);
+  return core::launch_fwd(a, w.plan.fwd, st);
 }
 
 // Backward of lfi_seq_train_fwd.  dx == nullptr: parameter gradients only (lfi_seq_train_bwd).  Otherwise (lfi_seq_train_bwd_dx)
@@ -680,21 +672,22 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   a.dx = w.dx; a.dh = w.dh; a.dc = w.dc; a.dG = w.dG; a.dAh = w.dAh; a.dO = w.dO; a.dzf = w.dzf;
   a.g_an_bias = g->an_bias; a.g_an_logs = g->an_logs; a.g_b_hh = g->b_hh; a.g_bf = g->bf; a.g_lf = g->lf;
   a.flags = w.flags; a.flags_bytes = kFlagInts * sizeof(int);
-  if (w.cp) {
+  const bool hybrid = w.plan.fwd == core::CoreKernel::WaveHybrid;
+  if (w.plan.planes) {
     a.dG = nullptr; a.dAh = nullptr; a.dO = nullptr; a.dzf = nullptr;
     a.pdG_hi = w.dG_hi; a.pdG_lo = w.dG_lo; a.pdAh_hi = w.dAh_hi; a.pdAh_lo = w.dAh_lo;
     a.pdO_hi = w.dO_hi; a.pdO_lo = w.dO_lo; a.pdzf_hi = w.dzf_hi; a.pdzf_lo = w.dzf_lo;
     a.g_b_ih = g->b_ih;
   }
-  a.stash_tiled = w.st_tiled ? 1 : 0;
-  if (w.wave_tc) { a.pdAh_hi = w.dAh_hi; a.pdAh_lo = w.dAh_lo; a.dAh = nullptr; }  // the cells write dA_h as operand planes only
-  if (w.wave_tc) {  // planes of W_hh were built by the forward call of this step
+  a.stash_tiled = w.plan.tiled ? 1 : 0;
+  if (hybrid) {  // the cells write dA_h as operand planes only; the planes of W_hh were built by the forward call of this step
+    a.pdAh_hi = w.dAh_hi; a.pdAh_lo = w.dAh_lo; a.dAh = nullptr;
     a.wtc.mode = gemm_mode; a.wtc.whh_hi = w.wt_hi; a.wtc.whh_lo = w.wt_lo; a.wtc.ghbuf = w.ghbuf; a.wtc.gws = gws; a.wtc.gws_bytes = gws_bytes;
   }
   // d(flow input) of every frame into the step-0 slot of the hand-off buffer, which nothing else writes or reads
   float *dflow = (dx && dx[0]) ? w.dx : nullptr;
   a.dx_in = dflow;
-  LFI_TRY(core::launch_bwd(a, st));
+  LFI_TRY(core::launch_bwd(a, w.plan.bwd, st));
 
   // 2. weight gradients of the per-step matrices as batched (over k) reductions over the M rows.  With every operand in
   //    plane form (no shared scratch) they are independent of the rest of the backward pass: they run on a side stream,
@@ -704,7 +697,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   LFI_TRY(dev_res(&dr));
   cudaStream_t wg_stream = dr->wg_stream;
   cudaEvent_t wg_fork = dr->wg_fork, wg_join = dr->wg_join;
-  const bool wg_par = w.cp;
+  const bool wg_par = w.plan.planes;
   cudaStream_t st_main = st;
   if (wg_par) {
     LFI_CUDA(cudaEventRecord(wg_fork, st_main));
@@ -718,7 +711,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
                    int ldc, long sC, PlaneRef pa = PlaneRef{nullptr, nullptr, 0, 0}, PlaneRef pb = PlaneRef{nullptr, nullptr, 0, 0}) -> int {
     GemmArgs q = gemm_args(1, 0, Mo, No, (int)red, A, lda, Bm, ldb, Cm, ldc, LFI_EPI_ACCUM);
     q.batch = K; q.sA = sA; q.sB = sB; q.sC = sC;
-    if (w.cp || w.wave_tc) { q.pA = pa; q.pB = pb; }  // (a plane reference with a null pointer means: split the fp32 operand)
+    if (w.plan.planes || hybrid) { q.pA = pa; q.pB = pb; }  // (a plane reference with a null pointer means: split the fp32 operand)
     return gemm_dispatch(bmode, q, gws, gws_bytes, st);
   };
   const PlaneRef pdG = plane_ref(w.dG_hi, w.dG_lo, K * GH, GH), ph = plane_ref(w.h_hi, w.h_lo, H, (long)(M * H));
@@ -733,8 +726,8 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
                 plane_ref(w.dO_hi, w.dO_lo, Co, (long)(M * Co)), ph));                                                 // dWf
   LFI_TRY(wgrad(C, C, M, w.st.y, C, (long)(M * C), w.dzf, C, (long)(M * C), g->w, C, (long)C * C,
                 plane_ref(w.y_hi, w.y_lo, C, (long)(M * C)), plane_ref(w.dzf_hi, w.dzf_lo, C, (long)(M * C))));       // dW (1x1 conv)
-  if (!w.cp) LFI_TRY(aux::colsum(g->b_ih, w.dG, K * GH, (int)M, K * GH, 1.0f, st));  // (planes: reduced inside the core kernel ...
-  if (w.st_tiled && core::pipe_bwd_tc_supported(d)) {
+  if (!w.plan.planes) LFI_TRY(aux::colsum(g->b_ih, w.dG, K * GH, (int)M, K * GH, 1.0f, st));  // (planes: reduced inside the core kernel ...
+  if (w.plan.bwd == core::CoreKernel::PipeTc) {
     // ... except with the tensor-core backward pipeline, which leaves the RNN bias gradients to column sums of its planes:
     // d b_ih = colsum(dG) (r, u parts also are d b_hh's), d b_hh n part = colsum of the n columns of dA_h)
     LFI_TRY(aux::colsum_planes(g->b_ih, g->b_hh, GH, 2 * H, 0, w.dG_hi, w.cp_lo ? w.dG_lo : nullptr, K * GH, 0, 1, (int)M, 0, K * GH, st));
@@ -746,17 +739,17 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   {
     GemmArgs q = gemm_args(0, 0, (int)M, D, GH, w.dG, K * GH, p->w_ih + Ci, In, w.dC, K * D, LFI_EPI_LRELU_BWD);
     q.batch = K; q.sA = GH; q.sB = (long)GH * In; q.sC = D; q.aux = w.Cact; q.ldaux = K * D; q.sAux = D;
-    if (w.cp) {  // planes in, planes out; LeakyReLU' from the sign of the activation plane; d b_c reduced in the epilogue
+    if (w.plan.planes) {  // planes in, planes out; LeakyReLU' from the sign of the activation plane; d b_c reduced in the epilogue
       q.pA = pdG; q.pOut = plane_ref(w.dC_hi, w.dC_lo, K * D, D); q.C = nullptr;
       q.aux = nullptr; q.auxp = w.cact_hi; q.ldauxp = K * D; q.sAuxp = D;
       q.colsum = g->bc; q.sColsum = D;
     }
     LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
-    if (!w.cp) LFI_TRY(aux::colsum(g->bc, w.dC, K * D, (int)M, K * D, 1.0f, st));
+    if (!w.plan.planes) LFI_TRY(aux::colsum(g->bc, w.dC, K * D, (int)M, K * D, 1.0f, st));
     // d W_c = dC^T cond: not needed by the rest of the backward pass.  With the side stream available it runs there, next to the
     // encoder backward (its operand-plane scratch sits behind the region the d cond GEMM of the main stream uses).
     GemmArgs r = gemm_args(1, 0, K * D, d.Fe, (int)M, w.dC, K * D, w.cond, d.Fe, w.dWcF, d.Fe, 0);
-    if (w.cp) r.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
+    if (w.plan.planes) r.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
     size_t side_off = 0;
     bool wc_side = false;
     if (wg_par) {
@@ -793,7 +786,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   if (enc_lo < 0 && !none_dx) { join_wgrads(); return LFI_OK; }
   auto dcond_gemm = [&](int lo, int hi) -> int {
     GemmArgs q = gemm_args(0, 0, (int)M, hi - lo, K * D, w.dC, K * D, WcF + lo, d.Fe, w.dcond + lo, d.Fe, 0);
-    if (w.cp) q.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
+    if (w.plan.planes) q.pA = plane_ref(w.dC_hi, w.dC_lo, K * D);
     return gemm_dispatch(bmode, q, gws, gws_bytes, st);
   };
   if (enc_lo >= 0) LFI_TRY(dcond_gemm(enc_lo, d.Fe));
@@ -1098,7 +1091,7 @@ static int flowstep_impl(const lfi_shape *s, const void *derived, const lfi_para
     a.st_h = h_out - koffH; a.st_c = c_out ? c_out - koffH : nullptr;
     a.ld = logdet; a.ld_accumulate = 1; a.nll = nullptr; a.z_out = y;
     a.scale_out = scale_out ? scale_out - (size_t)k * B * d.Cz : nullptr;
-    return core::launch_fwd(a, st);
+    return core::launch_fwd(a, core::CoreKernel::Wave, st);
   }
   // reverse: state is read and written in place by the persistent kernel
   if (h_in) LFI_CUDA(cudaMemcpyAsync(h_out, h_in, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -1320,7 +1313,7 @@ int lfi_flowstep_fwd_train(const lfi_shape *s, const void *derived, const lfi_pa
   a.st_gates = q.gates - kB * d.GH; a.st_ahn = d.G == 3 ? q.ahn - kB * d.H : nullptr; a.st_o = q.o - kB * d.Co;
   a.ld = logdet; a.ld_accumulate = 1; a.nll = nullptr; a.z_out = y;
   a.scale_out = scale_out ? scale_out - kB * d.Cz : nullptr;
-  LFI_TRY(core::launch_fwd(a, st));
+  LFI_TRY(core::launch_fwd(a, core::CoreKernel::Wave, st));
   LFI_CUDA(cudaMemcpyAsync(h_out, q.h, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
   if (d.G == 4) LFI_CUDA(cudaMemcpyAsync(c_out, q.c, (size_t)B * d.H * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return LFI_OK;
