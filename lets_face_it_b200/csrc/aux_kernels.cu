@@ -329,32 +329,6 @@ int enc_gate_fwd(const EncStep &a, cudaStream_t st) {
   return LFI_OK;
 }
 
-__global__ void enc_gate_bwd_kernel(EncStepBwd a) {
-  const int E = a.E;
-  const size_t n = (size_t)a.M * E;
-  for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < n; idx += (size_t)gridDim.x * blockDim.x) {
-    const int e = (int)(idx % E);
-    const size_t m = idx / E;
-    float dh = a.dh[idx];
-    if (a.dh_extra) dh += a.dh_extra[m * a.dh_extra_ld + e];
-    const float *g = a.gates + m * 3 * E;
-    const float rg = g[e], ug = g[E + e], ng = g[2 * E + e];
-    const float hp = a.hprev ? a.hprev[idx] : 0.f;
-    const float an = a.ahn[idx];
-    const float dn = dh * (1.0f - ug), du = dh * (hp - ng);
-    const float dan = dn * (1.0f - ng * ng), dau = du * ug * (1.0f - ug), dar = dan * an * rg * (1.0f - rg);
-    float *di = a.dai + m * 3 * E, *dhh = a.dah + m * 3 * E;
-    di[e] = dar; di[E + e] = dau; di[2 * E + e] = dan;
-    dhh[e] = dar; dhh[E + e] = dau; dhh[2 * E + e] = dan * rg;
-    a.dh[idx] = dh * ug;
-  }
-}
-int enc_gate_bwd(const EncStepBwd &a, cudaStream_t st) {
-  enc_gate_bwd_kernel<<<blocks_for((size_t)a.M * a.E), TB, 0, st>>>(a);
-  LFI_LAUNCH_CHECK();
-  return LFI_OK;
-}
-
 // thread = hidden unit e (coalesced over e), block = a strip of rows; the four bias-gradient sums stay in registers
 // kPart: the block adds its sums into its own row of part [blocks][4E] instead of issuing atomics
 template <bool kPart>

@@ -45,15 +45,6 @@ struct EncStep {
 };
 int enc_gate_fwd(const EncStep &a, cudaStream_t st);
 
-struct EncStepBwd {
-  const float *gates, *ahn, *hprev;  // stash of this step (hprev nullptr at s == 0)
-  float *dh;                         // [M][E] in: dL/dh_s ; out: dh * u (direct path to h_{s-1})
-  const float *dh_extra; int dh_extra_ld;  // optional extra dL/dh_s added first (d cond columns), nullable
-  float *dai, *dah;                  // [M][3E]
-  int M, E;
-};
-int enc_gate_bwd(const EncStepBwd &a, cudaStream_t st);
-
 // Gate backward of one window step for all M windows, writing the gate gradients in the form the batched weight-gradient
 // GEMMs consume (fp32, or bf16 planes in the tensor-core modes) and accumulating the bias gradients in-kernel:
 //   dah [M][3E] = (da_r, da_u, da_n * r)   (h-side pre-activations: dW_hh, dh_prev, db_hh)

@@ -81,15 +81,28 @@ static int derive_impl(const lfi_shape *s, const lfi_params *p, const float *win
 }
 
 // ------------------------------------------------------------------------------------------------
+// How the window GRU of one modality runs (plan_enc)
+enum class EncStepKind {
+  Unfused,  // per step: the recurrent GEMM into the shared gh scratch, then enc_gate_fwd
+  Fused,    // steps s >= 1: LFI_FUSE_GRU_FWD GEMMs; step 0 (zero state): enc_gate_fwd on the xp rows
+  FusedX,   // every step: a LFI_FUSE_GRU_FWD_X GEMM (input projection inside the step GEMM); step 0: the input part alone
+  Persist,  // all steps in one enc_gru_fwd_persist launch (enc_persist.cu)
+};
+struct EncPlan {
+  bool planes;       // bf16 operand planes, written by the producers themselves, never re-split
+  EncStepKind step;
+  bool stash;        // training: every step keeps h, gates and ahn for the backward pass (else h ping-pongs)
+  bool gates16;      // the gate stash in 16-bit fixed point (the fp32 mode keeps exact fp32 gates)
+};
+
 // workspace layouts
 struct EncWs {
   float *xp;     // [B*Tx][3E]
   float *hs;     // [hist][M][E]   (training) or [2][M][E] ping-pong (sampling)
   float *gates;  // [hist][M][3E]  (training only)
   float *ahn;    // [hist][M][E]   (training only)
-  // tensor-core modes (planes == true): bf16 operand planes written by the producers themselves, never re-split; the
-  // training stash keeps the gates in 16-bit fixed point (the fp32 mode keeps exact fp32 gates)
-  bool planes;
+  EncPlan plan;
+  // planes only
   void *hp_hi, *hp_lo;    // h          [hist | 2][M][E]
   void *whh_hi, *whh_lo;  // W_hh       [3E][E]  (K-major B of the step GEMM, MN-major B of dh_prev = dA_h W_hh)
   // backward (training only): gate gradients of every window step, kept for the batched weight-gradient GEMMs
@@ -97,33 +110,42 @@ struct EncWs {
   void *dah_hi, *dah_lo, *dan_hi, *dan_lo;  // planes, same shapes
   void *xg_hi, *xg_lo;    // masked window inputs [hist][M][round_up(dim, 8)]
   void *wih_hi, *wih_lo;  // W_ih       [3E][round_up(dim, 8)]  (input part of the fused forward step, LFI_FUSE_GRU_FWD_X)
-  bool xfuse;             // the forward steps take their input projection inside the step GEMM (planes, training, per-step path)
   float *xg32;            // the same in fp32 [hist][M][dim] (split source / fp32-mode operand)
   float *dhe;             // [M][E] running d h of the window recurrence
-  // persistent window-GRU forward (enc_persist.cu; sampling / feature encoding only): xp is time-major and row-interleaved
-  bool persist;
+  // Persist: xp is time-major and row-interleaved
   float *xT;              // [T*B][dim] raw frames in time-major order (input of the projection GEMM)
 };
 
-// A modality's encoder runs on operand planes when every GEMM it issues is taken by the tcgen05 tiles.
-static bool enc_use_planes(const lfi_shape *s, int m, size_t M, int mode) {
-  if (mode == LFI_GEMM_FP32) return false;
+// The path of modality m's window GRU over M windows (BT raw frames), for a training call (stash for the backward pass) or not.
+// The layouts (plan_enc_train, plan_sample) and every launch of build_cond, enc_bwd and seq_train_bwd follow it.
+//   planes   tensor-core mode, E >= 32, E % 8 == 0, dim >= 16, M >= 128, and the step GEMM [M, E] x [E, 3E] taken by the
+//            tcgen05 tiles (gemm_tc_wants): every GEMM of the encoder then runs there
+//   step     Persist  not training, planes, LFI_ENC_PERSIST_SAMPLE, encp::fwd_supported, and the projection GEMM
+//                     [BT, dim] x [dim, 3E] taken by the tcgen05 tiles (only those write the row-interleaved xp).  No stash to
+//                     store: 4 % faster than the per-step launches
+//            FusedX   training, planes, E % 64 == 0, LFI_ENC_XFUSE: the masked window inputs are gathered as operand planes in
+//                     the forward pass (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand
+//            Fused    planes, E % 64 == 0 (the fused GRU epilogue's tile of 64 hidden units)
+//            Unfused  otherwise
+//   stash    training
+//   gates16  training and planes
+// LFI_ENC_PERSIST_SAMPLE and LFI_ENC_XFUSE are read here only, at call time.
+static EncPlan plan_enc(const lfi_shape *s, int m, size_t M, size_t BT, int mode, bool training) {
   const int E = s->ehid[m], dim = s->dim[m];
-  if (E < 32 || E % 8 != 0 || dim < 16 || M < 128) return false;
-  GemmArgs g = gemm_args(0, 1, (int)M, 3 * E, E, nullptr, E, nullptr, E, nullptr, 3 * E);
-  return gemm_tc_wants(g);
-}
-// The persistent window-GRU forward kernel takes over a modality in sampling / feature encoding (no stash to store: 4 % faster
-// than the per-step launches; LFI_ENC_PERSIST_SAMPLE=0 turns it off, read at call time) when its encoder runs on operand planes,
-// the shape fits the kernel and the projection GEMM is taken by the tcgen05 tiles (only those write the row-interleaved xp).
-// Training always runs the per-step launches, which write the stash of the backward pass.
-static bool enc_use_persist(const lfi_shape *s, int m, size_t M, size_t BT, int mode) {
-  if (!env_flag("LFI_ENC_PERSIST_SAMPLE", true)) return false;
-  if (!enc_use_planes(s, m, M, mode)) return false;
-  const int E = s->ehid[m], hist = s->hist[m];
-  if (!encp::fwd_supported(E, hist, M, mode)) return false;
-  GemmArgs g = gemm_args(0, 1, (int)BT, 3 * E, s->dim[m], nullptr, s->dim[m], nullptr, s->dim[m], nullptr, 3 * E);
-  return gemm_tc_wants(g);
+  EncPlan p;
+  p.planes = mode != LFI_GEMM_FP32 && E >= 32 && E % 8 == 0 && dim >= 16 && M >= 128 &&
+             gemm_tc_wants(gemm_args(0, 1, (int)M, 3 * E, E, nullptr, E, nullptr, E, nullptr, 3 * E));
+  const bool fused = p.planes && E % 64 == 0;
+  if (!training && p.planes && env_flag("LFI_ENC_PERSIST_SAMPLE", true) && encp::fwd_supported(E, s->hist[m], M, mode) &&
+      gemm_tc_wants(gemm_args(0, 1, (int)BT, 3 * E, dim, nullptr, dim, nullptr, dim, nullptr, 3 * E)))
+    p.step = EncStepKind::Persist;
+  else if (fused && training && env_flag("LFI_ENC_XFUSE", true))
+    p.step = EncStepKind::FusedX;
+  else
+    p.step = fused ? EncStepKind::Fused : EncStepKind::Unfused;
+  p.stash = training;
+  p.gates16 = training && p.planes;
+  return p;
 }
 static void *take_bf16(Bump &b, size_t n) { return (void *)b.take<uint16_t>(n); }
 constexpr size_t kFlagInts = 1024;
@@ -159,8 +181,8 @@ static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t
   e.hs = S.take<float>(h * M * E);
   e.gates = S.take<float>(h * M * 3 * E);
   e.ahn = S.take<float>(h * M * E);
-  e.planes = enc_use_planes(s, m, M, mode);
-  if (e.planes) {
+  e.plan = plan_enc(s, m, M, B * T, mode, true);
+  if (e.plan.planes) {
     const bool lo = mode == LFI_GEMM_BF16X3;
     const size_t dimp = round_up(s->dim[m], 8);
     e.hp_hi = take_bf16(S, h * M * E);            e.hp_lo = lo ? take_bf16(S, h * M * E) : nullptr;
@@ -169,9 +191,6 @@ static void plan_enc_train(const lfi_shape *s, int m, size_t B, size_t T, size_t
     e.dan_hi = take_bf16(K, h * M * E);           e.dan_lo = lo ? take_bf16(K, h * M * E) : nullptr;
     e.xg_hi = take_bf16(S, h * M * dimp);         e.xg_lo = lo ? take_bf16(S, h * M * dimp) : nullptr;
     e.wih_hi = take_bf16(W, 3 * E * dimp);        e.wih_lo = lo ? take_bf16(W, 3 * E * dimp) : nullptr;
-    // input projection inside the fused step GEMM: the masked window inputs are gathered as operand planes in the forward pass
-    // (the backward pass needs them anyway for dW_ih) and W_ih joins the B operand; step 0 (no state yet) keeps the xp rows
-    e.xfuse = E % 64 == 0 && env_flag("LFI_ENC_XFUSE", true);
   } else {
     e.dah32 = K.take<float>(h * M * 3 * E);
     e.dan32 = K.take<float>(h * M * E);
@@ -285,14 +304,28 @@ static int dev_res(DevRes **out) {
   *out = &r;
   return LFI_OK;
 }
+// Fork / join of n modality chains: chain i >= 1 runs on r.enc_side[i], chain 0 on st.  The join records and waits without
+// checking, so that it also runs after an error.
+static int enc_fork(const DevRes &r, int n, cudaStream_t st) {
+  LFI_CUDA(cudaEventRecord(r.enc_fork, st));
+  for (int i = 1; i < n; ++i) LFI_CUDA(cudaStreamWaitEvent(r.enc_side[i], r.enc_fork, 0));
+  return LFI_OK;
+}
+static void enc_join(const DevRes &r, int n, cudaStream_t st) {
+  for (int i = 1; i < n; ++i) {
+    cudaEventRecord(r.enc_join[i], r.enc_side[i]);
+    cudaStreamWaitEvent(st, r.enc_join[i], 0);
+  }
+}
 
 // Encoders + "enc: none" windows into the folded feature matrix cond[M][Fe] for frames
 // t = t0 .. t0+Tp-1 (ModalityEncoder / FeatureEncoder, models.py:55-80, 127-145).
 //   x stream m: [B][Tx][dim] ;  skip_p1: leave the p1_face columns alone (autoregressive sampler)
-//   stash != 0: keep every step's h / gates / ahn (training); else ping-pong h
+//   project: also the window-independent input projections and W_hh planes (the sampler's later chunks reuse them)
+//   enc[m].plan: the path of each GRU modality (plan_enc)
 static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, const lfi_batch *bt, int t0, int Tp,
-                      float *cond, EncWs *enc, float *gh, bool stash, bool skip_p1, bool project, int mode, void *gws,
-                      size_t gws_bytes, cudaStream_t st) {
+                      float *cond, EncWs *enc, float *gh, bool skip_p1, bool project, int mode, void *gws, size_t gws_bytes,
+                      cudaStream_t st) {
   const int B = bt->B, T = bt->T;
   const size_t M = (size_t)Tp * B;
   const bool lo = mode == LFI_GEMM_BF16X3;
@@ -309,27 +342,28 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       LFI_TRY(aux::gather_windows(cond + d.enc_offe[m], d.Fe, 0, bt->x[m], bt->mask[m], B, T, dim, hist, m == 0 ? 0 : 1, t0, Tp, st));
       continue;
     }
+    EncWs &ew = enc[m];
+    const EncStepKind kind = ew.plan.step;
     // input projection for every raw frame (window independent): xp = x @ W_ih^T
-    if (project && enc[m].persist) {
+    if (project && kind == EncStepKind::Persist) {
       // raw frames in time-major order (row tau * B + b), projected into the row-interleaved layout the persistent kernel reads
-      LFI_TRY(aux::gather_windows(enc[m].xT, dim, 1, bt->x[m], nullptr, B, T, dim, 1, 1, 0, T, st));
-      GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, enc[m].xT, dim, p->enc_w_ih[m], dim, enc[m].xp, 3 * E);
+      LFI_TRY(aux::gather_windows(ew.xT, dim, 1, bt->x[m], nullptr, B, T, dim, 1, 1, 0, T, st));
+      GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, ew.xT, dim, p->enc_w_ih[m], dim, ew.xp, 3 * E);
       g.c_tiled32 = 1;
       LFI_TRY(gemm_dispatch(mode, g, gws, gws_bytes, st));
-    } else if (project && !(stash && enc[m].xfuse)) {  // (fused into the step GEMMs otherwise)
-      GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, bt->x[m], dim, p->enc_w_ih[m], dim, enc[m].xp, 3 * E);
+    } else if (project && kind != EncStepKind::FusedX) {  // (FusedX: inside the step GEMMs)
+      GemmArgs g = gemm_args(0, 1, B * T, 3 * E, dim, bt->x[m], dim, p->enc_w_ih[m], dim, ew.xp, 3 * E);
       LFI_TRY(gemm_dispatch(mode, g, gws, gws_bytes, st));
     }
-    EncWs &ew = enc[m];
-    if (ew.planes && project)  // W_hh planes: once per call (weights change every optimizer step)
+    if (ew.plan.planes && project)  // W_hh planes: once per call (weights change every optimizer step)
       LFI_TRY(split_to_planes(p->enc_w_hh[m], 3 * E, E, E, 0, 1, ew.whh_hi, lo ? ew.whh_lo : nullptr, st));
-    if (stash && ew.xfuse) {
+    if (kind == EncStepKind::FusedX) {
       const int dimp = round_up(dim, 8);
       LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
       LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * E, dim, dim, 0, 1, ew.wih_hi, lo ? ew.wih_lo : nullptr, st));
     }
     mods[nmods++] = m;
-    all_fused = all_fused && ew.planes && (ew.persist || E % 64 == 0);
+    all_fused = all_fused && kind != EncStepKind::Unfused;
   }
   // ---- phase 2: the window recurrences.  With the fused GRU launches (operands in plane form, no shared scratch) the
   //      modalities are independent chains: they run on parallel streams forked from / joined to the caller's, so that the
@@ -337,7 +371,8 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
   auto chain = [&](int m, cudaStream_t cs) -> int {
     const int hist = s->hist[m], E = s->ehid[m];
     EncWs &ew = enc[m];
-    if (ew.persist) {
+    const EncPlan &pl = ew.plan;
+    if (pl.step == EncStepKind::Persist) {
       // persistent window GRU: all `hist` steps of a 128-window tile in one launch, state resident in shared memory
       encp::FwdArgs a;
       memset(&a, 0, sizeof(a));
@@ -348,72 +383,60 @@ static int build_cond(const lfi_shape *s, const Dims &d, const lfi_params *p, co
       return encp::launch_fwd(a, cs);
     }
     for (int sidx = 0; sidx < hist; ++sidx) {
-      float *hprev = nullptr, *hcur;
-      const int cur = stash ? sidx : (sidx & 1), prv = stash ? sidx - 1 : ((sidx - 1) & 1);
-      hcur = ew.hs + (size_t)cur * M * E;
-      if (sidx) hprev = ew.hs + (size_t)prv * M * E;
-      const bool xf = stash && ew.xfuse;  // input projection inside the step GEMM: also step 0 (input part alone)
-      const bool fused = ew.planes && E % 64 == 0 && (sidx || xf);
-      if (sidx && !fused) {
-        GemmArgs gg = gemm_args(0, 1, (int)M, 3 * E, E, hprev, E, p->enc_w_hh[m], E, gh, 3 * E);
-        if (ew.planes) {
-          gg.pA = plane_ref((uint16_t *)ew.hp_hi + (size_t)prv * M * E, lo ? (uint16_t *)ew.hp_lo + (size_t)prv * M * E : nullptr, E);
-          gg.pB = plane_ref(ew.whh_hi, ew.whh_lo, E);
+      const int cur = pl.stash ? sidx : (sidx & 1), prv = pl.stash ? sidx - 1 : ((sidx - 1) & 1);
+      float *hprev = sidx ? ew.hs + (size_t)prv * M * E : nullptr, *hcur = ew.hs + (size_t)cur * M * E;
+      const size_t pslot = sidx ? (size_t)prv : 0;  // (step 0 reads no state: its plane reference only shapes the tensor map)
+      const PlaneRef ph = plane_ref(off16(ew.hp_hi, pslot * M * E), off16(ew.hp_lo, pslot * M * E), E);
+      const PlaneRef pw = plane_ref(ew.whh_hi, ew.whh_lo, E);
+      auto fill = [&](auto &q) {  // the arguments aux::EncStep and GruEpi share
+        q.xp = ew.xp; q.b_ih = p->enc_b_ih[m]; q.b_hh = p->enc_b_hh[m]; q.mask = bt->mask[m]; q.hprev = hprev; q.h = hcur;
+        q.gates = pl.stash ? ew.gates + (size_t)sidx * M * 3 * E : nullptr;
+        q.ahn = pl.stash ? ew.ahn + (size_t)sidx * M * E : nullptr;
+        q.cond = (sidx == hist - 1) ? cond + d.enc_offe[m] : nullptr; q.cond_ld = d.Fe;
+        q.h_hi = off16(ew.hp_hi, (size_t)cur * M * E); q.h_lo = off16(ew.hp_lo, (size_t)cur * M * E);
+        q.s = sidx; q.hist = hist; q.B = B; q.T = T; q.t0 = t0; q.E = E; q.gates16 = pl.gates16 ? 1 : 0;
+      };
+      auto gate_step = [&]() -> int {  // (s >= 1: after the recurrent product into the shared gh scratch)
+        if (sidx) {
+          GemmArgs gg = gemm_args(0, 1, (int)M, 3 * E, E, hprev, E, p->enc_w_hh[m], E, gh, 3 * E);
+          if (pl.planes) { gg.pA = ph; gg.pB = pw; }
+          LFI_TRY(gemm_dispatch(mode, gg, gws, gws_bytes, cs));
         }
-        LFI_TRY(gemm_dispatch(mode, gg, gws, gws_bytes, cs));
-      }
-      aux::EncStep a;
-      a.xp = ew.xp; a.gh = sidx ? gh : nullptr; a.b_ih = p->enc_b_ih[m]; a.b_hh = p->enc_b_hh[m];
-      a.mask = bt->mask[m]; a.hprev = hprev; a.h = hcur;
-      a.gates = stash ? ew.gates + (size_t)sidx * M * 3 * E : nullptr;
-      a.ahn = stash ? ew.ahn + (size_t)sidx * M * E : nullptr;
-      a.cond = (sidx == hist - 1) ? cond + d.enc_offe[m] : nullptr; a.cond_ld = d.Fe;
-      a.h_hi = ew.planes ? (void *)((uint16_t *)ew.hp_hi + (size_t)cur * M * E) : nullptr;
-      a.h_lo = (ew.planes && lo) ? (void *)((uint16_t *)ew.hp_lo + (size_t)cur * M * E) : nullptr;
-      a.s = sidx; a.hist = hist; a.B = B; a.T = T; a.Tp = Tp; a.t0 = t0; a.E = E;
-      a.gates16 = (stash && ew.planes) ? 1 : 0;
-      if (fused) {
-        // recurrent product and gate math in one launch: the [M, 3E] pre-activations stay in TMEM
+        aux::EncStep a;
+        fill(a);
+        a.gh = sidx ? gh : nullptr; a.Tp = Tp;
+        return aux::enc_gate_fwd(a, cs);
+      };
+      auto fused_step = [&](int fuse) -> int {  // recurrent product and gate math in one launch: the [M, 3E] pre-activations stay in TMEM
         GemmArgs gg = gemm_args(0, 1, (int)M, 3 * E, E, nullptr, E, nullptr, E, nullptr, 3 * E);
-        const size_t pslot = sidx ? (size_t)prv : 0;  // (step 0 reads no state: the plane reference only shapes the tensor map)
-        gg.pA = plane_ref((uint16_t *)ew.hp_hi + pslot * M * E, lo ? (uint16_t *)ew.hp_lo + pslot * M * E : nullptr, E);
-        gg.pB = plane_ref(ew.whh_hi, ew.whh_lo, E);
-        gg.fuse = LFI_FUSE_GRU_FWD;
+        gg.pA = ph; gg.pB = pw; gg.fuse = fuse;
         GruEpi &q = gg.gru;
-        if (xf) {
+        fill(q);
+        if (fuse == LFI_FUSE_GRU_FWD_X) {
           const int dimp = round_up(s->dim[m], 8);
-          gg.fuse = LFI_FUSE_GRU_FWD_X;
-          q.xa_hi = (uint16_t *)ew.xg_hi + (size_t)sidx * M * dimp; q.xa_lo = lo ? (uint16_t *)ew.xg_lo + (size_t)sidx * M * dimp : nullptr;
-          q.xb_hi = ew.wih_hi; q.xb_lo = lo ? ew.wih_lo : nullptr; q.xa_ld = dimp; q.xb_ld = dimp; q.xk = dimp;
+          q.xa_hi = off16(ew.xg_hi, (size_t)sidx * M * dimp); q.xa_lo = off16(ew.xg_lo, (size_t)sidx * M * dimp);
+          q.xb_hi = ew.wih_hi; q.xb_lo = ew.wih_lo; q.xa_ld = dimp; q.xb_ld = dimp; q.xk = dimp;
           q.x_only = sidx == 0 ? 1 : 0;
         }
-        q.E = E; q.s = sidx; q.hist = hist; q.B = B; q.T = T; q.t0 = t0; q.gates16 = a.gates16;
-        q.xp = a.xp; q.b_ih = a.b_ih; q.b_hh = a.b_hh; q.mask = a.mask; q.hprev = a.hprev;
-        q.h = a.h; q.gates = a.gates; q.ahn = a.ahn; q.cond = a.cond; q.cond_ld = a.cond_ld; q.h_hi = a.h_hi; q.h_lo = a.h_lo;
-        LFI_TRY(gemm_dispatch(mode, gg, gws, gws_bytes, cs));
-        continue;
+        return gemm_dispatch(mode, gg, gws, gws_bytes, cs);
+      };
+      switch (pl.step) {
+        case EncStepKind::FusedX: LFI_TRY(fused_step(LFI_FUSE_GRU_FWD_X)); break;
+        case EncStepKind::Fused: LFI_TRY(sidx ? fused_step(LFI_FUSE_GRU_FWD) : gate_step()); break;
+        default: LFI_TRY(gate_step()); break;  // Unfused (Persist returned above)
       }
-      LFI_TRY(aux::enc_gate_fwd(a, cs));
     }
     return LFI_OK;
   };
   const bool par = nmods > 1 && all_fused;
-  if (!par) {
-    for (int i = 0; i < nmods; ++i) LFI_TRY(chain(mods[i], st));
-    return LFI_OK;
-  }
   DevRes *dr = nullptr;
-  LFI_TRY(dev_res(&dr));
-  cudaStream_t *side = dr->enc_side;
-  cudaEvent_t ev_fork = dr->enc_fork, *ev_join = dr->enc_join;
-  LFI_CUDA(cudaEventRecord(ev_fork, st));
-  for (int i = 1; i < nmods; ++i) LFI_CUDA(cudaStreamWaitEvent(side[i], ev_fork, 0));
-  int rc = LFI_OK;
-  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = chain(mods[i], i == 0 ? st : side[i]);
-  for (int i = 1; i < nmods; ++i) {  // always join, also on error
-    cudaEventRecord(ev_join[i], side[i]);
-    cudaStreamWaitEvent(st, ev_join[i], 0);
+  if (par) {
+    LFI_TRY(dev_res(&dr));
+    LFI_TRY(enc_fork(*dr, nmods, st));
   }
+  int rc = LFI_OK;
+  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = chain(mods[i], par && i ? dr->enc_side[i] : st);
+  if (par) enc_join(*dr, nmods, st);  // always join, also on error
   return rc;
 }
 
@@ -437,9 +460,9 @@ static int enc_bwd(const lfi_shape *s, const Dims &d, const lfi_params *p, const
   const bool det = o.part != nullptr;
   const int wepi = det ? 0 : LFI_EPI_ACCUM;
   const int dimp = round_up(dim, 8);
-  if (ew.planes && ew.xfuse) {
+  if (ew.plan.step == EncStepKind::FusedX) {
     // (gathered by the forward pass, which fed them to its fused step GEMMs)
-  } else if (ew.planes)  // masked window inputs straight into the operand planes of the dW_ih GEMMs
+  } else if (ew.plan.planes)  // masked window inputs straight into the operand planes of the dW_ih GEMMs
     LFI_TRY(aux::gather_windows_planes(ew.xg_hi, lo ? ew.xg_lo : nullptr, dimp, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
   else
     LFI_TRY(aux::gather_windows(ew.xg32, dim, 1, bt->x[m], bt->mask[m], B, T, dim, hist, 1, t0, Tp, st));
@@ -451,17 +474,17 @@ static int enc_bwd(const lfi_shape *s, const Dims &d, const lfi_params *p, const
     e.gates = ew.gates + (size_t)sidx * M * 3 * E; e.ahn = ew.ahn + (size_t)sidx * M * E;
     e.hprev = sidx ? ew.hs + (size_t)(sidx - 1) * M * E : nullptr;
     e.dh = ew.dhe; e.dh_extra = (sidx == hist - 1) ? dcond + d.enc_offe[m] : nullptr; e.dh_extra_ld = d.Fe;
-    if (ew.planes) {
+    if (ew.plan.planes) {
       e.dah_hi = off16(ew.dah_hi, (size_t)sidx * M * 3 * E); e.dah_lo = lo ? off16(ew.dah_lo, (size_t)sidx * M * 3 * E) : nullptr;
       e.dan_hi = off16(ew.dan_hi, (size_t)sidx * M * E);     e.dan_lo = lo ? off16(ew.dan_lo, (size_t)sidx * M * E) : nullptr;
     } else {
       e.dah32 = ew.dah32 + (size_t)sidx * M * 3 * E; e.dan32 = ew.dan32 + (size_t)sidx * M * E;
     }
-    e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.planes ? 1 : 0;
+    e.gb_ih = g->enc_b_ih[m]; e.gb_hh = g->enc_b_hh[m]; e.M = (int)M; e.E = E; e.gates16 = ew.plan.gates16 ? 1 : 0;
     LFI_TRY(aux::enc_gate_bwd2(e, st, o.part));
     if (sidx) {  // dh_{s-1} += dA_h W_hh
       GemmArgs t = gemm_args(0, 0, (int)M, E, 3 * E, e.dah32, 3 * E, p->enc_w_hh[m], E, ew.dhe, E, det ? LFI_EPI_ACCUM_PRE : LFI_EPI_ACCUM);
-      if (ew.planes) { t.pA = plane_ref(e.dah_hi, e.dah_lo, 3 * E); t.pB = plane_ref(ew.whh_hi, ew.whh_lo, E); }
+      if (ew.plan.planes) { t.pA = plane_ref(e.dah_hi, e.dah_lo, 3 * E); t.pB = plane_ref(ew.whh_hi, ew.whh_lo, E); }
       LFI_TRY(gemm_dispatch(bmode, t, gws, gws_bytes, st));
     }
   }
@@ -469,23 +492,23 @@ static int enc_bwd(const lfi_shape *s, const Dims &d, const lfi_params *p, const
   const int Kall = (int)(hist * M), Khh = (int)((hist - 1) * M);
   if (hist > 1) {  // dW_hh += sum_{s>=1} dA_h[s]^T h[s-1]
     GemmArgs q = gemm_args(1, 0, 3 * E, E, Khh, ew.dah32 ? ew.dah32 + M * 3 * E : nullptr, 3 * E, ew.hs, E, g->enc_w_hh[m], E, wepi);
-    if (ew.planes) { q.pA = plane_ref(off16(ew.dah_hi, M * 3 * E), lo ? off16(ew.dah_lo, M * 3 * E) : nullptr, 3 * E); q.pB = plane_ref(ew.hp_hi, ew.hp_lo, E); }
+    if (ew.plan.planes) { q.pA = plane_ref(off16(ew.dah_hi, M * 3 * E), lo ? off16(ew.dah_lo, M * 3 * E) : nullptr, 3 * E); q.pB = plane_ref(ew.hp_hi, ew.hp_lo, E); }
     LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
   } else if (det) {
     LFI_CUDA(cudaMemsetAsync(g->enc_w_hh[m], 0, (size_t)3 * E * E * sizeof(float), st));
   }
   {  // dW_ih rows [0,2E) += dA_h[:, :2E]^T x  (r, u blocks coincide with the i-side gradients); rows [2E,3E) += dA_n^T x
     GemmArgs q = gemm_args(1, 0, 2 * E, dim, Kall, ew.dah32, 3 * E, ew.xg32, dim, g->enc_w_ih[m], dim, wepi);
-    if (ew.planes) { q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
+    if (ew.plan.planes) { q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
     LFI_TRY(gemm_dispatch(bmode, q, gws, gws_bytes, st));
     GemmArgs r = gemm_args(1, 0, E, dim, Kall, ew.dan32, E, ew.xg32, dim, g->enc_w_ih[m] + (size_t)2 * E * dim, dim, wepi);
-    if (ew.planes) { r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E); r.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
+    if (ew.plan.planes) { r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E); r.pB = plane_ref(ew.xg_hi, ew.xg_lo, dimp); }
     LFI_TRY(gemm_dispatch(bmode, r, gws, gws_bytes, st));
   }
   if (o.dx) {  // dXg = dA_h[:, :2E] W_ih[:2E] + dA_n W_ih[2E:] (ACCUM_PRE: neither launch splits K), then the adjoint of the gather
     GemmArgs q = gemm_args(0, 0, Kall, dim, 2 * E, ew.dah32, 3 * E, p->enc_w_ih[m], dim, o.dxg, dim, 0);
     GemmArgs r = gemm_args(0, 0, Kall, dim, E, ew.dan32, E, p->enc_w_ih[m] + (size_t)2 * E * dim, dim, o.dxg, dim, LFI_EPI_ACCUM_PRE);
-    if (ew.planes) {
+    if (ew.plan.planes) {
       q.pA = plane_ref(ew.dah_hi, ew.dah_lo, 3 * E); q.pB = plane_ref(ew.wih_hi, ew.wih_lo, dimp);
       r.pA = plane_ref(ew.dan_hi, ew.dan_lo, E);
       r.pB = plane_ref(off16(ew.wih_hi, (size_t)2 * E * dimp), lo ? off16(ew.wih_lo, (size_t)2 * E * dimp) : nullptr, dimp);
@@ -592,7 +615,7 @@ int lfi_seq_train_fwd(const lfi_shape *s, const void *derived, const lfi_params 
   const DerivedLayout L = derived_layout(d);
   const float *WcF = (const float *)derived + L.WcF;
 
-  LFI_TRY(build_cond(s, d, p, bt, d.start_ts, Tp, w.cond, w.enc, w.gh, true, false, true, gemm_mode, gws, gws_bytes, st));
+  LFI_TRY(build_cond(s, d, p, bt, d.start_ts, Tp, w.cond, w.enc, w.gh, false, true, gemm_mode, gws, gws_bytes, st));
   // the encoders read their parameters directly; the derived cache (composed 1x1 weights, folded W_c, transposes) is first needed
   // here - a caller that rebuilds it on another stream hands over the event to wait for (lfi_set_derived_ready_event)
   if (g_derived_ready_event) LFI_CUDA(cudaStreamWaitEvent(st, g_derived_ready_event, 0));
@@ -810,7 +833,7 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   auto enc_chain = [&](int m, cudaStream_t cs) -> int {
     float *dxm = dx ? dx[m] : nullptr;
     EncWs &ew = w.enc[m];
-    if (dxm && ew.planes && !ew.xfuse)  // (the fused forward steps built the W_ih planes already)
+    if (dxm && ew.plan.planes && ew.plan.step != EncStepKind::FusedX)  // (FusedX: the forward steps built the W_ih planes)
       LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * s->ehid[m], s->dim[m], s->dim[m], 0, 1, ew.wih_hi,
                               gemm_mode == LFI_GEMM_BF16X3 ? ew.wih_lo : nullptr, cs));
     const EncBwdOpts o = {nullptr, 0, dxm ? xw.dxg[m] : nullptr, dxm};
@@ -819,26 +842,13 @@ static int seq_train_bwd(const lfi_shape *s, const void *derived, const lfi_para
   int mods[LFI_NMOD], nmods = 0;
   bool all_planes = true;
   for (int m = 0; m < LFI_NMOD; ++m)
-    if (s->hist[m] > 0 && s->ehid[m] > 0) { mods[nmods++] = m; all_planes = all_planes && w.enc[m].planes; }
-  cudaStream_t *side = dr->enc_side;
-  cudaEvent_t ev_fork = dr->enc_fork, *ev_join = dr->enc_join;
+    if (s->hist[m] > 0 && s->ehid[m] > 0) { mods[nmods++] = m; all_planes = all_planes && w.enc[m].plan.planes; }
   const bool par = nmods > 1 && all_planes;
-  if (!par) {
-    int rc = LFI_OK;
-    for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], st);
-    if (rc == LFI_OK) rc = none_grads();
-    join_wgrads();
-    return rc;
-  }
-  LFI_CUDA(cudaEventRecord(ev_fork, st));
-  for (int i = 1; i < nmods; ++i) LFI_CUDA(cudaStreamWaitEvent(side[i], ev_fork, 0));
+  if (par) LFI_TRY(enc_fork(*dr, nmods, st));
   int rc = LFI_OK;
-  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], i == 0 ? st : side[i]);
+  for (int i = 0; i < nmods && rc == LFI_OK; ++i) rc = enc_chain(mods[i], par && i ? dr->enc_side[i] : st);
   if (rc == LFI_OK) rc = none_grads();
-  for (int i = 1; i < nmods; ++i) {  // always join, also on error
-    cudaEventRecord(ev_join[i], side[i]);
-    cudaStreamWaitEvent(st, ev_join[i], 0);
-  }
+  if (par) enc_join(*dr, nmods, st);  // always join, also on error
   join_wgrads();
   return rc;
 }
@@ -898,10 +908,9 @@ static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chu
     EncWs &e = w->enc[m];
     e.xp = b.take<float>(encp::tiled_rows((size_t)B * T) * 3 * E);
     e.hs = b.take<float>(2 * Mc * E);
-    e.planes = enc_use_planes(s, m, Mc, mode);
-    e.persist = enc_use_persist(s, m, Mc, (size_t)B * T, mode);
-    e.xT = e.persist ? b.take<float>((size_t)B * T * s->dim[m]) : nullptr;
-    if (e.planes) {
+    e.plan = plan_enc(s, m, Mc, (size_t)B * T, mode, false);
+    e.xT = e.plan.step == EncStepKind::Persist ? b.take<float>((size_t)B * T * s->dim[m]) : nullptr;
+    if (e.plan.planes) {
       const bool lo = mode == LFI_GEMM_BF16X3;
       e.hp_hi = take_bf16(b, 2 * Mc * E);  e.hp_lo = lo ? take_bf16(b, 2 * Mc * E) : nullptr;
       e.whh_hi = take_bf16(b, 3 * E * E);  e.whh_lo = lo ? take_bf16(b, 3 * E * E) : nullptr;
@@ -942,7 +951,7 @@ int lfi_feature_encode(const lfi_shape *s, const lfi_params *p, const lfi_batch 
   LFI_REQUIRE(ws_bytes >= w.bytes + gemm_scratch_bound(s, d, (size_t)Tp * bt->B, (size_t)bt->B * bt->T, gemm_mode), LFI_ERR_WORKSPACE,
               "feature workspace too small");
   void *gws = (char *)ws + w.bytes;
-  return build_cond(s, d, p, bt, t0, Tp, cond, w.enc, w.gh, false, false, true, gemm_mode, gws, ws_bytes - w.bytes, st);
+  return build_cond(s, d, p, bt, t0, Tp, cond, w.enc, w.gh, false, true, gemm_mode, gws, ws_bytes - w.bytes, st);
 }
 
 size_t lfi_sample_ws_bytes(const lfi_shape *s, int B, int T, int chunk, int gemm_mode) {
@@ -980,7 +989,7 @@ int lfi_seq_sample(const lfi_shape *s, const void *derived, const lfi_params *p,
     const int Tc = (Tgen - c0 < chunk) ? (Tgen - c0) : chunk;
     const size_t Mc = (size_t)Tc * B;
     const int t0 = d.start_ts + c0;
-    LFI_TRY(build_cond(s, d, p, bt, t0, Tc, w.cond, w.enc, w.gh, false, !teacher_forced, c0 == 0, gemm_mode, gws, gws_bytes, st));
+    LFI_TRY(build_cond(s, d, p, bt, t0, Tc, w.cond, w.enc, w.gh, !teacher_forced, c0 == 0, gemm_mode, gws, gws_bytes, st));
     core::InvArgs a;
     memset(&a, 0, sizeof(a));
     a.d = d; a.dv = make_view(d, derived, p); a.B = B; a.Tc = Tc; a.k_hi = K - 1; a.k_lo = 0; a.g_k0 = 0;
@@ -1427,7 +1436,7 @@ static size_t feature_bwd_scratch(const lfi_shape *s, const FeatPlan &f, int Tp,
   size_t need = 0;
   const int M = Tp * B;
   for (int m = 0; m < LFI_NMOD; ++m) {
-    if (s->hist[m] <= 0 || s->ehid[m] <= 0 || f.enc[m].planes) continue;
+    if (s->hist[m] <= 0 || s->ehid[m] <= 0 || f.enc[m].plan.planes) continue;
     const int E = s->ehid[m], dim = s->dim[m], h = s->hist[m];
     const GemmArgs gs[] = {gemm_args(0, 0, M, E, 3 * E, nullptr, 3 * E, nullptr, E, nullptr, E),
                            gemm_args(1, 0, 3 * E, E, (h - 1) * M, nullptr, 3 * E, nullptr, E, nullptr, E),
@@ -1507,7 +1516,7 @@ int lfi_feature_encode_fwd_train(const lfi_shape *s, const lfi_params *p, const 
               f.stash_bytes);
   const size_t need = feature_ws_need(s, d, bt->B, bt->T, Tp, gemm_mode);
   LFI_REQUIRE(ws_bytes >= need, LFI_ERR_WORKSPACE, "lfi_feature_encode_fwd_train: workspace too small: %zu < %zu", ws_bytes, need);
-  return build_cond(s, d, p, bt, t0, Tp, cond, f.enc, f.gh, true, false, true, gemm_mode, (char *)ws + f.ws_bytes, ws_bytes - f.ws_bytes, st);
+  return build_cond(s, d, p, bt, t0, Tp, cond, f.enc, f.gh, false, true, gemm_mode, (char *)ws + f.ws_bytes, ws_bytes - f.ws_bytes, st);
 }
 
 int lfi_feature_encode_bwd(const lfi_shape *s, const lfi_params *p, const lfi_batch *bt, int t0, int Tp, const float *dcond,
@@ -1536,7 +1545,7 @@ int lfi_feature_encode_bwd(const lfi_shape *s, const lfi_params *p, const lfi_ba
       continue;
     }
     EncWs &ew = f.enc[m];
-    if (ew.planes) {  // the operand planes of W_hh (dh_prev) and W_ih (dXg) belong to this call's workspace
+    if (ew.plan.planes) {  // the operand planes of W_hh (dh_prev) and W_ih (dXg) belong to this call's workspace
       LFI_TRY(split_to_planes(p->enc_w_hh[m], 3 * E, E, E, 0, 1, ew.whh_hi, lo ? ew.whh_lo : nullptr, st));
       if (dxm) LFI_TRY(split_to_planes(p->enc_w_ih[m], 3 * E, dim, dim, 0, 1, ew.wih_hi, lo ? ew.wih_lo : nullptr, st));
     }
