@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 9
+#define LFI_ABI_VERSION 10
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -337,6 +337,28 @@ int lfi_clip_adam(float *theta, float *grad, float *m, float *v, size_t n, float
  * (SURVEY.md section 8(f) rank 2: graph-capturable optimizer step; train.py: GraphedStep). */
 int lfi_clip_adam_dev(float *theta, float *grad, float *m, float *v, size_t n, const float *hyper, float beta1, float beta2,
                       float eps, float max_norm, float grad_scale, float *norm_scratch, void *stream);
+
+/* The same clip followed by torch.optim.SGD or torch.optim.RMSprop (single-tensor semantics of torch 2.x), each as two
+ * launches over the flat buffer (the norm pass, then the update) with the per-step scalars read from device memory, so that
+ * eager and captured steps run the same launch.  After the clip (g = grad * grad_scale * coef, as lfi_clip_adam):
+ *   SGD      g += weight_decay * theta;  with momentum != 0: buf = g on the first momentum step, else
+ *            buf = momentum * buf + (1 - dampening) * g, and g = g + momentum * buf (nesterov) or g = buf;  theta -= lr * g
+ *   RMSprop  g += weight_decay * theta;  sq = alpha * sq + (1 - alpha) * g^2;  centered (grad_avg given): grad_avg moves
+ *            towards g with weight 1 - alpha (torch's lerp_) and avg = sqrt(sq - grad_avg^2) + eps, else avg = sqrt(sq) + eps;
+ *            with momentum > 0: buf = momentum * buf + g / avg, theta -= lr * buf, else theta -= lr * g / avg
+ * lfi_clip_sgd_dev:     hyper[0] = learning rate, hyper[1] = 1 on the first momentum step (buf holds no value yet and is
+ *                       written without being read), else 0.  buf [n] is given exactly when momentum != 0.
+ * lfi_clip_rmsprop_dev: hyper[0] = learning rate.  square_avg [n] always; grad_avg [n] or NULL (not centered); buf [n] is
+ *                       given exactly when momentum > 0.
+ * Bad arguments return LFI_ERR_ARG before anything is launched: a null required pointer, n == 0, a buffer missing for (or
+ * given without) the configuration that uses it, a negative momentum / weight_decay (/ alpha / eps), and nesterov without
+ * momentum > 0 or with dampening != 0 (torch refuses these too).  The update has no atomics: given the same gradient and
+ * norm it is bitwise reproducible.  norm_scratch: 2 floats, as lfi_clip_adam. */
+int lfi_clip_sgd_dev(float *theta, float *grad, float *buf, size_t n, const float *hyper, float momentum, float dampening,
+                     float weight_decay, int nesterov, float max_norm, float grad_scale, float *norm_scratch, void *stream);
+int lfi_clip_rmsprop_dev(float *theta, float *grad, float *square_avg, float *grad_avg, float *buf, size_t n, const float *hyper,
+                         float alpha, float eps, float weight_decay, float momentum, float max_norm, float grad_scale,
+                         float *norm_scratch, void *stream);
 
 /* generic batched GEMM used by the time-parallel phases (exposed for unit parity of the tcgen05 path)
  * C[b] = op(A[b]) op(B[b]) : transA: A stored [K,M]; transB: B stored [N,K]. epilogue flags below. */

@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "liblfi_b200.so")
 NMOD = 4
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 GEMM_FP32, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
 EPI_BIAS, EPI_LRELU, EPI_ACCUM, EPI_LRELU_BWD = 1, 2, 4, 8
@@ -111,6 +111,8 @@ SYMBOLS = {
     "lfi_jerk": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "lfi_clip_adam": (_I, [_P, _P, _P, _P, _SZ, _F, _F, _F, _F, _F, _F, _I, _P, _P]),
     "lfi_clip_adam_dev": (_I, [_P, _P, _P, _P, _SZ, _P, _F, _F, _F, _F, _F, _P, _P]),
+    "lfi_clip_sgd_dev": (_I, [_P, _P, _P, _SZ, _P, _F, _F, _F, _I, _F, _F, _P, _P]),
+    "lfi_clip_rmsprop_dev": (_I, [_P, _P, _P, _P, _P, _SZ, _P, _F, _F, _F, _F, _F, _F, _P, _P]),
     "lfi_gemm": (_I, [_I, _I, _I, _I, _I, _I, _P, _I, _L, _P, _I, _L, _P, _I, _L, _P, _L, _P, _I, _L, _I, _I, _P, _SZ, _P]),
 }
 

@@ -627,16 +627,28 @@ int sumsq(float *out2, const float *g, size_t n, cudaStream_t st) {
   return LFI_OK;
 }
 
+namespace {
+// the gradient's factor: grad_scale times the clip_grad_norm_ coefficient (max_norm / (norm + 1e-6), clamped to 1;
+// max_norm <= 0: no clipping), norm = sqrt(sumsq) * grad_scale
+__device__ __forceinline__ float clip_grad_scale(const float *sumsq_in, float grad_scale, float max_norm) {
+  const float norm = sqrtf(sumsq_in[0]) * grad_scale;
+  float coef = 1.0f;
+  if (max_norm > 0.f) coef = fminf(max_norm / (norm + 1e-6f), 1.0f);
+  return grad_scale * coef;
+}
+__device__ __forceinline__ float4 ld4_or0(const float *p, size_t e) {
+  return p ? reinterpret_cast<const float4 *>(p)[e] : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+__device__ __forceinline__ bool aligned16(const void *p) { return ((uintptr_t)p & 15) == 0; }
+}  // namespace
+
 // torch.nn.utils.clip_grad_norm_ (coef = max_norm / (norm + 1e-6), clamped to 1) followed by torch.optim.Adam
 // (no weight decay, no amsgrad): the reference's configure_optimizers + gradient_clip_val.
 __global__ void clip_adam_kernel(float *theta, const float *grad, float *m, float *v, size_t n, float lr, float b1, float b2,
                                  float omb1, float omb2, float eps, float max_norm, float grad_scale, float bc1,
                                  float bc2_sqrt, const float *sumsq_in, const float *hyper) {
   if (hyper) { lr = hyper[0]; bc1 = hyper[1]; bc2_sqrt = hyper[2]; }  // captured launches: the per-step scalars live on the device
-  const float norm = sqrtf(sumsq_in[0]) * grad_scale;
-  float coef = 1.0f;
-  if (max_norm > 0.f) coef = fminf(max_norm / (norm + 1e-6f), 1.0f);
-  const float gs = grad_scale * coef;
+  const float gs = clip_grad_scale(sumsq_in, grad_scale, max_norm);
   const float step = lr / bc1;
   auto upd = [&](float &th, float gr, float &mo, float &ve) {
     const float g = gr * gs;
@@ -665,6 +677,100 @@ int clip_adam(float *theta, const float *grad, float *m, float *v, size_t n, flo
   clip_adam_kernel<<<blocks_for((n + 3) / 4, TB, 148 * 8), TB, 0, st>>>(theta, grad, m, v, n, lr, b1, b2, (float)(1.0 - b1d),
                                                                (float)(1.0 - b2d), eps, max_norm, grad_scale, bc1, bc2s,
                                                                sumsq_in, hyper);
+  LFI_LAUNCH_CHECK();
+  return LFI_OK;
+}
+
+// clip_grad_norm_ followed by torch.optim.SGD (single-tensor semantics).  hyper[0] = lr; hyper[1] != 0: the buffer holds no
+// value yet (torch's first momentum step, buf = g), so it is written without being read.
+__global__ void clip_sgd_kernel(float *theta, const float *grad, float *buf, size_t n, float momentum, float omd, float wd,
+                                int nesterov, float max_norm, float grad_scale, const float *sumsq_in, const float *hyper) {
+  const float lr = hyper[0];
+  const bool first = hyper[1] != 0.f;
+  const float gs = clip_grad_scale(sumsq_in, grad_scale, max_norm);
+  auto upd = [&](float &th, float gr, float &bu) {
+    float g = gr * gs;
+    if (wd != 0.f) g += wd * th;
+    if (buf) {
+      bu = first ? g : momentum * bu + omd * g;
+      g = nesterov ? g + momentum * bu : bu;
+    }
+    th -= lr * g;
+  };
+  const float *bin = first ? nullptr : buf;
+  const bool vec = aligned16(theta) && aligned16(grad) && aligned16(buf);
+  const size_t n4 = vec ? n / 4 : 0;  // 128-bit accesses over the aligned body
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n4; e += (size_t)gridDim.x * blockDim.x) {
+    float4 t4 = reinterpret_cast<float4 *>(theta)[e], b4 = ld4_or0(bin, e);
+    const float4 g4 = reinterpret_cast<const float4 *>(grad)[e];
+    upd(t4.x, g4.x, b4.x); upd(t4.y, g4.y, b4.y); upd(t4.z, g4.z, b4.z); upd(t4.w, g4.w, b4.w);
+    reinterpret_cast<float4 *>(theta)[e] = t4;
+    if (buf) reinterpret_cast<float4 *>(buf)[e] = b4;
+  }
+  for (size_t e = 4 * n4 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+    float bu = bin ? bin[e] : 0.f;
+    upd(theta[e], grad[e], bu);
+    if (buf) buf[e] = bu;
+  }
+}
+int clip_sgd(float *theta, const float *grad, float *buf, size_t n, const float *hyper, float momentum, float dampening,
+             float weight_decay, int nesterov, float max_norm, float grad_scale, const float *sumsq_in, cudaStream_t st) {
+  clip_sgd_kernel<<<blocks_for((n + 3) / 4, TB, 148 * 8), TB, 0, st>>>(theta, grad, buf, n, momentum, (float)(1.0 - (double)dampening),
+                                                                        weight_decay, nesterov, max_norm, grad_scale, sumsq_in, hyper);
+  LFI_LAUNCH_CHECK();
+  return LFI_OK;
+}
+
+// clip_grad_norm_ followed by torch.optim.RMSprop (single-tensor semantics; grad_avg != nullptr: centered, buf != nullptr:
+// momentum).  hyper[0] = lr.  The centered average moves as torch's lerp_ does (weight 1 - alpha).
+__global__ void clip_rmsprop_kernel(float *theta, const float *grad, float *sq, float *ga, float *buf, size_t n, float alpha,
+                                    float oma, float eps, float wd, float momentum, float max_norm, float grad_scale,
+                                    const float *sumsq_in, const float *hyper) {
+  const float lr = hyper[0];
+  const float gs = clip_grad_scale(sumsq_in, grad_scale, max_norm);
+  auto upd = [&](float &th, float gr, float &s, float &a, float &bu) {
+    float g = gr * gs;
+    if (wd != 0.f) g += wd * th;
+    s = alpha * s + oma * g * g;
+    float avg;
+    if (ga) {
+      a = oma < 0.5f ? a + oma * (g - a) : g - (g - a) * (1.0f - oma);
+      avg = sqrtf(s - a * a) + eps;
+    } else {
+      avg = sqrtf(s) + eps;
+    }
+    if (buf) {
+      bu = momentum * bu + g / avg;
+      th -= lr * bu;
+    } else {
+      th -= lr * (g / avg);
+    }
+  };
+  const bool vec = aligned16(theta) && aligned16(grad) && aligned16(sq) && aligned16(ga) && aligned16(buf);
+  const size_t n4 = vec ? n / 4 : 0;  // 128-bit accesses over the aligned body
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n4; e += (size_t)gridDim.x * blockDim.x) {
+    float4 t4 = reinterpret_cast<float4 *>(theta)[e], s4 = reinterpret_cast<float4 *>(sq)[e];
+    float4 a4 = ld4_or0(ga, e), b4 = ld4_or0(buf, e);
+    const float4 g4 = reinterpret_cast<const float4 *>(grad)[e];
+    upd(t4.x, g4.x, s4.x, a4.x, b4.x); upd(t4.y, g4.y, s4.y, a4.y, b4.y);
+    upd(t4.z, g4.z, s4.z, a4.z, b4.z); upd(t4.w, g4.w, s4.w, a4.w, b4.w);
+    reinterpret_cast<float4 *>(theta)[e] = t4; reinterpret_cast<float4 *>(sq)[e] = s4;
+    if (ga) reinterpret_cast<float4 *>(ga)[e] = a4;
+    if (buf) reinterpret_cast<float4 *>(buf)[e] = b4;
+  }
+  for (size_t e = 4 * n4 + blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+    float a = ga ? ga[e] : 0.f, bu = buf ? buf[e] : 0.f;
+    upd(theta[e], grad[e], sq[e], a, bu);
+    if (ga) ga[e] = a;
+    if (buf) buf[e] = bu;
+  }
+}
+int clip_rmsprop(float *theta, const float *grad, float *square_avg, float *grad_avg, float *buf, size_t n, const float *hyper,
+                 float alpha, float eps, float weight_decay, float momentum, float max_norm, float grad_scale, const float *sumsq_in,
+                 cudaStream_t st) {
+  clip_rmsprop_kernel<<<blocks_for((n + 3) / 4, TB, 148 * 8), TB, 0, st>>>(theta, grad, square_avg, grad_avg, buf, n, alpha,
+                                                                            (float)(1.0 - (double)alpha), eps, weight_decay, momentum,
+                                                                            max_norm, grad_scale, sumsq_in, hyper);
   LFI_LAUNCH_CHECK();
   return LFI_OK;
 }

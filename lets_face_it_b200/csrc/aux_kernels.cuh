@@ -82,6 +82,13 @@ int lu_mask_grads(float *dl, float *du, float *dlog_s, const float *dL, const fl
 int sumsq(float *out2, const float *g, size_t n, cudaStream_t st);
 int clip_adam(float *theta, const float *grad, float *m, float *v, size_t n, float lr, float b1, float b2, float eps,
               float max_norm, float grad_scale, int step, const float *sumsq_in, cudaStream_t st, const float *hyper = nullptr);
+// clip_grad_norm_ + torch.optim.SGD / RMSprop over a flat buffer, per-step scalars read from hyper (lfi_clip_sgd_dev /
+// lfi_clip_rmsprop_dev give the layouts); buf, grad_avg nullptr = no momentum / not centered
+int clip_sgd(float *theta, const float *grad, float *buf, size_t n, const float *hyper, float momentum, float dampening,
+             float weight_decay, int nesterov, float max_norm, float grad_scale, const float *sumsq_in, cudaStream_t st);
+int clip_rmsprop(float *theta, const float *grad, float *square_avg, float *grad_avg, float *buf, size_t n, const float *hyper,
+                 float alpha, float eps, float weight_decay, float momentum, float max_norm, float grad_scale, const float *sumsq_in,
+                 cudaStream_t st);
 
 int fill(float *p, float v, size_t n, cudaStream_t st);
 

@@ -1248,6 +1248,32 @@ int lfi_clip_adam_dev(float *theta, float *grad, float *m, float *v, size_t n, c
   return aux::clip_adam(theta, grad, m, v, n, 0.f, beta1, beta2, eps, max_norm, grad_scale, 1, norm_scratch, st, hyper);
 }
 
+int lfi_clip_sgd_dev(float *theta, float *grad, float *buf, size_t n, const float *hyper, float momentum, float dampening,
+                     float weight_decay, int nesterov, float max_norm, float grad_scale, float *norm_scratch, void *stream) {
+  LFI_REQUIRE(theta && grad && hyper && norm_scratch && n > 0, LFI_ERR_ARG, "lfi_clip_sgd_dev: bad argument");
+  LFI_REQUIRE(momentum >= 0.f && weight_decay >= 0.f, LFI_ERR_ARG, "lfi_clip_sgd_dev: negative momentum or weight_decay");
+  LFI_REQUIRE((buf != nullptr) == (momentum != 0.f), LFI_ERR_ARG, "lfi_clip_sgd_dev: buf must be given exactly when momentum != 0");
+  LFI_REQUIRE(!nesterov || (momentum > 0.f && dampening == 0.f), LFI_ERR_ARG,
+              "lfi_clip_sgd_dev: nesterov needs momentum > 0 and dampening 0");
+  cudaStream_t st = (cudaStream_t)stream;
+  LFI_TRY(aux::sumsq(norm_scratch, grad, n, st));
+  return aux::clip_sgd(theta, grad, buf, n, hyper, momentum, dampening, weight_decay, nesterov ? 1 : 0, max_norm, grad_scale,
+                       norm_scratch, st);
+}
+
+int lfi_clip_rmsprop_dev(float *theta, float *grad, float *square_avg, float *grad_avg, float *buf, size_t n, const float *hyper,
+                         float alpha, float eps, float weight_decay, float momentum, float max_norm, float grad_scale,
+                         float *norm_scratch, void *stream) {
+  LFI_REQUIRE(theta && grad && square_avg && hyper && norm_scratch && n > 0, LFI_ERR_ARG, "lfi_clip_rmsprop_dev: bad argument");
+  LFI_REQUIRE(alpha >= 0.f && eps >= 0.f && momentum >= 0.f && weight_decay >= 0.f, LFI_ERR_ARG,
+              "lfi_clip_rmsprop_dev: negative alpha, eps, momentum or weight_decay");
+  LFI_REQUIRE((buf != nullptr) == (momentum > 0.f), LFI_ERR_ARG, "lfi_clip_rmsprop_dev: buf must be given exactly when momentum > 0");
+  cudaStream_t st = (cudaStream_t)stream;
+  LFI_TRY(aux::sumsq(norm_scratch, grad, n, st));
+  return aux::clip_rmsprop(theta, grad, square_avg, grad_avg, buf, n, hyper, alpha, eps, weight_decay, momentum, max_norm, grad_scale,
+                           norm_scratch, st);
+}
+
 int lfi_gemm(int mode, int transA, int transB, int M, int N, int Kd, const float *A, int lda, long strideA, const float *Bm,
              int ldb, long strideB, float *Cm, int ldc, long strideC, const float *bias, long strideBias, const float *auxm,
              int ldaux, long strideAux, int batch, int epi, void *ws, size_t ws_bytes, void *stream) {

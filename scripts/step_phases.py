@@ -22,8 +22,8 @@ for _ in range(N):
     tr.gflat.zero_()
     eng.train_backward(z, tr._dnll[(56, 256, 1.0)], tr.gflat)
     ev[2].record()
-    tr.step_count += 1
-    cabi.check(cabi.lib().lfi_clip_adam(eng.theta.data_ptr(), tr.gflat.data_ptr(), tr.m.data_ptr(), tr.v.data_ptr(), eng.n_theta, tr.lr, tr.betas[0], tr.betas[1], tr.eps, tr.max_norm, 1.0, tr.step_count, tr.scratch.data_ptr(), cabi.stream_ptr()), "x")
+    tr._advance()
+    tr._update(tr.gflat[:eng.n_theta], None)
     ev[3].record()
     torch.cuda.synchronize()
     for i in range(3): acc[i] += ev[i].elapsed_time(ev[i + 1])
