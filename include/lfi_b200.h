@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LFI_ABI_VERSION 10
+#define LFI_ABI_VERSION 11
 #define LFI_NMOD 4 /* p1_face, p2_face, p1_speech, p2_speech — concat order of models.py:127-145 */
 
 typedef enum lfi_status {
@@ -152,6 +152,19 @@ size_t lfi_train_dx_ws_bytes(const lfi_shape *s, int B, int T, int gemm_mode);
 int lfi_seq_train_bwd_dx(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *b,
                          const float *z, const float *dnll, lfi_params *g, void *ws, size_t ws_bytes, float *const dx[LFI_NMOD],
                          void *dws, size_t dws_bytes, int gemm_mode, void *stream);
+
+/* ---- SeqGlow.forward without gradients, in chunks of frames (models.py:534-561 under torch.no_grad()) ---------------------
+ * z [T',B,C] and nll [T',B] as lfi_seq_train_fwd (nll without the parameter-only constant, which the host adds); scale_out NULL
+ * or [K,B,C-C/2]: the last frame's coupling scale per step.  Dropout masks come in b->mask in the training layout [T',B,hist].
+ * The frames are scored `chunk` at a time: per chunk the conditioning, the gate-ih pre-activations, then the forward flow core,
+ * which starts from the RNN state the previous chunk left.  Nothing is kept for a backward pass, so the workspace
+ * (lfi_eval_ws_bytes) grows with T only by the encoders' per-raw-frame input projections; everything else is sized by the chunk.
+ * At final_model.yaml, B = 256 and 56 frames per chunk it is about 2.4 GB in bf16x3, against 11.9 GB for lfi_seq_train_fwd at
+ * T = 80.  lfi_eval_ws_bytes returns 0 for a bad shape, chunk < 1 or T <= start_ts.  Null pointers, chunk < 1 or T <= start_ts
+ * (LFI_ERR_ARG) and a short workspace (LFI_ERR_WORKSPACE) return a status before anything is launched. */
+size_t lfi_eval_ws_bytes(const lfi_shape *s, int B, int T, int chunk, int gemm_mode);
+int lfi_seq_eval(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *b, int chunk, float *z,
+                 float *nll, float *scale_out, void *ws, size_t ws_bytes, int gemm_mode, void *stream);
 
 /* ---- SeqGlow.inference (models.py:567-596): persistent autoregressive sampler ---------------
  * faces [B, seq_len, C] in/out: the first start_ts frames hold the seed (data["p1_face"]), frames

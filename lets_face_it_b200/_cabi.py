@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "liblfi_b200.so")
 NMOD = 4
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 GEMM_FP32, GEMM_BF16X3, GEMM_BF16 = 0, 1, 2
 EPI_BIAS, EPI_LRELU, EPI_ACCUM, EPI_LRELU_BWD = 1, 2, 4, 8
@@ -90,6 +90,8 @@ SYMBOLS = {
     "lfi_train_dx_ws_bytes": (_SZ, [_SH, _I, _I, _I]),
     "lfi_seq_train_bwd_dx": (_I, [_SH, _P, _PR, _BT, _P, _P, _PR, _P, _SZ, C.POINTER(_P), _P, _SZ, _I, _P]),
     "lfi_seq_sample": (_I, [_SH, _P, _PR, _BT, _I, _P, _P, _P, _I, _I, _P, _SZ, _I, _P]),
+    "lfi_eval_ws_bytes": (_SZ, [_SH, _I, _I, _I, _I]),
+    "lfi_seq_eval": (_I, [_SH, _P, _PR, _BT, _I, _P, _P, _P, _P, _SZ, _I, _P]),
     "lfi_feature_encode": (_I, [_SH, _PR, _BT, _I, _I, _P, _P, _SZ, _I, _P]),
     "lfi_feature_stash_bytes": (_SZ, [_SH, _I, _I, _I, _I]),
     "lfi_feature_bwd_ws_bytes": (_SZ, [_SH, _I, _I, _I, _I]),

@@ -55,7 +55,13 @@ struct FwdArgs {
   // LSTM): the recurrent product h[k][t-1] W_hh[k]^T of every cell of a wavefront is ONE batched tcgen05 GEMM issued before the
   // wavefront's launch (core_fwd.cu: launch_fwd_t), and the cell kernel adds the result instead of streaming W_hh through FFMA.
   WaveTc wtc;
-  const float *gh_pre;        // set per wavefront by the launcher: [K][B][GH] products of this wavefront's cells (cells with t >= 1)
+  union {
+    const float *gh_pre;      // hybrid wavefronts, set per wavefront by the launcher: [K][B][GH] products of this wavefront's cells (t >= 1)
+    // stage pipelines, with h0: the carry instantiation (time-chunked evaluation, lfi_seq_eval) runs; every sequence starts from
+    // h0 and its state after frame Tp - 1 goes to h_last [K][B][H], st_h is not written.  (Sharing gh_pre's storage keeps the
+    // argument block's size, so the kernels without a carried state are unchanged; launch_fwd refuses h_last for the wavefronts.)
+    float *h_last;
+  };
 };
 
 struct InvArgs {
@@ -137,6 +143,7 @@ struct CorePlan {
 // The one place that decides the flow-core path of whole-sequence training (core_plan.cu): shape, GEMM mode, the switches of
 // DESIGN.md §9.  The forward and backward calls of a training step plan alike, so they agree on the workspace layout.
 CorePlan plan_core(const Dims &d, int B, int gemm_mode);
+CorePlan plan_core_eval(const Dims &d, int B, int gemm_mode);  // time-chunked evaluation (lfi_seq_eval): fwd is Wave, Pipe or PipeTc
 
 int fwd_smem_bytes(const Dims &d, int R);
 int choose_rpt(const Dims &d, int B, bool bwd, bool sampler);

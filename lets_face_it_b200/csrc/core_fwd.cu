@@ -427,16 +427,24 @@ static int launch_fwd_wave(const FwdArgs &a, bool tcw, cudaStream_t st) {
 }
 
 int launch_fwd(const FwdArgs &a, CoreKernel kern, cudaStream_t st) {
-  // only the plain wavefronts start from a given state (module API); the other kernels run whole-sequence training
-  LFI_REQUIRE(kern == CoreKernel::Wave || (!a.h0 && !a.c0), LFI_ERR_ARG, "flow core: only the wavefront kernels take an initial state");
+  // Initial state: the plain wavefronts read h0 / c0 (module API, time-chunked evaluation; the caller takes the final state
+  // from st_h / st_c).  The stage pipelines (GRU only) run their carry instantiation when given h0 and h_last.  The hybrid
+  // wavefronts start from zeros: their batched recurrent product would need h0 as operand planes.
   switch (kern) {
-    case CoreKernel::Wave: return launch_fwd_wave(a, false, st);
+    case CoreKernel::Wave:
+      LFI_REQUIRE(!a.h_last, LFI_ERR_ARG, "flow core: the wavefront kernels do not write h_last");
+      return launch_fwd_wave(a, false, st);
     case CoreKernel::WaveHybrid:
+      LFI_REQUIRE(!a.h0 && !a.c0 && !a.h_last, LFI_ERR_ARG, "flow core: the hybrid wavefronts take no initial state");
       LFI_REQUIRE(a.k_first == 0 && a.wtc.mode && a.wtc.whh_hi && a.wtc.ghbuf, LFI_ERR_ARG,
                   "flow core: hybrid wavefronts need W_hh planes and product buffers from step 0");
       return launch_fwd_wave(a, true, st);
-    case CoreKernel::Pipe: return launch_fwd_pipe(a, st);
-    case CoreKernel::PipeTc: return launch_fwd_pipe_tc(a, st);
+    case CoreKernel::Pipe:
+      LFI_REQUIRE(!a.c0, LFI_ERR_ARG, "flow core: the stage pipelines carry no LSTM cell state");
+      return launch_fwd_pipe(a, st);
+    case CoreKernel::PipeTc:
+      LFI_REQUIRE(!a.c0, LFI_ERR_ARG, "flow core: the stage pipelines carry no LSTM cell state");
+      return launch_fwd_pipe_tc(a, st);
   }
   set_error("flow core: unknown kernel %d", (int)kern);
   return LFI_ERR_ARG;

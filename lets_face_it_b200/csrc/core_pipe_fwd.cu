@@ -18,6 +18,9 @@ __device__ __forceinline__ void st_release_gpu(int *p, int v) {
 }
 
 // grid = (2, number of steps, pipelines); cluster = the two CTAs along x.
+// kCarry: every tile starts from the state a.h0 [K][B][H] and leaves its last frame's state in a.h_last [K][B][H] (time-chunked
+// evaluation, lfi_seq_eval); there is no st_h stash.  The instantiation without it starts from zeros and stores st_h.
+template <bool kCarry>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PNT, 1)
 core_fwd_pipe(const FwdArgs a, const int P, const int ntiles, int *progress) {
   extern __shared__ __align__(16) float sm[];
@@ -68,10 +71,33 @@ core_fwd_pipe(const FwdArgs a, const int P, const int ntiles, int *progress) {
     const int row0 = tile * PR, nrows = min(PR, B - row0);
     const int nmy = max(0, min(PRH, nrows - lr0));
     float hreg[8][2];
+    if constexpr (kCarry) {
+      // the carried state of this thread's rows and units, into both CTAs' h (the per-frame update's layout); rows past the
+      // batch are zero.  The two CTAs together write every unit and row of h, so nothing is zeroed first.
 #pragma unroll
-    for (int r = 0; r < 8; ++r) hreg[r][0] = hreg[r][1] = 0.f;
-    for (int e = tid; e < H * PHS; e += PNT) hs[e] = 0.f;  // models.py:196-202: state None = zeros
-    __syncthreads();
+      for (int r = 0; r < 8; ++r) {
+        const bool ok = 8 * rg + r < nrows;
+        const float *src = a.h0 + ((size_t)k * B + row0 + 8 * rg + r) * H + PUC * c + u0;
+        const float2 v = ok ? *reinterpret_cast<const float2 *>(src) : make_float2(0.f, 0.f);
+        hreg[r][0] = v.x; hreg[r][1] = v.y;
+      }
+#pragma unroll
+      for (int x = 0; x < 2; ++x) {
+        const float4 v0 = make_float4(hreg[0][x], hreg[1][x], hreg[2][x], hreg[3][x]);
+        const float4 v1 = make_float4(hreg[4][x], hreg[5][x], hreg[6][x], hreg[7][x]);
+        const int off = pl.h + (PUC * c + u0 + x) * PHS + 8 * rg;
+        *reinterpret_cast<float4 *>(sm + off) = v0;
+        *reinterpret_cast<float4 *>(sm + off + 4) = v1;
+        *reinterpret_cast<float4 *>(peer + off) = v0;
+        *reinterpret_cast<float4 *>(peer + off + 4) = v1;
+      }
+      cluster.sync();  // both halves of the state are in both CTAs before the first recurrent product
+    } else {
+#pragma unroll
+      for (int r = 0; r < 8; ++r) hreg[r][0] = hreg[r][1] = 0.f;
+      for (int e = tid; e < H * PHS; e += PNT) hs[e] = 0.f;  // models.py:196-202: state None = zeros
+      __syncthreads();
+    }
 
     for (int t = 0; t < Tp; ++t, ++it) {
       const size_t cell = (size_t)k * Tp + t;
@@ -241,7 +267,12 @@ core_fwd_pipe(const FwdArgs a, const int P, const int ntiles, int *progress) {
               *reinterpret_cast<float2 *>(gq + 2 * H) = make_float2(ani[r][0], ani[r][1]);
             }
             if (a.st_ahn) *reinterpret_cast<float2 *>(a.st_ahn + (rb + r) * H + uo) = make_float2(anh[r][0], anh[r][1]);
-            *reinterpret_cast<float2 *>(a.st_h + (rb + r) * H + uo) = make_float2(hreg[r][0], hreg[r][1]);
+            if constexpr (kCarry) {
+              if (t == Tp - 1)
+                *reinterpret_cast<float2 *>(a.h_last + ((size_t)k * B + row0 + 8 * rg + r) * H + uo) = make_float2(hreg[r][0], hreg[r][1]);
+            } else {
+              *reinterpret_cast<float2 *>(a.st_h + (rb + r) * H + uo) = make_float2(hreg[r][0], hreg[r][1]);
+            }
             if (a.ph_hi) put_plane2(a.ph_hi, a.ph_lo, (rb + r) * H + uo, hreg[r][0], hreg[r][1]);
           }
         }
@@ -354,7 +385,12 @@ bool pipe_supported(const Dims &d, bool bwd) {
 
 int launch_fwd_pipe(const FwdArgs &a, cudaStream_t st) {
   const int nk = a.k_last - a.k_first + 1;
-  return launch_pipe(core_fwd_pipe, a, PNT, plan_pipe(a.d).total * (int)sizeof(float), nk, nk, "core_fwd_pipe", st);
+  const int smem = plan_pipe(a.d).total * (int)sizeof(float);
+  if (a.h0 || a.h_last) {
+    LFI_REQUIRE(a.h0 && a.h_last, LFI_ERR_ARG, "core_fwd_pipe: a carried state needs both h0 and h_last");
+    return launch_pipe(core_fwd_pipe<true>, a, PNT, smem, nk, nk, "core_fwd_pipe", st);
+  }
+  return launch_pipe(core_fwd_pipe<false>, a, PNT, smem, nk, nk, "core_fwd_pipe", st);
 }
 
 }  // namespace core

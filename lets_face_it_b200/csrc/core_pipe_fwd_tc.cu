@@ -95,6 +95,9 @@ __host__ __device__ inline PlanTC plan_tc(const Dims &d) {
 
 }  // namespace
 
+// kCarry: every tile starts from the state a.h0 [K][B][H] and leaves its last frame's state in a.h_last [K][B][H] (time-chunked
+// evaluation, lfi_seq_eval); there is no st_h stash.  The instantiation without it starts from zeros and stores st_h.
+template <bool kCarry>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(FNT, 1)
 core_fwd_pipe_tc(const FwdArgs a, const int P, const int ntiles, int *progress) {
   extern __shared__ __align__(16) uint8_t smraw[];
@@ -193,9 +196,36 @@ core_fwd_pipe_tc(const FwdArgs a, const int P, const int ntiles, int *progress) 
     const int row0 = tile * PR, nrows = min(PR, B - row0);
     const int nmy = max(0, min(PRH, nrows - lr0));
     float hreg[16];
+    if constexpr (kCarry) {
+      // the carried state of this thread's sequence and 16 units, as operand planes of this CTA's k-block in both CTAs (the
+      // per-frame update's layout); rows past the batch are zero.  The compute threads of the two CTAs together write both
+      // k-blocks whole, so nothing is zeroed first.
+      if (!mma_warp) {
+        const bool ok = row < nrows;
+        const float *src = a.h0 + ((size_t)k * B + row0 + row) * H + PUC * c + ub;
 #pragma unroll
-    for (int j = 0; j < 16; ++j) hreg[j] = 0.f;
-    for (int e = tid; e < 2 * kAHPlane / 16; e += FNT) reinterpret_cast<uint4 *>(smb + kAH)[e] = make_uint4(0u, 0u, 0u, 0u);  // state None = zeros
+        for (int i = 0; i < 4; ++i) {
+          const float4 v = ok ? *reinterpret_cast<const float4 *>(src + 4 * i) : make_float4(0.f, 0.f, 0.f, 0.f);
+          hreg[4 * i] = v.x; hreg[4 * i + 1] = v.y; hreg[4 * i + 2] = v.z; hreg[4 * i + 3] = v.w;
+        }
+        uint4 hi0, lo0, hi1, lo1;
+        {
+          const float v0[8] = {hreg[0], hreg[1], hreg[2], hreg[3], hreg[4], hreg[5], hreg[6], hreg[7]};
+          const float v1[8] = {hreg[8], hreg[9], hreg[10], hreg[11], hreg[12], hreg[13], hreg[14], hreg[15]};
+          split8(v0, hi0, lo0);
+          split8(v1, hi1, lo1);
+        }
+        const uint32_t o0 = kAH + (uint32_t)c * (64 * 128) + sw128_off(row, ub >> 3), o1 = kAH + (uint32_t)c * (64 * 128) + sw128_off(row, (ub >> 3) + 1);
+        *reinterpret_cast<uint4 *>(smb + o0) = hi0; *reinterpret_cast<uint4 *>(smb + o0 + kAHPlane) = lo0;
+        *reinterpret_cast<uint4 *>(smb + o1) = hi1; *reinterpret_cast<uint4 *>(smb + o1 + kAHPlane) = lo1;
+        *reinterpret_cast<uint4 *>(peerb + o0) = hi0; *reinterpret_cast<uint4 *>(peerb + o0 + kAHPlane) = lo0;
+        *reinterpret_cast<uint4 *>(peerb + o1) = hi1; *reinterpret_cast<uint4 *>(peerb + o1 + kAHPlane) = lo1;
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < 16; ++j) hreg[j] = 0.f;
+      for (int e = tid; e < 2 * kAHPlane / 16; e += FNT) reinterpret_cast<uint4 *>(smb + kAH)[e] = make_uint4(0u, 0u, 0u, 0u);  // state None = zeros
+    }
     fence_async_smem();
     cluster.sync();
 
@@ -467,7 +497,13 @@ core_fwd_pipe_tc(const FwdArgs a, const int P, const int ntiles, int *progress) 
 #pragma unroll
           for (int i = 0; i < 4; ++i) *reinterpret_cast<float4 *>(ap + i * 256) = make_float4(vh[4 * i], vh[4 * i + 1], vh[4 * i + 2], vh[4 * i + 3]);
         }
-        {
+        if constexpr (kCarry) {
+          if (t == Tp - 1 && rowok) {
+            float *hp = a.h_last + ((size_t)k * B + row0 + row) * H + PUC * c + ub;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) *reinterpret_cast<float4 *>(hp + 4 * i) = make_float4(hreg[4 * i], hreg[4 * i + 1], hreg[4 * i + 2], hreg[4 * i + 3]);
+          }
+        } else {
           float *hp = a.st_h + stash_tiled_off(cell, ntiles, tile, c, hs, 1, 0, 0) + 4 * row;
 #pragma unroll
           for (int i = 0; i < 4; ++i) *reinterpret_cast<float4 *>(hp + i * 256) = make_float4(hreg[4 * i], hreg[4 * i + 1], hreg[4 * i + 2], hreg[4 * i + 3]);
@@ -578,7 +614,11 @@ int launch_fwd_pipe_tc(const FwdArgs &a, cudaStream_t st) {
   static const int timing = getenv("LFI_CORE_TIMING") ? atoi(getenv("LFI_CORE_TIMING")) : 0;
   if (timing) cudaMemcpyToSymbolAsync(g_core_timing, &timing, sizeof(int), 0, cudaMemcpyHostToDevice, st);
   const int nk = a.k_last - a.k_first + 1;
-  return launch_pipe(core_fwd_pipe_tc, a, FNT, plan_tc(a.d).total, nk, nk, "core_fwd_pipe_tc", st);
+  if (a.h0 || a.h_last) {
+    LFI_REQUIRE(a.h0 && a.h_last, LFI_ERR_ARG, "core_fwd_pipe_tc: a carried state needs both h0 and h_last");
+    return launch_pipe(core_fwd_pipe_tc<true>, a, FNT, plan_tc(a.d).total, nk, nk, "core_fwd_pipe_tc", st);
+  }
+  return launch_pipe(core_fwd_pipe_tc<false>, a, FNT, plan_tc(a.d).total, nk, nk, "core_fwd_pipe_tc", st);
 }
 
 }  // namespace core

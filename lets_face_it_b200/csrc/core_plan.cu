@@ -1,6 +1,6 @@
-// Which flow-core kernels run.  Whole-sequence training picks one kernel per direction here (plan_core), the sampler picks its
-// inverse kernel here (use_inv_rows); the launchers run what they are given.  The switches of DESIGN.md §9 that select these
-// paths are read here only, at call time (the tests toggle them between calls).
+// Which flow-core kernels run.  Whole-sequence training picks one kernel per direction here (plan_core), time-chunked evaluation
+// its forward kernel (plan_core_eval), the sampler its inverse kernel (use_inv_rows); the launchers run what they are given.
+// The switches of DESIGN.md §9 that select these paths are read here only, at call time (the tests toggle them between calls).
 #include "core_pipe.cuh"
 
 namespace lfi {
@@ -38,6 +38,15 @@ CorePlan plan_core(const Dims &d, int B, int gemm_mode) {
   p.fwd = p.tiled ? CoreKernel::PipeTc : pipe_fwd ? CoreKernel::Pipe : wave;
   const bool bwd_tc = p.tiled && env_flag("LFI_CORE_TC_BWD", true) && pipe_bwd_tc_supported(d);
   p.bwd = bwd_tc ? CoreKernel::PipeTc : pipe_bwd ? CoreKernel::Pipe : wave;
+  return p;
+}
+
+// Time-chunked evaluation (lfi_seq_eval): the forward kernel and operand-plane choice of training, run from a carried state.  The
+// hybrid wavefronts take no initial state, so their shapes run the plain wavefronts.  (No backward pass: bwd repeats fwd.)
+CorePlan plan_core_eval(const Dims &d, int B, int gemm_mode) {
+  CorePlan p = plan_core(d, B, gemm_mode);
+  if (p.fwd == CoreKernel::WaveHybrid) p.fwd = CoreKernel::Wave;
+  p.bwd = p.fwd;
   return p;
 }
 

@@ -10,6 +10,7 @@
 #include "core_api.cuh"
 #include "core_pipe.cuh"
 #include "enc_persist.cuh"
+#include <algorithm>
 #include <cstdlib>
 
 namespace lfi {
@@ -892,20 +893,15 @@ struct SampleWs {
 static bool sample_tc_ar(const Dims &d, int mode) {
   return mode != LFI_GEMM_FP32 && d.Far > 0 && d.Far % 8 == 0 && d.D % 8 == 0;
 }
-static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chunk, int mode, void *ws, SampleWs *w) {
-  Bump b(ws, 0);
-  const size_t Mc = (size_t)chunk * B, K = d.K;
-  w->cond = b.take<float>(Mc * d.Fe);
-  w->Cs = b.take<float>(Mc * K * d.D);
-  w->G = b.take<float>(Mc * K * d.GH);
-  w->hstate = b.take<float>(K * B * d.H);
-  w->cstate = d.G == 4 ? b.take<float>(K * B * d.H) : nullptr;
+// The encoders of a call without gradients over chunks of Mc windows (sampling, feature encoding, evaluation): the input
+// projections of all B*T raw frames (computed once per call), the window state ping-pong, and the shared gh scratch.
+static void plan_enc_nograd(const lfi_shape *s, int B, int T, size_t Mc, int mode, Bump &b, EncWs *enc, float **gh) {
   size_t ghmax = 0;
   for (int m = 0; m < LFI_NMOD; ++m) {
-    memset(&w->enc[m], 0, sizeof(EncWs));
+    memset(&enc[m], 0, sizeof(EncWs));
     if (s->hist[m] <= 0 || s->ehid[m] <= 0) continue;
     const size_t E = s->ehid[m];
-    EncWs &e = w->enc[m];
+    EncWs &e = enc[m];
     e.xp = b.take<float>(encp::tiled_rows((size_t)B * T) * 3 * E);
     e.hs = b.take<float>(2 * Mc * E);
     e.plan = plan_enc(s, m, Mc, (size_t)B * T, mode, false);
@@ -917,7 +913,17 @@ static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chu
     }
     if (Mc * 3 * E > ghmax) ghmax = Mc * 3 * E;
   }
-  w->gh = b.take<float>(ghmax);
+  *gh = b.take<float>(ghmax);
+}
+static void plan_sample(const lfi_shape *s, const Dims &d, int B, int T, int chunk, int mode, void *ws, SampleWs *w) {
+  Bump b(ws, 0);
+  const size_t Mc = (size_t)chunk * B, K = d.K;
+  w->cond = b.take<float>(Mc * d.Fe);
+  w->Cs = b.take<float>(Mc * K * d.D);
+  w->G = b.take<float>(Mc * K * d.GH);
+  w->hstate = b.take<float>(K * B * d.H);
+  w->cstate = d.G == 4 ? b.take<float>(K * B * d.H) : nullptr;
+  plan_enc_nograd(s, B, T, Mc, mode, b, w->enc, &w->gh);
   w->tc_ar = sample_tc_ar(d, mode);
   if (w->tc_ar) {
     const bool lo = mode == LFI_GEMM_BF16X3;
@@ -1043,6 +1049,113 @@ int lfi_seq_sample(const lfi_shape *s, const void *derived, const lfi_params *p,
       continue;
     }
     LFI_TRY(core::launch_inv(a, st));
+  }
+  return LFI_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// likelihood evaluation in chunks of frames: no stash, no gradients, the RNN state of the K flow steps carried between chunks
+struct EvalWs {
+  float *cond, *Cact, *G, *ld, *xin, *gh;
+  void *cact_hi, *cact_lo;   // the cond_transform activations as operand planes (plan.planes), as in training
+  float *hstate[2], *cstate[2];  // [K][B][H] carried state, ping-pong: chunk i reads slot i % 2 and leaves its final state in the other
+  float *st_h, *st_c;        // Wave only: [K][chunk][B][H], the states the wavefront kernel passes between frames
+  int *flags;
+  EncWs enc[LFI_NMOD];
+  core::CorePlan plan;
+  size_t bytes;
+};
+// Everything but the encoders' input projections (plan_enc_nograd) is sized by the chunk, not by T.
+static void plan_eval(const lfi_shape *s, const Dims &d, int B, int T, int chunk, int mode, void *ws, EvalWs *w) {
+  Bump b(ws, 0);
+  const size_t Mc = (size_t)chunk * B, K = d.K, KBH = K * B * d.H;
+  w->plan = core::plan_core_eval(d, B, mode);
+  const bool planes = w->plan.planes, wave = w->plan.fwd == core::CoreKernel::Wave;
+  w->cond = b.take<float>(Mc * d.Fe);
+  w->Cact = planes ? nullptr : b.take<float>(Mc * K * d.D);
+  w->cact_hi = planes ? take_bf16(b, Mc * K * d.D) : nullptr;
+  w->cact_lo = planes && mode == LFI_GEMM_BF16X3 ? take_bf16(b, Mc * K * d.D) : nullptr;
+  w->G = b.take<float>(round_up_sz(Mc, 32) * K * d.GH);  // (whole 32-row blocks: the row-interleaved layout of the tensor-core core)
+  w->ld = b.take<float>(Mc);
+  w->xin = b.take<float>(K * Mc * d.C);
+  w->flags = b.take<int>(kFlagInts);
+  for (int i = 0; i < 2; ++i) {
+    w->hstate[i] = b.take<float>(KBH);
+    w->cstate[i] = d.G == 4 ? b.take<float>(KBH) : nullptr;
+  }
+  w->st_h = wave ? b.take<float>(K * Mc * d.H) : nullptr;
+  w->st_c = wave && d.G == 4 ? b.take<float>(K * Mc * d.H) : nullptr;
+  plan_enc_nograd(s, B, T, Mc, mode, b, w->enc, &w->gh);
+  w->bytes = round_up_sz(b.off, 256);
+}
+
+size_t lfi_eval_ws_bytes(const lfi_shape *s, int B, int T, int chunk, int gemm_mode) {
+  Dims d;
+  if (make_dims(s, &d) != LFI_OK || B < 1 || chunk < 1 || T <= d.start_ts) return 0;
+  chunk = std::min(chunk, T - d.start_ts);
+  EvalWs w;
+  plan_eval(s, d, B, T, chunk, gemm_mode, nullptr, &w);
+  return w.bytes + gemm_scratch_bound(s, d, (size_t)chunk * B, (size_t)B * T, gemm_mode);
+}
+
+// SeqGlow.forward without gradients (models.py:534-561 under torch.no_grad()), chunk frames at a time: per chunk the conditioning
+// (build_cond, the encoder paths of a call without gradients), the gate-ih pre-activations, then the forward flow core from the
+// state the previous chunk left.  Stream-ordered throughout, no host round trip.
+int lfi_seq_eval(const lfi_shape *s, const void *derived, const lfi_params *p, const lfi_batch *bt, int chunk, float *z,
+                 float *nll, float *scale_out, void *ws, size_t ws_bytes, int gemm_mode, void *stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  Dims d;
+  LFI_TRY(make_dims(s, &d));
+  LFI_REQUIRE(derived && p && bt && z && nll && ws, LFI_ERR_ARG, "lfi_seq_eval: null argument");
+  LFI_REQUIRE(chunk >= 1, LFI_ERR_ARG, "lfi_seq_eval: chunk=%d must be >= 1", chunk);
+  LFI_REQUIRE(bt->B >= 1 && bt->T > d.start_ts, LFI_ERR_ARG, "lfi_seq_eval: B=%d, T=%d (T must exceed the longest history %d)",
+              bt->B, bt->T, d.start_ts);
+  LFI_REQUIRE(bt->x[0], LFI_ERR_ARG, "lfi_seq_eval: batch: p1_face missing");
+  const int B = bt->B, T = bt->T, Tp = T - d.start_ts, K = d.K;
+  chunk = std::min(chunk, Tp);
+  EvalWs w;
+  plan_eval(s, d, B, T, chunk, gemm_mode, ws, &w);
+  const size_t gneed = gemm_scratch_bound(s, d, (size_t)chunk * B, (size_t)B * T, gemm_mode);
+  LFI_REQUIRE(ws_bytes >= w.bytes + gneed, LFI_ERR_WORKSPACE, "eval workspace too small: %zu < %zu", ws_bytes, w.bytes + gneed);
+  void *gws = (char *)ws + w.bytes;
+  const size_t gws_bytes = ws_bytes - w.bytes;
+  const float *WcF = (const float *)derived + derived_layout(d).WcF;
+  const bool wave = w.plan.fwd == core::CoreKernel::Wave;
+  const size_t KBH = (size_t)K * B * d.H;
+
+  LFI_CUDA(cudaMemsetAsync(w.hstate[0], 0, KBH * sizeof(float), st));  // models.py:196-202: state None = zeros
+  if (w.cstate[0]) LFI_CUDA(cudaMemsetAsync(w.cstate[0], 0, KBH * sizeof(float), st));
+  lfi_batch bc = *bt;
+  for (int c0 = 0, cur = 0; c0 < Tp; c0 += chunk, cur ^= 1) {
+    const int Tc = std::min(chunk, Tp - c0);
+    const size_t Mc = (size_t)Tc * B;
+    // the window kernels index the masks [T'][B][hist] by the window's index within the call
+    for (int m = 0; m < LFI_NMOD; ++m) bc.mask[m] = bt->mask[m] ? bt->mask[m] + (size_t)c0 * B * s->hist[m] : nullptr;
+    // (the input projections of the encoders do not depend on the window: computed once, on the first chunk)
+    LFI_TRY(build_cond(s, d, p, &bc, d.start_ts + c0, Tc, w.cond, w.enc, w.gh, false, c0 == 0, gemm_mode, gws, gws_bytes, st));
+    LFI_TRY(cond_to_gates(d, p, WcF, w.cond, Mc, w.Cact, w.G, gemm_mode, gws, gws_bytes, st, w.cact_hi, w.cact_lo, w.plan.tiled));
+    core::FwdArgs a;
+    memset(&a, 0, sizeof(a));
+    a.d = d; a.dv = make_view(d, derived, p); a.B = B; a.Tp = Tc; a.k_first = 0; a.k_last = K - 1;
+    a.x0 = bt->x[0] + (size_t)(d.start_ts + c0) * d.C; a.x_sb = (long)T * d.C; a.x_st = d.C;
+    a.G = w.G; a.g_ld = (long)K * d.GH; a.g_k0 = 0;
+    a.xin = w.xin; a.ld = w.ld; a.ld_accumulate = 0;
+    a.nll = nll + (size_t)c0 * B; a.z_out = z + (size_t)c0 * B * d.C; a.scale_out = scale_out;
+    a.flags = w.flags; a.flags_bytes = kFlagInts * sizeof(int);
+    a.stash_tiled = a.g_tiled = w.plan.tiled ? 1 : 0;
+    a.h0 = w.hstate[cur];
+    if (wave) {
+      a.c0 = w.cstate[cur]; a.st_h = w.st_h; a.st_c = w.st_c;
+    } else {
+      a.h_last = w.hstate[cur ^ 1];
+    }
+    LFI_TRY(core::launch_fwd(a, w.plan.fwd, st));
+    if (wave && c0 + Tc < Tp) {  // the state after the chunk's last frame: cell (k, Tc - 1) of every step
+      const size_t row = (size_t)B * d.H * sizeof(float), pitch = (size_t)Tc * row;
+      LFI_CUDA(cudaMemcpy2DAsync(w.hstate[cur ^ 1], row, w.st_h + (size_t)(Tc - 1) * B * d.H, pitch, row, K, cudaMemcpyDeviceToDevice, st));
+      if (w.st_c)
+        LFI_CUDA(cudaMemcpy2DAsync(w.cstate[cur ^ 1], row, w.st_c + (size_t)(Tc - 1) * B * d.H, pitch, row, K, cudaMemcpyDeviceToDevice, st));
+    }
   }
   return LFI_OK;
 }

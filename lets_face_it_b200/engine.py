@@ -416,6 +416,44 @@ class Engine:
         self.ensure()
         return [p for p, _, _ in self._views]
 
+    # ------------------------------------------------------------------ SeqGlow.evaluate
+    def eval_chunk(self, B, T):
+        """Default frames per chunk of `evaluate`: as many as keep the chunk-dependent part of its workspace within 2.5 GB, so that
+        a training window (56 frames at B = 256, 2.2 GB in bf16x3 at final_model.yaml shapes) is one chunk.  Shorter chunks spend
+        a growing share of the time in the flow-core pipeline's fill and drain (K - 1 stage periods per chunk)."""
+        Tp = T - self.start_ts
+        if Tp <= 8:
+            return max(1, Tp)
+        L = cabi.lib()
+        size = lambda c: L.lfi_eval_ws_bytes(ctypes.byref(self.shape), B, T, c, self.gemm_mode)
+        per_frame = max(1.0, (size(8) - size(1)) / 7.0)
+        return max(1, min(Tp, int(2.5e9 // per_frame)))
+
+    @_on_own_device
+    def evaluate(self, batch, masks=None, chunk=None, scale_out=None):
+        """Returns (z [T',B,C], nll_core [T',B]) as train_forward does, without gradients: the frames are scored `chunk` at a time
+        (lfi_seq_eval) and nothing is kept for a backward pass, so the workspace does not grow with T except for the encoders'
+        per-raw-frame input projections.  nll_core lacks the parameter-only log-det constant."""
+        P = self.refresh(False)
+        L, st = cabi.lib(), cabi.stream_ptr()
+        dev = self.theta.device
+        x0 = batch["p1_face"]
+        B, T = x0.shape[0], x0.shape[1]
+        Tp = T - self.start_ts
+        if Tp < 1:
+            raise AssertionError("Sequence length %d must exceed the longest history %d (utils.py:116-122)" % (T, self.start_ts))
+        chunk = self.eval_chunk(B, T) if chunk is None else int(chunk)
+        if chunk < 1:
+            raise ValueError("chunk must be >= 1, got %d" % chunk)
+        bt, keep = self._batch_struct(batch, B, T, masks)
+        z = torch.empty(Tp, B, self.C, dtype=torch.float32, device=dev)
+        nll = torch.empty(Tp, B, dtype=torch.float32, device=dev)
+        ws = self._workspace(("eval",), L.lfi_eval_ws_bytes(ctypes.byref(self.shape), B, T, chunk, self.gemm_mode))
+        cabi.check(L.lfi_seq_eval(ctypes.byref(self.shape), self._derived.data_ptr(), ctypes.byref(P), ctypes.byref(bt), chunk,
+                                  z.data_ptr(), nll.data_ptr(), scale_out.data_ptr() if scale_out is not None else None,
+                                  ws.data_ptr(), ws.numel(), self.gemm_mode, st), "lfi_seq_eval")
+        return z, nll
+
     # ------------------------------------------------------------------ SeqGlow.inference / invert
     @_on_own_device
     def sample(self, data, seq_len, noise=None, teacher_forced=False, chunk=None, want_logdet=False):

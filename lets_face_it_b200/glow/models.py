@@ -740,6 +740,34 @@ class SeqGlow(nn.Module):
         z_seq = list(z.detach().unbind(0))
         return z_seq, loss.unsqueeze(-1), losses
 
+    def evaluate(self, batch, chunk=None):
+        """Likelihood of sequences of any length: returns what `with torch.no_grad(): forward(batch)` returns, (z_seq, loss [1],
+        losses), with the same dropout masks (drawn in training mode, `injected_masks` when set), ActNorm initialisation and
+        FlowStep.scale.  The frames are scored `chunk` at a time with the flow's RNN state carried from chunk to chunk, and nothing
+        is kept for a backward pass, so memory does not grow with the sequence the way a no-grad `forward` does (that one lays out
+        the training workspace).  chunk None: Engine.eval_chunk.  Always runs without autograd and returns detached tensors; use
+        `forward` for gradients."""
+        eng = self.engine()
+        self.glow.init_rnn_hidden()
+        with torch.no_grad():
+            x0 = batch["p1_face"]
+            B, T = x0.shape[0], x0.shape[1]
+            Tp = T - eng.start_ts
+            masks = self._masks(Tp, B, eng.theta.device)
+            if self.training and not all(l.actnorm.inited for l in self.glow.flow.layers):
+                self._ddi(eng, batch, masks)
+            scale_out = None
+            if self.hparams.Validation["scale_logging"] and eng.affine:
+                scale_out = torch.empty(eng.K, B, eng.Cz, device=eng.theta.device)
+            z, nll = eng.evaluate(batch, masks, chunk, scale_out)
+            nll = nll - eng.logdet_const() / LN2
+            if scale_out is not None:
+                for k, layer in enumerate(self.glow.flow.layers):
+                    layer.scale = scale_out[k]
+            loss = nll.mean(dim=1).sum() / Tp
+            losses = list(nll.cpu().unbind(0))  # one device->host copy
+            return list(z.unbind(0)), loss.unsqueeze(-1), losses
+
     def loss(self, objective, z):
         """-(logdet + log N(z; 0, I)) / ln 2 per sample (models.py:563-565); mutates `objective` like the reference."""
         objective += GaussianDiag.logp_simplified(z)
